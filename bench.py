@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                    # + a seeded sample of the last timed step's frames
 
 HEADLINE.  A "step" is a batch of --frames-per-step frames PER GPU of the workload BASELINE.json's metric is quoted
 on (configs[1]: 1920x1080, ground plane + 16 spheres, hard shadows, 1 spp, no recursion; a camera dolly).  Metric:
@@ -232,6 +233,8 @@ def run_reference(args, rank, world_size):
         f = sc.render(cd, opts, threads=cores, want_rgb=False, want_hit=False)
         rays += f.stats["rays"] + f.stats["shadow_queries"]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:  # the window the step rendered
+        dump_frames(args.dump_outputs, f.rgba[None, :, win[0]:win[2]], x0=win[0])
     value = rays / dt / 1e6
     frac = (win[2] - win[0]) / W
     sample = "window x in [%d,%d) of %dx%d (%.0f%% of the frame) per step, %d column strips" % (
@@ -278,6 +281,30 @@ def bind_to_gpu_numa_node(index):
 
 def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+DUMP_PIXELS = 1 << 21  # 2 Mi pixels: the two files take 48 MB
+
+
+def dump_frames(out_dir, frames, x0=0):
+    """`--dump-outputs`: the 8-bit frames [F, H, W, 3 or 4] a step delivered, as two float32 files in `out_dir`:
+    frames_sample.npy [n, 3] (R, G, B values 0..255; the constant alpha of RGBA8 is left out) and
+    frames_sample_index.npy [n, 3] (frame, y, x) of those pixels, x counted in the full frame (`frames` starts at
+    column x0).  Both arms write the same layout, so their dumps pair pixel for pixel.  n = min(F*H*W, DUMP_PIXELS)
+    pixels chosen with a fixed seed and kept in row-major order, so the same arguments sample the same pixels in
+    every run and two builds compare output for output."""
+    F, H, W, Ch = frames.shape
+    n_px = F * H * W
+    if n_px <= DUMP_PIXELS:
+        idx = np.arange(n_px)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(n_px, size=DUMP_PIXELS, replace=False))
+    values = frames.reshape(n_px, Ch)[idx, :3].astype(np.float32)
+    f, y, x = np.unravel_index(idx, (F, H, W))
+    where = np.stack([f, y, x + x0], axis=1).astype(np.float32)  # exact: every index < 2**24
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frames_sample.npy"), values)
+    np.save(os.path.join(out_dir, "frames_sample_index.npy"), where)
 
 
 class Ctx:
@@ -603,6 +630,12 @@ def run_ours(args, rank, local_rank, world_size):
     frames_total = n_slots  # frames finished per step by the whole job
     value = rays_total * args.steps / (total_ms * 1e-3) / 1e6
 
+    # ---- --dump-outputs (outside the timed region): the frames of the last timed step, as rank 0's slots hold them ----
+    if args.dump_outputs and rank == 0:
+        got = np.zeros((H * n_slots, W, 4), np.uint8)
+        r.framebuffer_download(W, H * n_slots, got)
+        dump_frames(args.dump_outputs, got.reshape(n_slots, slot_bytes)[:, :frame_bytes].reshape(n_slots, H, W, bpp))
+
     # ---- gather parity (N > 1, outside the timed region): what is in rank 0's slots after the last timed step
     # against the same frames rendered by rank 0 alone into a scratch renderer ----
     gather = None
@@ -814,7 +847,13 @@ def main():
     ap.add_argument("--cpu-fraction", type=float, default=1.0, help="fraction of the frame width the CPU legs render")
     ap.add_argument("--sustained-seconds", type=float, default=2.0, help="length of the back-to-back companion run (0 = skip)")
     ap.add_argument("--headline-only", action="store_true", help="skip the per-config and strong-scaling records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed seeded sample of the pixels of the frames the last step "
+                         "delivered: DIR/frames_sample.npy (R, G, B) and DIR/frames_sample_index.npy (frame, y, x), "
+                         "float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))

@@ -7,6 +7,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -74,6 +75,61 @@ def test_reference_arm_prints_the_contract_line():
     out = subprocess.check_output([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--config", "1",
                                    "--steps", "1", "--warmup", "0"], env=env, cwd=ROOT, timeout=120).decode()
     assert out.strip() == ""
+
+
+def test_dump_outputs_writes_the_last_step_frames(tmp_path):
+    """`--dump-outputs DIR` (reference arm here): float32 pixel values of the last timed step's frame with their
+    (frame, y, x), at most 64 MB, identical from run to run with the same arguments."""
+    from raytracing_rb_b200 import Camera, make_opts
+    from oracle import oracle
+    dumps = []
+    for k in range(2):
+        out = tmp_path / ("d%d" % k)
+        subprocess.check_call([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--config", "1",
+                               "--steps", "1", "--warmup", "0", "--cpu-fraction", "0.25", "--dump-outputs", str(out)],
+                              cwd=ROOT, timeout=300, stdout=subprocess.DEVNULL)
+        dumps.append({n: np.load(out / (n + ".npy")) for n in ("frames_sample", "frames_sample_index")})
+        assert sum(f.stat().st_size for f in out.iterdir()) <= 64 << 20
+    for d in dumps:
+        assert all(a.dtype == np.float32 for a in d.values())
+        assert np.array_equal(d["frames_sample"], dumps[0]["frames_sample"])
+        assert np.array_equal(d["frames_sample_index"], dumps[0]["frames_sample_index"])
+    world, cdoc, _ = bench.workload(1)
+    cd = Camera(world, cdoc).camera_desc()
+    win = bench.cpu_window(cd.width, cd.height, 0.25, 1)
+    want = oracle.OracleScene(world.to_scene_desc()).render(cd, make_opts(seed=1, window=win)).rgba
+    vals, where = dumps[0]["frames_sample"], dumps[0]["frames_sample_index"].astype(np.int64)
+    assert vals.shape == (cd.height * (win[2] - win[0]), 3) and (where[:, 0] == 0).all()
+    assert where[:, 2].min() == win[0] and where[:, 2].max() == win[2] - 1  # x in the full frame
+    assert np.array_equal(vals, want[where[:, 1], where[:, 2], :3].astype(np.float32))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("pixel_format", ["rgb8", "rgba8"])
+def test_gpu_arm_dump_outputs_are_the_frames_of_the_last_step(tmp_path, pixel_format):
+    """`--dump-outputs DIR` on the CUDA arm: the frame slots read back after the timed steps, cut to each frame's
+    bytes in either pixel format, must give the pixels a direct render of the same batch cameras gives."""
+    from raytracing_rb_b200 import PREC_FAST64, Renderer, _abi, make_opts
+    B = 3
+    subprocess.check_call([sys.executable, os.path.join(ROOT, "bench.py"), "--small", "--steps", "2", "--warmup", "1",
+                           "--frames-per-step", str(B), "--pixel-format", pixel_format, "--headline-only",
+                           "--sustained-seconds", "0", "--dump-outputs", str(tmp_path)],
+                          cwd=ROOT, timeout=600, stdout=subprocess.DEVNULL)
+    vals = np.load(tmp_path / "frames_sample.npy")
+    where = np.load(tmp_path / "frames_sample_index.npy").astype(np.int64)
+    world, cdoc, _ = bench.workload(2, small=True)
+    cams = bench.batch_cameras(world, cdoc, B)
+    W, H = cams[0].width, cams[0].height
+    assert vals.dtype == np.float32 and vals.shape == (B * H * W, 3)  # small enough to be dumped whole
+    r = Renderer(world.to_scene_desc(), 0)
+    fmt = _abi.FMT_RGB8 if pixel_format == "rgb8" else _abi.FMT_RGBA8
+    for f in range(B):
+        want = r.render(cams[f], make_opts(seed=1, precision=PREC_FAST64, pixel_format=fmt),
+                        want_rgb=False, want_hit=False).rgba
+        m = where[:, 0] == f
+        assert m.sum() == H * W
+        assert np.array_equal(vals[m], want[where[m, 1], where[m, 2], :3].astype(np.float32)), f
+    r.close()
 
 
 def test_gpu_arm_fails_loudly_without_a_gpu():

@@ -165,7 +165,7 @@ def test_multi_gpu_tiles_compose_in_process():
     from raytracing_rb_b200 import device_count
     n = device_count()
     if n < 2:
-        pytest.skip("needs >= 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     world, cam = load_scene(3, width=640, height=360)
     one = cam.render_frame(gpus=1, seed=5, count_detail=True)
     many = cam.render_frame(gpus=min(n, 8), seed=5, count_detail=True)
