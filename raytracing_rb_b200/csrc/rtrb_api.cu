@@ -769,9 +769,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   // 12.7 GB for one 4K / 64 spp frame) and no resolve launch.
   const bool strict_mode = opts.precision == RTRB_PREC_STRICT;
   int fuse = (S == 1 && cam->variant_threshold > 0) ? 1 : 0;
-#ifndef RTRB_NO_FUSE2  // (build-time A/B switch, profiles/README.md)
   if (!strict_mode && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0) fuse = 2;
-#endif
   const bool need_samples = fuse == 0;
   if ((need_samples && n_slots * (size_t)S * 3 * sizeof(double) > ((size_t)96 << 30)) || n_slots * (size_t)E * 3 * sizeof(double) > ((size_t)64 << 30))
     return fail(RTRB_ERR_UNSUPPORTED, "sample buffer would exceed the per-frame memory budget");

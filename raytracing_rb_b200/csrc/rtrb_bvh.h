@@ -42,10 +42,7 @@ inline void grow(Box& b, const BvhBuildSphere& s) {
   }
 }
 
-#ifndef RTRB_BVH_LEAF
-#define RTRB_BVH_LEAF 4
-#endif
-constexpr int kLeafSize = RTRB_BVH_LEAF;
+constexpr int kLeafSize = 4;
 
 // Recursively builds over order[first, first+count); returns the child reference for this subtree and its box.
 inline int32_t build(std::vector<BvhNode>& nodes, std::vector<BvhBuildSphere>& sph, int first, int count, Box* box_out) {

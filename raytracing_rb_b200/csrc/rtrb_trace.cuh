@@ -25,23 +25,78 @@ namespace rtrb {
 
 struct d3 { double x, y, z; };
 
-// libm's FP64 transcendentals are 100-500 SASS instructions each; inlined at every call site they push the
-// ray-tree kernels past 160 KB of code and the warps stall on instruction fetch (ncu: no_instruction is the
-// top stall of the depth-8 kernel).  One out-of-line copy each would keep more of the hot loop in the instruction
-// cache; results are unchanged (same routines).  MEASURED (round 1): out-of-line copies made configs 3-5
-// 4-5 % SLOWER (4.38 -> 4.62 ms on config 3), so the inlined form stays the default;
-// -DRTRB_OUTLINE_LIBM selects the out-of-line form.
-#ifndef RTRB_OUTLINE_LIBM
-#define RTRB_LIBM __device__ __forceinline__
-#else
-#define RTRB_LIBM static __device__ __noinline__
-#endif
-RTRB_LIBM double m_sin(double x) { return sin(x); }
-RTRB_LIBM double m_cos(double x) { return cos(x); }
-RTRB_LIBM double m_asin(double x) { return asin(x); }
-RTRB_LIBM double m_acos(double x) { return acos(x); }
-RTRB_LIBM double m_pow(double x, double y) { return pow(x, y); }
-RTRB_LIBM double m_fmod(double x, double y) { return fmod(x, y); }
+// ---- build policies ------------------------------------------------------------------------------------------------
+// What a kernel build knows at compile time.  The policy is the first template argument of every function whose code
+// depends on it, from the kernel body down.  STRICT is one build; the FAST64 kernels exist in several builds that differ
+// only in what is known about the scene (checked when it is baked, FrameParams::scene_class) or the frame, so that code
+// the class cannot reach is not compiled in.  Same source, same arithmetic, bit-identical results; what changes is code
+// size, register pressure and - these kernels being bound by instruction fetch and dependent issue - speed:
+//   fast          the exact-preserving shortcuts of FAST64 inside the shared STRICT functions (sphere_intersect).
+//   one_light     exactly one light and soft_shadow_exponent == 2 (every BASELINE.json config): no loops over
+//                 lights, no division by the number of matching / lit lights (x / 1.0 == x), no pow.
+//                 Ray-tree kernels: configs 3 / 4 / 5 -8.6 / -9.1 / -4.3 %.
+//   no_mc         monte_carlo_diffusion_times == 0: no Monte-Carlo ray code (configs 3 / 5 a further -1.6 / -4.9 %).
+//   lean          one_light plus: the light's radius is exactly 0 (hard shadows) and no object is textured: no
+//                 texture lookup, no penumbra branch in Sphere#cover_area.  Depth-1 kernels (config 2): -13 %.
+//   outline_libm  the FAST64 depth-1 builds (at<1>).  libm's FP64 transcendentals are 100-500 SASS instructions each.
+//                 In a depth-1 frame they (acos / sin of the penumbra and highlight fallbacks, pow, fmod) are cold, yet
+//                 inlined they put ~1 700 instructions between the hot blocks of a kernel whose top stall after `wait`
+//                 is `no_instruction`; as one out-of-line copy each (and the exact highlight test out of line) they sit
+//                 behind the kernel (config 2: -2 %).  The ray-tree kernels, where these calls are warm, keep them
+//                 inline: out of line measured +2 % .. +5 % there (round 1: config 3 4.38 -> 4.62 ms).
+template <bool FAST, bool ONE_LIGHT, bool LEAN, bool NO_MC, bool OUTLINE_LIBM = false>
+struct Policy {
+  static_assert(!LEAN || ONE_LIGHT, "a lean scene is a one-light scene");
+  static constexpr bool fast = FAST, one_light = ONE_LIGHT, lean = LEAN, no_mc = NO_MC, outline_libm = OUTLINE_LIBM;
+  // CTAs per SM that the depth-1 kernel's __launch_bounds__ asks for (128 threads each).  Generic: 5 (96 registers;
+  // config 2: 0.101 ms at 4 CTAs / 128 registers, 0.095 - 0.098 at 5 .. 8 CTAs / 96 .. 64 registers; 256 x 2: 0.103).
+  // Lean (124 registers unconstrained): 8, from 0.086 / 0.080 / 0.078 / 0.076 / 0.078 / 0.088 ms on config 2 at
+  // 4 / 5 / 7 / 8 / 10 / 12 CTAs per SM (124 / 96 / 72 / 64 / 48 / 40 registers).
+  static constexpr int d1_min_blocks = LEAN ? 8 : 5;
+  // this class's build for a work stack of MAXS items
+  template <int MAXS>
+  using at = Policy<FAST, ONE_LIGHT, LEAN, NO_MC, FAST && MAXS == 1>;
+
+  // FrameParams / material fields, or the constant the class fixes
+  __device__ static __forceinline__ int n_lights(const FrameParams& P) { return ONE_LIGHT ? 1 : P.n_lights; }
+  __device__ static __forceinline__ double shadow_exponent(const FrameParams& P) { return ONE_LIGHT ? 2.0 : P.soft_shadow_exponent; }
+  __device__ static __forceinline__ bool textured(const DevMat& M) { return LEAN ? false : M.tex != nullptr; }
+  __device__ static __forceinline__ int mc(const FrameParams& P) { return NO_MC ? 0 : P.mc; }
+};
+using Strict = Policy<false, false, false, false>;
+using Generic = Policy<true, false, false, false>;
+using OneLight = Policy<true, true, false, false>;
+using OneLightNoMc = Policy<true, true, false, true>;
+using Lean = Policy<true, true, true, false>;
+
+// libm wrappers: m_sin<Pol>(x) calls the one out-of-line copy cold::sin in the Policy::outline_libm builds and inlines
+// libm's sin in all others.  Likewise for the other functions.
+namespace cold {
+static __device__ __noinline__ double sin(double x) { return ::sin(x); }
+static __device__ __noinline__ double cos(double x) { return ::cos(x); }
+static __device__ __noinline__ double asin(double x) { return ::asin(x); }
+static __device__ __noinline__ double acos(double x) { return ::acos(x); }
+static __device__ __noinline__ double pow(double x, double y) { return ::pow(x, y); }
+static __device__ __noinline__ double fmod(double x, double y) { return ::fmod(x, y); }
+}  // namespace cold
+template <class Pol> __device__ __forceinline__ double m_sin(double x) {
+  if constexpr (Pol::outline_libm) return cold::sin(x); else return ::sin(x);
+}
+template <class Pol> __device__ __forceinline__ double m_cos(double x) {
+  if constexpr (Pol::outline_libm) return cold::cos(x); else return ::cos(x);
+}
+template <class Pol> __device__ __forceinline__ double m_asin(double x) {
+  if constexpr (Pol::outline_libm) return cold::asin(x); else return ::asin(x);
+}
+template <class Pol> __device__ __forceinline__ double m_acos(double x) {
+  if constexpr (Pol::outline_libm) return cold::acos(x); else return ::acos(x);
+}
+template <class Pol> __device__ __forceinline__ double m_pow(double x, double y) {
+  if constexpr (Pol::outline_libm) return cold::pow(x, y); else return ::pow(x, y);
+}
+template <class Pol> __device__ __forceinline__ double m_fmod(double x, double y) {
+  if constexpr (Pol::outline_libm) return cold::fmod(x, y); else return ::fmod(x, y);
+}
 
 __device__ __forceinline__ d3 mk(double x, double y, double z) { d3 r; r.x = x; r.y = y; r.z = z; return r; }
 __device__ __forceinline__ d3 ld3(const double* p) { return mk(p[0], p[1], p[2]); }
@@ -91,12 +146,14 @@ __device__ __forceinline__ double rb_sqrt(double x, ThreadCtx& ctx) {
   if (x < 0) ctx.status |= RTRB_ST_MATH_DOMAIN;
   return sqrt(x);
 }
+template <class Pol>
 __device__ __forceinline__ double rb_acos(double x, ThreadCtx& ctx) {
   if (x < -1 || x > 1) ctx.status |= RTRB_ST_MATH_DOMAIN;
-  return m_acos(x);
+  return m_acos<Pol>(x);
 }
 // Float ** exponent (world.rb:76).  pow(x, 2.0) is the correctly rounded x*x.
-__device__ __forceinline__ double rb_pow(double x, double y) { return (y == 2.0) ? x * x : m_pow(x, y); }
+template <class Pol>
+__device__ __forceinline__ double rb_pow(double x, double y) { return (y == 2.0) ? x * x : m_pow<Pol>(x, y); }
 
 // ---- counter RNG: Philox4x32-10 keyed by (seed; pixel, sample, ray path, purpose) ---------------
 __device__ __forceinline__ void philox4x32_10(uint32_t k0, uint32_t k1, uint32_t& c0, uint32_t& c1, uint32_t& c2,
@@ -124,6 +181,7 @@ struct HitRec {
 };
 
 // Sphere#intersect (sphere.rb:60-85).  d_r = |d|, dn = d / d_r are ray invariants.
+template <class Pol>
 __device__ __forceinline__ bool sphere_intersect(const DevGeom& g, d3 o, d3 d, double d_r, d3 dn, HitRec& h) {
   d3 c = mk(g.px, g.py, g.pz);
   d3 oc = c - o;
@@ -135,18 +193,18 @@ __device__ __forceinline__ bool sphere_intersect(const DevGeom& g, d3 o, d3 d, d
   double hh = sqrt(g.radius * g.radius - nd * nd);
   d3 vec = dn * hh;
   // from_inner = |O - C| <= R (|O - C| == |C - O| bit for bit)
-#ifdef RTRB_FAST_TU
-  // FAST64 translation units: sqrt is monotone and correctly rounded, so away from the surface the comparison of the
-  // squares decides (1e-14 >> 2^-52 covers the roundings of R*R and of the sum); inside that band, and for NaNs,
-  // negative or overflowing radii, the reference's own expression is evaluated.
-  const double oc2 = sumsq(oc), rr2 = g.radius * g.radius;
   bool from_inner;
-  if (g.radius >= 0 && rr2 < 1e300 && oc2 < rr2 * (1.0 - 1e-14)) from_inner = true;
-  else if (g.radius >= 0 && rr2 < 1e300 && oc2 > rr2 * (1.0 + 1e-14)) from_inner = false;
-  else from_inner = sqrt(oc2) <= g.radius;
-#else
-  const bool from_inner = norm(oc) <= g.radius;
-#endif
+  if constexpr (Pol::fast) {
+    // FAST64: sqrt is monotone and correctly rounded, so away from the surface the comparison of the squares decides
+    // (1e-14 >> 2^-52 covers the roundings of R*R and of the sum); inside that band, and for NaNs, negative or
+    // overflowing radii, the reference's own expression is evaluated.
+    const double oc2 = sumsq(oc), rr2 = g.radius * g.radius;
+    if (g.radius >= 0 && rr2 < 1e300 && oc2 < rr2 * (1.0 - 1e-14)) from_inner = true;
+    else if (g.radius >= 0 && rr2 < 1e300 && oc2 > rr2 * (1.0 + 1e-14)) from_inner = false;
+    else from_inner = sqrt(oc2) <= g.radius;
+  } else {
+    from_inner = norm(oc) <= g.radius;
+  }
   h.dir_in = !from_inner;
   h.p = h.dir_in ? (np - vec) : (np + vec);
   if (!from_inner && t < 0) return false;
@@ -229,14 +287,14 @@ __device__ __forceinline__ CoverRay make_cover_ray(d3 target, const DevLight& L)
 // KIND tells what the caller already knows about g.type, so that the other branches are not compiled into its loop
 // (the sphere branch with its penumbra code is 800 instructions): 0 = anything (the reference's own scan), 1 = a sphere
 // or a box (an entry of the sphere filter), 2 = a plane.
-template <bool BOX = true, int KIND = 0>
+template <class Pol, bool BOX = true, int KIND = 0>
 __device__ __forceinline__ double cover_object_exact(const FrameParams& P, const DevGeom& g, const CoverRay& c,
                                                      double light_radius, ThreadCtx& ctx) {
   if (KIND != 2 && g.type == RTRB_OBJ_SPHERE) {
     RTRB_COUNT(ctx, RTRB_CNT_COV_SPH);
     HitRec h;
     int factor = 0;
-    if (sphere_intersect(g, c.target, c.lt, c.lt_r, c.ltn, h) && dot(h.p - c.lp, c.tl) > 0) factor = 1;
+    if (sphere_intersect<Pol>(g, c.target, c.lt, c.lt_r, c.ltn, h) && dot(h.p - c.lp, c.tl) > 0) factor = 1;
     d3 cc = mk(g.px, g.py, g.pz);
     double t = dot(cc - c.target, c.lt) / (c.lt_r * c.lt_r);
     d3 x1 = c.target + c.lt * t;
@@ -244,20 +302,19 @@ __device__ __forceinline__ double cover_object_exact(const FrameParams& P, const
     double dd = norm(x1 - cc);
     if (dd >= r1 + g.radius) return 0;
     double s1 = RTRB_PI * r1 * r1;
-#ifdef RTRB_SCENE_LEAN
-    // light_radius == 0.0, so r1 is a zero or a NaN (0 * inf).  Past the test above dd < R (or a comparison with a NaN
-    // failed); then `dd > |R - r1|` = `dd > |R|` cannot hold (R >= 0: dd < R; R < 0: no dd >= 0 is < R; NaN: false), so
-    // the partial-overlap branch (sphere.rb:37-47) is unreachable and its acos / sin / divisions are not compiled in
-    if (false) {
-#else
-    if (dd > fabs(g.radius - r1)) {
-#endif
-      RTRB_COUNT(ctx, RTRB_CNT_COV_SPH_PEN);
-      double ct1 = fmin((r1 * r1 + dd * dd - g.radius * g.radius) / (2 * r1 * dd), 1.0);
-      double ct2 = fmin((g.radius * g.radius + dd * dd - r1 * r1) / (2 * g.radius * dd), 1.0);
-      double th1 = rb_acos(ct1, ctx), th2 = rb_acos(ct2, ctx);
-      double delta_s = ((th1 - m_sin(th1)) * r1 * r1 + (th2 - m_sin(th2)) * g.radius * g.radius) / 2;
-      return factor * delta_s / s1;
+    // Lean scenes: light_radius == 0.0, so r1 is a zero or a NaN (0 * inf).  Past the test above dd < R (or a comparison
+    // with a NaN failed); then `dd > |R - r1|` = `dd > |R|` cannot hold (R >= 0: dd < R; R < 0: no dd >= 0 is < R; NaN:
+    // false), so the partial-overlap branch (sphere.rb:37-47) is unreachable and its acos / sin / divisions are not
+    // compiled in
+    if constexpr (!Pol::lean) {
+      if (dd > fabs(g.radius - r1)) {
+        RTRB_COUNT(ctx, RTRB_CNT_COV_SPH_PEN);
+        double ct1 = fmin((r1 * r1 + dd * dd - g.radius * g.radius) / (2 * r1 * dd), 1.0);
+        double ct2 = fmin((g.radius * g.radius + dd * dd - r1 * r1) / (2 * g.radius * dd), 1.0);
+        double th1 = rb_acos<Pol>(ct1, ctx), th2 = rb_acos<Pol>(ct2, ctx);
+        double delta_s = ((th1 - m_sin<Pol>(th1)) * r1 * r1 + (th2 - m_sin<Pol>(th2)) * g.radius * g.radius) / 2;
+        return factor * delta_s / s1;
+      }
     }
     RTRB_COUNT(ctx, RTRB_CNT_COV_SPH_FULL);
     if (r1 > g.radius) return factor * RTRB_PI * g.radius * g.radius / s1;
@@ -274,26 +331,29 @@ __device__ __forceinline__ double cover_object_exact(const FrameParams& P, const
       return 0;
     }
   }
-  if constexpr (KIND == 1) return 0;  // (unreachable: the sphere filter only lists spheres and boxes)
-  RTRB_COUNT(ctx, RTRB_CNT_COV_PL);
-  HitRec h;
-  double den;
-  if (plane_intersect(g, c.target, c.lt, h, den) && dot(h.p - c.lp, c.tl) > 0) {
-    RTRB_COUNT(ctx, RTRB_CNT_COV_PL_ACC);
-    return 1;
+  if constexpr (KIND == 1) {
+    return 0;  // (unreachable: the sphere filter only lists spheres and boxes)
+  } else {
+    RTRB_COUNT(ctx, RTRB_CNT_COV_PL);
+    HitRec h;
+    double den;
+    if (plane_intersect(g, c.target, c.lt, h, den) && dot(h.p - c.lp, c.tl) > 0) {
+      RTRB_COUNT(ctx, RTRB_CNT_COV_PL_ACC);
+      return 1;
+    }
+    return 0;
   }
-  return 0;
 }
 
 // World#lit_area (world.rb:62-69) for one light seen from `target`:
 // max(1 - sum over ALL objects of cover_area, 0), subtraction in world_objects order.
-template <bool BOX = true>
+template <class Pol, bool BOX = true>
 static __device__ __noinline__ double lit_area(const FrameParams& P, d3 target, const DevLight& L, ThreadCtx& ctx) {
   const CoverRay c = make_cover_ray(target, L);
   double total = 1;
   for (int i = 0; i < P.n_objects; ++i) {
     const DevGeom g = P.geom[i];
-    total -= cover_object_exact<BOX>(P, g, c, L.radius, ctx);
+    total -= cover_object_exact<Pol, BOX>(P, g, c, L.radius, ctx);
   }
   return fmax(total, 0.0);
 }
@@ -311,21 +371,23 @@ __device__ __forceinline__ d3 a_vertical_vector(d3 n, ThreadCtx& ctx) {
 // Float#to_i then Integer#% (texture.rb:24-25): truncation toward zero, then FLOORED modulo by a positive size.
 // `t` is already truncated.  Values that fit 32 bits take the integer path (the remainder of an integer division is
 // exact either way, so the result equals fmod's: -2.6 % instructions on config 3); anything larger goes through fmod.
+template <class Pol>
 __device__ __forceinline__ int trunc_mod(double t, int n) {
   if (fabs(t) < 2147483648.0) {
     int m = (int)t % n;
     return m < 0 ? m + n : m;
   }
-  double m = m_fmod(t, (double)n);
+  double m = m_fmod<Pol>(t, (double)n);
   if (m < 0) m += n;
   return (int)m;
 }
 
 // Texture#color (texture.rb:23-28)
+template <class Pol>
 __device__ __forceinline__ d3 texture_color(const DevMat& m, double uu, double vv, ThreadCtx& ctx) {
   double fu = (uu + m.uoff) / m.hscale, fv = (vv + m.voff) / m.vscale;
   if (!isfinite(fu) || !isfinite(fv)) { ctx.status |= RTRB_ST_NAN_TO_INT; return mk(0, 0, 0); }
-  const int u = trunc_mod(trunc(fu), m.tex_w), v = trunc_mod(trunc(fv), m.tex_h);
+  const int u = trunc_mod<Pol>(trunc(fu), m.tex_w), v = trunc_mod<Pol>(trunc(fv), m.tex_h);
   const uint8_t* p = m.tex + ((size_t)v * m.tex_w + u) * 3;
   return mk(__ldg(p) / 256.0, __ldg(p + 1) / 256.0, __ldg(p + 2) / 256.0);
 }
@@ -352,7 +414,7 @@ struct StackItem {
 
 // RayTracer#trace_sync for one sample.  Returns the summed colour; *primary_hit gets the root ray's
 // World#intersect winner (-1 miss, -2 highlight-terminated).
-template <int MAXS, bool MT = false>
+template <class Pol, int MAXS, bool MT = false>
 __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                            ThreadCtx& ctx, int* primary_hit, MtCursor* mt = nullptr) {
   StackItem stack[MAXS];
@@ -384,7 +446,7 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
       const DevLight& L = P.lights[l];
       d3 a = mk(L.px, L.py, L.pz) - o;
       double ct = vcos(d, a, ctx);
-      double ang = rb_acos(ct, ctx);
+      double ang = rb_acos<Pol>(ct, ctx);
       if (ang < L.hl_threshold) { hl_mask |= 1ull << l; hl_n++; }
     }
     if (hl_n > 0) {
@@ -411,7 +473,7 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
       bool ok;
       if (g.type == RTRB_OBJ_SPHERE) {
         RTRB_COUNT(ctx, RTRB_CNT_SPH_TEST);
-        ok = sphere_intersect(g, o, d, d_r, dn, h);
+        ok = sphere_intersect<Pol>(g, o, d, d_r, dn, h);
         if (ok) RTRB_COUNT(ctx, RTRB_CNT_SPH_ACC);
       } else if (g.type == RTRB_OBJ_BOX) {
         RTRB_COUNT(ctx, RTRB_CNT_BOX_TEST);
@@ -470,8 +532,8 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
       double sin_r = sin_i / rate;
       if (!(sin_r >= 1)) {
         if (sin_r < -1 || sin_r > 1) ctx.status |= RTRB_ST_MATH_DOMAIN;
-        double r = m_asin(sin_r);
-        refr_dir = nn * (-m_cos(r)) + normalize(refl_dir + d, ctx) * sin_r;
+        double r = m_asin<Pol>(sin_r);
+        refr_dir = nn * (-m_cos<Pol>(r)) + normalize(refl_dir + d, ctx) * sin_r;
         refr_org = bh.p - nn * RTRB_EPSILON;
         has_refr = true;
       }
@@ -503,9 +565,9 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
     for (int l = 0; l < P.n_lights; ++l) {
       const DevLight& L = P.lights[l];
       ctx.shadow++;
-      double area = lit_area(P, shade_from, L, ctx);
+      double area = lit_area<Pol>(P, shade_from, L, ctx);
       if (area > 0) {
-        d3 lc = ld3(L.color) * (rb_pow(area, P.soft_shadow_exponent) / (double)P.n_lights);
+        d3 lc = ld3(L.color) * (rb_pow<Pol>(area, P.soft_shadow_exponent) / (double)P.n_lights);
         d3 lv = normalize(mk(L.px, L.py, L.pz) - bh.p, ctx);  // shading point is WITHOUT delta (:152)
         double ldn = dot(lv, nn);
         if (ldn > 1) ldn = 1.0; else if (ldn < 0) ldn = 0.0;
@@ -530,7 +592,7 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
             u_theta = res53(c0, c1); u_phi = res53(c2, c3);
           }
           double theta = u_theta * RTRB_PI / 2, phi = u_phi * RTRB_PI * 2;
-          d3 dir = nn * m_sin(theta) + (leftv * m_cos(phi) + upv * m_sin(phi)) * m_cos(theta);
+          d3 dir = nn * m_sin<Pol>(theta) + (leftv * m_cos<Pol>(phi) + upv * m_sin<Pol>(phi)) * m_cos<Pol>(theta);
           RTRB_COUNT(ctx, RTRB_CNT_MC);
           StackItem& s = stack[sp++];
           d3 a2 = att * att_pt;
@@ -561,7 +623,7 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
           v = dot(rel, ld3(M.e1)) / M.v_unit;
         }
         RTRB_COUNT(ctx, RTRB_CNT_TEXEL);
-        filter = texture_color(M, u, v, ctx) * filter;
+        filter = texture_color<Pol>(M, u, v, ctx) * filter;
       }
       d3 local = ((contrib * ld3(M.diffuse)) * filter) + ld3(M.ambient);
       d3 c = att * local;  // ray_tracer.rb:152
@@ -573,6 +635,7 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
 }
 
 // Camera#lens_func (camera.rb:129-151) for pixel (x, y) and aperture angle theta.
+template <class Pol>
 __device__ __forceinline__ void lens_ray(const FrameParams& P, int x, int y, double theta, d3& ro, d3& rd) {
   d3 pos = ld3(P.pos), left = ld3(P.left), upn = ld3(P.up_n), front = ld3(P.front);
   // host-built tables of 2.0 * (x.to_f / width - 0.5) * retina_width and the y analogue (camera.rb:133-134)
@@ -583,7 +646,7 @@ __device__ __forceinline__ void lens_ray(const FrameParams& P, int x, int y, dou
   // adding a zero of either sign to `pos` gives `pos` (up to the sign of an exact zero, which no later
   // expression can observe), so the two FP64 transcendentals are skipped.
   d3 rand_vector = mk(0.0, 0.0, 0.0);
-  if (P.aperture_radius != 0.0) rand_vector = (ld3(P.left_n) * m_cos(theta) + upn * m_sin(theta)) * P.aperture_radius;
+  if (P.aperture_radius != 0.0) rand_vector = (ld3(P.left_n) * m_cos<Pol>(theta) + upn * m_sin<Pol>(theta)) * P.aperture_radius;
   d3 aperture = pos + rand_vector;
   d3 rf = pos - retina_position;  // ray retina -> lens centre
   double t = dot(ld3(P.focal_point) - retina_position, front) / dot(front, rf);  // intersect_plane :123-127
@@ -698,23 +761,22 @@ __device__ __forceinline__ void merge_ctx(ThreadCtx& ctx, const ThreadCtx& t) {
 }
 
 // FAST64 entry point, defined in rtrb_trace_fast.cuh (only instantiated by that translation unit).
-template <int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                                 ThreadCtx& ctx, int* primary_hit);
 
-// MODE: 0 = STRICT, 1 = FAST64 with the linear filter, 2 = FAST64 with the sphere BVH.
+// BVH: FAST64 with the sphere BVH instead of the linear filter.
 // BOX: the FAST64 kernels carry the Box code only in their full-counter (DETAIL) variants; scenes with a
 // box are always dispatched there (rtrb_api.cu), so the lean hot kernels stay sphere/plane-only.
-template <int MAXS, int MODE, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                              ThreadCtx& ctx, int* primary_hit) {
-  if constexpr (MODE == 2) return trace_sample_fast<MAXS, true, BOX>(P, ro, rd, pixel, sample, ctx, primary_hit);
-  else if constexpr (MODE == 1) return trace_sample_fast<MAXS, false, BOX>(P, ro, rd, pixel, sample, ctx, primary_hit);
-  else return trace_sample<MAXS>(P, ro, rd, pixel, sample, ctx, primary_hit);
+  if constexpr (Pol::fast) return trace_sample_fast<Pol, MAXS, BVH, BOX>(P, ro, rd, pixel, sample, ctx, primary_hit);
+  else return trace_sample<Pol, MAXS>(P, ro, rd, pixel, sample, ctx, primary_hit);
 }
 
 // One thread per (pixel, sample j < pre_sample_times): the first loop of render_at (camera.rb:73-78).
-template <int MAXS, bool DETAIL, int MODE = 0>
+template <class Pol, int MAXS, bool DETAIL, bool BVH = false>
 __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
   const uint32_t S = (uint32_t)P.pre;
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -737,9 +799,9 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
         theta = res53(c0, c1);  // Random.rand, camera.rb:135
       }
       d3 ro, rd;
-      lens_ray(P, x, y, theta, ro, rd);
+      lens_ray<Pol>(P, x, y, theta, ro, rd);
       int ph;
-      d3 col = trace_dispatch<MAXS, MODE, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
+      d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
       if (P.fuse_resolve) {
         // one sample, positive threshold: mean = s / 1.0 = s and variance = 0 < threshold (camera.rb:80-87)
@@ -756,7 +818,7 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
 
 // Extra samples j in [pre, max) of the pixels that failed the variance test (camera.rb:88-93);
 // persistent grid-stride loop because the pixel count is only known on the device.
-template <int MAXS, bool DETAIL, int MODE = 0>
+template <class Pol, int MAXS, bool DETAIL, bool BVH = false>
 __device__ __forceinline__ void trace_extra_body(const FrameParams& P) {
   const uint32_t E = (uint32_t)(P.max_samples - P.pre);
   const unsigned long long total = (unsigned long long)(*P.extra_count) * E;
@@ -778,9 +840,9 @@ __device__ __forceinline__ void trace_extra_body(const FrameParams& P) {
       theta = res53(c0, c1);
     }
     d3 ro, rd;
-    lens_ray(P, x, y, theta, ro, rd);
+    lens_ray<Pol>(P, x, y, theta, ro, rd);
     int ph;
-    d3 col = trace_dispatch<MAXS, MODE, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
+    d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
     RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
     double* out = P.extra_samples + w * 3ull;
     out[0] = col.x; out[1] = col.y; out[2] = col.z;
@@ -813,7 +875,7 @@ __device__ __forceinline__ void pre_mean(const FrameParams& P, uint32_t slot, do
 // aperture is 0), its Monte-Carlo draws in LIFO ray order, then the next sample, then the adaptive samples.
 // The thread reads its draws from mt_stream starting at mt_offset[pixel order] and reports how many it used;
 // the host iterates offsets = prefix sums of the counts until they stop changing (rtrb_api.cu).
-template <int MAXS, bool DETAIL>
+template <class Pol, int MAXS, bool DETAIL>
 __device__ __forceinline__ void trace_mt_body(const FrameParams& P) {
   const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
   ThreadCtx ctx;
@@ -832,9 +894,9 @@ __device__ __forceinline__ void trace_mt_body(const FrameParams& P) {
     for (int j = 0; j < S; ++j) {
       const double theta = cur.next();
       d3 ro, rd;
-      lens_ray(P, x, y, theta, ro, rd);
+      lens_ray<Pol>(P, x, y, theta, ro, rd);
       int ph;
-      d3 col = trace_sample<MAXS, true>(P, ro, rd, pixel, (uint32_t)j, ctx, &ph, &cur);
+      d3 col = trace_sample<Pol, MAXS, true>(P, ro, rd, pixel, (uint32_t)j, ctx, &ph, &cur);
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
       smp[j * 3 + 0] = col.x; smp[j * 3 + 1] = col.y; smp[j * 3 + 2] = col.z;
       if (j == 0 && P.hit) P.hit[(size_t)y * P.width + x] = ph;
@@ -847,9 +909,9 @@ __device__ __forceinline__ void trace_mt_body(const FrameParams& P) {
       for (int j = S; j < P.max_samples; ++j) {
         const double theta = cur.next();
         d3 ro, rd;
-        lens_ray(P, x, y, theta, ro, rd);
+        lens_ray<Pol>(P, x, y, theta, ro, rd);
         int ph;
-        d3 col = trace_sample<MAXS, true>(P, ro, rd, pixel, (uint32_t)j, ctx, &ph, &cur);
+        d3 col = trace_sample<Pol, MAXS, true>(P, ro, rd, pixel, (uint32_t)j, ctx, &ph, &cur);
         RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
         cx += col.x; cy += col.y; cz += col.z;
       }

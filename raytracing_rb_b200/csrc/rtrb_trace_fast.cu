@@ -1,38 +1,57 @@
-// rtrb_trace_fast.cu — RTRB_PREC_FAST64 dispatch (FP32 filter + exact FP64 refine).  The kernels are instantiated
-// per work-stack capacity in rtrb_trace_fast_{d1,t10,t32,t128}.cu and, for the scene / frame classes of
-// rtrb_trace_fast.cuh, once more in the *_l1 / *_l1n / d1lean translation units (all compiled -fmad=false: the exact
-// parts must round like STRICT; the filter uses explicit fmaf()).
-#include "rtrb_launch.h"
-
-#define RTRB_DECLARE_NS(ns)                                       \
-  namespace ns {                                                  \
-  cudaError_t pre_d1(const FrameParams& P, cudaStream_t s);       \
-  cudaError_t extra_d1(const FrameParams& P, cudaStream_t s);     \
-  cudaError_t pre_t10(const FrameParams& P, cudaStream_t s);      \
-  cudaError_t extra_t10(const FrameParams& P, cudaStream_t s);    \
-  cudaError_t pre_t32(const FrameParams& P, cudaStream_t s);      \
-  cudaError_t extra_t32(const FrameParams& P, cudaStream_t s);    \
-  cudaError_t pre_t128(const FrameParams& P, cudaStream_t s);     \
-  cudaError_t extra_t128(const FrameParams& P, cudaStream_t s);   \
-  }
-RTRB_DECLARE_NS(rtrb_fast)       // generic: d1, t10, t32, t128
-RTRB_DECLARE_NS(rtrb_fast_lean)  // d1 only
-RTRB_DECLARE_NS(rtrb_fast_l1)    // t10, t32
-RTRB_DECLARE_NS(rtrb_fast_l1n)   // t10, t32
+// rtrb_trace_fast.cu — RTRB_PREC_FAST64 dispatch (FP32 filter + exact FP64 refine).  The kernels of each class build
+// and work-stack capacity are instantiated in their own translation unit (rtrb_trace_fast_launch.cuh).
+#include "rtrb_trace_fast_launch.cuh"
 
 // A persistent-THREAD variant (single lanes refetch a new sample when their stack empties) was measured in round 1
 // and rejected: it mixed unrelated rays into one warp (22.9 instead of 29.1 of 32 lanes active on config 3).  Round 2
 // measured warp-granular refill as well (profiles/README.md): also rejected.
 
-#define RTRB_FAST_DISPATCH(fn)                                                                              \
-  const bool one_light = (P.scene_class & RTRB_SCENE_CLASS_ONE_LIGHT) != 0;                                 \
-  if (P.trace_depth <= 1)                                                                                   \
-    return (P.scene_class & RTRB_SCENE_CLASS_LEAN) ? rtrb_fast_lean::fn##_d1(P, s) : rtrb_fast::fn##_d1(P, s); \
-  if (stack_need <= 10)                                                                                     \
-    return !one_light ? rtrb_fast::fn##_t10(P, s) : (P.mc == 0 ? rtrb_fast_l1n::fn##_t10(P, s) : rtrb_fast_l1::fn##_t10(P, s)); \
-  if (stack_need <= 32)                                                                                     \
-    return !one_light ? rtrb_fast::fn##_t32(P, s) : (P.mc == 0 ? rtrb_fast_l1n::fn##_t32(P, s) : rtrb_fast_l1::fn##_t32(P, s)); \
-  return rtrb_fast::fn##_t128(P, s);
+namespace {
 
-cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cudaStream_t s) { RTRB_FAST_DISPATCH(pre) }
-cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int stack_need, cudaStream_t s) { RTRB_FAST_DISPATCH(extra) }
+// Every build that exists, the most specialised class first within each capacity: a frame runs the first build of
+// its capacity whose class it belongs to.
+const FastKernels* const kBuilds[] = {
+    &rtrb_fast_lean::d1, &rtrb_fast::d1,
+    &rtrb_fast_l1n::t10, &rtrb_fast_l1::t10, &rtrb_fast::t10,
+    &rtrb_fast_l1n::t32, &rtrb_fast_l1::t32, &rtrb_fast::t32,
+    &rtrb_fast::t128,
+};
+
+const FastKernels* build_for(const FrameParams& P, int stack_need) {
+  const int capacity = P.trace_depth <= 1 ? 1 : stack_capacity(stack_need);
+  const bool one_light = (P.scene_class & RTRB_SCENE_CLASS_ONE_LIGHT) != 0;
+  const bool lean = (P.scene_class & RTRB_SCENE_CLASS_LEAN) != 0;
+  for (const FastKernels* k : kBuilds)
+    if (k->capacity == capacity && (one_light || !k->one_light) && (lean || !k->lean) && (P.mc == 0 || !k->no_mc)) return k;
+  return nullptr;
+}
+
+}  // namespace
+
+cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cudaStream_t s) {
+  const FastKernels* k = build_for(P, stack_need);
+  if (!k) return cudaErrorInvalidValue;
+  const TraceKernel kernel = k->pre[P.count_detail != 0][P.use_bvh != 0];
+  // one thread per (pixel, sample); the ray-tree kernels run lockstep CTAs (rtrb_trace_fast.cuh, trace_pre_tree_body),
+  // more and smaller ones on small frames
+  const unsigned long long threads = pre_threads(P);
+  if (threads == 0) return cudaSuccess;
+  int block = kFastBlock;
+  if (k->capacity > 1) block = threads < 4ull * (unsigned long long)sm_count() * kTreeBlock ? RTRB_TREE_MIN_BLOCK : kTreeBlock;
+  const long long blocks = grid_size(threads, block);
+  if (blocks < 0) return cudaErrorInvalidConfiguration;
+  // in-CTA resolve (fuse_resolve == 2, ray-tree frames only): the host only selects it for sample counts that divide
+  // both CTA sizes
+  if (P.fuse_resolve == 2 && (block % P.pre) != 0) return cudaErrorInvalidConfiguration;
+  const size_t smem = P.fuse_resolve == 2 ? (size_t)block * 3u * sizeof(double) : 0u;
+  kernel<<<(unsigned)blocks, block, smem, s>>>(P);
+  return cudaGetLastError();
+}
+
+cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int stack_need, cudaStream_t s) {
+  const FastKernels* k = build_for(P, stack_need);
+  if (!k) return cudaErrorInvalidValue;
+  const TraceKernel kernel = k->extra[P.count_detail != 0][P.use_bvh != 0];
+  kernel<<<extra_grid(), kFastBlock, 0, s>>>(P);
+  return cudaGetLastError();
+}

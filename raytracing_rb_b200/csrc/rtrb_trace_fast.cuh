@@ -12,41 +12,11 @@
 //   * children that cannot survive the cut at ray_tracer.rb:52 are not computed;
 //   * divisions by exactly 1.0 (one light) are skipped; the attenuation cut avoids its sqrt
 //     outside a narrow band around the threshold.
+// What a scene / frame class fixes comes from the build policy (rtrb_trace.cuh, "build policies").
 //
 // Compiled with -fmad=false as well: the exact parts must not contract; the FP32 filter uses
 // explicit fmaf().
 #pragma once
-#define RTRB_FAST_TU 1  // exact-preserving shortcuts inside the shared STRICT functions (rtrb_trace.cuh)
-// SCENE / FRAME CLASSES.  The kernels exist in several builds that differ only in what is known at compile time about
-// the scene (checked when it is baked, FrameParams::scene_class) or the frame, so that code the class cannot reach is
-// not compiled in.  Same source, same arithmetic, bit-identical results; what changes is code size, register pressure
-// and - these kernels being bound by instruction fetch and dependent issue - speed:
-//   RTRB_SCENE_ONE_LIGHT  exactly one light and soft_shadow_exponent == 2 (every BASELINE.json config): no loops over
-//                         lights, no division by the number of matching / lit lights (x / 1.0 == x), no pow.
-//                         Ray-tree kernels: configs 3 / 4 / 5 -8.6 / -9.1 / -4.3 %.
-//   RTRB_FRAME_NO_MC      monte_carlo_diffusion_times == 0: no Monte-Carlo ray code (configs 3 / 5 a further -1.6 / -4.9 %).
-//   RTRB_SCENE_LEAN       ONE_LIGHT plus: the light's radius is exactly 0 (hard shadows) and no object is textured: no
-//                         texture lookup, no penumbra branch in Sphere#cover_area.  Depth-1 kernels (config 2): -13 %.
-#ifdef RTRB_SCENE_LEAN
-#define RTRB_SCENE_ONE_LIGHT 1
-#endif
-#ifdef RTRB_SCENE_ONE_LIGHT
-#define RTRB_NL(P) 1
-#define RTRB_EXP(P) 2.0
-#else
-#define RTRB_NL(P) (P).n_lights
-#define RTRB_EXP(P) (P).soft_shadow_exponent
-#endif
-#ifdef RTRB_SCENE_LEAN
-#define RTRB_TEX(M) false
-#else
-#define RTRB_TEX(M) ((M).tex != nullptr)
-#endif
-#ifdef RTRB_FRAME_NO_MC
-#define RTRB_MC(P) 0
-#else
-#define RTRB_MC(P) (P).mc
-#endif
 #include "rtrb_trace.cuh"
 
 namespace rtrb {
@@ -185,7 +155,7 @@ struct Pack8 {
 };
 
 // The reference's own scan (world.rb:44-57); used when the filter keeps more survivors than fit.
-template <bool BOX>
+template <class Pol, bool BOX>
 static __device__ __noinline__ int closest_hit_scan(const FrameParams& P, d3 o, d3 d, HitRec& bh, ThreadCtx& ctx) {
   const double d_r = norm(d);
   const d3 dn = mk(d.x / d_r, d.y / d_r, d.z / d_r);
@@ -196,7 +166,7 @@ static __device__ __noinline__ int closest_hit_scan(const FrameParams& P, d3 o, 
     HitRec h;
     bool ok;
     double den;
-    if (g.type == RTRB_OBJ_SPHERE) ok = sphere_intersect(g, o, d, d_r, dn, h);
+    if (g.type == RTRB_OBJ_SPHERE) ok = sphere_intersect<Pol>(g, o, d, d_r, dn, h);
     else if (BOX && g.type == RTRB_OBJ_BOX) ok = box_intersect(P.boxes[g.aux], o, d, h);
     else ok = plane_intersect(g, o, d, h, den);
     RTRB_COUNT(ctx, RTRB_CNT_EXACT);
@@ -211,22 +181,22 @@ static __device__ __noinline__ int closest_hit_scan(const FrameParams& P, d3 o, 
 // The out-of-line fallbacks get TEMPORARIES for everything they take by reference: a thread's own hit record and
 // counter block must never have their address taken, or they live in local memory for the whole kernel (ncu:
 // 36 local loads/stores per thread on the config 2 kernel before this) instead of registers.
-template <bool BOX>
+template <class Pol, bool BOX>
 __device__ __forceinline__ int closest_hit_scan_call(const FrameParams& P, d3 o, d3 d, HitRec& bh, ThreadCtx& ctx) {
   HitRec h;
   h.p = mk(0, 0, 0); h.dir_in = false; h.face = 0;
   ThreadCtx t;
   init_ctx(t, ctx.detail);
-  const int i = closest_hit_scan<BOX>(P, o, d, h, t);
+  const int i = closest_hit_scan<Pol, BOX>(P, o, d, h, t);
   if (i >= 0) keep_hit<BOX>(bh, h);
   merge_ctx(ctx, t);
   return i;
 }
-template <bool BOX>
+template <class Pol, bool BOX>
 __device__ __forceinline__ double lit_area_call(const FrameParams& P, d3 target, const DevLight& L, ThreadCtx& ctx) {
   ThreadCtx t;
   init_ctx(t, ctx.detail);
-  const double a = lit_area<BOX>(P, target, L, t);
+  const double a = lit_area<Pol, BOX>(P, target, L, t);
   merge_ctx(ctx, t);
   return a;
 }
@@ -306,12 +276,12 @@ __device__ __forceinline__ bool bvh_traverse(const FrameParams& P, const BvhRay&
 }
 
 // World#intersect (world.rb:37-59) = FP32 filter (planes + sphere BVH) + exact test of the survivors.
-template <bool BOX>
+template <class Pol, bool BOX>
 __device__ __forceinline__ int closest_hit_bvh(const FrameParams& P, d3 o, d3 d, const CullRay& r, HitRec& bh,
                                                 ThreadCtx& ctx) {
   // Pack8 keeps survivor slots in 16 bits: the BVH filter serves scenes of up to 65 536 bounded objects (larger ones
   // take the reference's own scan: correct, but brute force)
-  if (P.n_sph > 0x10000 || P.n_pl > 8) return closest_hit_scan_call<BOX>(P, o, d, bh, ctx);
+  if (P.n_sph > 0x10000 || P.n_pl > 8) return closest_hit_scan_call<Pol, BOX>(P, o, d, bh, ctx);
   // pass 1a: planes bound the search first (nothing at or beyond max_distance can win, world.rb:39)
   float best_hi = P.max_distance_f;
   for (int k = 0; k < P.n_pl; ++k) {
@@ -333,7 +303,7 @@ __device__ __forceinline__ int closest_hit_bvh(const FrameParams& P, d3 o, d3 d,
         if (kind == 2 && hi < best_hi) { best_hi = hi; tmax = hi + r.E; }
       }
     });
-    if (!ok || S.overflow()) return closest_hit_scan_call<BOX>(P, o, d, bh, ctx);
+    if (!ok || S.overflow()) return closest_hit_scan_call<Pol, BOX>(P, o, d, bh, ctx);
   }
   // pass 2: exact FP64 evaluation of whatever can still win; (distance, index) lexicographic order
   // reproduces the strict `<` scan in world_objects order.
@@ -352,7 +322,7 @@ __device__ __forceinline__ int closest_hit_bvh(const FrameParams& P, d3 o, d3 d,
     const DevGeom g = P.geom[i];
     HitRec h;
     RTRB_COUNT(ctx, RTRB_CNT_EXACT);
-    if ((BOX && g.type == RTRB_OBJ_BOX) ? box_intersect(P.boxes[g.aux], o, d, h) : sphere_intersect(g, o, d, d_r, dn, h)) {
+    if ((BOX && g.type == RTRB_OBJ_BOX) ? box_intersect(P.boxes[g.aux], o, d, h) : sphere_intersect<Pol>(g, o, d, d_r, dn, h)) {
       const double new_dis = norm(o - h.p);
       if (new_dis < best || (new_dis == best && best_i >= 0 && i < best_i)) { best = new_dis; best_i = i; keep_hit<BOX>(bh, h); }
     }
@@ -378,7 +348,7 @@ __device__ __forceinline__ int closest_hit_bvh(const FrameParams& P, d3 o, d3 d,
 // An object the probe ray certainly misses (or certainly meets beyond the light) has factor 0, hence
 // cover exactly 0 (sphere.rb:29,45-53 multiply everything by factor; world_object.rb:43-47), and
 // total - 0 == total, so skipping it leaves the running difference bit-identical.
-template <bool BOX>
+template <class Pol, bool BOX>
 __device__ __forceinline__ double lit_area_bvh(const FrameParams& P, d3 target, const DevLight& L, ThreadCtx& ctx) {
   CoverRay c;
   c.target = target;
@@ -392,7 +362,7 @@ __device__ __forceinline__ double lit_area_bvh(const FrameParams& P, d3 target, 
     const float lx = (float)c.lt.x, ly = (float)c.lt.y, lz = (float)c.lt.z;
     far = sqrt_approx(fmaf(lz, lz, fmaf(ly, ly, lx * lx))) * 1.00001f + 2.0f * r.E;
   }
-  if (P.n_sph > 0x10000 || P.n_pl > 0xFFFF) return lit_area_call<BOX>(P, target, L, ctx);
+  if (P.n_sph > 0x10000 || P.n_pl > 0xFFFF) return lit_area_call<Pol, BOX>(P, target, L, ctx);
   Pack8 S, Q;
   S.clear();
   Q.clear();
@@ -405,14 +375,14 @@ __device__ __forceinline__ double lit_area_bvh(const FrameParams& P, d3 target, 
       const int kind = classify_sphere<BOX>(s, r, lo, hi);
       if (kind != 0 && !(lo > far)) S.push(k);
     });
-    if (!ok) return lit_area_call<BOX>(P, target, L, ctx);
+    if (!ok) return lit_area_call<Pol, BOX>(P, target, L, ctx);
   }
   for (int k = 0; k < P.n_pl; ++k) {
     float lo, hi;
     const int kind = classify_plane(__ldg(&P.cull_pl[2 * k]), __ldg(&P.cull_pl[2 * k + 1]), r, lo, hi);
     if (kind != 0 && !(lo > far)) Q.push((uint32_t)k);
   }
-  if (S.overflow() || Q.overflow()) return lit_area_call<BOX>(P, target, L, ctx);
+  if (S.overflow() || Q.overflow()) return lit_area_call<Pol, BOX>(P, target, L, ctx);
   double total = 1;
   bool have_n = false;
   // visit the survivors in ascending world_objects index (selection over <= 16 entries)
@@ -440,8 +410,8 @@ __device__ __forceinline__ double lit_area_bvh(const FrameParams& P, d3 target, 
       }
     }
     RTRB_COUNT(ctx, RTRB_CNT_EXACT);
-    if (best_k >= 0) total -= cover_object_exact<BOX, 1>(P, P.geom[best_idx], c, L.radius, ctx);
-    else total -= cover_object_exact<BOX, 2>(P, P.geom[best_idx], c, L.radius, ctx);
+    if (best_k >= 0) total -= cover_object_exact<Pol, BOX, 1>(P, P.geom[best_idx], c, L.radius, ctx);
+    else total -= cover_object_exact<Pol, BOX, 2>(P, P.geom[best_idx], c, L.radius, ctx);
   }
   return fmax(total, 0.0);
 }
@@ -509,10 +479,10 @@ __device__ __forceinline__ uint32_t line_survivors_light(const FrameParams& P, c
 }
 
 // World#intersect (world.rb:37-59) = FP32 filter over every object + exact test of the survivors.
-template <bool BOX, bool KT>
+template <class Pol, bool BOX, bool KT>
 __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3 d, const CullRay& r, HitRec& bh,
                                                 ThreadCtx& ctx, const bool through_lens) {
-  if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return closest_hit_scan_call<BOX>(P, o, d, bh, ctx);
+  if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return closest_hit_scan_call<Pol, BOX>(P, o, d, bh, ctx);
   const uint32_t mask = (through_lens && P.cam_tab_valid) ? line_survivors_camera(P, r) : line_survivors_generic<KT>(P, r);
   // pass 1 (only when something can be pruned): the smallest certain upper bound; nothing at or beyond
   // max_distance can win (world.rb:39)
@@ -552,7 +522,7 @@ __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3
     const DevGeom g = P.geom[i];
     HitRec h;
     RTRB_COUNT(ctx, RTRB_CNT_EXACT);
-    if ((BOX && g.type == RTRB_OBJ_BOX) ? box_intersect(P.boxes[g.aux], o, d, h) : sphere_intersect(g, o, d, d_r, dn, h)) {
+    if ((BOX && g.type == RTRB_OBJ_BOX) ? box_intersect(P.boxes[g.aux], o, d, h) : sphere_intersect<Pol>(g, o, d, d_r, dn, h)) {
       const double new_dis = norm(o - h.p);
       if (new_dis < best || (new_dis == best && best_i >= 0 && i < best_i)) { best = new_dis; best_i = i; keep_hit<BOX>(bh, h); }
     }
@@ -581,7 +551,7 @@ __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3
 // An object the probe ray certainly misses (or certainly meets beyond the light) has factor 0, hence
 // cover exactly 0 (sphere.rb:29,45-53 multiply everything by factor; world_object.rb:43-47), and
 // total - 0 == total, so skipping it leaves the running difference bit-identical.
-template <bool BOX, bool KT>
+template <class Pol, bool BOX, bool KT>
 __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 target, const DevLight& L, const int light_index,
                                                   ThreadCtx& ctx) {
   CoverRay c;
@@ -596,7 +566,7 @@ __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 targe
     const float lx = (float)c.lt.x, ly = (float)c.lt.y, lz = (float)c.lt.z;
     far = sqrt_approx(fmaf(lz, lz, fmaf(ly, ly, lx * lx))) * 1.00001f + 2.0f * r.E;
   }
-  if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return lit_area_call<BOX>(P, target, L, ctx);
+  if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return lit_area_call<Pol, BOX>(P, target, L, ctx);
   // the probe ray's line passes through the light: apex table of this light when there is one
   uint32_t sm = (P.k_has_light_tab != 0) ? line_survivors_light<KT>(P, light_index, r) : line_survivors_generic<KT>(P, r);
   uint32_t qm = 0u;
@@ -623,11 +593,11 @@ __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 targe
         have_n = true;
       }
       RTRB_COUNT(ctx, RTRB_CNT_EXACT);
-      total -= cover_object_exact<BOX, 1>(P, P.geom[is], c, L.radius, ctx);
+      total -= cover_object_exact<Pol, BOX, 1>(P, P.geom[is], c, L.radius, ctx);
     } else {
       qm &= qm - 1u;
       RTRB_COUNT(ctx, RTRB_CNT_EXACT);
-      total -= cover_object_exact<BOX, 2>(P, P.geom[iq], c, L.radius, ctx);
+      total -= cover_object_exact<Pol, BOX, 2>(P, P.geom[iq], c, L.radius, ctx);
     }
   }
   return fmax(total, 0.0);
@@ -648,33 +618,35 @@ __device__ __forceinline__ const DevLightF& light_f_at(const FrameParams& P, int
 
 // Compile-time choice: kernels are instantiated once per filter so each stays compact (the linear
 // scan wins below ~32 spheres: measured 5.56 vs 6.05 ms on config 3; the BVH wins 5x on config 5).
-template <bool BVH, bool BOX, bool KT>
+template <class Pol, bool BVH, bool BOX, bool KT>
 __device__ __forceinline__ int closest_hit_fast(const FrameParams& P, d3 o, d3 d, const CullRay& r, HitRec& bh,
                                                 ThreadCtx& ctx, const bool through_lens) {
-  if constexpr (BVH) return closest_hit_bvh<BOX>(P, o, d, r, bh, ctx);
-  else return closest_hit_linear<BOX, KT>(P, o, d, r, bh, ctx, through_lens);
+  if constexpr (BVH) return closest_hit_bvh<Pol, BOX>(P, o, d, r, bh, ctx);
+  else return closest_hit_linear<Pol, BOX, KT>(P, o, d, r, bh, ctx, through_lens);
 }
-template <bool BVH, bool BOX, bool KT>
+template <class Pol, bool BVH, bool BOX, bool KT>
 __device__ __forceinline__ double lit_area_fast(const FrameParams& P, d3 target, const DevLight& L, const int light_index,
                                                 ThreadCtx& ctx) {
-  if constexpr (BVH) return lit_area_bvh<BOX>(P, target, L, ctx);
-  else return lit_area_linear<BOX, KT>(P, target, L, light_index, ctx);
+  if constexpr (BVH) return lit_area_bvh<Pol, BOX>(P, target, L, ctx);
+  else return lit_area_linear<Pol, BOX, KT>(P, target, L, light_index, ctx);
 }
 
-// The reference's own expression of the highlight match (world.rb:86-93), register-only interface.
+// The reference's own expression of the highlight match (world.rb:86-93), register-only interface.  Only the depth-1
+// builds call it (Policy::outline_libm), so its acos is their out-of-line copy.
 static __device__ __noinline__ bool highlight_match_exact(double lx, double ly, double lz, double threshold, double ox, double oy,
                                                          double oz, double dx, double dy, double dz, uint32_t* status) {
   ThreadCtx t;
   t.status = 0; t.detail = false;
   const d3 a = mk(lx, ly, lz) - mk(ox, oy, oz);
   const double ct = vcos(mk(dx, dy, dz), a, t);
-  const double ang = rb_acos(ct, t);
+  const double ang = rb_acos<Generic::at<1>>(ct, t);
   *status = t.status;
   return ang < threshold;
 }
 
 // World#high_lights match for one light (world.rb:86-93): acos(|cos|) < threshold, filtered in FP32 on
 // cos^2 against cos^2(threshold); the exact FP64 expression decides only inside the error band.
+template <class Pol>
 __device__ __forceinline__ bool highlight_match_fast(const DevLight& L, const DevLightF& F, d3 o, d3 d,
                                                      const CullRay& r, ThreadCtx& ctx) {
   const float eps = 5.9604645e-8f;
@@ -690,19 +662,19 @@ __device__ __forceinline__ bool highlight_match_fast(const DevLight& L, const De
     if (c2 + tol < F.cos2_thr) return false;
   }
   // exact (also reached for thresholds outside (0, 90 degrees), NaNs, and rays starting at the light)
-#ifdef RTRB_OUTLINE_LIBM
-  // depth-1 translation unit: rare there, and out of line so that its two divisions, square root and acos do not sit
-  // between the hot blocks (config 2: -1 %; the ray-tree kernels lose 1 % with it and keep the inline form)
-  uint32_t st = 0u;
-  const bool hit = highlight_match_exact(L.px, L.py, L.pz, L.hl_threshold, o.x, o.y, o.z, d.x, d.y, d.z, &st);
-  ctx.status |= st;
-  return hit;
-#else
-  d3 a = mk(L.px, L.py, L.pz) - o;
-  double ct = vcos(d, a, ctx);
-  double ang = rb_acos(ct, ctx);
-  return ang < L.hl_threshold;
-#endif
+  if constexpr (Pol::outline_libm) {
+    // depth-1 builds: rare there, and out of line so that its two divisions, square root and acos do not sit between
+    // the hot blocks (config 2: -1 %; the ray-tree kernels lose 1 % with it and keep the inline form)
+    uint32_t st = 0u;
+    const bool hit = highlight_match_exact(L.px, L.py, L.pz, L.hl_threshold, o.x, o.y, o.z, d.x, d.y, d.z, &st);
+    ctx.status |= st;
+    return hit;
+  } else {
+    d3 a = mk(L.px, L.py, L.pz) - o;
+    double ct = vcos(d, a, ctx);
+    double ang = rb_acos<Pol>(ct, ctx);
+    return ang < L.hl_threshold;
+  }
 }
 
 // `attenuation.r < 0.0001` (ray_tracer.rb:52) without the square root outside a narrow band.
@@ -719,7 +691,7 @@ __device__ __forceinline__ bool attenuation_dead(d3 att) {
 //            here (dead, terminated by a highlight, or a miss);
 //   phase B  intersect_parameters, the children (pushed onto `stack`), World#local_lights and local_lighting.
 // Emitted colours are added to `sum` in emission order.
-template <int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackItem& it, d3& sum, ThreadCtx& ctx, bool is_first,
                                             int* primary_hit, HitRec& bh) {
   constexpr bool KT = !BVH && MAXS == 1;  // constant-bank tables: depth-1 linear-filter kernels only (see pl_rec)
@@ -733,10 +705,10 @@ __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackIte
   {
     unsigned long long hl_mask = 0ull;
     int hl_n = 0;
-    for (int l = 0; l < RTRB_NL(P); ++l)
-      if (highlight_match_fast(light_at<KT>(P, l), light_f_at<KT>(P, l), o, d, r, ctx)) { hl_mask |= 1ull << l; hl_n++; }
+    for (int l = 0; l < Pol::n_lights(P); ++l)
+      if (highlight_match_fast<Pol>(light_at<KT>(P, l), light_f_at<KT>(P, l), o, d, r, ctx)) { hl_mask |= 1ull << l; hl_n++; }
     if (hl_n > 0) {
-      for (int l = 0; l < RTRB_NL(P); ++l) {
+      for (int l = 0; l < Pol::n_lights(P); ++l) {
         if (!((hl_mask >> l) & 1ull)) continue;
         d3 c = att * ld3(light_at<KT>(P, l).color_hl);
         if (hl_n != 1) c = c / (double)hl_n;  // x / 1.0 == x
@@ -752,7 +724,7 @@ __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackIte
   // ---- World#intersect ----
   bh.p = mk(0, 0, 0); bh.dir_in = false;
   if constexpr (BOX) bh.face = 0;
-  const int best_i = closest_hit_fast<BVH, BOX, KT>(P, o, d, r, bh, ctx, is_first);
+  const int best_i = closest_hit_fast<Pol, BVH, BOX, KT>(P, o, d, r, bh, ctx, is_first);
   if (best_i < 0) return -1;
   if (is_first) *primary_hit = best_i;
   RTRB_COUNT(ctx, RTRB_CNT_HITS);
@@ -780,11 +752,11 @@ static __device__ __noinline__ uint32_t born_dead_children_status(double dx, dou
   return t.status;
 }
 
-template <int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackItem& it, const int best_i, const HitRec& bh,
                                              StackItem* stack, int& sp, d3& sum, ThreadCtx& ctx, uint32_t pixel,
                                              uint32_t sample) {
-  const uint32_t K = (uint32_t)(RTRB_MC(P) + 2);
+  const uint32_t K = (uint32_t)(Pol::mc(P) + 2);
   constexpr bool KT = !BVH && MAXS == 1;
   {
     const d3 o = mk(it.ox, it.oy, it.oz), d = mk(it.dx, it.dy, it.dz), att = mk(it.ax, it.ay, it.az);
@@ -856,8 +828,8 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
         const double sin_r = sin_i / rate;
         if (!(sin_r >= 1)) {
           if (sin_r < -1 || sin_r > 1) ctx.status |= RTRB_ST_MATH_DOMAIN;
-          const double rr = m_asin(sin_r);
-          const d3 refr_dir = nn * (-m_cos(rr)) + normalize(refl_dir + d, ctx) * sin_r;
+          const double rr = m_asin<Pol>(sin_r);
+          const d3 refr_dir = nn * (-m_cos<Pol>(rr)) + normalize(refl_dir + d, ctx) * sin_r;
           const d3 refr_org = bh.p - nn * RTRB_EPSILON;
           RTRB_COUNT(ctx, RTRB_CNT_REFR);
           StackItem& s = stack[sp++];
@@ -873,13 +845,13 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
     const d3 shade_from = bh.p + delta;
     d3 contrib = mk(0.0, 0.0, 0.0);
     int n_lit = 0;
-    for (int l = 0; l < RTRB_NL(P); ++l) {
+    for (int l = 0; l < Pol::n_lights(P); ++l) {
       const DevLight& L = light_at<KT>(P, l);
       ctx.shadow++;
-      const double area = lit_area_fast<BVH, BOX, KT>(P, shade_from, L, l, ctx);
+      const double area = lit_area_fast<Pol, BVH, BOX, KT>(P, shade_from, L, l, ctx);
       if (area > 0) {
-        double w = rb_pow(area, RTRB_EXP(P));
-        if (RTRB_NL(P) != 1) w = w / (double)RTRB_NL(P);  // x / 1.0 == x
+        double w = rb_pow<Pol>(area, Pol::shadow_exponent(P));
+        if (Pol::n_lights(P) != 1) w = w / (double)Pol::n_lights(P);  // x / 1.0 == x
         d3 lc = ld3(L.color) * w;
         d3 lv = normalize(mk(L.px, L.py, L.pz) - bh.p, ctx);
         double ldn = dot(lv, nn);
@@ -889,22 +861,22 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
       }
     }
     if (n_lit == 0) {
-      if (MAXS == 1 && RTRB_MC(P) > 0 && ctx.detail) ctx.c[RTRB_CNT_MC] += RTRB_MC(P);  // spawned, born dead
-      if (MAXS > 1 && RTRB_MC(P) > 0) {
-        if (sp + RTRB_MC(P) > MAXS) { ctx.status |= RTRB_ST_STACK_OVERFLOW; return; }
-        const d3 att_pt = ld3(M.diffuse) / (double)RTRB_MC(P);
+      if (MAXS == 1 && Pol::mc(P) > 0 && ctx.detail) ctx.c[RTRB_CNT_MC] += Pol::mc(P);  // spawned, born dead
+      if (MAXS > 1 && Pol::mc(P) > 0) {
+        if (sp + Pol::mc(P) > MAXS) { ctx.status |= RTRB_ST_STACK_OVERFLOW; return; }
+        const d3 att_pt = ld3(M.diffuse) / (double)Pol::mc(P);
         const d3 a2 = att * att_pt;
         const bool mc_alive = depth_ok && !(sumsq(a2) < 0.99e-8);
         const d3 vv = a_vertical_vector(n, ctx);
         if (mc_alive || sumsq(vv) == 0) {
           const d3 leftv = normalize(vv, ctx);
           const d3 upv = cross(nn, leftv);
-          for (int m = 0; m < RTRB_MC(P); ++m) {
+          for (int m = 0; m < Pol::mc(P); ++m) {
             uint32_t child = it.path * K + (uint32_t)(2 + m);
             uint32_t c0 = pixel, c1 = sample, c2 = child, c3 = 1u;
             philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
             double theta = res53(c0, c1) * RTRB_PI / 2, phi = res53(c2, c3) * RTRB_PI * 2;
-            d3 dir = nn * m_sin(theta) + (leftv * m_cos(phi) + upv * m_sin(phi)) * m_cos(theta);
+            d3 dir = nn * m_sin<Pol>(theta) + (leftv * m_cos<Pol>(phi) + upv * m_sin<Pol>(phi)) * m_cos<Pol>(theta);
             StackItem& s = stack[sp++];
             s.ox = shade_from.x; s.oy = shade_from.y; s.oz = shade_from.z;
             s.dx = dir.x; s.dy = dir.y; s.dz = dir.z;
@@ -912,14 +884,14 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
             s.depth = it.depth - 1; s.path = child;
           }
         }
-        if (ctx.detail) ctx.c[RTRB_CNT_MC] += RTRB_MC(P);
+        if (ctx.detail) ctx.c[RTRB_CNT_MC] += Pol::mc(P);
       }
     } else {
       RTRB_COUNT(ctx, RTRB_CNT_LOCAL);
       if (ctx.detail) ctx.c[RTRB_CNT_LIT] += n_lit;
       if (n_lit != 1) contrib = contrib / (double)n_lit;  // x / 1.0 == x
       d3 filter = mk(1.0, 1.0, 1.0);
-      if (RTRB_TEX(M)) {
+      if (Pol::textured(M)) {
         double u, v;
         if (g.type == RTRB_OBJ_SPHERE) {
           d3 vec = bh.p - mk(g.px, g.py, g.pz);
@@ -935,7 +907,7 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
           v = dot(rel, ld3(M.e1)) / M.v_unit;
         }
         RTRB_COUNT(ctx, RTRB_CNT_TEXEL);
-        filter = texture_color(M, u, v, ctx) * filter;
+        filter = texture_color<Pol>(M, u, v, ctx) * filter;
       }
       d3 local = ((contrib * ld3(M.diffuse)) * filter) + ld3(M.ambient);
       d3 c = att * local;
@@ -945,17 +917,17 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
   }
 }
 
-template <int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ void process_item_fast(const FrameParams& P, const StackItem& it, StackItem* stack, int& sp,
                                                   d3& sum, ThreadCtx& ctx, uint32_t pixel, uint32_t sample,
                                                   bool is_first, int* primary_hit) {
   HitRec bh;
-  const int best_i = item_phase_a<MAXS, BVH, BOX>(P, it, sum, ctx, is_first, primary_hit, bh);
-  if (best_i >= 0) item_phase_b<MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
+  const int best_i = item_phase_a<Pol, MAXS, BVH, BOX>(P, it, sum, ctx, is_first, primary_hit, bh);
+  if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
 }
 
 // RayTracer#trace_sync for one sample (non-persistent form; used by tools and kept for reference).
-template <int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                                 ThreadCtx& ctx, int* primary_hit) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
@@ -971,7 +943,7 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
   *primary_hit = -1;
   ctx.max_stack = max(ctx.max_stack, 1u);
   while (true) {
-    process_item_fast<MAXS, BVH, BOX>(P, it, stack, sp, sum, ctx, pixel, sample, first, primary_hit);
+    process_item_fast<Pol, MAXS, BVH, BOX>(P, it, stack, sp, sum, ctx, pixel, sample, first, primary_hit);
     first = false;
     if (MAXS == 1 || sp == 0) break;
     if ((uint32_t)sp > ctx.max_stack) ctx.max_stack = (uint32_t)sp;
@@ -994,7 +966,7 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
 // mean, variance of the signed maximum, adaptive decision, quantisation.  No per-sample FP64 buffer crosses HBM
 // (24 B per sample: 12.7 GB for one 4K / 64 spp frame) and no resolve kernel runs.  FrameParams::fuse_resolve == 2
 // selects it; other sample counts (3, 10, ...) write the sample buffer for resolve_kernel as before.
-template <int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                                          ThreadCtx& ctx, int* primary_hit, bool active) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
@@ -1012,14 +984,14 @@ __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d
   while (__syncthreads_or(have ? 1 : 0)) {
     HitRec bh;
     int best_i = -1;
-    if (have) best_i = item_phase_a<MAXS, BVH, BOX>(P, it, sum, ctx, first, primary_hit, bh);
+    if (have) best_i = item_phase_a<Pol, MAXS, BVH, BOX>(P, it, sum, ctx, first, primary_hit, bh);
     // phase boundary: with the BVH filter the whole CTA also moves from intersection to shading together when a warp
     // holds several pixels (config 5 at 4 spp: 3.90 -> 3.53 ms); with a whole warp on one pixel (>= 32 spp) the warps are
     // even enough without it (config 5 at 64 spp: 956 -> 944 ms without), and with the linear filter the second
     // barrier costs more than it saves (config 3: +3 %)
     if constexpr (BVH) { if (mid_barrier) __syncthreads(); }
     if (have) {
-      if (best_i >= 0) item_phase_b<MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
+      if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
       first = false;
       if (sp == 0) have = false;
       else {
@@ -1032,7 +1004,7 @@ __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d
 }
 
 // Kernel body: the first loop of render_at (camera.rb:73-78) for the CTA's samples, then (fuse_resolve == 2) its tail.
-template <int MAXS, bool BVH, bool DETAIL>
+template <class Pol, int MAXS, bool BVH, bool DETAIL>
 __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
   extern __shared__ double rtrb_cta_samples[];  // [blockDim.x][3] when fuse_resolve == 2
   const uint32_t S = (uint32_t)P.pre;
@@ -1057,11 +1029,11 @@ __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
         philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
         theta = res53(c0, c1);  // Random.rand, camera.rb:135
       }
-      lens_ray(P, x, y, theta, ro, rd);
+      lens_ray<Pol>(P, x, y, theta, ro, rd);
     }
   }
   int ph = -1;
-  const d3 col = trace_sample_fast_lockstep<MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph, active);
+  const d3 col = trace_sample_fast_lockstep<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph, active);
   if (active) {
     RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
     if (j == 0 && P.hit) P.hit[(size_t)y * P.width + x] = ph;

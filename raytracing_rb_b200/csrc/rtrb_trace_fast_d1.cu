@@ -1,17 +1,3 @@
-// FAST64, trace_depth <= 1: the stackless depth-1 kernels (config 2's kernel lives here).  -fmad=false.
-// In a depth-1 frame the FP64 transcendentals (acos / sin of the penumbra and highlight fallbacks, pow, fmod) are cold, yet
-// inlined they put ~1 700 instructions between the hot blocks of a kernel whose top stall after `wait` is
-// `no_instruction`; as real functions they sit behind the kernel (config 2: -2 %).  The ray-tree kernels, where these
-// calls are warm, keep them inline (measured +2 % .. +5 % out of line).
-#ifndef RTRB_D1_INLINE_LIBM
-#define RTRB_OUTLINE_LIBM 1
-#endif
+// FAST64 depth-1 kernels (trace_depth <= 1, stackless; config 2's kernel lives here), generic scenes.  -fmad=false.
 #include "rtrb_trace_fast_launch.cuh"
-namespace RTRB_FAST_NS {
-cudaError_t pre_d1(const FrameParams& P, cudaStream_t s) {
-  return P.count_detail ? launch_pre_d1<true>(P, s) : launch_pre_d1<false>(P, s);
-}
-cudaError_t extra_d1(const FrameParams& P, cudaStream_t s) {
-  return P.count_detail ? launch_extra<1, true>(P, s) : launch_extra<1, false>(P, s);
-}
-}  // namespace RTRB_FAST_NS
+namespace rtrb_fast { const FastKernels d1 = kernels<1>(); }

@@ -1,5 +1,3 @@
-// FAST64, trace_depth <= 1, LEAN scenes (RTRB_SCENE_CLASS_LEAN: one light of radius 0, no textures, exponent 2): the same
-// source as rtrb_trace_fast_d1.cu compiled with RTRB_SCENE_LEAN, in namespace rtrb_fast_lean.  -fmad=false.
-#define RTRB_SCENE_LEAN 1
-#define RTRB_FAST_NS rtrb_fast_lean
-#include "rtrb_trace_fast_d1.cu"
+// FAST64 depth-1 kernels, lean scenes (rtrb::Lean: one light of radius 0, no textures, exponent 2).  -fmad=false.
+#include "rtrb_trace_fast_launch.cuh"
+namespace rtrb_fast_lean { const FastKernels d1 = kernels<1>(); }

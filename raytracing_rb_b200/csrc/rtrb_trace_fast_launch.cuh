@@ -1,109 +1,121 @@
-// rtrb_trace_fast_launch.cuh — kernels and launchers of the FAST64 trace path, instantiated per stack capacity
-// in separate translation units (rtrb_trace_fast_d1.cu, _t10.cu, _t32.cu, _t128.cu) so they compile in parallel.
+// rtrb_trace_fast_launch.cuh — the FAST64 kernels of every class build (rtrb_trace.cuh, "build policies").  The
+// kernels carry their class as a namespace: rtrb_fast (generic), rtrb_fast_lean, rtrb_fast_l1 (one light) and
+// rtrb_fast_l1n (one light, no Monte-Carlo rays).  Each rtrb_trace_fast_*.cu translation unit instantiates one
+// (class, work-stack capacity) pair, so `make -j` compiles them in parallel; rtrb_trace_fast.cu launches them.
 #pragma once
 #include "rtrb_launch.h"
 #include "rtrb_trace_fast.cuh"
 
-#ifndef RTRB_FAST_NS
-#define RTRB_FAST_NS rtrb_fast  // the lean-scene build of the depth-1 kernels lives in rtrb_fast_lean
-#endif
-namespace RTRB_FAST_NS {
-
 // Launch shape per kernel family (16 warps per SM at 128 registers either way; measured on B200, profiles/README.md):
-//   depth-1 kernels (MAXS == 1): 128 threads x 5 CTAs per SM = 96 registers (round 2, config 2: 0.101 ms at 4 CTAs /
-//                                128 registers, 0.095 - 0.098 at 5 .. 8 CTAs / 96 .. 64 registers; 256 x 2: 0.103).
-//                                The extra-sample kernels keep 4 CTAs (config 1: 0.707 vs 0.735 ms)
+//   depth-1 kernels (MAXS == 1): 128 threads x Policy::d1_min_blocks CTAs per SM.  The extra-sample kernels keep 4
+//                                CTAs (config 1: 0.707 vs 0.735 ms)
 //   ray-tree kernels (MAXS > 1): lockstep item loop, so the CTA is the unit that shares the instruction caches:
 //                                512 threads x 1 CTA per SM on frames of more than a few waves (config 4: 4.44 / 3.78 /
 //                                3.57 ms and config 5: 5.13 / 4.61 / 4.24 ms with 128 / 256 / 512 threads; config 3:
-//                                3.87 / 3.44 / 3.52), 128 threads on small frames
-#ifndef RTRB_TREE_BLOCK
-#define RTRB_TREE_BLOCK 512
-#endif
-#ifndef RTRB_FAST_MIN_BLOCKS
-#ifdef RTRB_SCENE_LEAN
-#define RTRB_FAST_MIN_BLOCKS 8  // lean depth-1 kernel (124 registers unconstrained): 0.086 / 0.080 / 0.078 / 0.076 / 0.078 / 0.088 ms
-#else                           // on config 2 at 4 / 5 / 7 / 8 / 10 / 12 CTAs per SM (124 / 96 / 72 / 64 / 48 / 40 registers)
-#define RTRB_FAST_MIN_BLOCKS 5
-#endif
-#endif
-constexpr int kFastBlock = 128, kFastMinBlocks = RTRB_FAST_MIN_BLOCKS, kExtraMinBlocks = 4, kTreeBlock = RTRB_TREE_BLOCK, kTreeMinBlocks = 512 / RTRB_TREE_BLOCK > 0 ? 512 / RTRB_TREE_BLOCK : 1;
+//                                3.87 / 3.44 / 3.52), RTRB_TREE_MIN_BLOCK threads on small frames
+constexpr int kFastBlock = 128, kExtraMinBlocks = 4, kTreeBlock = 512;
 
+// One class build's kernels for one work-stack capacity (1: the stackless depth-1 kernels), indexed
+// [count_detail][use_bvh], and the class they were compiled for.
+struct FastKernels {
+  bool one_light, lean, no_mc;
+  int capacity;
+  TraceKernel pre[2][2], extra[2][2];
+};
+
+namespace rtrb_fast {
+using Pol = rtrb::Generic;
 template <int MAXS, bool DETAIL, bool BVH>
-__global__ void __launch_bounds__(kFastBlock, kFastMinBlocks) trace_pre_fast_kernel(const __grid_constant__ FrameParams P) {
-  rtrb::trace_pre_body<MAXS, DETAIL, BVH ? 2 : 1>(P);
+__global__ void __launch_bounds__(kFastBlock, Pol::d1_min_blocks) trace_pre_fast_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_pre_body<Pol::at<MAXS>, MAXS, DETAIL, BVH>(P);
 }
 template <int MAXS, bool DETAIL, bool BVH>
-__global__ void __launch_bounds__(kTreeBlock, kTreeMinBlocks) trace_pre_tree_kernel(const __grid_constant__ FrameParams P) {
-  rtrb::trace_pre_tree_body<MAXS, BVH, DETAIL>(P);
+__global__ void __launch_bounds__(kTreeBlock, 1) trace_pre_tree_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_pre_tree_body<Pol::at<MAXS>, MAXS, BVH, DETAIL>(P);
 }
 template <int MAXS, bool DETAIL, bool BVH>
 __global__ void __launch_bounds__(kFastBlock, kExtraMinBlocks) trace_extra_fast_kernel(const __grid_constant__ FrameParams P) {
-  rtrb::trace_extra_body<MAXS, DETAIL, BVH ? 2 : 1>(P);
+  rtrb::trace_extra_body<Pol::at<MAXS>, MAXS, DETAIL, BVH>(P);
 }
-
-inline int sm_count() {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return sms;
+template <int MAXS, bool DETAIL, bool BVH>
+TraceKernel pre_kernel() {
+  if constexpr (MAXS == 1) return trace_pre_fast_kernel<1, DETAIL, BVH>;
+  else return trace_pre_tree_kernel<MAXS, DETAIL, BVH>;
 }
-
-// depth-1 frames: one thread per (pixel, sample)
-template <bool DETAIL>
-cudaError_t launch_pre_d1(const FrameParams& P, cudaStream_t s) {
-  const unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * (unsigned long long)P.pre;
-  if (total == 0) return cudaSuccess;
-  const unsigned long long blocks = (total + kFastBlock - 1) / kFastBlock;
-  if (blocks > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  if (P.use_bvh) trace_pre_fast_kernel<1, DETAIL, true><<<(unsigned)blocks, kFastBlock, 0, s>>>(P);
-  else trace_pre_fast_kernel<1, DETAIL, false><<<(unsigned)blocks, kFastBlock, 0, s>>>(P);
-  return cudaGetLastError();
+template <int MAXS>
+FastKernels kernels() {
+  return {Pol::one_light, Pol::lean, Pol::no_mc, MAXS,
+          {{pre_kernel<MAXS, false, false>(), pre_kernel<MAXS, false, true>()},
+           {pre_kernel<MAXS, true, false>(), pre_kernel<MAXS, true, true>()}},
+          {{trace_extra_fast_kernel<MAXS, false, false>, trace_extra_fast_kernel<MAXS, false, true>},
+           {trace_extra_fast_kernel<MAXS, true, false>, trace_extra_fast_kernel<MAXS, true, true>}}};
 }
+}  // namespace rtrb_fast
 
-// ray-tree frames: one thread per (pixel, sample), lockstep CTAs (rtrb_trace_fast.cuh, trace_pre_tree_body)
-template <int MAXS, bool DETAIL>
-cudaError_t launch_pre_tree(const FrameParams& P, cudaStream_t s) {
-  const unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * (unsigned long long)P.pre;
-  if (total == 0) return cudaSuccess;
-  int block = kTreeBlock;
-  if (total < 4ull * (unsigned long long)sm_count() * kTreeBlock) block = 128;  // small frames: more, smaller CTAs
-  const unsigned long long blocks = (total + block - 1) / block;
-  if (blocks > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  // in-CTA resolve (fuse_resolve == 2): the host only selects it for sample counts that divide both CTA sizes
-  if (P.fuse_resolve == 2 && (block % P.pre) != 0) return cudaErrorInvalidConfiguration;
-  const size_t smem = P.fuse_resolve == 2 ? (size_t)block * 3u * sizeof(double) : 0u;
-  if (P.use_bvh) trace_pre_tree_kernel<MAXS, DETAIL, true><<<(unsigned)blocks, block, smem, s>>>(P);
-  else trace_pre_tree_kernel<MAXS, DETAIL, false><<<(unsigned)blocks, block, smem, s>>>(P);
-  return cudaGetLastError();
+// depth-1 kernels only
+namespace rtrb_fast_lean {
+using Pol = rtrb::Lean;
+template <int MAXS, bool DETAIL, bool BVH>
+__global__ void __launch_bounds__(kFastBlock, Pol::d1_min_blocks) trace_pre_fast_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_pre_body<Pol::at<MAXS>, MAXS, DETAIL, BVH>(P);
 }
-
-template <int MAXS, bool DETAIL>
-cudaError_t launch_extra(const FrameParams& P, cudaStream_t s) {
-  const int sms = sm_count();
-  if (P.use_bvh) trace_extra_fast_kernel<MAXS, DETAIL, true><<<sms * 8, kFastBlock, 0, s>>>(P);
-  else trace_extra_fast_kernel<MAXS, DETAIL, false><<<sms * 8, kFastBlock, 0, s>>>(P);
-  return cudaGetLastError();
+template <int MAXS, bool DETAIL, bool BVH>
+__global__ void __launch_bounds__(kFastBlock, kExtraMinBlocks) trace_extra_fast_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_extra_body<Pol::at<MAXS>, MAXS, DETAIL, BVH>(P);
 }
+template <int MAXS>
+FastKernels kernels() {
+  return {Pol::one_light, Pol::lean, Pol::no_mc, MAXS,
+          {{trace_pre_fast_kernel<MAXS, false, false>, trace_pre_fast_kernel<MAXS, false, true>},
+           {trace_pre_fast_kernel<MAXS, true, false>, trace_pre_fast_kernel<MAXS, true, true>}},
+          {{trace_extra_fast_kernel<MAXS, false, false>, trace_extra_fast_kernel<MAXS, false, true>},
+           {trace_extra_fast_kernel<MAXS, true, false>, trace_extra_fast_kernel<MAXS, true, true>}}};
+}
+}  // namespace rtrb_fast_lean
 
-// per-capacity entry points, one translation unit each
-cudaError_t pre_d1(const FrameParams& P, cudaStream_t s);
-cudaError_t extra_d1(const FrameParams& P, cudaStream_t s);
-cudaError_t pre_t10(const FrameParams& P, cudaStream_t s);
-cudaError_t extra_t10(const FrameParams& P, cudaStream_t s);
-cudaError_t pre_t32(const FrameParams& P, cudaStream_t s);
-cudaError_t extra_t32(const FrameParams& P, cudaStream_t s);
-cudaError_t pre_t128(const FrameParams& P, cudaStream_t s);
-cudaError_t extra_t128(const FrameParams& P, cudaStream_t s);
+// ray-tree kernels only (the depth-1 frames of these classes run the generic build)
+namespace rtrb_fast_l1 {
+using Pol = rtrb::OneLight;
+template <int MAXS, bool DETAIL, bool BVH>
+__global__ void __launch_bounds__(kTreeBlock, 1) trace_pre_tree_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_pre_tree_body<Pol, MAXS, BVH, DETAIL>(P);
+}
+template <int MAXS, bool DETAIL, bool BVH>
+__global__ void __launch_bounds__(kFastBlock, kExtraMinBlocks) trace_extra_fast_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_extra_body<Pol, MAXS, DETAIL, BVH>(P);
+}
+template <int MAXS>
+FastKernels kernels() {
+  return {Pol::one_light, Pol::lean, Pol::no_mc, MAXS,
+          {{trace_pre_tree_kernel<MAXS, false, false>, trace_pre_tree_kernel<MAXS, false, true>},
+           {trace_pre_tree_kernel<MAXS, true, false>, trace_pre_tree_kernel<MAXS, true, true>}},
+          {{trace_extra_fast_kernel<MAXS, false, false>, trace_extra_fast_kernel<MAXS, false, true>},
+           {trace_extra_fast_kernel<MAXS, true, false>, trace_extra_fast_kernel<MAXS, true, true>}}};
+}
+}  // namespace rtrb_fast_l1
 
-}  // namespace RTRB_FAST_NS
+namespace rtrb_fast_l1n {
+using Pol = rtrb::OneLightNoMc;
+template <int MAXS, bool DETAIL, bool BVH>
+__global__ void __launch_bounds__(kTreeBlock, 1) trace_pre_tree_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_pre_tree_body<Pol, MAXS, BVH, DETAIL>(P);
+}
+template <int MAXS, bool DETAIL, bool BVH>
+__global__ void __launch_bounds__(kFastBlock, kExtraMinBlocks) trace_extra_fast_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_extra_body<Pol, MAXS, DETAIL, BVH>(P);
+}
+template <int MAXS>
+FastKernels kernels() {
+  return {Pol::one_light, Pol::lean, Pol::no_mc, MAXS,
+          {{trace_pre_tree_kernel<MAXS, false, false>, trace_pre_tree_kernel<MAXS, false, true>},
+           {trace_pre_tree_kernel<MAXS, true, false>, trace_pre_tree_kernel<MAXS, true, true>}},
+          {{trace_extra_fast_kernel<MAXS, false, false>, trace_extra_fast_kernel<MAXS, false, true>},
+           {trace_extra_fast_kernel<MAXS, true, false>, trace_extra_fast_kernel<MAXS, true, true>}}};
+}
+}  // namespace rtrb_fast_l1n
 
-#define RTRB_FAST_TREE_TU(N)                                                                         \
-  namespace RTRB_FAST_NS {                                                                              \
-  cudaError_t pre_t##N(const FrameParams& P, cudaStream_t s) {                                       \
-    return P.count_detail ? launch_pre_tree<N, true>(P, s) : launch_pre_tree<N, false>(P, s);        \
-  }                                                                                                  \
-  cudaError_t extra_t##N(const FrameParams& P, cudaStream_t s) {                                     \
-    return P.count_detail ? launch_extra<N, true>(P, s) : launch_extra<N, false>(P, s);              \
-  }                                                                                                  \
-  }
+// The builds, one object each (rtrb_trace_fast_{d1,d1lean,t10,t10_l1,t10_l1n,t32,t32_l1,t32_l1n,t128}.cu).
+namespace rtrb_fast { extern const FastKernels d1, t10, t32, t128; }
+namespace rtrb_fast_lean { extern const FastKernels d1; }
+namespace rtrb_fast_l1 { extern const FastKernels t10, t32; }
+namespace rtrb_fast_l1n { extern const FastKernels t10, t32; }

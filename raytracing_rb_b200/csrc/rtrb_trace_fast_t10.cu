@@ -1,3 +1,3 @@
-// FAST64 ray-tree kernels with a work stack of up to 10 items (trace_depth * (1 + mc) + 1 <= 10).  -fmad=false.
+// FAST64 ray-tree kernels with a work stack of up to 10 items, generic scenes.  -fmad=false.
 #include "rtrb_trace_fast_launch.cuh"
-RTRB_FAST_TREE_TU(10)
+namespace rtrb_fast { const FastKernels t10 = kernels<10>(); }

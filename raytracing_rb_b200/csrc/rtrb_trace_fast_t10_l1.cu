@@ -1,5 +1,3 @@
-// FAST64 ray-tree kernels (work stack <= 10 items) for scenes with ONE light and soft_shadow_exponent == 2
-// (RTRB_SCENE_CLASS_ONE_LIGHT), namespace rtrb_fast_l1.  Same source as rtrb_trace_fast_t10.cu.  -fmad=false.
-#define RTRB_SCENE_ONE_LIGHT 1
-#define RTRB_FAST_NS rtrb_fast_l1
-#include "rtrb_trace_fast_t10.cu"
+// FAST64 ray-tree kernels (work stack <= 10 items), one-light scenes (rtrb::OneLight).  -fmad=false.
+#include "rtrb_trace_fast_launch.cuh"
+namespace rtrb_fast_l1 { const FastKernels t10 = kernels<10>(); }

@@ -1,7 +1,4 @@
-// FAST64 ray-tree kernels (work stack <= 10 items) for scenes with ONE light and soft_shadow_exponent == 2, frames
-// without Monte-Carlo rays (monte_carlo_diffusion_times == 0), namespace rtrb_fast_l1n.  Same source as
-// rtrb_trace_fast_t10.cu.  -fmad=false.
-#define RTRB_SCENE_ONE_LIGHT 1
-#define RTRB_FRAME_NO_MC 1
-#define RTRB_FAST_NS rtrb_fast_l1n
-#include "rtrb_trace_fast_t10.cu"
+// FAST64 ray-tree kernels (work stack <= 10 items), one-light scenes in frames without Monte-Carlo rays
+// (rtrb::OneLightNoMc).  -fmad=false.
+#include "rtrb_trace_fast_launch.cuh"
+namespace rtrb_fast_l1n { const FastKernels t10 = kernels<10>(); }

@@ -1,3 +1,3 @@
-// FAST64 ray-tree kernels with a work stack of up to 128 items (trace_depth * (1 + mc) + 1 <= 128).  -fmad=false.
+// FAST64 ray-tree kernels with a work stack of up to 128 items, generic scenes.  -fmad=false.
 #include "rtrb_trace_fast_launch.cuh"
-RTRB_FAST_TREE_TU(128)
+namespace rtrb_fast { const FastKernels t128 = kernels<128>(); }

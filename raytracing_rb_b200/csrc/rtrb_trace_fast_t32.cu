@@ -1,3 +1,3 @@
-// FAST64 ray-tree kernels with a work stack of up to 32 items (trace_depth * (1 + mc) + 1 <= 32).  -fmad=false.
+// FAST64 ray-tree kernels with a work stack of up to 32 items, generic scenes.  -fmad=false.
 #include "rtrb_trace_fast_launch.cuh"
-RTRB_FAST_TREE_TU(32)
+namespace rtrb_fast { const FastKernels t32 = kernels<32>(); }

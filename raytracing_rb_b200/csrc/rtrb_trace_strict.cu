@@ -9,63 +9,53 @@ constexpr int kBlock = 128;
 
 template <int MAXS, bool DETAIL>
 __global__ void __launch_bounds__(kBlock) trace_pre_strict_kernel(const __grid_constant__ FrameParams P) {
-  rtrb::trace_pre_body<MAXS, DETAIL>(P);
+  rtrb::trace_pre_body<rtrb::Strict, MAXS, DETAIL>(P);
 }
 template <int MAXS, bool DETAIL>
 __global__ void __launch_bounds__(kBlock) trace_extra_strict_kernel(const __grid_constant__ FrameParams P) {
-  rtrb::trace_extra_body<MAXS, DETAIL>(P);
+  rtrb::trace_extra_body<rtrb::Strict, MAXS, DETAIL>(P);
 }
-
 template <int MAXS, bool DETAIL>
 __global__ void __launch_bounds__(kBlock) trace_mt_strict_kernel(const __grid_constant__ FrameParams P) {
-  rtrb::trace_mt_body<MAXS, DETAIL>(P);
-}
-template <int MAXS, bool DETAIL>
-cudaError_t launch_mt(const FrameParams& P, cudaStream_t s) {
-  unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS;  // one thread per PIXEL
-  if (total == 0) return cudaSuccess;
-  unsigned long long blocks = (total + kBlock - 1) / kBlock;
-  if (blocks > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  trace_mt_strict_kernel<MAXS, DETAIL><<<(unsigned)blocks, kBlock, 0, s>>>(P);
-  return cudaGetLastError();
+  rtrb::trace_mt_body<rtrb::Strict, MAXS, DETAIL>(P);
 }
 
+struct StrictKernels {
+  TraceKernel pre, extra, mt;
+};
 template <int MAXS, bool DETAIL>
-cudaError_t launch_pre(const FrameParams& P, cudaStream_t s) {
-  unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * (unsigned long long)P.pre;
-  if (total == 0) return cudaSuccess;
-  unsigned long long blocks = (total + kBlock - 1) / kBlock;
-  if (blocks > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  trace_pre_strict_kernel<MAXS, DETAIL><<<(unsigned)blocks, kBlock, 0, s>>>(P);
-  return cudaGetLastError();
+const StrictKernels kKernels = {trace_pre_strict_kernel<MAXS, DETAIL>, trace_extra_strict_kernel<MAXS, DETAIL>,
+                                trace_mt_strict_kernel<MAXS, DETAIL>};
+
+// the kernels of capacity stack_capacity(stack_need), with or without the detailed counters
+const StrictKernels& kernels(const FrameParams& P, int stack_need) {
+  const bool det = P.count_detail != 0;
+  switch (stack_capacity(stack_need)) {
+    case 10: return det ? kKernels<10, true> : kKernels<10, false>;
+    case 32: return det ? kKernels<32, true> : kKernels<32, false>;
+    default: return det ? kKernels<128, true> : kKernels<128, false>;
+  }
 }
-template <int MAXS, bool DETAIL>
-cudaError_t launch_extra(const FrameParams& P, cudaStream_t s) {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  trace_extra_strict_kernel<MAXS, DETAIL><<<sms * 8, kBlock, 0, s>>>(P);
+
+// `k` with one thread for each of `threads`
+cudaError_t launch_cover(TraceKernel k, unsigned long long threads, const FrameParams& P, cudaStream_t s) {
+  const long long blocks = grid_size(threads, kBlock);
+  if (blocks <= 0) return blocks == 0 ? cudaSuccess : cudaErrorInvalidConfiguration;
+  k<<<(unsigned)blocks, kBlock, 0, s>>>(P);
   return cudaGetLastError();
 }
 
 }  // namespace
 
-int rtrb_max_stack_supported(void) { return 128; }
-
-#define RTRB_DISPATCH(fn, P, need, s)                                         \
-  do {                                                                        \
-    const bool det = (P).count_detail != 0;                                   \
-    if ((need) <= 10) return det ? fn<10, true>(P, s) : fn<10, false>(P, s);  \
-    if ((need) <= 32) return det ? fn<32, true>(P, s) : fn<32, false>(P, s);  \
-    return det ? fn<128, true>(P, s) : fn<128, false>(P, s);                  \
-  } while (0)
-
 cudaError_t rtrb_launch_trace_pre_strict(const FrameParams& P, int stack_need, cudaStream_t s) {
-  RTRB_DISPATCH(launch_pre, P, stack_need, s);
+  return launch_cover(kernels(P, stack_need).pre, pre_threads(P), P, s);
 }
 cudaError_t rtrb_launch_trace_extra_strict(const FrameParams& P, int stack_need, cudaStream_t s) {
-  RTRB_DISPATCH(launch_extra, P, stack_need, s);
+  const TraceKernel k = kernels(P, stack_need).extra;
+  k<<<extra_grid(), kBlock, 0, s>>>(P);
+  return cudaGetLastError();
 }
 cudaError_t rtrb_launch_trace_mt_strict(const FrameParams& P, int stack_need, cudaStream_t s) {
-  RTRB_DISPATCH(launch_mt, P, stack_need, s);
+  // one thread per PIXEL
+  return launch_cover(kernels(P, stack_need).mt, (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS, P, s);
 }

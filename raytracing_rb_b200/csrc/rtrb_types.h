@@ -106,7 +106,7 @@ struct FrameParams {
   const struct BvhNode* bvh;   // sphere BVH over cull_sph[] (rtrb_bvh.h); node 0 = root
   int32_t n_sph, n_pl;
   int32_t use_bvh;             // > RTRB_BVH_MIN_SPHERES spheres: BVH kernels; else the linear-scan kernels
-  int32_t scene_class;         // what is known about the scene (rtrb_trace_fast.cuh, "scene / frame classes"):
+  int32_t scene_class;         // what is known about the scene (rtrb_trace.cuh, "build policies"):
                                // bit 0 = exactly one light and soft_shadow_exponent == 2; bit 1 = that and: the
                                // light's radius is exactly 0 and no object is textured.  Selects kernel builds
                                // without the code the class cannot reach; results are the generic kernels' bit for bit

@@ -39,6 +39,27 @@ def test_kernel_name_follows_the_dispatch():
         assert bench.kernel_name(cd, n_sph, klass) == want
 
 
+def test_kernel_names_exist_in_the_library():
+    """Every name bench.kernel_name gives for configs 1-5, with the linear filter and with the BVH, is a kernel of the
+    built library (bench.py reports it as the kernel that ran)."""
+    import re
+    import shutil
+    from raytracing_rb_b200 import Camera, _lib
+    if not os.path.exists(_lib.LIB_PATH) or shutil.which("cuobjdump") is None:
+        pytest.skip("needs the built library and cuobjdump")
+    out = subprocess.run(["cuobjdump", "-res-usage", _lib.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    functions = set(re.findall(r"Function (\S+):", out))
+    for cid in range(1, 6):
+        world, cdoc, _ = bench.workload(cid)
+        cd = Camera(world, cdoc).camera_desc()
+        for n_sph in (0, 33):  # linear filter, BVH
+            name = bench.kernel_name(cd, n_sph, bench.scene_class(world))
+            ns, fn, cap, detail, bvh = re.fullmatch(r"(\w+)::(\w+)<(\d+),(true|false),(true|false)>", name).groups()
+            mangled = "_ZN%d%s%d%sILi%sELb%dELb%dEEEv11FrameParams" % (len(ns), ns, len(fn), fn, cap, detail == "true",
+                                                                        bvh == "true")
+            assert mangled in functions, name
+
+
 def test_cpu_window_is_a_centred_full_height_strip():
     assert bench.cpu_window(1920, 1080, 1.0, 16) == (0, 0, 1920, 1080)
     assert bench.cpu_window(1920, 1080, 0.25, 16) == (720, 0, 1200, 1080)

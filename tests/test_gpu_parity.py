@@ -415,7 +415,7 @@ def test_more_spheres_than_the_filter_can_index(oracle_mod):
 @pytest.mark.parametrize("seed", range(8))
 def test_lean_scene_kernels_match_the_generic_path(oracle_mod, seed):
     """Scenes with ONE light of radius exactly 0, no textures and soft_shadow_exponent 2 run depth-1 frames on kernels
-    compiled without the code such a scene cannot reach (rtrb_trace_fast_d1lean.cu: light loops, pow, texture lookup,
+    compiled without the code such a scene cannot reach (the rtrb::Lean build policy: light loops, pow, texture lookup,
     the penumbra branch of Sphere#cover_area).  They must reproduce STRICT bit for bit and the oracle's frame, also
     with the camera inside a sphere, spheres cut by planes, a glassy plane, 1 and 3 samples per pixel and the adaptive
     pass; a light radius of 1e-300 or a second light must fall back to the generic kernels with the same result."""
