@@ -13,6 +13,8 @@
  *   Rtrb::Renderer.new(world)                      -> bakes the scene on GPU 0 (rtrb_renderer_create)
  *   renderer.render(camera, seed = 1, precision = 1) -> String of H*W*3 RGB8 bytes, row = y, col = x
  *                                                     (RTRB_FMT_RGB8: alpha is always 255, camera.rb:155)
+ *   renderer.render_png(camera, seed = 1, precision = 1) -> binary String: the frame as an 8-bit RGB PNG file,
+ *                                                     encoded on the GPU (only the file crosses PCIe)
  *   renderer.stats                                 -> Hash of the last frame's counters
  */
 #include <ruby.h>
@@ -191,6 +193,7 @@ typedef struct {
   rtrb_render_opts opts;
   uint8_t* rgba;
   int rc;
+  size_t capacity, png_bytes;  /* render_png */
 } render_call;
 
 static void* render_without_gvl(void* p) {   /* one blocking call per frame; the GVL is released */
@@ -199,7 +202,19 @@ static void* render_without_gvl(void* p) {   /* one blocking call per frame; the
   return NULL;
 }
 
-static VALUE renderer_render(int argc, VALUE* argv, VALUE self) {
+static void* render_png_without_gvl(void* p) {  /* render into device memory, encode there, fetch the file */
+  render_call* c = (render_call*)p;
+  c->rc = rtrb_render_device(c->s->r, &c->cam, &c->opts, &c->s->last);
+  if (c->rc != RTRB_OK && c->rc != RTRB_ERR_RAISED) return NULL;
+  const int raised = c->rc == RTRB_ERR_RAISED;
+  c->rc = rtrb_encode_png(c->s->r, NULL, c->cam.width, c->cam.height, c->opts.pixel_format, NULL, c->rgba, c->capacity,
+                          &c->png_bytes);
+  if (c->rc == RTRB_OK && raised) c->rc = RTRB_ERR_RAISED;
+  return NULL;
+}
+
+/* (camera, seed = 1, precision = 1) -> the frame call's camera and options (RTRB_FMT_RGB8) */
+static void frame_call(int argc, VALUE* argv, VALUE self, render_call* cp) {
   VALUE camera, seed, precision;
   rb_scan_args(argc, argv, "12", &camera, &seed, &precision);
   shim_renderer* s;
@@ -220,12 +235,31 @@ static VALUE renderer_render(int argc, VALUE* argv, VALUE self) {
   c.opts.seed = NIL_P(seed) ? 1 : NUM2ULL(seed);                 /* main.rb:10 Random.srand(1) */
   c.opts.precision = NIL_P(precision) ? RTRB_PREC_DEFAULT : NUM2INT(precision);
   c.opts.pixel_format = RTRB_FMT_RGB8;                           /* alpha = 255 never crosses PCIe */
+  *cp = c;
+}
+
+static VALUE renderer_render(int argc, VALUE* argv, VALUE self) {
+  render_call c;
+  frame_call(argc, argv, self, &c);
   size_t bytes = (size_t)c.cam.width * c.cam.height * 3;
   VALUE out = rb_str_new(NULL, (long)bytes);
   c.rgba = (uint8_t*)RSTRING_PTR(out);
   rb_thread_call_without_gvl(render_without_gvl, &c, RUBY_UBF_IO, NULL);
   if (c.rc == RTRB_ERR_RAISED) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());  /* ray_tracer.rb:295 et al. */
   if (c.rc != RTRB_OK) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());
+  return out;
+}
+
+static VALUE renderer_render_png(int argc, VALUE* argv, VALUE self) {
+  render_call c;
+  frame_call(argc, argv, self, &c);
+  c.opts.skip_outputs = RTRB_SKIP_RGB | RTRB_SKIP_HIT;           /* only the 8-bit frame is needed */
+  if (rtrb_png_max_bytes(c.cam.width, c.cam.height, &c.capacity) != RTRB_OK) rb_raise(rb_eArgError, "%s", rtrb_last_error());
+  VALUE out = rb_str_new(NULL, (long)c.capacity);
+  c.rgba = (uint8_t*)RSTRING_PTR(out);
+  rb_thread_call_without_gvl(render_png_without_gvl, &c, RUBY_UBF_IO, NULL);
+  if (c.rc != RTRB_OK) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());  /* RTRB_ERR_RAISED included, as render */
+  rb_str_set_len(out, (long)c.png_bytes);  /* rb_str_new strings are binary (ASCII-8BIT) */
   return out;
 }
 
@@ -247,6 +281,7 @@ void Init_rtrb_b200(void) {
   rb_define_alloc_func(cRenderer, renderer_alloc);
   rb_define_method(cRenderer, "initialize", renderer_initialize, 1);
   rb_define_method(cRenderer, "render", renderer_render, -1);
+  rb_define_method(cRenderer, "render_png", renderer_render_png, -1);
   rb_define_method(cRenderer, "stats", renderer_stats, 0);
   rb_define_const(mRtrb, "ABI_VERSION", INT2NUM(rtrb_abi_version()));
 }

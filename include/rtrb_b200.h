@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define RTRB_ABI_VERSION 3
+#define RTRB_ABI_VERSION 4
 
 /* ---- status codes ------------------------------------------------------------------------- */
 enum {
@@ -235,6 +235,32 @@ int rtrb_render(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
 int rtrb_submit(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* rgba_host,
                 int* ticket_out);
 int rtrb_wait(rtrb_renderer* r, int ticket, rtrb_stats* stats_out);
+
+/* -- PNG files encoded on the device (ABI 4) ------------------------------------------------------ */
+/* The encoder writes 8-bit RGB PNG files (colour type 2, no interlace; alpha is not stored because it is always 255).
+ * Every row takes the PNG filter (None, Sub, Up, Average, Paeth) with the smallest sum of |signed byte|, ties to the
+ * lowest type.  The filtered stream is cut into segments of RTRB_PNG_SEGMENT_BYTES that are deflated independently on
+ * the device, each into the smallest of a stored, fixed-Huffman or dynamic-Huffman block (matches may reach 32 KiB
+ * back into earlier segments) and one IDAT chunk; the zlib header and the Adler-32 trailer are IDAT chunks of their
+ * own.  The same image always gives the same bytes. */
+#define RTRB_PNG_SEGMENT_BYTES 32768
+
+/* bytes that always suffice for a device-encoded PNG of width x height (stored-block worst case; pure host) */
+int rtrb_png_max_bytes(int width, int height, size_t* bytes_out);
+
+/* Encodes a width x height image in `pixel_format` that is in device memory: `src_device` or, if NULL, the start of
+ * the renderer's framebuffer (its last frame, or a frame that tile ranks gathered there).  Ordered after the work on
+ * `stream` (NULL = the renderer's own).  Blocks until exactly *bytes_out bytes of PNG file are in png_host. */
+int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int height, int pixel_format, void* stream,
+                    uint8_t* png_host, size_t capacity, size_t* bytes_out);
+
+/* Pipelined form (the rtrb_submit slots and tickets; completed by the unchanged rtrb_wait, which also stores the
+ * byte count into *png_bytes_out).  png_host must be page-locked and device-mapped.  Only the encoded bytes cross
+ * PCIe: device stores through the mapped alias, as publish_ctl_kernel already does for the control block.
+ * opts->pixel_format is RTRB_FMT_RGBA8 or RTRB_FMT_RGB8; opts->rgba_device_out is rejected.  The frame is encoded on
+ * the renderer's copy stream, so the next frame renders meanwhile.  A frame that raises still yields its PNG. */
+int rtrb_submit_png(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* png_host,
+                    size_t capacity, size_t* png_bytes_out, int* ticket_out);
 
 /* -- multi-GPU tile gather without a collective ----------------------------------------------- */
 /* Device pointer of the renderer's RGBA8 framebuffer for (width,height) (allocates it if needed).  From this

@@ -5,6 +5,7 @@ module Rtrb
     # method stubs
     def initialize(world); raise NotImplementedError; end
     def render(camera, seed = 1, precision = 1); raise NotImplementedError; end
+    def render_png(camera, seed = 1, precision = 1); raise NotImplementedError; end
     def stats; raise NotImplementedError; end
   end
 end
@@ -27,6 +28,12 @@ module Alex
         end
       end
       save_image(file_path)
+    end
+
+    # save_image's file without the canvas: the GPU renders and encodes the PNG (8-bit RGB), only the file crosses PCIe
+    def render_cuda_png(file_path, seed = 1)
+      @rtrb ||= Rtrb::Renderer.new(@world)
+      File.binwrite(file_path, @rtrb.render_png(self, seed))
     end
   end
 end

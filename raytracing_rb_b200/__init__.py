@@ -11,7 +11,7 @@ from .configurable_object import ConfigurableObject
 from .lights import Light, SpotLight
 from .objects import Box, Plane, Sphere, WorldObject
 from .renderer import (Frame, Renderer, deal_frames, device_count, ipc_close, ipc_open, make_opts, measure_fma_peak,
-                       render_multi, tile_partition)
+                       png_max_bytes, render_multi, tile_partition)
 from .texture import Texture
 from .vec3 import Vec3
 from .world import World
@@ -20,5 +20,6 @@ __all__ = [
     "Camera", "World", "Sphere", "Plane", "Box", "WorldObject", "Light", "SpotLight", "Texture", "Vec3",
     "ConfigurableObject", "Renderer", "Frame", "make_opts", "render_multi", "measure_fma_peak",
     "device_count", "deal_frames", "ipc_open", "ipc_close", "write_png", "write_png_scanlines", "tile_partition",
+    "png_max_bytes",
     "PREC_STRICT", "PREC_FAST64", "PREC_DEFAULT", "RNG_CTR", "RNG_MT",
 ]

@@ -2,7 +2,7 @@
 for field; tests/test_abi.py checks sizeof() against the values the compiled library reports."""
 import ctypes as C
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 RTRB_OK, RTRB_ERR_INVALID, RTRB_ERR_CUDA, RTRB_ERR_RAISED, RTRB_ERR_UNSUPPORTED = 0, 1, 2, 3, 4
 
@@ -18,6 +18,7 @@ RNG_CTR, RNG_MT = 0, 1
 PREC_STRICT, PREC_FAST64 = 0, 1
 PREC_DEFAULT = PREC_FAST64
 SKIP_RGB, SKIP_HIT = 1, 2
+PNG_SEGMENT_BYTES = 32768  # RTRB_PNG_SEGMENT_BYTES: the deflate segment of the device PNG encoder
 
 D3 = C.c_double * 3
 

@@ -16,6 +16,7 @@ EXPORTS = (
     "rtrb_framebuffer_device_ptr", "rtrb_framebuffer_download", "rtrb_framebuffer_copy_async", "rtrb_framebuffer_ipc_export", "rtrb_ipc_open", "rtrb_ipc_close",
     "rtrb_peer_push", "rtrb_peer_push_join",
     "rtrb_render_multi", "rtrb_tile_partition", "rtrb_measure_fma_peak", "rtrb_launch_count", "rtrb_last_mt_passes",
+    "rtrb_png_max_bytes", "rtrb_encode_png", "rtrb_submit_png",
 )
 
 _lib = None
@@ -62,6 +63,11 @@ def lib():
     L.rtrb_measure_fma_peak.argtypes = [C.c_int, C.c_int, P(C.c_double)]
     L.rtrb_launch_count.restype = C.c_uint64
     L.rtrb_last_mt_passes.argtypes = [C.c_void_p]
+    L.rtrb_png_max_bytes.argtypes = [C.c_int, C.c_int, P(C.c_size_t)]
+    L.rtrb_encode_png.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
+                                  P(C.c_size_t)]
+    L.rtrb_submit_png.argtypes = [C.c_void_p, P(_abi.CameraDesc), P(_abi.RenderOpts), C.c_void_p, C.c_size_t,
+                                  P(C.c_size_t), P(C.c_int)]
     for name in EXPORTS:
         getattr(L, name)
     if L.rtrb_abi_version() != _abi.ABI_VERSION:

@@ -103,6 +103,15 @@ class Camera(ConfigurableObject):
         self.last_frame = frame
         return frame
 
+    @staticmethod
+    def _raise_for(stats):
+        names = [n for b, n in ((_abi.ST_COLOR_GT_1, "color greater than 1"),
+                                (_abi.ST_ZERO_VECTOR, "zero vector detected"),
+                                (_abi.ST_MATH_DOMAIN, "Math::DomainError"),
+                                (_abi.ST_STACK_OVERFLOW, "device bounce stack overflow"),
+                                (_abi.ST_NAN_TO_INT, "FloatDomainError")) if stats["status"] & b]
+        raise RuntimeError("%s at pixel (%d, %d)" % (", ".join(names), stats["first_bad_x"], stats["first_bad_y"]))
+
     def render_cuda(self, file_path=None, gpus=1, seed=1, **kw):
         """Drop-in for render_sync(file_path) / render_fork(file_path, n) (camera.rb:41-68,101-110).
         Raises RuntimeError where the reference would have raised mid-frame (ray_tracer.rb:294-296,
@@ -112,14 +121,25 @@ class Camera(ConfigurableObject):
         if file_path:
             self.save_image(file_path)
         if frame.raised:
-            names = [n for b, n in ((_abi.ST_COLOR_GT_1, "color greater than 1"),
-                                    (_abi.ST_ZERO_VECTOR, "zero vector detected"),
-                                    (_abi.ST_MATH_DOMAIN, "Math::DomainError"),
-                                    (_abi.ST_STACK_OVERFLOW, "device bounce stack overflow"),
-                                    (_abi.ST_NAN_TO_INT, "FloatDomainError")) if frame.status & b]
-            raise RuntimeError("%s at pixel (%d, %d)" % (", ".join(names), frame.stats["first_bad_x"],
-                                                         frame.stats["first_bad_y"]))
+            self._raise_for(frame.stats)
         return frame
+
+    def render_png(self, file_path, seed=1, **kw):
+        """render_cuda(file_path) with the PNG encoded on the GPU: one GPU renders the frame in RGB8 and deflates it in
+        device memory, and only the file crosses PCIe (8-bit RGB, where save_image writes RGBA with alpha 255; the
+        pixels are the same).  `canvas` is left as it was.  Raises RuntimeError as render_cuda does, after the file
+        has been written.  Returns the frame's stats dict."""
+        opts = make_opts(seed=seed, skip_outputs=_abi.SKIP_RGB | _abi.SKIP_HIT, pixel_format=_abi.FMT_RGB8, **kw)
+        r = self.renderer()
+        stats, code = r.render_device(self.camera_desc(), opts)
+        png = r.encode_png(self.width, self.height, _abi.FMT_RGB8)
+        d = os.path.dirname(os.path.abspath(file_path))
+        os.makedirs(d, exist_ok=True)
+        with open(file_path, "wb") as f:
+            f.write(png)
+        if code == _abi.RTRB_ERR_RAISED:
+            self._raise_for(stats)
+        return stats
 
     def render_fork(self, file_path, threads, out_dir="out", seed=1, **kw):
         """Drop-in for render_fork(file_path, threads) (camera.rb:41-68) for tooling that consumes its

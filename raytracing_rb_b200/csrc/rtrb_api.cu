@@ -19,6 +19,7 @@
 
 #include "../../include/rtrb_b200.h"
 #include "rtrb_launch.h"
+#include "rtrb_png.h"
 #include "rtrb_trace.cuh"
 #include "rtrb_types.h"
 
@@ -133,6 +134,7 @@ struct FrameCtl {
   unsigned long long* h_dev = nullptr;  // ... and the address the device stores to (publish_ctl_kernel)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, evt0 = nullptr, evt1 = nullptr, copied = nullptr, ctl_copied = nullptr;
   DevBuf<uint8_t> rgba;             // pipeline slots own a framebuffer; the main slot uses rtrb_renderer::rgba
+  size_t* png_bytes_out = nullptr;  // rtrb_submit_png frames: where rtrb_wait stores h[RTRB_FCB_WORDS], the file size
   // facts of the frame in flight, needed to finish its stats later
   int W = 0, H = 0, S = 0, E = 0, n_tiles = 0;
   bool detail = false, in_flight = false, timed = false;
@@ -141,7 +143,7 @@ struct FrameCtl {
   int init() {
     cudaError_t e;
     if ((e = d.ensure(RTRB_FCB_WORDS)) != cudaSuccess) return (int)e;
-    if ((e = cudaHostAlloc((void**)&h, RTRB_FCB_WORDS * sizeof(unsigned long long), cudaHostAllocMapped)) != cudaSuccess) return (int)e;
+    if ((e = cudaHostAlloc((void**)&h, (RTRB_FCB_WORDS + 1) * sizeof(unsigned long long), cudaHostAllocMapped)) != cudaSuccess) return (int)e;
     if ((e = cudaHostGetDevicePointer((void**)&h_dev, h, 0)) != cudaSuccess) return (int)e;
     cudaEvent_t* evs[6] = {&ev0, &ev1, &evt0, &evt1, &copied, &ctl_copied};
     for (auto ev : evs)
@@ -161,6 +163,8 @@ struct rtrb_renderer {
   int device = 0;
   cudaStream_t stream = nullptr, copy_stream = nullptr;
   cudaEvent_t push_ev = nullptr, push_done_ev = nullptr;  // rtrb_peer_push ordering (no timing)
+  cudaEvent_t png_ev = nullptr;  // rtrb_encode_png waits for the pipelined encodes that share png
+  RtrbPngScratch png;            // device PNG encoder scratch (rtrb_png.cu)
   FrameCtl main_ctl;       // synchronous calls
   FrameCtl pipe_ctl[RTRB_PIPE_SLOTS];  // rtrb_submit / rtrb_wait frame slots
   bool pipe_ready = false;
@@ -989,6 +993,61 @@ int finish_stats(rtrb_renderer* r, FrameCtl& fc, rtrb_stats* stats_out) {
   return RTRB_OK;
 }
 
+
+// First half of rtrb_submit / rtrb_submit_png: takes the next pipeline slot and launches the frame into its
+// framebuffer on the render stream.
+int submit_render(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, FrameCtl** fc_out,
+                  uint8_t** frame_out) {
+  CUDA_TRY(cudaSetDevice(r->device));
+  if (!r->pipe_ready) {
+    for (int i = 0; i < RTRB_PIPE_SLOTS; ++i) {
+      cudaError_t e = (cudaError_t)r->pipe_ctl[i].init();
+      if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "pipeline slot init failed: %s", cudaGetErrorString(e));
+    }
+    r->pipe_ready = true;
+  }
+  const unsigned ticket = r->next_ticket;
+  FrameCtl& fc = r->pipe_ctl[ticket % RTRB_PIPE_SLOTS];
+  if (fc.in_flight) return fail(RTRB_ERR_INVALID, "%d frames are already in flight: call rtrb_wait first", RTRB_PIPE_SLOTS);
+  const size_t slot_bytes = (size_t)cam->width * cam->height * 4;
+  if (cam->width > 0 && cam->height > 0 && fc.rgba.n < slot_bytes) {
+    CUDA_TRY(fc.rgba.ensure(slot_bytes));
+    CUDA_TRY(cudaMemsetAsync(fc.rgba.p, 0, slot_bytes, r->stream));
+  }
+  rtrb_render_opts o;
+  memset(&o, 0, sizeof(o));
+  if (opts) o = *opts;
+  else { o.seed = 1; o.precision = RTRB_PREC_DEFAULT; }
+  o.stream = nullptr;  // the pipeline owns its streams
+  FrameTargets tg;
+  tg.rgba = o.rgba_device_out ? (uint8_t*)o.rgba_device_out : fc.rgba.p;
+  tg.want_rgb = false; tg.want_hit = false;
+  int rc = render_impl(r, cam, &o, &tg, nullptr, &fc);
+  if (rc) return rc;
+  *fc_out = &fc;
+  *frame_out = tg.rgba;
+  return RTRB_OK;
+}
+
+// Second half: publishes the control block and hands out the ticket (the frame's copy or encode is queued).
+int submit_finish(rtrb_renderer* r, FrameCtl& fc, int* ticket_out) {
+  // The 1.3 KB control block does not go through the copy engine at all: a one-block kernel behind the frame's kernels
+  // stores it straight into the pinned (device-mapped) host mirror.  As a DMA of its own - even on its own stream - it
+  // sat between the 6.2 MB frame copies of a PCIe-bound sequence and cost 6 % of the frame rate (8 057 -> 8 540 frames/s
+  // on config 2); behind the frame on the copy stream it cost 14 % (round 1).
+  publish_ctl_kernel<<<1, 256, 0, r->stream>>>(fc.h_dev, fc.d.p, RTRB_FCB_WORDS);
+  CUDA_TRY(cudaGetLastError());
+  g_launches++;
+  CUDA_TRY(cudaEventRecord(fc.ctl_copied, r->stream));
+  // (the slot is reused only after rtrb_wait has host-synchronised on `copied`, so no stream wait is needed)
+  const unsigned ticket = r->next_ticket;
+  fc.in_flight = true;
+  fc.ticket = ticket;
+  r->next_ticket = ticket + 1;
+  *ticket_out = (int)ticket;
+  return RTRB_OK;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -1047,6 +1106,8 @@ int rtrb_renderer_destroy(rtrb_renderer* r) {
   r->extra_samples.release(); r->pre_avg.release(); r->rgb.release(); r->extra_list.release(); r->hit.release(); r->rgba.release();
   r->main_ctl.destroy();
   for (int i = 0; i < RTRB_PIPE_SLOTS; ++i) r->pipe_ctl[i].destroy();
+  r->png.release();
+  if (r->png_ev) cudaEventDestroy(r->png_ev);
   for (uint8_t* t : r->textures) cudaFree(t);
   if (r->push_ev) cudaEventDestroy(r->push_ev);
   if (r->push_done_ev) cudaEventDestroy(r->push_done_ev);
@@ -1104,52 +1165,55 @@ int rtrb_render(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
 int rtrb_submit(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* rgba_host,
                 int* ticket_out) {
   if (!r || !cam || !rgba_host || !ticket_out) return fail(RTRB_ERR_INVALID, "bad argument");
-  CUDA_TRY(cudaSetDevice(r->device));
-  if (!r->pipe_ready) {
-    for (int i = 0; i < RTRB_PIPE_SLOTS; ++i) {
-      cudaError_t e = (cudaError_t)r->pipe_ctl[i].init();
-      if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "pipeline slot init failed: %s", cudaGetErrorString(e));
-    }
-    r->pipe_ready = true;
-  }
-  const unsigned ticket = r->next_ticket;
-  FrameCtl& fc = r->pipe_ctl[ticket % RTRB_PIPE_SLOTS];
-  if (fc.in_flight) return fail(RTRB_ERR_INVALID, "%d frames are already in flight: call rtrb_wait first", RTRB_PIPE_SLOTS);
-  const size_t bytes = RTRB_FRAME_BYTES(cam->width, cam->height, opts ? opts->pixel_format : RTRB_FMT_RGBA8);
-  const size_t slot_bytes = (size_t)cam->width * cam->height * 4;
-  if (cam->width > 0 && cam->height > 0 && fc.rgba.n < slot_bytes) {
-    CUDA_TRY(fc.rgba.ensure(slot_bytes));
-    CUDA_TRY(cudaMemsetAsync(fc.rgba.p, 0, slot_bytes, r->stream));
-  }
-  rtrb_render_opts o;
-  memset(&o, 0, sizeof(o));
-  if (opts) o = *opts;
-  else { o.seed = 1; o.precision = RTRB_PREC_DEFAULT; }
-  o.stream = nullptr;  // the pipeline owns its streams
-  FrameTargets tg;
-  tg.rgba = o.rgba_device_out ? (uint8_t*)o.rgba_device_out : fc.rgba.p;
-  tg.want_rgb = false; tg.want_hit = false;
-  int rc = render_impl(r, cam, &o, &tg, nullptr, &fc);
+  FrameCtl* fcp = nullptr;
+  uint8_t* frame = nullptr;
+  int rc = submit_render(r, cam, opts, &fcp, &frame);
   if (rc) return rc;
+  FrameCtl& fc = *fcp;
+  const size_t bytes = RTRB_FRAME_BYTES(cam->width, cam->height, opts ? opts->pixel_format : RTRB_FMT_RGBA8);
   // the copy stream picks the frame up as soon as its kernels are done; the render stream is free
   // to start the next frame into the other slot meanwhile
   CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, fc.ev1, 0));
-  CUDA_TRY(cudaMemcpyAsync(rgba_host, tg.rgba, bytes, cudaMemcpyDeviceToHost, r->copy_stream));
+  CUDA_TRY(cudaMemcpyAsync(rgba_host, frame, bytes, cudaMemcpyDeviceToHost, r->copy_stream));
   CUDA_TRY(cudaEventRecord(fc.copied, r->copy_stream));
-  // The 1.3 KB control block does not go through the copy engine at all: a one-block kernel behind the frame's kernels
-  // stores it straight into the pinned (device-mapped) host mirror.  As a DMA of its own - even on its own stream - it
-  // sat between the 6.2 MB frame copies of a PCIe-bound sequence and cost 6 % of the frame rate (8 057 -> 8 540 frames/s
-  // on config 2); behind the frame on the copy stream it cost 14 % (round 1).
-  publish_ctl_kernel<<<1, 256, 0, r->stream>>>(fc.h_dev, fc.d.p, RTRB_FCB_WORDS);
-  CUDA_TRY(cudaGetLastError());
-  g_launches++;
-  CUDA_TRY(cudaEventRecord(fc.ctl_copied, r->stream));
-  // (the slot is reused only after rtrb_wait has host-synchronised on `copied`, so no stream wait is needed)
-  fc.in_flight = true;
-  fc.ticket = ticket;
-  r->next_ticket = ticket + 1;
-  *ticket_out = (int)ticket;
-  return RTRB_OK;
+  fc.png_bytes_out = nullptr;
+  return submit_finish(r, fc, ticket_out);
+}
+
+int rtrb_submit_png(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* png_host,
+                    size_t capacity, size_t* png_bytes_out, int* ticket_out) {
+  if (!r || !cam || !png_host || !png_bytes_out || !ticket_out) return fail(RTRB_ERR_INVALID, "bad argument");
+  const int fmt = opts ? opts->pixel_format : RTRB_FMT_RGBA8;
+  if (fmt != RTRB_FMT_RGBA8 && fmt != RTRB_FMT_RGB8)
+    return fail(RTRB_ERR_INVALID, "rtrb_submit_png encodes RTRB_FMT_RGBA8 or RTRB_FMT_RGB8 frames, not format %d", fmt);
+  if (opts && opts->rgba_device_out)
+    return fail(RTRB_ERR_INVALID, "rgba_device_out does not combine with rtrb_submit_png (the frame stays in its slot)");
+  size_t need = 0;
+  int rc = rtrb_png_max_bytes(cam->width, cam->height, &need);
+  if (rc) return rc;
+  if (capacity < need) return fail(RTRB_ERR_INVALID, "png capacity %zu < %zu bytes (rtrb_png_max_bytes)", capacity, need);
+  CUDA_TRY(cudaSetDevice(r->device));
+  void* host_dev = nullptr;
+  if (cudaHostGetDevicePointer(&host_dev, png_host, 0) != cudaSuccess) {
+    cudaGetLastError();  // not sticky: clear it so that later launch checks do not report it
+    return fail(RTRB_ERR_INVALID, "png_host is not page-locked, device-mapped host memory");
+  }
+  FrameCtl* fcp = nullptr;
+  uint8_t* frame = nullptr;
+  rc = submit_render(r, cam, opts, &fcp, &frame);
+  if (rc) return rc;
+  FrameCtl& fc = *fcp;
+  // encoded on the copy stream behind the frame's kernels: the render stream goes on with the next frame, and only the
+  // file crosses PCIe (device stores into png_host, the byte count into the slot's mapped control word)
+  CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, fc.ev1, 0));
+  unsigned long long launches = 0;
+  cudaError_t e = rtrb_png_encode(r->png, frame, cam->width, cam->height, fmt, r->copy_stream, (uint8_t*)host_dev,
+                                  fc.h_dev + RTRB_FCB_WORDS, &launches);
+  g_launches += launches;
+  if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "PNG encoder: %s", cudaGetErrorString(e));
+  CUDA_TRY(cudaEventRecord(fc.copied, r->copy_stream));
+  fc.png_bytes_out = png_bytes_out;
+  return submit_finish(r, fc, ticket_out);
 }
 
 int rtrb_wait(rtrb_renderer* r, int ticket, rtrb_stats* stats_out) {
@@ -1160,6 +1224,7 @@ int rtrb_wait(rtrb_renderer* r, int ticket, rtrb_stats* stats_out) {
   CUDA_TRY(cudaEventSynchronize(fc.copied));
   CUDA_TRY(cudaEventSynchronize(fc.ctl_copied));
   fc.in_flight = false;
+  if (fc.png_bytes_out) *fc.png_bytes_out = (size_t)fc.h[RTRB_FCB_WORDS];
   rtrb_stats local;
   return finish_stats(r, fc, stats_out ? stats_out : &local);
 }
@@ -1328,6 +1393,53 @@ int rtrb_render_multi(rtrb_renderer* const* renderers, int n, const rtrb_camera_
   if (rc) return rc;
   if (worst == RTRB_ERR_RAISED) g_last_error = keep;
   return worst;
+}
+
+int rtrb_png_max_bytes(int width, int height, size_t* bytes_out) {
+  if (!bytes_out || width <= 0 || height <= 0) return fail(RTRB_ERR_INVALID, "bad argument");
+  *bytes_out = rtrb_png_bound(width, height);
+  return RTRB_OK;
+}
+
+int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int height, int pixel_format, void* stream,
+                    uint8_t* png_host, size_t capacity, size_t* bytes_out) {
+  if (!png_host || !bytes_out) return fail(RTRB_ERR_INVALID, "bad argument");
+  if (pixel_format != RTRB_FMT_RGBA8 && pixel_format != RTRB_FMT_RGB8 && pixel_format != RTRB_FMT_PNG_RGB8)
+    return fail(RTRB_ERR_INVALID, "unknown pixel format %d", pixel_format);
+  size_t need = 0;
+  int rc = rtrb_png_max_bytes(width, height, &need);
+  if (rc) return rc;
+  if (capacity < need) return fail(RTRB_ERR_INVALID, "png capacity %zu < %zu bytes (rtrb_png_max_bytes)", capacity, need);
+  int n = 0;
+  cudaError_t e = cudaGetDeviceCount(&n);
+  if (e != cudaSuccess || n == 0) {
+    cudaGetLastError();
+    return fail(RTRB_ERR_CUDA, "no CUDA device (%s); this library has no CPU fallback", cudaGetErrorString(e));
+  }
+  if (!r) return fail(RTRB_ERR_INVALID, "renderer is NULL");
+  CUDA_TRY(cudaSetDevice(r->device));
+  const uint8_t* src = (const uint8_t*)src_device;
+  if (!src) {
+    if (r->rgba.n < RTRB_FRAME_BYTES(width, height, pixel_format))
+      return fail(RTRB_ERR_INVALID, "the framebuffer (%zu bytes) is smaller than a %dx%d frame", r->rgba.n, width, height);
+    src = r->rgba.p;
+  }
+  cudaStream_t s = stream ? (cudaStream_t)stream : r->stream;
+  if (!r->png_ev) CUDA_TRY(cudaEventCreateWithFlags(&r->png_ev, cudaEventDisableTiming));
+  CUDA_TRY(cudaEventRecord(r->png_ev, r->copy_stream));  // pipelined encodes use the same scratch
+  CUDA_TRY(cudaStreamWaitEvent(s, r->png_ev, 0));
+  unsigned long long launches = 0;
+  e = rtrb_png_encode(r->png, src, width, height, pixel_format, s, nullptr, nullptr, &launches);
+  g_launches += launches;
+  if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "PNG encoder: %s", cudaGetErrorString(e));
+  unsigned long long total = 0;
+  CUDA_TRY(cudaMemcpyAsync(&total, r->png.total, sizeof(total), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  if (total > capacity) return fail(RTRB_ERR_CUDA, "PNG encoder produced %llu bytes, more than its bound %zu", total, need);
+  CUDA_TRY(cudaMemcpyAsync(png_host, r->png.file, total, cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  *bytes_out = (size_t)total;
+  return RTRB_OK;
 }
 
 int rtrb_tile_partition(int width, int height, const int32_t* window, int tile_rank, int tile_world,

@@ -44,6 +44,7 @@ class Renderer:
         self._scene = scene  # SceneDescHolder; only needed during create, kept for introspection
         self._h = C.c_void_p()
         self.device = device
+        self._png_pending = {}  # submit_png ticket -> (host buffer, byte count that rtrb_wait fills in)
         check(lib().rtrb_renderer_create(C.byref(scene.desc), device, C.byref(self._h)))
 
     def close(self):
@@ -108,6 +109,35 @@ class Renderer:
         code = lib().rtrb_wait(self._h, ticket, C.byref(st))
         check(code, allow_raised=True)
         return st.as_dict(), code
+
+    def encode_png(self, width, height, pixel_format=_abi.FMT_RGB8, src=None, stream=None):
+        """PNG file (bytes) of a width x height image in device memory, encoded on the device: `src` (a device pointer)
+        or, if None, the renderer's framebuffer; ordered after the work on `stream` (None = the renderer's own)."""
+        cap = png_max_bytes(width, height)
+        out = np.empty(cap, np.uint8)
+        n = C.c_size_t()
+        check(lib().rtrb_encode_png(self._h, C.c_void_p(src) if src else None, width, height, pixel_format,
+                                    C.c_void_p(stream) if stream else None, out.ctypes.data, cap, C.byref(n)))
+        return out[:n.value].tobytes()
+
+    def submit_png(self, cam, out_pinned, opts=None):
+        """Pipelined frame encoded as a PNG file on the device: returns a ticket at once; the file lands in `out_pinned`
+        (a uint8 numpy view of page-locked, device-mapped host memory of at least png_max_bytes(W, H) bytes) by the time
+        `wait_png(ticket)` returns.  Shares the four slots and the ticket order of `submit`."""
+        opts = opts or make_opts()
+        t = C.c_int()
+        n = C.c_size_t()
+        check(lib().rtrb_submit_png(self._h, C.byref(cam), C.byref(opts), out_pinned.ctypes.data, out_pinned.nbytes,
+                                    C.byref(n), C.byref(t)))
+        self._png_pending[t.value] = (out_pinned, n)
+        return t.value
+
+    def wait_png(self, ticket):
+        """-> (PNG bytes, stats dict, status code) of a submit_png frame."""
+        out, n = self._png_pending.get(ticket, (None, None))
+        stats, code = self.wait(ticket)
+        del self._png_pending[ticket]
+        return out[:n.value].tobytes(), stats, code
 
     def peer_push(self, src_ptr, dst_peer_ptr, nbytes, after_stream=None):
         """Copy-engine gather: queue a D2D copy to a peer mapping behind `after_stream` (see rtrb_peer_push)."""
@@ -187,6 +217,13 @@ def deal_frames(rank, world, frames_per_gpu):
         raise ValueError("bad rank/world/frames_per_gpu")
     first = rank * frames_per_gpu
     return [(first + f, first + f) for f in range(frames_per_gpu)]
+
+
+def png_max_bytes(width, height):
+    """Bytes that always suffice for a device-encoded PNG of width x height.  Pure host logic."""
+    n = C.c_size_t()
+    check(lib().rtrb_png_max_bytes(width, height, C.byref(n)))
+    return n.value
 
 
 def measure_fma_peak(device=0, fp64=True):
