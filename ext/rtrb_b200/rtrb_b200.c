@@ -15,7 +15,12 @@
  *                                                     (RTRB_FMT_RGB8: alpha is always 255, camera.rb:155)
  *   renderer.render_png(camera, seed = 1, precision = 1) -> binary String: the frame as an 8-bit RGB PNG file,
  *                                                     encoded on the GPU (only the file crosses PCIe)
- *   renderer.stats                                 -> Hash of the last frame's counters
+ *   renderer.stats                                 -> Hash of the last frame's (or ray batch's) counters
+ *   renderer.trace_rays(packed_rays, trace_depth, mc, seed = 1) -> [rgb, hits]: RayTracer#trace_sync on n rays given as
+ *                                                     n*6 doubles (position, front; Array#pack("d*")); rgb = n*3 doubles,
+ *                                                     hits = n int32 root-ray winners (unpack("d*") / unpack("l*"))
+ *   renderer.intersect_rays(packed_rays)           -> String of n rtrb_ray_hit records (unpack("l4d7") each):
+ *                                                     World#intersect's object, :in?, box face, distance, point, delta
  */
 #include <ruby.h>
 #include <ruby/thread.h>
@@ -263,6 +268,70 @@ static VALUE renderer_render_png(int argc, VALUE* argv, VALUE self) {
   return out;
 }
 
+typedef struct {
+  shim_renderer* s;
+  rtrb_ray_opts opts;
+  int n;
+  const rtrb_ray* rays;
+  double* rgb;
+  int32_t* hit;
+  rtrb_ray_hit* hits;
+  int rc;
+} ray_call;
+
+static void* trace_rays_without_gvl(void* p) {   /* one blocking call per batch; the GVL is released */
+  ray_call* c = (ray_call*)p;
+  c->rc = rtrb_trace_rays(c->s->r, &c->opts, c->n, c->rays, NULL, c->rgb, c->hit, &c->s->last);
+  return NULL;
+}
+
+static void* intersect_rays_without_gvl(void* p) {
+  ray_call* c = (ray_call*)p;
+  c->rc = rtrb_intersect_rays(c->s->r, &c->opts, c->n, c->rays, c->hits);
+  return NULL;
+}
+
+/* packed_rays: a String of n * 6 doubles -> the call's rays (the String must stay referenced while the call runs) */
+static void ray_call_init(VALUE self, VALUE packed_rays, ray_call* c) {
+  StringValue(packed_rays);
+  if (RSTRING_LEN(packed_rays) % (long)sizeof(rtrb_ray) != 0)
+    rb_raise(rb_eArgError, "packed rays must be a multiple of 48 bytes (6 doubles: position, front)");
+  memset(c, 0, sizeof(*c));
+  Data_Get_Struct(self, shim_renderer, c->s);
+  c->n = (int)(RSTRING_LEN(packed_rays) / (long)sizeof(rtrb_ray));
+  c->rays = (const rtrb_ray*)RSTRING_PTR(packed_rays);
+  c->opts.precision = RTRB_PREC_DEFAULT;
+}
+
+static VALUE renderer_trace_rays(int argc, VALUE* argv, VALUE self) {
+  VALUE packed, depth, mc, seed;
+  rb_scan_args(argc, argv, "31", &packed, &depth, &mc, &seed);
+  ray_call c;
+  ray_call_init(self, packed, &c);
+  c.opts.trace_depth = NUM2INT(depth);
+  c.opts.monte_carlo_diffusion_times = NUM2INT(mc);
+  c.opts.seed = NIL_P(seed) ? 1 : NUM2ULL(seed);
+  VALUE rgb = rb_str_new(NULL, (long)c.n * 3 * (long)sizeof(double));
+  VALUE hit = rb_str_new(NULL, (long)c.n * (long)sizeof(int32_t));
+  c.rgb = (double*)RSTRING_PTR(rgb);
+  c.hit = (int32_t*)RSTRING_PTR(hit);
+  rb_thread_call_without_gvl(trace_rays_without_gvl, &c, RUBY_UBF_IO, NULL);
+  RB_GC_GUARD(packed);
+  if (c.rc != RTRB_OK) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());  /* RTRB_ERR_RAISED included, as render */
+  return rb_ary_new_from_args(2, rgb, hit);
+}
+
+static VALUE renderer_intersect_rays(VALUE self, VALUE packed) {
+  ray_call c;
+  ray_call_init(self, packed, &c);
+  VALUE out = rb_str_new(NULL, (long)c.n * (long)sizeof(rtrb_ray_hit));
+  c.hits = (rtrb_ray_hit*)RSTRING_PTR(out);
+  rb_thread_call_without_gvl(intersect_rays_without_gvl, &c, RUBY_UBF_IO, NULL);
+  RB_GC_GUARD(packed);
+  if (c.rc != RTRB_OK) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());
+  return out;
+}
+
 static VALUE renderer_stats(VALUE self) {
   shim_renderer* s;
   Data_Get_Struct(self, shim_renderer, s);
@@ -283,5 +352,7 @@ void Init_rtrb_b200(void) {
   rb_define_method(cRenderer, "render", renderer_render, -1);
   rb_define_method(cRenderer, "render_png", renderer_render_png, -1);
   rb_define_method(cRenderer, "stats", renderer_stats, 0);
+  rb_define_method(cRenderer, "trace_rays", renderer_trace_rays, -1);
+  rb_define_method(cRenderer, "intersect_rays", renderer_intersect_rays, 1);
   rb_define_const(mRtrb, "ABI_VERSION", INT2NUM(rtrb_abi_version()));
 }

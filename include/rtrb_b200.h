@@ -262,6 +262,66 @@ int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int hei
 int rtrb_submit_png(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* png_host,
                     size_t capacity, size_t* png_bytes_out, int* ticket_out);
 
+/* -- ray-level queries on caller-supplied rays ---------------------------------------------------- */
+/* The layers below the camera, for callers with their own rays (other projections, picking, probes of one ray):
+ * RayTracer#trace_sync (ray_tracer.rb:16-46) and World#intersect (world.rb:37-59) on a batch of rays, one device
+ * thread per ray, and Camera#lens_func (camera.rb:129-151) for a window of pixels.  Same kernels' arithmetic as the
+ * frames: STRICT and FAST64 give the same bits.  The calls never touch the renderer's framebuffers, its last frame or
+ * its rtrb_submit slots (they have a control block and scratch of their own); they are not pipelined and draw their
+ * Monte-Carlo rays from the counter RNG only.  Every call fails with RTRB_ERR_CUDA when no CUDA device is usable. */
+
+/* Ray(front, position) of the reference (algebra.rb); `front` is NOT normalised, as the reference keeps it. */
+typedef struct rtrb_ray {
+  double position[3];
+  double front[3];
+} rtrb_ray;
+
+/* World#intersect's answer for one ray.  A miss has object -1, face -1 and zeros elsewhere. */
+typedef struct rtrb_ray_hit {
+  int32_t object;          /* index in world_objects, -1 = miss */
+  int32_t direction;       /* 1 = :in, 0 = :out */
+  int32_t face;            /* box: Box#intersect's data[:index] (box.rb:89: 0 up, 1 bottom, 2 front, 3 back, 4 left,
+                              5 right); -1 otherwise */
+  int32_t reserved0;
+  double distance;         /* Ray#distance(intersection) (algebra.rb:10-12) */
+  double intersection[3];
+  double delta[3];         /* sphere.rb:84 / plane.rb:50 (a box: the winning face's plane) */
+} rtrb_ray_hit;
+
+/* bytes of device scratch a host-buffer ray call may use (inputs and outputs staged on the device) */
+#define RTRB_RAY_SCRATCH_BUDGET ((size_t)16 << 30)
+
+typedef struct rtrb_ray_opts {
+  int32_t precision;       /* RTRB_PREC_* */
+  int32_t device_buffers;  /* 0: host pointers, blocking.  1: device pointers on the renderer's device, ordered on
+                              `stream`; synchronises only when stats_out != NULL (like rtrb_render_device) */
+  uint64_t seed;           /* Philox key, as rtrb_render_opts.seed */
+  int32_t trace_depth, monte_carlo_diffusion_times;  /* rtrb_trace_rays: the root item's depth, MC rays per bounce */
+  int32_t count_detail;    /* rtrb_trace_rays: 1 = fill every rtrb_stats counter */
+  int32_t x0, y0, x1, y1;  /* rtrb_camera_rays: window of pixels, x in [x0,x1), y in [y0,y1); all zero = whole frame */
+  int32_t reserved0;
+  void* stream;            /* cudaStream_t; NULL = the renderer's own stream */
+} rtrb_ray_opts;
+
+/* RayTracer#trace_sync on n rays: the root item has depth opts->trace_depth and attenuation (1, 1, 1).  Ray i draws its
+ * Monte-Carlo rays from the Philox counter (keys[2i], keys[2i+1], path, 1), keys_or_null = NULL meaning (i, 0); a
+ * frame's sample j of pixel (x, y) is keyed (y * W + x, j), so rays from rtrb_camera_rays traced with its keys reproduce
+ * the frame's samples bit for bit.  rgb_out: n x 3 doubles, the unclamped rt_reduce sum; hit_or_null: n root-ray
+ * World#intersect winners (-1 miss, -2 highlight-terminated).  stats_out: counters and status as for a frame of height
+ * 1, so first_bad_x is the lowest offending ray index and first_bad_y is 0.  RTRB_ERR_RAISED when a ray would have
+ * raised in the reference (every output is written); RTRB_ERR_UNSUPPORTED when trace_depth * (1 + mc) + 1 exceeds the
+ * device work stack (128 items, as for frames) or the host-buffer scratch exceeds RTRB_RAY_SCRATCH_BUDGET. */
+int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rtrb_ray* rays, const uint32_t* keys_or_null,
+                    double* rgb_out, int32_t* hit_or_null, rtrb_stats* stats_out);
+/* World#intersect on n rays (opts: precision, device_buffers, stream). */
+int rtrb_intersect_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rtrb_ray* rays, rtrb_ray_hit* hits_out);
+/* Camera#lens_func for every pixel (x, y) of the window and every sample j in [sample_begin, sample_end), with the
+ * aperture angle the frame draws for that sample (Philox counter (y * W + x, j, 0, 0)).  Ray (x, y, j) is at index
+ * ((y - y0) * (x1 - x0) + (x - x0)) * (sample_end - sample_begin) + (j - sample_begin); keys_or_null receives its
+ * (y * W + x, j) key.  The camera's sampling and tracing fields are not used. */
+int rtrb_camera_rays(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_ray_opts* opts, int sample_begin,
+                     int sample_end, rtrb_ray* rays_out, uint32_t* keys_or_null);
+
 /* -- multi-GPU tile gather without a collective ----------------------------------------------- */
 /* Device pointer of the renderer's RGBA8 framebuffer for (width,height) (allocates it if needed).  From this
  * call (or rtrb_framebuffer_ipc_export) on the framebuffer is PINNED: a later frame or request that needs a larger

@@ -7,6 +7,8 @@ module Rtrb
     def render(camera, seed = 1, precision = 1); raise NotImplementedError; end
     def render_png(camera, seed = 1, precision = 1); raise NotImplementedError; end
     def stats; raise NotImplementedError; end
+    def trace_rays(packed_rays, trace_depth, mc, seed = 1); raise NotImplementedError; end
+    def intersect_rays(packed_rays); raise NotImplementedError; end
   end
 end
 

@@ -80,6 +80,28 @@ class RenderOpts(C.Structure):
     ]
 
 
+class Ray(C.Structure):
+    _fields_ = [("position", D3), ("front", D3)]
+
+
+class RayHit(C.Structure):
+    _fields_ = [
+        ("object", C.c_int32), ("direction", C.c_int32), ("face", C.c_int32), ("reserved0", C.c_int32),
+        ("distance", C.c_double), ("intersection", D3), ("delta", D3),
+    ]
+
+
+class RayOpts(C.Structure):
+    _fields_ = [
+        ("precision", C.c_int32), ("device_buffers", C.c_int32), ("seed", C.c_uint64),
+        ("trace_depth", C.c_int32), ("monte_carlo_diffusion_times", C.c_int32),
+        ("count_detail", C.c_int32),
+        ("x0", C.c_int32), ("y0", C.c_int32), ("x1", C.c_int32), ("y1", C.c_int32),
+        ("reserved0", C.c_int32),
+        ("stream", C.c_void_p),
+    ]
+
+
 class Stats(C.Structure):
     _fields_ = [
         ("samples", C.c_uint64), ("rays", C.c_uint64), ("shadow_queries", C.c_uint64),

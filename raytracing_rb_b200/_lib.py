@@ -17,6 +17,7 @@ EXPORTS = (
     "rtrb_peer_push", "rtrb_peer_push_join",
     "rtrb_render_multi", "rtrb_tile_partition", "rtrb_measure_fma_peak", "rtrb_launch_count", "rtrb_last_mt_passes",
     "rtrb_png_max_bytes", "rtrb_encode_png", "rtrb_submit_png",
+    "rtrb_trace_rays", "rtrb_intersect_rays", "rtrb_camera_rays",
 )
 
 _lib = None
@@ -68,6 +69,11 @@ def lib():
                                   P(C.c_size_t)]
     L.rtrb_submit_png.argtypes = [C.c_void_p, P(_abi.CameraDesc), P(_abi.RenderOpts), C.c_void_p, C.c_size_t,
                                   P(C.c_size_t), P(C.c_int)]
+    L.rtrb_trace_rays.argtypes = [C.c_void_p, P(_abi.RayOpts), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                  P(_abi.Stats)]
+    L.rtrb_intersect_rays.argtypes = [C.c_void_p, P(_abi.RayOpts), C.c_int, C.c_void_p, C.c_void_p]
+    L.rtrb_camera_rays.argtypes = [C.c_void_p, P(_abi.CameraDesc), P(_abi.RayOpts), C.c_int, C.c_int, C.c_void_p,
+                                   C.c_void_p]
     for name in EXPORTS:
         getattr(L, name)
     if L.rtrb_abi_version() != _abi.ABI_VERSION:

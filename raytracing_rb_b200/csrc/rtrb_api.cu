@@ -20,6 +20,7 @@
 #include "../../include/rtrb_b200.h"
 #include "rtrb_launch.h"
 #include "rtrb_png.h"
+#include "rtrb_rays.h"
 #include "rtrb_trace.cuh"
 #include "rtrb_types.h"
 
@@ -226,6 +227,12 @@ struct rtrb_renderer {
   int last_format = RTRB_FMT_RGBA8;
   cudaStream_t last_stream = nullptr;
   bool timing_valid = false;
+  // ray-level calls (rtrb_trace_rays & co.): their own control block and scratch, never the frames'
+  FrameCtl ray_ctl;
+  bool ray_ready = false;
+  DevBuf<uint8_t> ray_scratch;         // host-buffer calls: inputs and outputs staged on the device
+  DevBuf<double> ray_lens;             // rtrb_camera_rays: lens tables
+  double ray_lens_key[4] = {0, 0, 0, 0};  // (W, H, retina_width, retina_height) ray_lens was built for
 };
 
 namespace {
@@ -630,6 +637,40 @@ void enumerate_tiles(int W, int x0, int y0, int x1, int y1, int rank, int world,
       if (i % world == rank) out.push_back(ty * stx_count + tx);
 }
 
+// The per-column / per-row scalars of camera.rb:133-134 in the reference's order: [W] x offsets, then [H] y offsets.
+std::vector<double> lens_table(const rtrb_camera_desc* cam) {
+  const int W = cam->width, H = cam->height;
+  std::vector<double> tab((size_t)W + H);
+  for (int x = 0; x < W; ++x) tab[x] = 2.0 * ((double)x / W - 0.5) * cam->retina_width;
+  for (int y = 0; y < H; ++y) tab[(size_t)W + y] = 2 * ((double)y / H - 0.5) * cam->retina_height;
+  return tab;
+}
+
+// The scene part of FrameParams: baked buffers, FP32 filter view, constant-bank tables of small scenes.  The camera
+// apex table is not part of it (it only holds for rays that start at the camera).
+void fill_scene_params(const rtrb_renderer* r, FrameParams& P) {
+  P.max_distance = r->max_distance; P.soft_shadow_exponent = r->soft_shadow_exponent;
+  P.n_objects = r->n_objects; P.n_lights = r->n_lights;
+  P.geom = r->geom.p; P.mat = r->mat.p; P.lights = r->lights.p; P.boxes = r->boxes.p;
+  P.cull_sph = r->cull_sph.p; P.sph_index = r->sph_index.p; P.cull_pl = r->cull_pl.p; P.pl_index = r->pl_index.p;
+  P.lights_f = r->lights_f.p; P.n_sph = r->n_sph; P.n_pl = r->n_pl; P.bvh = r->bvh.p;
+  P.m_scene = r->m_scene; P.max_distance_f = r->max_distance_f;
+  P.use_bvh = r->small_scene ? 0 : 1;
+  P.scene_class = r->scene_class;
+  if (r->small_scene) {
+    static_assert(sizeof(r->k.light_tab) == sizeof(P.k_light_tab) && sizeof(r->k.lights) == sizeof(P.k_lights), "table layout");
+    memcpy(P.k_light_tab, r->k.light_tab, sizeof(P.k_light_tab));
+    memcpy(P.k_cull_sph, r->k.cull_sph, sizeof(P.k_cull_sph));
+    memcpy(P.k_cull_pl, r->k.cull_pl, sizeof(P.k_cull_pl));
+    memcpy(P.k_lights, r->k.lights, sizeof(P.k_lights));
+    memcpy(P.k_lights_f, r->k.lights_f, sizeof(P.k_lights_f));
+    memcpy(P.k_pl_index, r->k.pl_index, sizeof(P.k_pl_index));
+    P.k_has_light_tab = r->k.has_light_tab;
+  }
+  P.light_tab = r->light_tab.p;  // nullptr unless the scene uses the linear filter
+  P.cam_tab_valid = 0;
+}
+
 struct FrameTargets {  // where this renderer writes (own buffers, or rank 0's through a peer mapping)
   uint8_t* rgba = nullptr;
   double* rgb = nullptr;
@@ -659,6 +700,15 @@ int ensure_framebuffers(rtrb_renderer* r, int w, int h, bool rgba, bool rgb, boo
 }
 
 int finish_stats(rtrb_renderer* r, FrameCtl& fc, rtrb_stats* stats_out);
+
+// The control-block words a launch reports into (layout: RTRB_FCB_WORDS).
+void bind_ctl(FrameParams& P, FrameCtl& fc) {
+  P.counters = fc.d.p; P.first_bad = fc.d.p + RTRB_CNT_N;
+  P.work_counter = fc.d.p + RTRB_CNT_N + 1;
+  P.status = reinterpret_cast<uint32_t*>(fc.d.p + RTRB_CNT_N + 3);
+  P.extra_count = reinterpret_cast<uint32_t*>(fc.d.p + RTRB_CNT_N + 4);
+  P.hot = fc.d.p + RTRB_CNT_N + 5;
+}
 
 int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts_in,
                 const FrameTargets* targets, rtrb_stats* stats_out, FrameCtl* ctl = nullptr) {
@@ -755,9 +805,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   {
     double lk[4] = {(double)W, (double)H, cam->retina_width, cam->retina_height};
     if (memcmp(lk, r->lens_key, sizeof(lk)) != 0 || !r->lens_tab.p) {
-      std::vector<double> tab((size_t)W + H);
-      for (int x = 0; x < W; ++x) tab[x] = 2.0 * ((double)x / W - 0.5) * cam->retina_width;
-      for (int y = 0; y < H; ++y) tab[(size_t)W + y] = 2 * ((double)y / H - 0.5) * cam->retina_height;
+      const std::vector<double> tab = lens_table(cam);
       CUDA_TRY(r->lens_tab.ensure(tab.size()));
       CUDA_TRY(cudaMemcpyAsync(r->lens_tab.p, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
       CUDA_TRY(cudaStreamSynchronize(stream));
@@ -786,26 +834,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   FrameParams P;
   memset(&P, 0, sizeof(P));
   bake_camera(P, cam);
-  P.max_distance = r->max_distance; P.soft_shadow_exponent = r->soft_shadow_exponent;
-  P.n_objects = r->n_objects; P.n_lights = r->n_lights;
-  P.geom = r->geom.p; P.mat = r->mat.p; P.lights = r->lights.p; P.boxes = r->boxes.p;
-  P.cull_sph = r->cull_sph.p; P.sph_index = r->sph_index.p; P.cull_pl = r->cull_pl.p; P.pl_index = r->pl_index.p;
-  P.lights_f = r->lights_f.p; P.n_sph = r->n_sph; P.n_pl = r->n_pl; P.bvh = r->bvh.p;
-  P.m_scene = r->m_scene; P.max_distance_f = r->max_distance_f;
-  P.use_bvh = r->small_scene ? 0 : 1;
-  P.scene_class = r->scene_class;
-  if (r->small_scene) {
-    static_assert(sizeof(r->k.light_tab) == sizeof(P.k_light_tab) && sizeof(r->k.lights) == sizeof(P.k_lights), "table layout");
-    memcpy(P.k_light_tab, r->k.light_tab, sizeof(P.k_light_tab));
-    memcpy(P.k_cull_sph, r->k.cull_sph, sizeof(P.k_cull_sph));
-    memcpy(P.k_cull_pl, r->k.cull_pl, sizeof(P.k_cull_pl));
-    memcpy(P.k_lights, r->k.lights, sizeof(P.k_lights));
-    memcpy(P.k_lights_f, r->k.lights_f, sizeof(P.k_lights_f));
-    memcpy(P.k_pl_index, r->k.pl_index, sizeof(P.k_pl_index));
-    P.k_has_light_tab = r->k.has_light_tab;
-  }
-  P.light_tab = r->light_tab.p;  // nullptr unless the scene uses the linear filter
-  P.cam_tab_valid = 0;
+  fill_scene_params(r, P);
   if (!P.use_bvh && r->n_sph > 0 && r->n_sph <= RTRB_APEX_MAX) {
     const double cm = fmax(fabs(cam->position[0]), fmax(fabs(cam->position[1]), fabs(cam->position[2])));
     for (int k = 0; k < r->n_sph; ++k)
@@ -820,11 +849,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   P.lens_sx = r->lens_tab.p; P.lens_sy = r->lens_tab.p + W;
   P.samples = need_samples ? r->samples.p : nullptr; P.rgb = tg.rgb; P.hit = tg.hit; P.rgba = tg.rgba;
   P.pre_avg = r->pre_avg.p;
-  P.counters = fc.d.p; P.first_bad = fc.d.p + RTRB_CNT_N;
-  P.work_counter = fc.d.p + RTRB_CNT_N + 1;
-  P.status = reinterpret_cast<uint32_t*>(fc.d.p + RTRB_CNT_N + 3);
-  P.extra_count = reinterpret_cast<uint32_t*>(fc.d.p + RTRB_CNT_N + 4);
-  P.hot = fc.d.p + RTRB_CNT_N + 5;
+  bind_ctl(P, fc);
   P.tiles_magic = (world == 1 && x0 == 0 && y0 == 0 && x1 == W && y1 == H) ? r->tiles_magic : 0u;
   P.extra_list = r->extra_list.p; P.extra_samples = r->extra_samples.p;
   // the Box code lives only in the full-counter kernel variants (rtrb_trace.cuh, trace_dispatch)
@@ -1048,6 +1073,71 @@ int submit_finish(rtrb_renderer* r, FrameCtl& fc, int* ticket_out) {
   return RTRB_OK;
 }
 
+// ---- ray-level calls ---------------------------------------------------------------------------------------------
+// Checks every ray call makes before it needs a device.
+int ray_args(const rtrb_ray_opts* opts, int n) {
+  if (!opts) return fail(RTRB_ERR_INVALID, "opts is NULL");
+  if (n < 0) return fail(RTRB_ERR_INVALID, "n = %d < 0", n);
+  if (opts->precision != RTRB_PREC_STRICT && opts->precision != RTRB_PREC_FAST64)
+    return fail(RTRB_ERR_INVALID, "unknown precision mode %d", opts->precision);
+  if (opts->device_buffers != 0 && opts->device_buffers != 1)
+    return fail(RTRB_ERR_INVALID, "device_buffers must be 0 or 1, not %d", opts->device_buffers);
+  return RTRB_OK;
+}
+
+// No device: RTRB_ERR_CUDA, as every computing entry point.  Otherwise selects the renderer's device and sets up the
+// ray calls' own control block on first use.
+int ray_device(rtrb_renderer* r) {
+  int n = 0;
+  cudaError_t e = cudaGetDeviceCount(&n);
+  if (e != cudaSuccess || n == 0) {
+    cudaGetLastError();
+    return fail(RTRB_ERR_CUDA, "no CUDA device (%s); this library has no CPU fallback", cudaGetErrorString(e));
+  }
+  if (!r) return fail(RTRB_ERR_INVALID, "renderer is NULL");
+  CUDA_TRY(cudaSetDevice(r->device));
+  if (!r->ray_ready) {
+    e = (cudaError_t)r->ray_ctl.init();
+    if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "ray control block init failed: %s", cudaGetErrorString(e));
+    r->ray_ready = true;
+  }
+  return RTRB_OK;
+}
+
+// device_buffers = 1: `p` (if not NULL) must be device memory of the renderer's device.
+int check_device_ptr(const rtrb_renderer* r, const void* p, const char* what) {
+  if (!p) return RTRB_OK;
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(RTRB_ERR_INVALID, "%s is not a device pointer", what);
+  }
+  if (a.type != cudaMemoryTypeDevice || a.device != r->device)
+    return fail(RTRB_ERR_INVALID, "%s is not device memory of the renderer's device %d", what, r->device);
+  return RTRB_OK;
+}
+
+// Host-buffer calls stage their k arrays of bytes[i] bytes (0 = absent: nullptr) in ray_scratch.
+int ray_stage(rtrb_renderer* r, const size_t* bytes, int k, uint8_t** out) {
+  size_t off[8], total = 0;
+  for (int i = 0; i < k; ++i) { off[i] = total; total += (bytes[i] + 255) & ~(size_t)255; }
+  if (total > RTRB_RAY_SCRATCH_BUDGET)
+    return fail(RTRB_ERR_UNSUPPORTED, "the call needs %zu bytes of device scratch, more than RTRB_RAY_SCRATCH_BUDGET (%zu); "
+                                      "split it or pass device buffers", total, RTRB_RAY_SCRATCH_BUDGET);
+  CUDA_TRY(r->ray_scratch.ensure(std::max<size_t>(1, total)));
+  for (int i = 0; i < k; ++i) out[i] = bytes[i] ? r->ray_scratch.p + off[i] : nullptr;
+  return RTRB_OK;
+}
+
+// Copies the ray call's control block back and turns it into stats (RTRB_ERR_RAISED when a ray raised).  Synchronises.
+int ray_finish(rtrb_renderer* r, cudaStream_t s, rtrb_stats* stats_out) {
+  FrameCtl& fc = r->ray_ctl;
+  CUDA_TRY(cudaMemcpyAsync(fc.h, fc.d.p, RTRB_FCB_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  rtrb_stats local;
+  return finish_stats(r, fc, stats_out ? stats_out : &local);
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -1105,6 +1195,7 @@ int rtrb_renderer_destroy(rtrb_renderer* r) {
   r->cull_sph.release(); r->cull_pl.release(); r->sph_index.release(); r->pl_index.release(); r->lights_f.release(); r->tiles.release(); r->samples.release();
   r->extra_samples.release(); r->pre_avg.release(); r->rgb.release(); r->extra_list.release(); r->hit.release(); r->rgba.release();
   r->main_ctl.destroy();
+  r->ray_ctl.destroy(); r->ray_scratch.release(); r->ray_lens.release();
   for (int i = 0; i < RTRB_PIPE_SLOTS; ++i) r->pipe_ctl[i].destroy();
   r->png.release();
   if (r->png_ev) cudaEventDestroy(r->png_ev);
@@ -1439,6 +1530,155 @@ int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int hei
   CUDA_TRY(cudaMemcpyAsync(png_host, r->png.file, total, cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   *bytes_out = (size_t)total;
+  return RTRB_OK;
+}
+
+int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rtrb_ray* rays, const uint32_t* keys_or_null,
+                    double* rgb_out, int32_t* hit_or_null, rtrb_stats* stats_out) {
+  int rc = ray_args(opts, n);
+  if (rc) return rc;
+  if (n > 0 && (!rays || !rgb_out)) return fail(RTRB_ERR_INVALID, "rays / rgb_out is NULL");
+  if (opts->trace_depth < 0 || opts->monte_carlo_diffusion_times < 0) return fail(RTRB_ERR_INVALID, "negative trace_depth / mc");
+  const long long need = (long long)opts->trace_depth * (1 + (long long)opts->monte_carlo_diffusion_times) + 1;
+  if (need > rtrb_max_stack_supported())
+    return fail(RTRB_ERR_UNSUPPORTED, "trace_depth*(1+mc)+1 = %lld exceeds the device stack limit %d", need, rtrb_max_stack_supported());
+  if ((rc = ray_device(r))) return rc;
+  const bool dev = opts->device_buffers == 1;
+  if (dev && ((rc = check_device_ptr(r, rays, "rays")) || (rc = check_device_ptr(r, keys_or_null, "keys")) ||
+              (rc = check_device_ptr(r, rgb_out, "rgb_out")) || (rc = check_device_ptr(r, hit_or_null, "hit"))))
+    return rc;
+  if (stats_out) { memset(stats_out, 0, sizeof(*stats_out)); stats_out->first_bad_x = stats_out->first_bad_y = -1; }
+  if (n == 0) return RTRB_OK;
+  cudaStream_t s = opts->stream ? (cudaStream_t)opts->stream : r->stream;
+  const size_t un = (size_t)n;
+  RayBatch B;
+  memset(&B, 0, sizeof(B));
+  B.n = n;
+  if (dev) {
+    B.rays = (const double*)rays; B.keys = keys_or_null; B.rgb = rgb_out; B.hit = hit_or_null;
+  } else {
+    const size_t bytes[4] = {un * sizeof(rtrb_ray), keys_or_null ? un * 2 * sizeof(uint32_t) : 0, un * 3 * sizeof(double),
+                             hit_or_null ? un * sizeof(int32_t) : 0};
+    uint8_t* p[4];
+    if ((rc = ray_stage(r, bytes, 4, p))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(p[0], rays, bytes[0], cudaMemcpyHostToDevice, s));
+    if (keys_or_null) CUDA_TRY(cudaMemcpyAsync(p[1], keys_or_null, bytes[1], cudaMemcpyHostToDevice, s));
+    B.rays = (const double*)p[0]; B.keys = (const uint32_t*)p[1]; B.rgb = (double*)p[2]; B.hit = (int32_t*)p[3];
+  }
+  FrameParams P;
+  memset(&P, 0, sizeof(P));
+  fill_scene_params(r, P);
+  P.trace_depth = opts->trace_depth; P.mc = opts->monte_carlo_diffusion_times;
+  P.width = 1; P.height = 1;  // status reports ray i as pixel (i, 0)
+  P.key0 = (uint32_t)opts->seed; P.key1 = (uint32_t)(opts->seed >> 32);
+  P.count_detail = (opts->count_detail || r->n_boxes > 0) ? 1 : 0;  // the Box code lives in the detailed kernels
+  FrameCtl& fc = r->ray_ctl;
+  bind_ctl(P, fc);
+  fc.timed = stats_out != nullptr;
+  fc.W = 1; fc.H = 1; fc.S = 1; fc.E = 0; fc.n_tiles = 1; fc.px_count = un; fc.detail = P.count_detail != 0;
+  if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev0, s));
+  CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, RTRB_FCB_WORDS * sizeof(unsigned long long), s));
+  if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
+  CUDA_TRY(rtrb_launch_trace_rays(P, B, opts->precision == RTRB_PREC_STRICT, (int)need, s));
+  g_launches++;
+  if (fc.timed) { CUDA_TRY(cudaEventRecord(fc.evt1, s)); CUDA_TRY(cudaEventRecord(fc.ev1, s)); }
+  if (!dev) {
+    CUDA_TRY(cudaMemcpyAsync(rgb_out, B.rgb, un * 3 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (hit_or_null) CUDA_TRY(cudaMemcpyAsync(hit_or_null, B.hit, un * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    return ray_finish(r, s, stats_out);
+  }
+  return stats_out ? ray_finish(r, s, stats_out) : RTRB_OK;
+}
+
+int rtrb_intersect_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rtrb_ray* rays, rtrb_ray_hit* hits_out) {
+  static_assert(sizeof(rtrb_ray) == 48 && sizeof(rtrb_ray_hit) == 72, "rtrb_ray / rtrb_ray_hit layout");
+  int rc = ray_args(opts, n);
+  if (rc) return rc;
+  if (n > 0 && (!rays || !hits_out)) return fail(RTRB_ERR_INVALID, "rays / hits_out is NULL");
+  if ((rc = ray_device(r))) return rc;
+  const bool dev = opts->device_buffers == 1;
+  if (dev && ((rc = check_device_ptr(r, rays, "rays")) || (rc = check_device_ptr(r, hits_out, "hits_out")))) return rc;
+  if (n == 0) return RTRB_OK;
+  cudaStream_t s = opts->stream ? (cudaStream_t)opts->stream : r->stream;
+  const size_t un = (size_t)n;
+  RayBatch B;
+  memset(&B, 0, sizeof(B));
+  B.n = n;
+  if (dev) {
+    B.rays = (const double*)rays; B.hits = hits_out;
+  } else {
+    const size_t bytes[2] = {un * sizeof(rtrb_ray), un * sizeof(rtrb_ray_hit)};
+    uint8_t* p[2];
+    if ((rc = ray_stage(r, bytes, 2, p))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(p[0], rays, bytes[0], cudaMemcpyHostToDevice, s));
+    B.rays = (const double*)p[0]; B.hits = (rtrb_ray_hit*)p[1];
+  }
+  FrameParams P;
+  memset(&P, 0, sizeof(P));
+  fill_scene_params(r, P);
+  CUDA_TRY(rtrb_launch_intersect_rays(P, B, opts->precision == RTRB_PREC_STRICT, s));
+  g_launches++;
+  if (!dev) {
+    CUDA_TRY(cudaMemcpyAsync(hits_out, B.hits, un * sizeof(rtrb_ray_hit), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+  }
+  return RTRB_OK;
+}
+
+int rtrb_camera_rays(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_ray_opts* opts, int sample_begin,
+                     int sample_end, rtrb_ray* rays_out, uint32_t* keys_or_null) {
+  int rc = ray_args(opts, 0);
+  if (rc) return rc;
+  if (!cam) return fail(RTRB_ERR_INVALID, "camera is NULL");
+  const int W = cam->width, H = cam->height;
+  if (W <= 0 || H <= 0) return fail(RTRB_ERR_INVALID, "bad frame size %dx%d", W, H);
+  int x0 = opts->x0, y0 = opts->y0, x1 = opts->x1, y1 = opts->y1;
+  if (x0 == 0 && y0 == 0 && x1 == 0 && y1 == 0) { x1 = W; y1 = H; }
+  if (x0 < 0 || y0 < 0 || x1 > W || y1 > H || x0 >= x1 || y0 >= y1) return fail(RTRB_ERR_INVALID, "bad window");
+  if (sample_begin < 0 || sample_end <= sample_begin)
+    return fail(RTRB_ERR_INVALID, "empty sample range [%d, %d)", sample_begin, sample_end);
+  if (!rays_out) return fail(RTRB_ERR_INVALID, "rays_out is NULL");
+  const unsigned long long n = (unsigned long long)(x1 - x0) * (unsigned long long)(y1 - y0) * (unsigned long long)(sample_end - sample_begin);
+  if (n > 0x7fffffffull) return fail(RTRB_ERR_UNSUPPORTED, "%llu rays: more than one ray call takes", n);
+  if ((rc = ray_device(r))) return rc;
+  const bool dev = opts->device_buffers == 1;
+  if (dev && ((rc = check_device_ptr(r, rays_out, "rays_out")) || (rc = check_device_ptr(r, keys_or_null, "keys")))) return rc;
+  cudaStream_t s = opts->stream ? (cudaStream_t)opts->stream : r->stream;
+  // lens tables of this camera (the frames' cache is not touched); re-uploaded when the camera's size changes
+  {
+    double lk[4] = {(double)W, (double)H, cam->retina_width, cam->retina_height};
+    if (memcmp(lk, r->ray_lens_key, sizeof(lk)) != 0 || !r->ray_lens.p) {
+      const std::vector<double> tab = lens_table(cam);
+      CUDA_TRY(r->ray_lens.ensure(tab.size()));
+      CUDA_TRY(cudaMemcpyAsync(r->ray_lens.p, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, s));
+      CUDA_TRY(cudaStreamSynchronize(s));
+      memcpy(r->ray_lens_key, lk, sizeof(lk));
+    }
+  }
+  RayBatch B;
+  memset(&B, 0, sizeof(B));
+  B.n = (long long)n; B.sample_begin = sample_begin; B.sample_end = sample_end;
+  if (dev) {
+    B.rays_out = (double*)rays_out; B.keys_out = keys_or_null;
+  } else {
+    const size_t bytes[2] = {(size_t)n * sizeof(rtrb_ray), keys_or_null ? (size_t)n * 2 * sizeof(uint32_t) : 0};
+    uint8_t* p[2];
+    if ((rc = ray_stage(r, bytes, 2, p))) return rc;
+    B.rays_out = (double*)p[0]; B.keys_out = (uint32_t*)p[1];
+  }
+  FrameParams P;
+  memset(&P, 0, sizeof(P));
+  bake_camera(P, cam);
+  P.x0 = x0; P.y0 = y0; P.x1 = x1; P.y1 = y1;
+  P.lens_sx = r->ray_lens.p; P.lens_sy = r->ray_lens.p + W;
+  P.key0 = (uint32_t)opts->seed; P.key1 = (uint32_t)(opts->seed >> 32);
+  CUDA_TRY(rtrb_launch_camera_rays(P, B, s));
+  g_launches++;
+  if (!dev) {
+    CUDA_TRY(cudaMemcpyAsync(rays_out, B.rays_out, (size_t)n * sizeof(rtrb_ray), cudaMemcpyDeviceToHost, s));
+    if (keys_or_null) CUDA_TRY(cudaMemcpyAsync(keys_or_null, B.keys_out, (size_t)n * 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+  }
   return RTRB_OK;
 }
 

@@ -39,6 +39,36 @@ def make_opts(rng_mode=_abi.RNG_CTR, precision=_abi.PREC_DEFAULT, seed=1, window
     return o
 
 
+# numpy view of rtrb_ray_hit (World#intersect's answer for one ray)
+RAY_HIT_DTYPE = np.dtype([("object", "<i4"), ("direction", "<i4"), ("face", "<i4"), ("reserved0", "<i4"),
+                          ("distance", "<f8"), ("intersection", "<f8", (3,)), ("delta", "<f8", (3,))])
+assert RAY_HIT_DTYPE.itemsize == C.sizeof(_abi.RayHit)
+
+
+def make_ray_opts(precision=_abi.PREC_DEFAULT, seed=1, trace_depth=1, mc=0, count_detail=False, window=None,
+                  device_buffers=False, stream=None):
+    o = _abi.RayOpts()
+    o.precision, o.seed = precision, seed
+    o.trace_depth, o.monte_carlo_diffusion_times = trace_depth, mc
+    o.count_detail = 1 if count_detail else 0
+    if window:
+        o.x0, o.y0, o.x1, o.y1 = window
+    o.device_buffers = 1 if device_buffers else 0
+    o.stream = stream
+    return o
+
+
+def _is_tensor(x):
+    return type(x).__module__.startswith("torch")
+
+
+def _torch_stream(device):
+    """torch.cuda.current_stream(device) as a cudaStream_t for the C ABI.  torch reports its default stream as 0, which
+    the ABI reads as "the renderer's own stream"; the legacy default stream's handle is cudaStreamLegacy (0x1)."""
+    import torch
+    return torch.cuda.current_stream(device).cuda_stream or 1
+
+
 class Renderer:
     def __init__(self, scene, device=0):
         self._scene = scene  # SceneDescHolder; only needed during create, kept for introspection
@@ -138,6 +168,91 @@ class Renderer:
         stats, code = self.wait(ticket)
         del self._png_pending[ticket]
         return out[:n.value].tobytes(), stats, code
+
+    # -- ray-level queries (rtrb_trace_rays / rtrb_intersect_rays / rtrb_camera_rays) ----------------------------------
+    # Rays are [n, 6] float64 rows (position, front).  numpy arrays take the blocking host-buffer path; CUDA torch
+    # tensors on this renderer's device take the device-buffer path on torch.cuda.current_stream() and give torch outputs.
+    def _device_rays(self, rays):
+        import torch
+        if not rays.is_cuda or rays.device.index != self.device:
+            raise ValueError("ray tensors must live on cuda:%d" % self.device)
+        return rays.to(torch.float64).reshape(-1, 6).contiguous(), _torch_stream(self.device)
+
+    def trace_rays(self, rays, trace_depth=1, mc=0, seed=1, keys=None, precision=_abi.PREC_DEFAULT, count_detail=False,
+                   want_stats=True):
+        """RayTracer#trace_sync on every ray -> (rgb [n, 3] float64, hit [n] int32, stats dict or None, status code).
+        keys: [n, 2] (pixel, sample) Philox keys of the Monte-Carlo rays; None keys ray i as (i, 0).  On the device
+        path the call synchronises only when want_stats (stats is None otherwise)."""
+        st = _abi.Stats()
+        if _is_tensor(rays):
+            import torch
+            rays, stream = self._device_rays(rays)
+            n = rays.shape[0]
+            if keys is not None:
+                keys = keys.reshape(-1, 2).to(device=rays.device, dtype=torch.int32).contiguous()
+                assert keys.shape[0] == n
+            rgb = torch.empty((n, 3), dtype=torch.float64, device=rays.device)
+            hit = torch.empty((n,), dtype=torch.int32, device=rays.device)
+            opts = make_ray_opts(precision, seed, trace_depth, mc, count_detail, device_buffers=True, stream=stream)
+            code = lib().rtrb_trace_rays(self._h, C.byref(opts), n, rays.data_ptr(), keys.data_ptr() if keys is not None else None,
+                                         rgb.data_ptr(), hit.data_ptr(), C.byref(st) if want_stats else None)
+        else:
+            rays = np.ascontiguousarray(rays, np.float64).reshape(-1, 6)
+            n = rays.shape[0]
+            if keys is not None:
+                keys = np.ascontiguousarray(keys, np.uint32).reshape(-1, 2)
+                assert keys.shape[0] == n
+            rgb = np.empty((n, 3), np.float64)
+            hit = np.empty((n,), np.int32)
+            opts = make_ray_opts(precision, seed, trace_depth, mc, count_detail)
+            code = lib().rtrb_trace_rays(self._h, C.byref(opts), n, rays.ctypes.data, keys.ctypes.data if keys is not None else None,
+                                         rgb.ctypes.data, hit.ctypes.data, C.byref(st))
+            want_stats = True
+        check(code, allow_raised=True)
+        return rgb, hit, (st.as_dict() if want_stats else None), code
+
+    def intersect_rays(self, rays, precision=_abi.PREC_DEFAULT):
+        """World#intersect on every ray.  numpy input -> structured array of RAY_HIT_DTYPE; torch input -> dict of
+        tensors (object, direction, face int32; distance float64; intersection, delta [n, 3] float64) that view one
+        [n, 9] float64 buffer of rtrb_ray_hit records."""
+        if _is_tensor(rays):
+            import torch
+            rays, stream = self._device_rays(rays)
+            n = rays.shape[0]
+            raw = torch.empty((n, 9), dtype=torch.float64, device=rays.device)
+            opts = make_ray_opts(precision, device_buffers=True, stream=stream)
+            check(lib().rtrb_intersect_rays(self._h, C.byref(opts), n, rays.data_ptr(), raw.data_ptr()))
+            ints = raw[:, :2].view(torch.int32)
+            return {"object": ints[:, 0], "direction": ints[:, 1], "face": ints[:, 2], "distance": raw[:, 2],
+                    "intersection": raw[:, 3:6], "delta": raw[:, 6:9], "raw": raw}
+        rays = np.ascontiguousarray(rays, np.float64).reshape(-1, 6)
+        out = np.empty(rays.shape[0], RAY_HIT_DTYPE)
+        opts = make_ray_opts(precision)
+        check(lib().rtrb_intersect_rays(self._h, C.byref(opts), rays.shape[0], rays.ctypes.data, out.ctypes.data))
+        return out
+
+    def camera_rays(self, cam, seed=1, window=None, samples=None, device_buffers=False):
+        """Camera#lens_func for every pixel of `window` (x0, y0, x1, y1; None = the whole frame) and every sample j in
+        `samples` = (begin, end) (None = the pre samples, (0, pre_sample_times)) -> (rays [n, 6], keys [n, 2]); ray
+        (x, y, j) is row ((y - y0) * (x1 - x0) + (x - x0)) * (end - begin) + (j - begin) and its key is (y * W + x, j).
+        numpy arrays (keys uint32), or with device_buffers torch tensors on this renderer's device (keys int32)."""
+        b, e = samples if samples is not None else (0, cam.pre_sample_times)
+        x0, y0, x1, y1 = window if window else (0, 0, cam.width, cam.height)
+        n = max(0, x1 - x0) * max(0, y1 - y0) * max(0, e - b)
+        if device_buffers:
+            import torch
+            dev = torch.device("cuda", self.device)
+            rays = torch.empty((n, 6), dtype=torch.float64, device=dev)
+            keys = torch.empty((n, 2), dtype=torch.int32, device=dev)
+            opts = make_ray_opts(seed=seed, window=window, device_buffers=True,
+                                 stream=_torch_stream(self.device))
+            check(lib().rtrb_camera_rays(self._h, C.byref(cam), C.byref(opts), b, e, rays.data_ptr(), keys.data_ptr()))
+            return rays, keys
+        rays = np.empty((n, 6), np.float64)
+        keys = np.empty((n, 2), np.uint32)
+        opts = make_ray_opts(seed=seed, window=window)
+        check(lib().rtrb_camera_rays(self._h, C.byref(cam), C.byref(opts), b, e, rays.ctypes.data, keys.ctypes.data))
+        return rays, keys
 
     def peer_push(self, src_ptr, dst_peer_ptr, nbytes, after_stream=None):
         """Copy-engine gather: queue a D2D copy to a peer mapping behind `after_stream` (see rtrb_peer_push)."""

@@ -1,7 +1,10 @@
 """Mirror of Alex::World (reference src/world.rb:10-34): YAML -> objects + lights.  The scene
 queries World#intersect / lit_area / local_lights / high_lights (:37-98) are device code; this
-class only builds the flat scene description handed to rtrb_renderer_create."""
+class builds the flat scene description handed to rtrb_renderer_create, and World#intersect is reachable on its own
+through `intersect` / `intersect_batch` (rtrb_intersect_rays)."""
 import ctypes as C
+
+from .vec3 import Vec3
 
 from . import _abi
 from .configurable_object import ConfigurableObject
@@ -26,6 +29,28 @@ class World(ConfigurableObject):
         super().__init__(config_file)
         self.world_objects = self.parse_objects(self.world_objects)  # world.rb:17
         self.lights = self.parse_lights(self.lights)                  # world.rb:18
+
+    def renderer(self, device=0):
+        """The scene baked on `device` for ray-level queries (one per device, made on first use)."""
+        rs = self.__dict__.setdefault("_renderers", {})
+        if device not in rs:
+            from .renderer import Renderer
+            rs[device] = Renderer(self.to_scene_desc(), device)
+        return rs[device]
+
+    def intersect_batch(self, rays, precision=_abi.PREC_DEFAULT, device=0):
+        """World#intersect on many rays (Ray objects or [n, 6] rows of position, front) -> RAY_HIT_DTYPE array."""
+        from .ray_tracer import rays_array
+        return self.renderer(device).intersect_rays(rays_array(rays), precision)
+
+    def intersect(self, ray, precision=_abi.PREC_DEFAULT, device=0):
+        """world.rb:37-59 -> (object, intersection, direction, delta) as the reference returns them: the winning world
+        object, Vec3, "in" / "out", Vec3; four Nones on a miss."""
+        h = self.intersect_batch([ray], precision, device)[0]
+        if h["object"] < 0:
+            return None, None, None, None
+        return (self.world_objects[int(h["object"])], Vec3(*[float(v) for v in h["intersection"]]),
+                "in" if h["direction"] else "out", Vec3(*[float(v) for v in h["delta"]]))
 
     def parse_lights(self, array):  # world.rb:21-27
         ret = []
