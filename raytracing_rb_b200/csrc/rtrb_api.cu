@@ -12,6 +12,7 @@
 #include <string.h>
 
 #include <atomic>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -106,59 +107,220 @@ struct HostMT {
   }
 };
 
-template <typename T>
-struct DevBuf {
-  T* p = nullptr;
-  size_t n = 0;
-  cudaError_t ensure(size_t want) {
-    if (want <= n && p) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr; n = 0;
-    if (want == 0) return cudaSuccess;
-    cudaError_t e = cudaMalloc((void**)&p, want * sizeof(T));
-    if (e == cudaSuccess) n = want;
-    return e;
-  }
-  void release() { if (p) cudaFree(p); p = nullptr; n = 0; }
+// Frame control block: every small per-frame device word in ONE buffer (one memset, one D2H copy).  The kernels
+// reach its fields through FrameParams (bind_ctl).
+struct CtlBlock {
+  unsigned long long counters[RTRB_CNT_N];      // RTRB_CNT_*
+  unsigned long long first_bad;                 // max over flagged pixels of ~(x * H + y), 0 = none
+  unsigned long long work[2];                   // work-claim counters
+  uint32_t status, max_stack;
+  uint32_t extra_count, pad;
+  unsigned long long hot[2 * RTRB_HOT_SLICES];  // sliced (rays, shadow) counters
+};
+static_assert(sizeof(CtlBlock) == (RTRB_CNT_N + 5 + 2 * RTRB_HOT_SLICES) * 8, "control block layout");
+
+// Pinned host mirror of a control block, mapped into the device's address space.
+struct CtlMirror {
+  CtlBlock blk;
+  unsigned long long png_bytes;  // rtrb_submit_png frames: the file size, stored by the encoder
 };
 
-}  // namespace
-
-// Frame control block: every small per-frame device word in ONE buffer (one memset, one D2H copy).
-// u64 words: [0, RTRB_CNT_N) counters | [N] first_bad | [N+1, N+2] work claims | [N+3] = {status, max_stack}
-// | [N+4] = {extra_count, pad} | [N+5, N+5+2*RTRB_HOT_SLICES) sliced (rays, shadow) counters
-#define RTRB_FCB_WORDS (RTRB_CNT_N + 5 + 2 * RTRB_HOT_SLICES)
 #define RTRB_PIPE_SLOTS 4  // frames that may be in flight between rtrb_submit and rtrb_wait
 struct FrameCtl {
-  DevBuf<unsigned long long> d;
-  unsigned long long* h = nullptr;  // pinned host mirror (mapped into the device's address space)
-  unsigned long long* h_dev = nullptr;  // ... and the address the device stores to (publish_ctl_kernel)
+  DevBuf<CtlBlock> d;
+  CtlMirror* h = nullptr;      // pinned host mirror
+  CtlMirror* h_dev = nullptr;  // ... and the address the device stores to (publish_ctl_kernel)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, evt0 = nullptr, evt1 = nullptr, copied = nullptr, ctl_copied = nullptr;
   DevBuf<uint8_t> rgba;             // pipeline slots own a framebuffer; the main slot uses rtrb_renderer::rgba
-  size_t* png_bytes_out = nullptr;  // rtrb_submit_png frames: where rtrb_wait stores h[RTRB_FCB_WORDS], the file size
+  size_t* png_bytes_out = nullptr;  // rtrb_submit_png frames: where rtrb_wait stores h->png_bytes
   // facts of the frame in flight, needed to finish its stats later
   int W = 0, H = 0, S = 0, E = 0, n_tiles = 0;
   bool detail = false, in_flight = false, timed = false;
   unsigned ticket = 0;              // the rtrb_submit ticket occupying this slot while in_flight
   size_t px_count = 0;
-  int init() {
+  // Allocates on first use, so that slots a renderer never uses cost nothing.
+  cudaError_t init() {
     cudaError_t e;
-    if ((e = d.ensure(RTRB_FCB_WORDS)) != cudaSuccess) return (int)e;
-    if ((e = cudaHostAlloc((void**)&h, (RTRB_FCB_WORDS + 1) * sizeof(unsigned long long), cudaHostAllocMapped)) != cudaSuccess) return (int)e;
-    if ((e = cudaHostGetDevicePointer((void**)&h_dev, h, 0)) != cudaSuccess) return (int)e;
-    cudaEvent_t* evs[6] = {&ev0, &ev1, &evt0, &evt1, &copied, &ctl_copied};
-    for (auto ev : evs)
-      if ((e = cudaEventCreate(ev)) != cudaSuccess) return (int)e;
-    return 0;
+    if ((e = d.ensure(1)) != cudaSuccess) return e;
+    if ((e = cudaHostAlloc((void**)&h, sizeof(CtlMirror), cudaHostAllocMapped)) != cudaSuccess) return e;
+    if ((e = cudaHostGetDevicePointer((void**)&h_dev, h, 0)) != cudaSuccess) return e;
+    for (cudaEvent_t* ev : {&ev0, &ev1, &evt0, &evt1, &copied, &ctl_copied})
+      if ((e = cudaEventCreate(ev)) != cudaSuccess) return e;
+    return cudaSuccess;
   }
-  void destroy() {
-    d.release(); rgba.release();
+  ~FrameCtl() {
     if (h) cudaFreeHost(h);
-    h = nullptr; h_dev = nullptr;
-    cudaEvent_t* evs[6] = {&ev0, &ev1, &evt0, &evt1, &copied, &ctl_copied};
-    for (auto ev : evs) { if (*ev) cudaEventDestroy(*ev); *ev = nullptr; }
+    for (cudaEvent_t ev : {ev0, ev1, evt0, evt1, copied, ctl_copied})
+      if (ev) cudaEventDestroy(ev);
   }
 };
+
+// The per-column / per-row scalars of camera.rb:133-134 in the reference's order: [W] x offsets, then [H] y offsets.
+std::vector<double> lens_table(const rtrb_camera_desc* cam) {
+  const int W = cam->width, H = cam->height;
+  std::vector<double> tab((size_t)W + H);
+  for (int x = 0; x < W; ++x) tab[x] = 2.0 * ((double)x / W - 0.5) * cam->retina_width;
+  for (int y = 0; y < H; ++y) tab[(size_t)W + y] = 2 * ((double)y / H - 0.5) * cam->retina_height;
+  return tab;
+}
+
+// Lens tables on the device (cached): evaluated on the host in the reference's order so the device does two loads
+// instead of two FP64 divisions per sample.
+struct LensTable {
+  DevBuf<double> tab;            // [W + H] per-column / per-row retina offsets
+  double key[4] = {0, 0, 0, 0};  // (W, H, retina_width, retina_height) the table was built for
+  int ensure(const rtrb_camera_desc* cam, cudaStream_t s) {
+    const double k[4] = {(double)cam->width, (double)cam->height, cam->retina_width, cam->retina_height};
+    if (memcmp(k, key, sizeof(k)) == 0 && tab.p) return RTRB_OK;
+    const std::vector<double> t = lens_table(cam);
+    CUDA_TRY(tab.ensure(t.size()));
+    CUDA_TRY(cudaMemcpyAsync(tab.p, t.data(), t.size() * sizeof(double), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    memcpy(key, k, sizeof(k));
+    return RTRB_OK;
+  }
+};
+
+// A window of a W x H frame, and the share of its super-tiles one rank renders.
+struct Window {
+  int x0, y0, x1, y1, rank, world;
+  bool whole;  // the whole frame on one rank
+};
+
+// {0, 0, 0, 0} is the whole frame; tile_world <= 1 is one rank.
+int make_window(int W, int H, int x0, int y0, int x1, int y1, int tile_rank, int tile_world, Window& w) {
+  if (x0 == 0 && y0 == 0 && x1 == 0 && y1 == 0) { x1 = W; y1 = H; }
+  if (x0 < 0 || y0 < 0 || x1 > W || y1 > H || x0 >= x1 || y0 >= y1) return fail(RTRB_ERR_INVALID, "bad window");
+  const int world = tile_world <= 1 ? 1 : tile_world, rank = world == 1 ? 0 : tile_rank;
+  if (rank < 0 || rank >= world) return fail(RTRB_ERR_INVALID, "tile_rank %d outside tile_world %d", rank, world);
+  w = Window{x0, y0, x1, y1, rank, world, x0 == 0 && y0 == 0 && x1 == W && y1 == H && world == 1};
+  return RTRB_OK;
+}
+
+void enumerate_tiles(int W, const Window& w, std::vector<int32_t>& out) {
+  const int stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER;
+  out.clear();
+  // deal the window's super-tiles round-robin in row-major order: shares differ by at most one tile
+  int i = 0;
+  for (int ty = w.y0 / RTRB_SUPER; ty <= (w.y1 - 1) / RTRB_SUPER; ++ty)
+    for (int tx = w.x0 / RTRB_SUPER; tx <= (w.x1 - 1) / RTRB_SUPER; ++tx, ++i)
+      if (i % w.world == w.rank) out.push_back(ty * stx_count + tx);
+}
+
+// The super-tiles of a window that one rank renders (cached: rebuilt when the frame size, window or partition changes).
+struct TileList {
+  DevBuf<int32_t> dev;             // packed tx | ty << 16
+  std::vector<int32_t> host;       // global ids ty * stx_count + tx
+  size_t px_count = 0;             // pixels of the window covered by host
+  uint32_t magic = 0;              // see FrameParams::tiles_magic (0 when the list is not plain row-major)
+  int key[8] = {-1, -1, -1, -1, -1, -1, -1, -1};
+  int ensure(int W, int H, const Window& w, cudaStream_t s) {
+    const int k[8] = {W, H, w.x0, w.y0, w.x1, w.y1, w.rank, w.world};
+    if (memcmp(k, key, sizeof(k)) == 0) return RTRB_OK;
+    const int stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER;
+    enumerate_tiles(W, w, host);
+    std::vector<int32_t> packed(host.size());
+    for (size_t i = 0; i < packed.size(); ++i) packed[i] = (host[i] % stx_count) | ((host[i] / stx_count) << 16);
+    CUDA_TRY(dev.ensure(std::max<size_t>(1, packed.size())));
+    if (!packed.empty())
+      CUDA_TRY(cudaMemcpyAsync(dev.p, packed.data(), packed.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    memcpy(key, k, sizeof(k));
+    magic = 0;
+    if (stx_count > 0 && stx_count < 65536 && host.size() < 65536) {
+      const uint32_t m = (uint32_t)((1ull << 32) / (unsigned)stx_count) + 1u;
+      bool ok = true;
+      for (size_t i = 0; i < host.size() && ok; ++i) {
+        const uint32_t ty = (uint32_t)(((unsigned long long)i * m) >> 32);
+        ok = host[i] == (int32_t)i && ty == (uint32_t)i / (unsigned)stx_count;
+      }
+      if (ok) magic = m;
+    }
+    px_count = 0;
+    for (int b : host) {
+      int tx = b % stx_count, ty = b / stx_count;
+      int ax0 = std::max(w.x0, tx * RTRB_SUPER), ax1 = std::min(w.x1, (tx + 1) * RTRB_SUPER);
+      int ay0 = std::max(w.y0, ty * RTRB_SUPER), ay1 = std::min(w.y1, (ty + 1) * RTRB_SUPER);
+      if (ax1 > ax0 && ay1 > ay0) px_count += (size_t)(ax1 - ax0) * (ay1 - ay0);
+    }
+    return RTRB_OK;
+  }
+};
+
+// RTRB_RNG_MT validation mode: serial by construction (every pixel's first draw depends on how many draws all earlier
+// pixels made), so the frame iterates to a fixed point of its per-pixel draw offsets.
+struct MtState {
+  DevBuf<double> draws;
+  DevBuf<uint32_t> offset, count;
+  std::vector<double> host;        // the first host.size() draws after init_genrand(seed)
+  HostMT gen;
+  uint64_t seed = ~0ull;
+  size_t uploaded = 0;
+  int iterations = 0;              // iterations the last MT frame needed to reach its fixed point
+
+  // Offsets = exclusive prefix sums of the per-pixel draw counts, iterated until stable.  The first pixel whose offset
+  // is wrong is right after the next pass (its predecessors no longer move), so the loop ends after at most one pass
+  // per pixel; in practice a handful of passes per data-dependent pixel.
+  int trace(FrameParams& P, FrameCtl& fc, uint64_t frame_seed, int stack_need, cudaStream_t s) {
+    const int S = P.pre;
+    const size_t npx = (size_t)(P.x1 - P.x0) * (size_t)(P.y1 - P.y0);
+    if (npx * (size_t)std::max(S, P.max_samples) > 0x3fffffffull) return fail(RTRB_ERR_UNSUPPORTED, "window too large for RTRB_RNG_MT");
+    CUDA_TRY(offset.ensure(npx));
+    CUDA_TRY(count.ensure(npx));
+    std::vector<uint32_t> off(npx), cnt(npx), nxt(npx);
+    for (size_t i = 0; i < npx; ++i) off[i] = (uint32_t)(i * (size_t)S);
+    if (seed != frame_seed) {
+      host.clear(); gen.seed((uint32_t)frame_seed); seed = frame_seed; uploaded = 0;
+    }
+    size_t want_len = npx * (size_t)(S + 1) + 4096;
+    const int max_iter = 200000;
+    int it = 0;
+    for (;; ++it) {
+      if (it >= max_iter) return fail(RTRB_ERR_UNSUPPORTED, "RTRB_RNG_MT did not reach its fixed point in %d passes", max_iter);
+      if (host.size() < want_len) {
+        host.reserve(want_len);
+        while (host.size() < want_len) host.push_back(gen.res53());
+      }
+      if (uploaded < host.size()) {
+        CUDA_TRY(draws.ensure(host.size()));
+        CUDA_TRY(cudaMemcpyAsync(draws.p, host.data(), host.size() * sizeof(double), cudaMemcpyHostToDevice, s));
+        uploaded = host.size();
+      }
+      P.mt_stream = draws.p; P.mt_len = (uint32_t)std::min<size_t>(host.size(), 0xfffffff0u);
+      P.mt_offset = offset.p; P.mt_count = count.p;
+      CUDA_TRY(cudaMemcpyAsync(offset.p, off.data(), npx * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+      CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, sizeof(CtlBlock), s));
+      if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
+      CUDA_TRY(rtrb_launch_trace_mt_strict(P, stack_need, s));
+      if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt1, s));
+      g_launches++;
+      CUDA_TRY(cudaMemcpyAsync(cnt.data(), count.p, npx * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+      CUDA_TRY(cudaStreamSynchronize(s));
+      bool overflow = false;
+      for (size_t i = 0; i < npx && !overflow; ++i) overflow = cnt[i] == 0xFFFFFFFFu;
+      if (overflow) {  // some pixel ran past the end of the stream: generate more and repeat the pass
+        want_len = host.size() * 2;
+        if (want_len > 0xfffffff0ull) return fail(RTRB_ERR_UNSUPPORTED, "RTRB_RNG_MT stream would exceed 2^32 draws");
+        continue;
+      }
+      size_t acc = 0;
+      bool same = true;
+      for (size_t i = 0; i < npx; ++i) {
+        nxt[i] = (uint32_t)acc;
+        same = same && nxt[i] == off[i];
+        acc += cnt[i];
+      }
+      if (acc > 0xfffffff0ull) return fail(RTRB_ERR_UNSUPPORTED, "RTRB_RNG_MT stream would exceed 2^32 draws");
+      if (same) break;
+      off.swap(nxt);
+      want_len = std::max(want_len, acc + 4096);
+    }
+    iterations = it + 1;
+    return RTRB_OK;
+  }
+};
+
+}  // namespace
 
 struct rtrb_renderer {
   int device = 0;
@@ -198,25 +360,13 @@ struct rtrb_renderer {
   DevBuf<DevLightF> lights_f;
   int n_sph = 0, n_pl = 0;
   float m_scene = 0.0f, max_distance_f = 0.0f;
-  std::vector<uint8_t*> textures;
-  // per-frame scratch
-  DevBuf<int32_t> tiles;
-  std::vector<int32_t> tiles_host;     // global ids ty * stx_count + tx
-  size_t tiles_px_count = 0;           // pixels of the window covered by tiles_host
-  uint32_t tiles_magic = 0;            // see FrameParams::tiles_magic (0 when the list is not plain row-major)
-  DevBuf<double> lens_tab;             // [W + H] per-column / per-row retina offsets
-  double lens_key[4] = {0, 0, 0, 0};   // (W, H, retina_width, retina_height) the table was built for
-  int tiles_key[8] = {-1, -1, -1, -1, -1, -1, -1, -1};
+  std::vector<DevBuf<uint8_t>> textures;  // DevMat::tex holds their addresses
+  // per-frame caches and scratch
+  TileList tiles;
+  LensTable lens;
   DevBuf<double> samples, extra_samples, pre_avg, rgb;
   DevBuf<uint32_t> extra_list;
-  // RTRB_RNG_MT validation mode
-  DevBuf<double> mt_stream;
-  DevBuf<uint32_t> mt_offset, mt_count;
-  std::vector<double> mt_host;         // the first mt_host.size() draws after init_genrand(mt_seed)
-  HostMT mt_gen;
-  uint64_t mt_seed = ~0ull;
-  size_t mt_uploaded = 0;
-  int mt_iterations = 0;               // iterations the last MT frame needed to reach its fixed point
+  MtState mt;
   DevBuf<int32_t> hit;
   DevBuf<uint8_t> rgba;
   bool fb_exported = false;            // its address / IPC handle has been handed out: it may no longer move
@@ -226,30 +376,31 @@ struct rtrb_renderer {
   bool last_has_rgb = false, last_has_hit = false, last_rgba_own = true;
   int last_format = RTRB_FMT_RGBA8;
   cudaStream_t last_stream = nullptr;
-  bool timing_valid = false;
-  // ray-level calls (rtrb_trace_rays & co.): their own control block and scratch, never the frames'
+  // ray-level calls (rtrb_trace_rays & co.): their own control block, scratch and lens tables, never the frames'
   FrameCtl ray_ctl;
   bool ray_ready = false;
   DevBuf<uint8_t> ray_scratch;         // host-buffer calls: inputs and outputs staged on the device
-  DevBuf<double> ray_lens;             // rtrb_camera_rays: lens tables
-  double ray_lens_key[4] = {0, 0, 0, 0};  // (W, H, retina_width, retina_height) ray_lens was built for
+  LensTable ray_lens;                  // rtrb_camera_rays
+  // The members free their own device memory; the renderer's device must be current (rtrb_renderer_destroy).
+  ~rtrb_renderer() {
+    for (cudaEvent_t ev : {push_ev, push_done_ev, png_ev})
+      if (ev) cudaEventDestroy(ev);
+    for (cudaStream_t s : {stream, copy_stream})
+      if (s) cudaStreamDestroy(s);
+  }
 };
 
 namespace {
 
 // ---- resolve kernels ---------------------------------------------------------------------------
-using rtrb::write_pixel;
-
-__device__ __forceinline__ bool slot_to_xy(const FrameParams& P, uint32_t slot, int& x, int& y) {
-  return rtrb::decode_pixel(P, slot, x, y);
-}
-
+using rtrb::decode_pixel;
 using rtrb::pre_mean;
+using rtrb::write_pixel;
 
 __global__ void __launch_bounds__(256) resolve_kernel(const __grid_constant__ FrameParams P) {
   const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
   int x = 0, y = 0;
-  const bool valid = slot < (uint32_t)P.n_tiles * RTRB_SUPER_PIXELS && slot_to_xy(P, slot, x, y);
+  const bool valid = slot < (uint32_t)P.n_tiles * RTRB_SUPER_PIXELS && decode_pixel(P, slot, x, y);
   double ax = 0, ay = 0, az = 0, variance = 0;
   if (valid) pre_mean(P, slot, ax, ay, az, variance);
   const bool adaptive = valid && variance >= P.variant_threshold;
@@ -286,7 +437,7 @@ __global__ void __launch_bounds__(256) resolve_extra_kernel(const __grid_constan
   for (uint32_t e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
     const uint32_t slot = P.extra_list[e];
     int x, y;
-    if (!slot_to_xy(P, slot, x, y)) continue;
+    if (!decode_pixel(P, slot, x, y)) continue;
     double ax, ay, az, variance;
     if (P.fuse_resolve == 2) { ax = P.pre_avg[(size_t)e * 3]; ay = P.pre_avg[(size_t)e * 3 + 1]; az = P.pre_avg[(size_t)e * 3 + 2]; }
     else pre_mean(P, slot, ax, ay, az, variance);
@@ -329,19 +480,21 @@ int measure_fma(int device, double* tflops_out) {
   CUDA_TRY(cudaSetDevice(device));
   int sms = 0;
   CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-  T* d = nullptr;
-  CUDA_TRY(cudaMalloc((void**)&d, sizeof(T)));
+  DevBuf<T> d;
+  CUDA_TRY(d.ensure(1));
   cudaEvent_t e0, e1;
   CUDA_TRY(cudaEventCreate(&e0));
+  std::unique_ptr<CUevent_st, decltype(&cudaEventDestroy)> own_e0(e0, cudaEventDestroy);
   CUDA_TRY(cudaEventCreate(&e1));
+  std::unique_ptr<CUevent_st, decltype(&cudaEventDestroy)> own_e1(e1, cudaEventDestroy);
   const int blocks = sms * 8, threads = 256, iters = 4096;
-  fma_peak_kernel<T><<<blocks, threads>>>(d, 64, (T)1.0000001, (T)1e-9);  // warm-up
+  fma_peak_kernel<T><<<blocks, threads>>>(d.p, 64, (T)1.0000001, (T)1e-9);  // warm-up
   g_launches++;
   CUDA_TRY(cudaDeviceSynchronize());
   double best = 0;
   for (int rep = 0; rep < 5; ++rep) {
     CUDA_TRY(cudaEventRecord(e0));
-    fma_peak_kernel<T><<<blocks, threads>>>(d, iters, (T)1.0000001, (T)1e-9);
+    fma_peak_kernel<T><<<blocks, threads>>>(d.p, iters, (T)1.0000001, (T)1e-9);
     g_launches++;
     CUDA_TRY(cudaEventRecord(e1));
     CUDA_TRY(cudaEventSynchronize(e1));
@@ -351,9 +504,6 @@ int measure_fma(int device, double* tflops_out) {
     double tf = flops / (ms * 1e-3) / 1e12;
     if (tf > best) best = tf;
   }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  cudaFree(d);
   *tflops_out = best;
   return RTRB_OK;
 }
@@ -400,11 +550,10 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
   }
   for (int i = 0; i < s->n_textures; ++i) {
     const rtrb_texture_desc& t = s->textures[i];
-    uint8_t* d = nullptr;
     size_t bytes = (size_t)t.width * t.height * 3;
-    CUDA_TRY(cudaMalloc((void**)&d, bytes));
-    r->textures.push_back(d);
-    CUDA_TRY(cudaMemcpy(d, t.rgb8, bytes, cudaMemcpyHostToDevice));
+    r->textures.emplace_back();
+    CUDA_TRY(r->textures.back().ensure(bytes));
+    CUDA_TRY(cudaMemcpy(r->textures.back().p, t.rgb8, bytes, cudaMemcpyHostToDevice));
   }
   std::vector<DevGeom> geom(s->n_objects);
   std::vector<DevMat> mat(s->n_objects);
@@ -472,7 +621,7 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
     m.hscale = o.texture_horizontal_scale; m.vscale = o.texture_vertical_scale;
     m.uoff = o.texture_u_offset; m.voff = o.texture_v_offset;
     if (o.texture >= 0 && o.type != RTRB_OBJ_BOX) {  // a box never samples its texture (box.rb has no local_lighting)
-      m.tex = r->textures[o.texture];
+      m.tex = r->textures[o.texture].p;
       m.tex_w = s->textures[o.texture].width;
       m.tex_h = s->textures[o.texture].height;
       if (o.type == RTRB_OBJ_SPHERE) {
@@ -627,25 +776,6 @@ void bake_camera(FrameParams& P, const rtrb_camera_desc* c) {
   P.trace_depth = c->trace_depth; P.mc = c->monte_carlo_diffusion_times;
 }
 
-void enumerate_tiles(int W, int x0, int y0, int x1, int y1, int rank, int world, std::vector<int32_t>& out) {
-  const int stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER;
-  out.clear();
-  // deal the window's super-tiles round-robin in row-major order: shares differ by at most one tile
-  int i = 0;
-  for (int ty = y0 / RTRB_SUPER; ty <= (y1 - 1) / RTRB_SUPER; ++ty)
-    for (int tx = x0 / RTRB_SUPER; tx <= (x1 - 1) / RTRB_SUPER; ++tx, ++i)
-      if (i % world == rank) out.push_back(ty * stx_count + tx);
-}
-
-// The per-column / per-row scalars of camera.rb:133-134 in the reference's order: [W] x offsets, then [H] y offsets.
-std::vector<double> lens_table(const rtrb_camera_desc* cam) {
-  const int W = cam->width, H = cam->height;
-  std::vector<double> tab((size_t)W + H);
-  for (int x = 0; x < W; ++x) tab[x] = 2.0 * ((double)x / W - 0.5) * cam->retina_width;
-  for (int y = 0; y < H; ++y) tab[(size_t)W + y] = 2 * ((double)y / H - 0.5) * cam->retina_height;
-  return tab;
-}
-
 // The scene part of FrameParams: baked buffers, FP32 filter view, constant-bank tables of small scenes.  The camera
 // apex table is not part of it (it only holds for rays that start at the camera).
 void fill_scene_params(const rtrb_renderer* r, FrameParams& P) {
@@ -699,24 +829,105 @@ int ensure_framebuffers(rtrb_renderer* r, int w, int h, bool rgba, bool rgb, boo
   return RTRB_OK;
 }
 
-int finish_stats(rtrb_renderer* r, FrameCtl& fc, rtrb_stats* stats_out);
+// RTRB_ERR_CUDA without a CUDA device: this library has no CPU fallback.  count_out (optional): the number of devices.
+int require_device(int* count_out = nullptr) {
+  int n = 0;
+  cudaError_t e = cudaGetDeviceCount(&n);
+  if (e != cudaSuccess || n == 0) {
+    cudaGetLastError();  // not sticky: clear it so that later launch checks do not report it
+    return fail(RTRB_ERR_CUDA, "no CUDA device (%s); this library has no CPU fallback", cudaGetErrorString(e));
+  }
+  if (count_out) *count_out = n;
+  return RTRB_OK;
+}
 
-// The control-block words a launch reports into (layout: RTRB_FCB_WORDS).
+// The caller's options, or the defaults (main.rb's Random.srand(1), the default precision) when it passes none.
+rtrb_render_opts opts_or_default(const rtrb_render_opts* in) {
+  rtrb_render_opts o;
+  memset(&o, 0, sizeof(o));
+  if (in) o = *in;
+  else { o.seed = 1; o.precision = RTRB_PREC_DEFAULT; }
+  return o;
+}
+
+// Partial frames: the hit ids of pixels outside the window read -3.
+void prefill_hits(int32_t* hit, int W, int H, cudaStream_t s) {
+  const size_t n = (size_t)W * H;
+  fill_i32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(hit, n, -3);
+  g_launches++;
+}
+
+// Where a launch reports into the control block.
 void bind_ctl(FrameParams& P, FrameCtl& fc) {
-  P.counters = fc.d.p; P.first_bad = fc.d.p + RTRB_CNT_N;
-  P.work_counter = fc.d.p + RTRB_CNT_N + 1;
-  P.status = reinterpret_cast<uint32_t*>(fc.d.p + RTRB_CNT_N + 3);
-  P.extra_count = reinterpret_cast<uint32_t*>(fc.d.p + RTRB_CNT_N + 4);
-  P.hot = fc.d.p + RTRB_CNT_N + 5;
+  CtlBlock* b = fc.d.p;
+  P.counters = b->counters; P.first_bad = &b->first_bad; P.work_counter = b->work;
+  P.status = &b->status; P.extra_count = &b->extra_count; P.hot = b->hot;
+}
+
+// Turns a copied-back control block into rtrb_stats (+ RTRB_ERR_RAISED when a status bit is set).
+int finish_stats(FrameCtl& fc, rtrb_stats* stats_out) {
+  rtrb_stats local;
+  if (!stats_out) stats_out = &local;
+  const CtlBlock& b = fc.h->blk;
+  const unsigned long long* c = b.counters;
+  memset(stats_out, 0, sizeof(*stats_out));
+  stats_out->rays = c[RTRB_CNT_RAYS]; stats_out->shadow_queries = c[RTRB_CNT_SHADOW];
+  for (int sl = 0; sl < RTRB_HOT_SLICES; ++sl) {
+    stats_out->rays += b.hot[2 * sl];
+    stats_out->shadow_queries += b.hot[2 * sl + 1];
+  }
+  stats_out->highlight_hits = c[RTRB_CNT_HIGHLIGHT]; stats_out->hits = c[RTRB_CNT_HITS];
+  stats_out->local_shaded = c[RTRB_CNT_LOCAL]; stats_out->lit_lights = c[RTRB_CNT_LIT];
+  stats_out->mc_rays = c[RTRB_CNT_MC]; stats_out->refractions = c[RTRB_CNT_REFR];
+  stats_out->texel_fetches = c[RTRB_CNT_TEXEL];
+  stats_out->sphere_tests = c[RTRB_CNT_SPH_TEST]; stats_out->sphere_accepts = c[RTRB_CNT_SPH_ACC];
+  stats_out->plane_tests = c[RTRB_CNT_PL_TEST]; stats_out->plane_accepts = c[RTRB_CNT_PL_ACC];
+  stats_out->cover_sphere = c[RTRB_CNT_COV_SPH]; stats_out->cover_sphere_full = c[RTRB_CNT_COV_SPH_FULL];
+  stats_out->cover_sphere_penumbra = c[RTRB_CNT_COV_SPH_PEN];
+  stats_out->cover_plane = c[RTRB_CNT_COV_PL]; stats_out->cover_plane_accepts = c[RTRB_CNT_COV_PL_ACC];
+  stats_out->adaptive_pixels = c[RTRB_CNT_ADAPTIVE]; stats_out->exact_tests = c[RTRB_CNT_EXACT];
+  stats_out->box_tests = c[RTRB_CNT_BOX_TEST]; stats_out->box_accepts = c[RTRB_CNT_BOX_ACC];
+  stats_out->cover_box = c[RTRB_CNT_COV_BOX]; stats_out->cover_box_accepts = c[RTRB_CNT_COV_BOX_ACC];
+  // samples: counted on the device with count_detail; otherwise a pure function of the window
+  stats_out->samples = fc.detail ? c[RTRB_CNT_SAMPLES]
+                                 : (uint64_t)fc.px_count * fc.S + (uint64_t)(fc.E > 0 ? c[RTRB_CNT_ADAPTIVE] * (uint64_t)fc.E : 0);
+  stats_out->status = b.status;
+  stats_out->max_stack = b.max_stack > 1u ? b.max_stack : (stats_out->rays ? 1u : 0u);  // blocks only report depths > 1
+  if (b.status && b.first_bad != 0ull) {  // stored complemented so that an all-zero block means "none"
+    const unsigned long long key = ~b.first_bad;
+    stats_out->first_bad_x = (int32_t)(key / (unsigned long long)fc.H);
+    stats_out->first_bad_y = (int32_t)(key % (unsigned long long)fc.H);
+  } else {
+    stats_out->first_bad_x = stats_out->first_bad_y = -1;
+  }
+  float ms = 0;
+  if (fc.timed) {
+    CUDA_TRY(cudaEventElapsedTime(&ms, fc.ev0, fc.ev1));
+    stats_out->device_ms = ms;
+  }
+  if (fc.timed && fc.n_tiles > 0) {
+    CUDA_TRY(cudaEventElapsedTime(&ms, fc.evt0, fc.evt1));
+    stats_out->trace_ms = ms;
+  }
+  if (b.status) {
+    fail(RTRB_ERR_RAISED, "the reference would have raised: status 0x%x at pixel (%d, %d)", b.status,
+         stats_out->first_bad_x, stats_out->first_bad_y);
+    return RTRB_ERR_RAISED;
+  }
+  return RTRB_OK;
+}
+
+// Copies the control block of the work queued on `s` back and finishes its stats.  Synchronises.
+int read_stats(FrameCtl& fc, cudaStream_t s, rtrb_stats* stats_out) {
+  CUDA_TRY(cudaMemcpyAsync(&fc.h->blk, fc.d.p, sizeof(CtlBlock), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  return finish_stats(fc, stats_out);
 }
 
 int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts_in,
                 const FrameTargets* targets, rtrb_stats* stats_out, FrameCtl* ctl = nullptr) {
   if (!r || !cam) return fail(RTRB_ERR_INVALID, "renderer/camera is NULL");
-  rtrb_render_opts opts;
-  memset(&opts, 0, sizeof(opts));
-  if (opts_in) opts = *opts_in;
-  else { opts.seed = 1; opts.precision = RTRB_PREC_DEFAULT; }
+  rtrb_render_opts opts = opts_or_default(opts_in);
   if (cam->width <= 0 || cam->height <= 0) return fail(RTRB_ERR_INVALID, "bad frame size %dx%d", cam->width, cam->height);
   if (cam->pre_sample_times < 1) return fail(RTRB_ERR_INVALID, "pre_sample_times must be >= 1");
   if (cam->max_sample_times < 0 || cam->monte_carlo_diffusion_times < 0 || cam->trace_depth < 0)
@@ -736,12 +947,9 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   if (opts.pixel_format != RTRB_FMT_RGBA8 && opts.pixel_format != RTRB_FMT_RGB8 && opts.pixel_format != RTRB_FMT_PNG_RGB8)
     return fail(RTRB_ERR_INVALID, "unknown pixel format %d", opts.pixel_format);
   const int W = cam->width, H = cam->height;
-  int x0 = opts.x0, y0 = opts.y0, x1 = opts.x1, y1 = opts.y1;
-  if (x0 == 0 && y0 == 0 && x1 == 0 && y1 == 0) { x1 = W; y1 = H; }
-  if (x0 < 0 || y0 < 0 || x1 > W || y1 > H || x0 >= x1 || y0 >= y1) return fail(RTRB_ERR_INVALID, "bad window");
-  int world = opts.tile_world <= 1 ? 1 : opts.tile_world;
-  int rank = world == 1 ? 0 : opts.tile_rank;
-  if (rank < 0 || rank >= world) return fail(RTRB_ERR_INVALID, "tile_rank %d outside tile_world %d", rank, world);
+  Window win;
+  int rc = make_window(W, H, opts.x0, opts.y0, opts.x1, opts.y1, opts.tile_rank, opts.tile_world, win);
+  if (rc) return rc;
   const int stack_need = cam->trace_depth * (1 + cam->monte_carlo_diffusion_times) + 1;
   if (stack_need > rtrb_max_stack_supported())
     return fail(RTRB_ERR_UNSUPPORTED, "trace_depth*(1+mc)+1 = %d exceeds the device stack limit %d", stack_need,
@@ -757,71 +965,25 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
     tg.want_hit = !(opts.skip_outputs & RTRB_SKIP_HIT);
   }
   if (!tg.rgba && opts.rgba_device_out) tg.rgba = (uint8_t*)opts.rgba_device_out;
-  {
-    int rc = ensure_framebuffers(r, W, H, tg.rgba == nullptr, tg.want_rgb && !tg.rgb, tg.want_hit && !tg.hit);
-    if (rc) return rc;
-  }
+  if ((rc = ensure_framebuffers(r, W, H, tg.rgba == nullptr, tg.want_rgb && !tg.rgb, tg.want_hit && !tg.hit))) return rc;
   if (!tg.rgba) tg.rgba = r->rgba.p;
   if (tg.want_rgb && !tg.rgb) tg.rgb = r->rgb.p;
   if (tg.want_hit && !tg.hit) tg.hit = r->hit.p;
   if (!tg.want_rgb) tg.rgb = nullptr;
   if (!tg.want_hit) tg.hit = nullptr;
 
-  // ---- tile list (cached) ----
-  const int stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER;
-  int key[8] = {W, H, x0, y0, x1, y1, rank, world};
-  if (memcmp(key, r->tiles_key, sizeof(key)) != 0) {
-    enumerate_tiles(W, x0, y0, x1, y1, rank, world, r->tiles_host);
-    CUDA_TRY(r->tiles.ensure(std::max<size_t>(1, r->tiles_host.size())));
-    if (!r->tiles_host.empty()) {
-      std::vector<int32_t> packed(r->tiles_host.size());
-      for (size_t i = 0; i < packed.size(); ++i)
-        packed[i] = (r->tiles_host[i] % stx_count) | ((r->tiles_host[i] / stx_count) << 16);
-      CUDA_TRY(cudaMemcpyAsync(r->tiles.p, packed.data(), packed.size() * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
-      CUDA_TRY(cudaStreamSynchronize(stream));
-    }
-    CUDA_TRY(cudaStreamSynchronize(stream));
-    memcpy(r->tiles_key, key, sizeof(key));
-    r->tiles_magic = 0;
-    if (stx_count > 0 && stx_count < 65536 && r->tiles_host.size() < 65536) {
-      const uint32_t magic = (uint32_t)((1ull << 32) / (unsigned)stx_count) + 1u;
-      bool ok = true;
-      for (size_t k = 0; k < r->tiles_host.size() && ok; ++k) {
-        const uint32_t ty = (uint32_t)(((unsigned long long)k * magic) >> 32);
-        ok = r->tiles_host[k] == (int32_t)k && ty == (uint32_t)k / (unsigned)stx_count;
-      }
-      if (ok) r->tiles_magic = magic;
-    }
-    r->tiles_px_count = 0;
-    for (int b : r->tiles_host) {
-      int tx = b % stx_count, ty = b / stx_count;
-      int ax0 = std::max(x0, tx * RTRB_SUPER), ax1 = std::min(x1, (tx + 1) * RTRB_SUPER);
-      int ay0 = std::max(y0, ty * RTRB_SUPER), ay1 = std::min(y1, (ty + 1) * RTRB_SUPER);
-      if (ax1 > ax0 && ay1 > ay0) r->tiles_px_count += (size_t)(ax1 - ax0) * (ay1 - ay0);
-    }
-  }
-  // ---- lens tables (cached): the per-column / per-row scalars of camera.rb:133-134, evaluated on the
-  // host in the reference's order so the device does two loads instead of two FP64 divisions per sample
-  {
-    double lk[4] = {(double)W, (double)H, cam->retina_width, cam->retina_height};
-    if (memcmp(lk, r->lens_key, sizeof(lk)) != 0 || !r->lens_tab.p) {
-      const std::vector<double> tab = lens_table(cam);
-      CUDA_TRY(r->lens_tab.ensure(tab.size()));
-      CUDA_TRY(cudaMemcpyAsync(r->lens_tab.p, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
-      CUDA_TRY(cudaStreamSynchronize(stream));
-      memcpy(r->lens_key, lk, sizeof(lk));
-    }
-  }
-  const int n_tiles = (int)r->tiles_host.size();
+  if ((rc = r->tiles.ensure(W, H, win, stream)) || (rc = r->lens.ensure(cam, stream))) return rc;
+  const int n_tiles = (int)r->tiles.host.size();
   const size_t n_slots = (size_t)n_tiles * RTRB_SUPER_PIXELS;
   const int S = cam->pre_sample_times;
   const int E = cam->max_sample_times > S ? cam->max_sample_times - S : 0;
   // Who finishes render_at (FrameParams::fuse_resolve).  The FAST64 ray-tree kernels resolve a pixel inside the CTA
   // that traced its samples whenever the sample count divides the CTA size: no FP64 sample buffer (24 B per sample:
-  // 12.7 GB for one 4K / 64 spp frame) and no resolve launch.
-  const bool strict_mode = opts.precision == RTRB_PREC_STRICT;
-  int fuse = (S == 1 && cam->variant_threshold > 0) ? 1 : 0;
-  if (!strict_mode && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0) fuse = 2;
+  // 12.7 GB for one 4K / 64 spp frame) and no resolve launch.  RTRB_RNG_MT frames always go through the sample
+  // buffer: trace_mt_body finishes render_at from it.
+  const bool strict = opts.precision == RTRB_PREC_STRICT;
+  int fuse = (!mt_mode && S == 1 && cam->variant_threshold > 0) ? 1 : 0;
+  if (!strict && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0) fuse = 2;
   const bool need_samples = fuse == 0;
   if ((need_samples && n_slots * (size_t)S * 3 * sizeof(double) > ((size_t)96 << 30)) || n_slots * (size_t)E * 3 * sizeof(double) > ((size_t)64 << 30))
     return fail(RTRB_ERR_UNSUPPORTED, "sample buffer would exceed the per-frame memory budget");
@@ -844,13 +1006,13 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
     P.cam_tab_valid = 1;
   }
   P.key0 = (uint32_t)opts.seed; P.key1 = (uint32_t)(opts.seed >> 32);
-  P.x0 = x0; P.y0 = y0; P.x1 = x1; P.y1 = y1;
-  P.n_tiles = n_tiles; P.stx_count = stx_count; P.tiles = r->tiles.p;
-  P.lens_sx = r->lens_tab.p; P.lens_sy = r->lens_tab.p + W;
+  P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
+  P.n_tiles = n_tiles; P.stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER; P.tiles = r->tiles.dev.p;
+  P.lens_sx = r->lens.tab.p; P.lens_sy = r->lens.tab.p + W;
   P.samples = need_samples ? r->samples.p : nullptr; P.rgb = tg.rgb; P.hit = tg.hit; P.rgba = tg.rgba;
   P.pre_avg = r->pre_avg.p;
   bind_ctl(P, fc);
-  P.tiles_magic = (world == 1 && x0 == 0 && y0 == 0 && x1 == W && y1 == H) ? r->tiles_magic : 0u;
+  P.tiles_magic = win.whole ? r->tiles.magic : 0u;
   P.extra_list = r->extra_list.p; P.extra_samples = r->extra_samples.p;
   // the Box code lives only in the full-counter kernel variants (rtrb_trace.cuh, trace_dispatch)
   P.count_detail = (opts.count_detail || r->n_boxes > 0) ? 1 : 0;
@@ -858,77 +1020,16 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   // (1: a single sample with a positive threshold can never take the adaptive branch, variance == 0)
   P.fuse_resolve = fuse;
 
-  const bool strict = strict_mode;
   // timing events only for the blocking calls that return stats: a timestamp between two kernels keeps
   // frame i+1 from starting under frame i's tail, so pipelined frames (rtrb_submit) are not timed and
   // report device_ms = trace_ms = 0
   const bool timed = stats_out != nullptr;
   fc.timed = timed;
   if (timed) CUDA_TRY(cudaEventRecord(fc.ev0, stream));
-  CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, RTRB_FCB_WORDS * sizeof(unsigned long long), stream));
-  const bool partial = !(x0 == 0 && y0 == 0 && x1 == W && y1 == H && world == 1);
-  if (partial && !tg.no_fill && tg.hit == r->hit.p && tg.hit) {
-    size_t n = (size_t)W * H;
-    fill_i32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(tg.hit, n, -3);
-    g_launches++;
-  }
+  CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, sizeof(CtlBlock), stream));
+  if (!win.whole && !tg.no_fill && tg.hit == r->hit.p && tg.hit) prefill_hits(tg.hit, W, H, stream);
   if (n_tiles > 0 && mt_mode) {
-    // ---- RTRB_RNG_MT: offsets = exclusive prefix sums of the per-pixel draw counts, iterated until stable.
-    // The first pixel whose offset is wrong is right after the next pass (its predecessors no longer move), so
-    // the loop ends after at most one pass per pixel; in practice a handful of passes per data-dependent pixel.
-    const size_t npx = (size_t)(x1 - x0) * (size_t)(y1 - y0);
-    if (npx * (size_t)std::max(S, cam->max_sample_times) > 0x3fffffffull) return fail(RTRB_ERR_UNSUPPORTED, "window too large for RTRB_RNG_MT");
-    CUDA_TRY(r->mt_offset.ensure(npx));
-    CUDA_TRY(r->mt_count.ensure(npx));
-    std::vector<uint32_t> off(npx), cnt(npx), nxt(npx);
-    for (size_t i = 0; i < npx; ++i) off[i] = (uint32_t)(i * (size_t)S);
-    if (r->mt_seed != opts.seed) {
-      r->mt_host.clear(); r->mt_gen.seed((uint32_t)opts.seed); r->mt_seed = opts.seed; r->mt_uploaded = 0;
-    }
-    size_t want_len = npx * (size_t)(S + 1) + 4096;
-    const int max_iter = 200000;
-    int it = 0;
-    for (;; ++it) {
-      if (it >= max_iter) return fail(RTRB_ERR_UNSUPPORTED, "RTRB_RNG_MT did not reach its fixed point in %d passes", max_iter);
-      if (r->mt_host.size() < want_len) {
-        r->mt_host.reserve(want_len);
-        while (r->mt_host.size() < want_len) r->mt_host.push_back(r->mt_gen.res53());
-      }
-      if (r->mt_uploaded < r->mt_host.size()) {
-        CUDA_TRY(r->mt_stream.ensure(r->mt_host.size()));
-        CUDA_TRY(cudaMemcpyAsync(r->mt_stream.p, r->mt_host.data(), r->mt_host.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
-        r->mt_uploaded = r->mt_host.size();
-      }
-      P.mt_stream = r->mt_stream.p; P.mt_len = (uint32_t)std::min<size_t>(r->mt_host.size(), 0xfffffff0u);
-      P.mt_offset = r->mt_offset.p; P.mt_count = r->mt_count.p;
-      CUDA_TRY(cudaMemcpyAsync(r->mt_offset.p, off.data(), npx * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
-      CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, RTRB_FCB_WORDS * sizeof(unsigned long long), stream));
-      if (timed) CUDA_TRY(cudaEventRecord(fc.evt0, stream));
-      CUDA_TRY(rtrb_launch_trace_mt_strict(P, stack_need, stream));
-      if (timed) CUDA_TRY(cudaEventRecord(fc.evt1, stream));
-      g_launches++;
-      CUDA_TRY(cudaMemcpyAsync(cnt.data(), r->mt_count.p, npx * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-      CUDA_TRY(cudaStreamSynchronize(stream));
-      bool overflow = false;
-      for (size_t i = 0; i < npx && !overflow; ++i) overflow = cnt[i] == 0xFFFFFFFFu;
-      if (overflow) {  // some pixel ran past the end of the stream: generate more and repeat the pass
-        want_len = r->mt_host.size() * 2;
-        if (want_len > 0xfffffff0ull) return fail(RTRB_ERR_UNSUPPORTED, "RTRB_RNG_MT stream would exceed 2^32 draws");
-        continue;
-      }
-      size_t acc = 0;
-      bool same = true;
-      for (size_t i = 0; i < npx; ++i) {
-        nxt[i] = (uint32_t)acc;
-        same = same && nxt[i] == off[i];
-        acc += cnt[i];
-      }
-      if (acc > 0xfffffff0ull) return fail(RTRB_ERR_UNSUPPORTED, "RTRB_RNG_MT stream would exceed 2^32 draws");
-      if (same) break;
-      off.swap(nxt);
-      want_len = std::max(want_len, acc + 4096);
-    }
-    r->mt_iterations = it + 1;
+    if ((rc = r->mt.trace(P, fc, opts.seed, stack_need, stream))) return rc;
   } else if (n_tiles > 0) {
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt0, stream));
     CUDA_TRY(strict ? rtrb_launch_trace_pre_strict(P, stack_need, stream) : rtrb_launch_trace_pre_fast(P, stack_need, stream));
@@ -957,67 +1058,9 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
 
   // facts needed to finish the stats once the control block has been copied back
   fc.W = W; fc.H = H; fc.S = S; fc.E = E; fc.n_tiles = n_tiles; fc.detail = P.count_detail != 0;
-  fc.px_count = r->tiles_px_count;
-  if (stats_out) {
-    CUDA_TRY(cudaMemcpyAsync(fc.h, fc.d.p, RTRB_FCB_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
-    CUDA_TRY(cudaStreamSynchronize(stream));
-    return finish_stats(r, fc, stats_out);
-  }
-  return RTRB_OK;
+  fc.px_count = r->tiles.px_count;
+  return stats_out ? read_stats(fc, stream, stats_out) : RTRB_OK;
 }
-
-// Turns a copied-back control block into rtrb_stats (+ RTRB_ERR_RAISED when a status bit is set).
-int finish_stats(rtrb_renderer* r, FrameCtl& fc, rtrb_stats* stats_out) {
-  (void)r;
-  const unsigned long long* c = fc.h;
-  const uint32_t* st = reinterpret_cast<const uint32_t*>(fc.h + RTRB_CNT_N + 3);
-  memset(stats_out, 0, sizeof(*stats_out));
-  stats_out->rays = c[RTRB_CNT_RAYS]; stats_out->shadow_queries = c[RTRB_CNT_SHADOW];
-  for (int sl = 0; sl < RTRB_HOT_SLICES; ++sl) {
-    stats_out->rays += c[RTRB_CNT_N + 5 + 2 * sl];
-    stats_out->shadow_queries += c[RTRB_CNT_N + 5 + 2 * sl + 1];
-  }
-  stats_out->highlight_hits = c[RTRB_CNT_HIGHLIGHT]; stats_out->hits = c[RTRB_CNT_HITS];
-  stats_out->local_shaded = c[RTRB_CNT_LOCAL]; stats_out->lit_lights = c[RTRB_CNT_LIT];
-  stats_out->mc_rays = c[RTRB_CNT_MC]; stats_out->refractions = c[RTRB_CNT_REFR];
-  stats_out->texel_fetches = c[RTRB_CNT_TEXEL];
-  stats_out->sphere_tests = c[RTRB_CNT_SPH_TEST]; stats_out->sphere_accepts = c[RTRB_CNT_SPH_ACC];
-  stats_out->plane_tests = c[RTRB_CNT_PL_TEST]; stats_out->plane_accepts = c[RTRB_CNT_PL_ACC];
-  stats_out->cover_sphere = c[RTRB_CNT_COV_SPH]; stats_out->cover_sphere_full = c[RTRB_CNT_COV_SPH_FULL];
-  stats_out->cover_sphere_penumbra = c[RTRB_CNT_COV_SPH_PEN];
-  stats_out->cover_plane = c[RTRB_CNT_COV_PL]; stats_out->cover_plane_accepts = c[RTRB_CNT_COV_PL_ACC];
-  stats_out->adaptive_pixels = c[RTRB_CNT_ADAPTIVE]; stats_out->exact_tests = c[RTRB_CNT_EXACT];
-  stats_out->box_tests = c[RTRB_CNT_BOX_TEST]; stats_out->box_accepts = c[RTRB_CNT_BOX_ACC];
-  stats_out->cover_box = c[RTRB_CNT_COV_BOX]; stats_out->cover_box_accepts = c[RTRB_CNT_COV_BOX_ACC];
-  // samples: counted on the device with count_detail; otherwise a pure function of the window
-  stats_out->samples = fc.detail ? c[RTRB_CNT_SAMPLES]
-                                 : (uint64_t)fc.px_count * fc.S + (uint64_t)(fc.E > 0 ? c[RTRB_CNT_ADAPTIVE] * (uint64_t)fc.E : 0);
-  stats_out->status = st[0];
-  stats_out->max_stack = st[1] > 1u ? st[1] : (stats_out->rays ? 1u : 0u);  // blocks only report depths > 1
-  if (st[0] && c[RTRB_CNT_N] != 0ull) {  // stored complemented so that an all-zero block means "none"
-    const unsigned long long key = ~c[RTRB_CNT_N];
-    stats_out->first_bad_x = (int32_t)(key / (unsigned long long)fc.H);
-    stats_out->first_bad_y = (int32_t)(key % (unsigned long long)fc.H);
-  } else {
-    stats_out->first_bad_x = stats_out->first_bad_y = -1;
-  }
-  float ms = 0;
-  if (fc.timed) {
-    CUDA_TRY(cudaEventElapsedTime(&ms, fc.ev0, fc.ev1));
-    stats_out->device_ms = ms;
-  }
-  if (fc.timed && fc.n_tiles > 0) {
-    CUDA_TRY(cudaEventElapsedTime(&ms, fc.evt0, fc.evt1));
-    stats_out->trace_ms = ms;
-  }
-  if (st[0]) {
-    fail(RTRB_ERR_RAISED, "the reference would have raised: status 0x%x at pixel (%d, %d)", st[0],
-         stats_out->first_bad_x, stats_out->first_bad_y);
-    return RTRB_ERR_RAISED;
-  }
-  return RTRB_OK;
-}
-
 
 // First half of rtrb_submit / rtrb_submit_png: takes the next pipeline slot and launches the frame into its
 // framebuffer on the render stream.
@@ -1026,7 +1069,7 @@ int submit_render(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_rend
   CUDA_TRY(cudaSetDevice(r->device));
   if (!r->pipe_ready) {
     for (int i = 0; i < RTRB_PIPE_SLOTS; ++i) {
-      cudaError_t e = (cudaError_t)r->pipe_ctl[i].init();
+      cudaError_t e = r->pipe_ctl[i].init();
       if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "pipeline slot init failed: %s", cudaGetErrorString(e));
     }
     r->pipe_ready = true;
@@ -1039,10 +1082,7 @@ int submit_render(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_rend
     CUDA_TRY(fc.rgba.ensure(slot_bytes));
     CUDA_TRY(cudaMemsetAsync(fc.rgba.p, 0, slot_bytes, r->stream));
   }
-  rtrb_render_opts o;
-  memset(&o, 0, sizeof(o));
-  if (opts) o = *opts;
-  else { o.seed = 1; o.precision = RTRB_PREC_DEFAULT; }
+  rtrb_render_opts o = opts_or_default(opts);
   o.stream = nullptr;  // the pipeline owns its streams
   FrameTargets tg;
   tg.rgba = o.rgba_device_out ? (uint8_t*)o.rgba_device_out : fc.rgba.p;
@@ -1060,7 +1100,8 @@ int submit_finish(rtrb_renderer* r, FrameCtl& fc, int* ticket_out) {
   // stores it straight into the pinned (device-mapped) host mirror.  As a DMA of its own - even on its own stream - it
   // sat between the 6.2 MB frame copies of a PCIe-bound sequence and cost 6 % of the frame rate (8 057 -> 8 540 frames/s
   // on config 2); behind the frame on the copy stream it cost 14 % (round 1).
-  publish_ctl_kernel<<<1, 256, 0, r->stream>>>(fc.h_dev, fc.d.p, RTRB_FCB_WORDS);
+  publish_ctl_kernel<<<1, 256, 0, r->stream>>>((unsigned long long*)&fc.h_dev->blk, (const unsigned long long*)fc.d.p,
+                                               (int)(sizeof(CtlBlock) / sizeof(unsigned long long)));
   CUDA_TRY(cudaGetLastError());
   g_launches++;
   CUDA_TRY(cudaEventRecord(fc.ctl_copied, r->stream));
@@ -1088,16 +1129,12 @@ int ray_args(const rtrb_ray_opts* opts, int n) {
 // No device: RTRB_ERR_CUDA, as every computing entry point.  Otherwise selects the renderer's device and sets up the
 // ray calls' own control block on first use.
 int ray_device(rtrb_renderer* r) {
-  int n = 0;
-  cudaError_t e = cudaGetDeviceCount(&n);
-  if (e != cudaSuccess || n == 0) {
-    cudaGetLastError();
-    return fail(RTRB_ERR_CUDA, "no CUDA device (%s); this library has no CPU fallback", cudaGetErrorString(e));
-  }
+  int rc = require_device();
+  if (rc) return rc;
   if (!r) return fail(RTRB_ERR_INVALID, "renderer is NULL");
   CUDA_TRY(cudaSetDevice(r->device));
   if (!r->ray_ready) {
-    e = (cudaError_t)r->ray_ctl.init();
+    cudaError_t e = r->ray_ctl.init();
     if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "ray control block init failed: %s", cudaGetErrorString(e));
     r->ray_ready = true;
   }
@@ -1129,13 +1166,14 @@ int ray_stage(rtrb_renderer* r, const size_t* bytes, int k, uint8_t** out) {
   return RTRB_OK;
 }
 
-// Copies the ray call's control block back and turns it into stats (RTRB_ERR_RAISED when a ray raised).  Synchronises.
-int ray_finish(rtrb_renderer* r, cudaStream_t s, rtrb_stats* stats_out) {
-  FrameCtl& fc = r->ray_ctl;
-  CUDA_TRY(cudaMemcpyAsync(fc.h, fc.d.p, RTRB_FCB_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaStreamSynchronize(s));
-  rtrb_stats local;
-  return finish_stats(r, fc, stats_out ? stats_out : &local);
+// Downloads the frame just rendered into host buffers.  A frame that raised (rc == RTRB_ERR_RAISED) keeps its error text.
+int download_frame(rtrb_renderer* r, int rc, uint8_t* rgba, double* rgb_or_null, int32_t* hit_or_null) {
+  if (rc != RTRB_OK && rc != RTRB_ERR_RAISED) return rc;
+  std::string keep = g_last_error;
+  int rc2 = rtrb_download(r, rgba, rgb_or_null, hit_or_null);
+  if (rc2) return rc2;
+  if (rc == RTRB_ERR_RAISED) g_last_error = keep;
+  return rc;
 }
 
 }  // namespace
@@ -1163,9 +1201,7 @@ int rtrb_renderer_create(const rtrb_scene_desc* scene, int device, rtrb_renderer
   int rc = validate_scene(scene);
   if (rc) return rc;
   int n = 0;
-  cudaError_t e = cudaGetDeviceCount(&n);
-  if (e != cudaSuccess || n == 0)
-    return fail(RTRB_ERR_CUDA, "no CUDA device (%s); this library has no CPU fallback", cudaGetErrorString(e));
+  if ((rc = require_device(&n))) return rc;
   if (device < 0 || device >= n) return fail(RTRB_ERR_INVALID, "device %d out of range (%d devices)", device, n);
   CUDA_TRY(cudaSetDevice(device));
   rtrb_renderer* r = new rtrb_renderer();
@@ -1175,7 +1211,7 @@ int rtrb_renderer_create(const rtrb_scene_desc* scene, int device, rtrb_renderer
       (ce = cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking)) != cudaSuccess ||
       (ce = cudaEventCreateWithFlags(&r->push_ev, cudaEventDisableTiming)) != cudaSuccess ||
       (ce = cudaEventCreateWithFlags(&r->push_done_ev, cudaEventDisableTiming)) != cudaSuccess ||
-      (ce = (cudaError_t)r->main_ctl.init()) != cudaSuccess) {
+      (ce = r->main_ctl.init()) != cudaSuccess) {
     rtrb_renderer_destroy(r);
     return fail(RTRB_ERR_CUDA, "stream/event creation failed: %s", cudaGetErrorString(ce));
   }
@@ -1189,21 +1225,6 @@ int rtrb_renderer_destroy(rtrb_renderer* r) {
   if (!r) return RTRB_OK;
   cudaSetDevice(r->device);
   cudaDeviceSynchronize();
-  r->mt_stream.release(); r->mt_offset.release(); r->mt_count.release();
-  r->geom.release(); r->mat.release(); r->lights.release(); r->lens_tab.release(); r->boxes.release();
-  r->bvh.release(); r->light_tab.release();
-  r->cull_sph.release(); r->cull_pl.release(); r->sph_index.release(); r->pl_index.release(); r->lights_f.release(); r->tiles.release(); r->samples.release();
-  r->extra_samples.release(); r->pre_avg.release(); r->rgb.release(); r->extra_list.release(); r->hit.release(); r->rgba.release();
-  r->main_ctl.destroy();
-  r->ray_ctl.destroy(); r->ray_scratch.release(); r->ray_lens.release();
-  for (int i = 0; i < RTRB_PIPE_SLOTS; ++i) r->pipe_ctl[i].destroy();
-  r->png.release();
-  if (r->png_ev) cudaEventDestroy(r->png_ev);
-  for (uint8_t* t : r->textures) cudaFree(t);
-  if (r->push_ev) cudaEventDestroy(r->push_ev);
-  if (r->push_done_ev) cudaEventDestroy(r->push_done_ev);
-  if (r->stream) cudaStreamDestroy(r->stream);
-  if (r->copy_stream) cudaStreamDestroy(r->copy_stream);
   delete r;
   return RTRB_OK;
 }
@@ -1244,13 +1265,8 @@ int rtrb_render(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   tg.want_rgb = rgb_or_null != nullptr;
   tg.want_hit = hit_or_null != nullptr;
   rtrb_stats local;
-  int rc = render_impl(r, cam, opts, &tg, stats_out ? stats_out : &local);
-  if (rc != RTRB_OK && rc != RTRB_ERR_RAISED) return rc;
-  std::string keep = g_last_error;
-  int rc2 = rtrb_download(r, rgba, rgb_or_null, hit_or_null);
-  if (rc2) return rc2;
-  if (rc == RTRB_ERR_RAISED) g_last_error = keep;
-  return rc;
+  const int rc = render_impl(r, cam, opts, &tg, stats_out ? stats_out : &local);
+  return download_frame(r, rc, rgba, rgb_or_null, hit_or_null);
 }
 
 int rtrb_submit(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* rgba_host,
@@ -1299,7 +1315,7 @@ int rtrb_submit_png(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_re
   CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, fc.ev1, 0));
   unsigned long long launches = 0;
   cudaError_t e = rtrb_png_encode(r->png, frame, cam->width, cam->height, fmt, r->copy_stream, (uint8_t*)host_dev,
-                                  fc.h_dev + RTRB_FCB_WORDS, &launches);
+                                  &fc.h_dev->png_bytes, &launches);
   g_launches += launches;
   if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "PNG encoder: %s", cudaGetErrorString(e));
   CUDA_TRY(cudaEventRecord(fc.copied, r->copy_stream));
@@ -1315,9 +1331,8 @@ int rtrb_wait(rtrb_renderer* r, int ticket, rtrb_stats* stats_out) {
   CUDA_TRY(cudaEventSynchronize(fc.copied));
   CUDA_TRY(cudaEventSynchronize(fc.ctl_copied));
   fc.in_flight = false;
-  if (fc.png_bytes_out) *fc.png_bytes_out = (size_t)fc.h[RTRB_FCB_WORDS];
-  rtrb_stats local;
-  return finish_stats(r, fc, stats_out ? stats_out : &local);
+  if (fc.png_bytes_out) *fc.png_bytes_out = (size_t)fc.h->png_bytes;
+  return finish_stats(fc, stats_out);
 }
 
 int rtrb_framebuffer_device_ptr(rtrb_renderer* r, int width, int height, void** ptr_out) {
@@ -1416,21 +1431,14 @@ int rtrb_render_multi(rtrb_renderer* const* renderers, int n, const rtrb_camera_
       return fail(RTRB_ERR_CUDA, "cudaDeviceEnablePeerAccess: %s", cudaGetErrorString(e));
     cudaGetLastError();
   }
-  rtrb_render_opts base;
-  memset(&base, 0, sizeof(base));
-  if (opts_in) base = *opts_in;
-  else { base.seed = 1; base.precision = RTRB_PREC_DEFAULT; }
-  {
-    const rtrb_render_opts& b = base;
-    const bool full = (b.x0 == 0 && b.y0 == 0 && b.x1 == 0 && b.y1 == 0) ||
-                      (b.x0 == 0 && b.y0 == 0 && b.x1 == cam->width && b.y1 == cam->height);
-    if (!full && want_hit) {
-      CUDA_TRY(cudaSetDevice(root->device));
-      size_t npx = (size_t)cam->width * cam->height;
-      fill_i32_kernel<<<(unsigned)((npx + 255) / 256), 256, 0, root->stream>>>(root->hit.p, npx, -3);
-      g_launches++;
-      CUDA_TRY(cudaStreamSynchronize(root->stream));
-    }
+  const rtrb_render_opts base = opts_or_default(opts_in);
+  // (a bad window is left to the ranks' render_impl to report)
+  Window win;
+  if (want_hit && make_window(cam->width, cam->height, base.x0, base.y0, base.x1, base.y1, 0, 1, win) == RTRB_OK &&
+      !win.whole) {
+    CUDA_TRY(cudaSetDevice(root->device));
+    prefill_hits(root->hit.p, cam->width, cam->height, root->stream);
+    CUDA_TRY(cudaStreamSynchronize(root->stream));
   }
   std::vector<rtrb_stats> st(n);
   std::vector<int> rcs(n, 0);
@@ -1460,10 +1468,12 @@ int rtrb_render_multi(rtrb_renderer* const* renderers, int n, const rtrb_camera_
   agg.first_bad_x = agg.first_bad_y = -1;
   long long best_key = -1;
   {
+    // the counters samples .. cover_box_accepts are summed as one array
+    static_assert(offsetof(rtrb_stats, status) - offsetof(rtrb_stats, samples) == 25 * sizeof(uint64_t), "rtrb_stats counters");
     uint64_t* a = &agg.samples;
     for (int i = 0; i < n; ++i) {
       const uint64_t* b = &st[i].samples;
-      for (int k = 0; k < 25; ++k) a[k] += b[k];  // samples .. cover_box_accepts
+      for (int k = 0; k < 25; ++k) a[k] += b[k];
       agg.status |= st[i].status;
       agg.max_stack = std::max(agg.max_stack, st[i].max_stack);
       agg.device_ms = std::max(agg.device_ms, st[i].device_ms);
@@ -1475,15 +1485,7 @@ int rtrb_render_multi(rtrb_renderer* const* renderers, int n, const rtrb_camera_
     }
   }
   if (stats_out) *stats_out = agg;
-  root->last_w = cam->width; root->last_h = cam->height;
-  root->last_has_rgb = want_rgb; root->last_has_hit = want_hit; root->last_rgba_own = true;
-  root->last_stream = root->stream;
-  root->last_format = base.pixel_format;
-  std::string keep = g_last_error;
-  rc = rtrb_download(root, rgba, rgb_or_null, hit_or_null);
-  if (rc) return rc;
-  if (worst == RTRB_ERR_RAISED) g_last_error = keep;
-  return worst;
+  return download_frame(root, worst, rgba, rgb_or_null, hit_or_null);  // rank 0's render_impl recorded the frame
 }
 
 int rtrb_png_max_bytes(int width, int height, size_t* bytes_out) {
@@ -1501,12 +1503,7 @@ int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int hei
   int rc = rtrb_png_max_bytes(width, height, &need);
   if (rc) return rc;
   if (capacity < need) return fail(RTRB_ERR_INVALID, "png capacity %zu < %zu bytes (rtrb_png_max_bytes)", capacity, need);
-  int n = 0;
-  cudaError_t e = cudaGetDeviceCount(&n);
-  if (e != cudaSuccess || n == 0) {
-    cudaGetLastError();
-    return fail(RTRB_ERR_CUDA, "no CUDA device (%s); this library has no CPU fallback", cudaGetErrorString(e));
-  }
+  if ((rc = require_device())) return rc;
   if (!r) return fail(RTRB_ERR_INVALID, "renderer is NULL");
   CUDA_TRY(cudaSetDevice(r->device));
   const uint8_t* src = (const uint8_t*)src_device;
@@ -1520,14 +1517,14 @@ int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int hei
   CUDA_TRY(cudaEventRecord(r->png_ev, r->copy_stream));  // pipelined encodes use the same scratch
   CUDA_TRY(cudaStreamWaitEvent(s, r->png_ev, 0));
   unsigned long long launches = 0;
-  e = rtrb_png_encode(r->png, src, width, height, pixel_format, s, nullptr, nullptr, &launches);
+  cudaError_t e = rtrb_png_encode(r->png, src, width, height, pixel_format, s, nullptr, nullptr, &launches);
   g_launches += launches;
   if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "PNG encoder: %s", cudaGetErrorString(e));
   unsigned long long total = 0;
-  CUDA_TRY(cudaMemcpyAsync(&total, r->png.total, sizeof(total), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaMemcpyAsync(&total, r->png.total.p, sizeof(total), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   if (total > capacity) return fail(RTRB_ERR_CUDA, "PNG encoder produced %llu bytes, more than its bound %zu", total, need);
-  CUDA_TRY(cudaMemcpyAsync(png_host, r->png.file, total, cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaMemcpyAsync(png_host, r->png.file.p, total, cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   *bytes_out = (size_t)total;
   return RTRB_OK;
@@ -1577,7 +1574,7 @@ int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rt
   fc.timed = stats_out != nullptr;
   fc.W = 1; fc.H = 1; fc.S = 1; fc.E = 0; fc.n_tiles = 1; fc.px_count = un; fc.detail = P.count_detail != 0;
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev0, s));
-  CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, RTRB_FCB_WORDS * sizeof(unsigned long long), s));
+  CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, sizeof(CtlBlock), s));
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
   CUDA_TRY(rtrb_launch_trace_rays(P, B, opts->precision == RTRB_PREC_STRICT, (int)need, s));
   g_launches++;
@@ -1585,9 +1582,9 @@ int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rt
   if (!dev) {
     CUDA_TRY(cudaMemcpyAsync(rgb_out, B.rgb, un * 3 * sizeof(double), cudaMemcpyDeviceToHost, s));
     if (hit_or_null) CUDA_TRY(cudaMemcpyAsync(hit_or_null, B.hit, un * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    return ray_finish(r, s, stats_out);
+    return read_stats(fc, s, stats_out);
   }
-  return stats_out ? ray_finish(r, s, stats_out) : RTRB_OK;
+  return stats_out ? read_stats(fc, s, stats_out) : RTRB_OK;
 }
 
 int rtrb_intersect_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rtrb_ray* rays, rtrb_ray_hit* hits_out) {
@@ -1632,29 +1629,19 @@ int rtrb_camera_rays(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_r
   if (!cam) return fail(RTRB_ERR_INVALID, "camera is NULL");
   const int W = cam->width, H = cam->height;
   if (W <= 0 || H <= 0) return fail(RTRB_ERR_INVALID, "bad frame size %dx%d", W, H);
-  int x0 = opts->x0, y0 = opts->y0, x1 = opts->x1, y1 = opts->y1;
-  if (x0 == 0 && y0 == 0 && x1 == 0 && y1 == 0) { x1 = W; y1 = H; }
-  if (x0 < 0 || y0 < 0 || x1 > W || y1 > H || x0 >= x1 || y0 >= y1) return fail(RTRB_ERR_INVALID, "bad window");
+  Window win;
+  if ((rc = make_window(W, H, opts->x0, opts->y0, opts->x1, opts->y1, 0, 1, win))) return rc;
   if (sample_begin < 0 || sample_end <= sample_begin)
     return fail(RTRB_ERR_INVALID, "empty sample range [%d, %d)", sample_begin, sample_end);
   if (!rays_out) return fail(RTRB_ERR_INVALID, "rays_out is NULL");
-  const unsigned long long n = (unsigned long long)(x1 - x0) * (unsigned long long)(y1 - y0) * (unsigned long long)(sample_end - sample_begin);
+  const unsigned long long n =
+      (unsigned long long)(win.x1 - win.x0) * (unsigned long long)(win.y1 - win.y0) * (unsigned long long)(sample_end - sample_begin);
   if (n > 0x7fffffffull) return fail(RTRB_ERR_UNSUPPORTED, "%llu rays: more than one ray call takes", n);
   if ((rc = ray_device(r))) return rc;
   const bool dev = opts->device_buffers == 1;
   if (dev && ((rc = check_device_ptr(r, rays_out, "rays_out")) || (rc = check_device_ptr(r, keys_or_null, "keys")))) return rc;
   cudaStream_t s = opts->stream ? (cudaStream_t)opts->stream : r->stream;
-  // lens tables of this camera (the frames' cache is not touched); re-uploaded when the camera's size changes
-  {
-    double lk[4] = {(double)W, (double)H, cam->retina_width, cam->retina_height};
-    if (memcmp(lk, r->ray_lens_key, sizeof(lk)) != 0 || !r->ray_lens.p) {
-      const std::vector<double> tab = lens_table(cam);
-      CUDA_TRY(r->ray_lens.ensure(tab.size()));
-      CUDA_TRY(cudaMemcpyAsync(r->ray_lens.p, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, s));
-      CUDA_TRY(cudaStreamSynchronize(s));
-      memcpy(r->ray_lens_key, lk, sizeof(lk));
-    }
-  }
+  if ((rc = r->ray_lens.ensure(cam, s))) return rc;  // the frames' lens tables are not touched
   RayBatch B;
   memset(&B, 0, sizeof(B));
   B.n = (long long)n; B.sample_begin = sample_begin; B.sample_end = sample_end;
@@ -1669,8 +1656,8 @@ int rtrb_camera_rays(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_r
   FrameParams P;
   memset(&P, 0, sizeof(P));
   bake_camera(P, cam);
-  P.x0 = x0; P.y0 = y0; P.x1 = x1; P.y1 = y1;
-  P.lens_sx = r->ray_lens.p; P.lens_sy = r->ray_lens.p + W;
+  P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
+  P.lens_sx = r->ray_lens.tab.p; P.lens_sy = r->ray_lens.tab.p + W;
   P.key0 = (uint32_t)opts->seed; P.key1 = (uint32_t)(opts->seed >> 32);
   CUDA_TRY(rtrb_launch_camera_rays(P, B, s));
   g_launches++;
@@ -1685,23 +1672,20 @@ int rtrb_camera_rays(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_r
 int rtrb_tile_partition(int width, int height, const int32_t* window, int tile_rank, int tile_world,
                         int32_t* tiles_out, int capacity, int* count_out) {
   if (width <= 0 || height <= 0 || !count_out) return fail(RTRB_ERR_INVALID, "bad argument");
-  int x0 = 0, y0 = 0, x1 = width, y1 = height;
-  if (window && !(window[0] == 0 && window[1] == 0 && window[2] == 0 && window[3] == 0)) {
-    x0 = window[0]; y0 = window[1]; x1 = window[2]; y1 = window[3];
-  }
-  if (x0 < 0 || y0 < 0 || x1 > width || y1 > height || x0 >= x1 || y0 >= y1) return fail(RTRB_ERR_INVALID, "bad window");
-  int world = tile_world <= 1 ? 1 : tile_world;
-  int rank = world == 1 ? 0 : tile_rank;
-  if (rank < 0 || rank >= world) return fail(RTRB_ERR_INVALID, "tile_rank %d outside tile_world %d", rank, world);
+  static const int32_t whole[4] = {0, 0, 0, 0};
+  if (!window) window = whole;
+  Window win;
+  int rc = make_window(width, height, window[0], window[1], window[2], window[3], tile_rank, tile_world, win);
+  if (rc) return rc;
   std::vector<int32_t> t;
-  enumerate_tiles(width, x0, y0, x1, y1, rank, world, t);
+  enumerate_tiles(width, win, t);
   *count_out = (int)t.size();
   if (tiles_out)
     for (int i = 0; i < (int)t.size() && i < capacity; ++i) tiles_out[i] = t[i];
   return RTRB_OK;
 }
 
-int rtrb_last_mt_passes(rtrb_renderer* r) { return r ? r->mt_iterations : 0; }
+int rtrb_last_mt_passes(rtrb_renderer* r) { return r ? r->mt.iterations : 0; }
 
 int rtrb_measure_fma_peak(int device, int which, double* tflops_out) {
   if (!tflops_out) return fail(RTRB_ERR_INVALID, "tflops_out is NULL");

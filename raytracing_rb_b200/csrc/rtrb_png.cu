@@ -733,50 +733,28 @@ __global__ void __launch_bounds__(256) png_publish_kernel(const uint8_t* __restr
   if (tid == 0) *count = n;
 }
 
-template <typename T>
-cudaError_t grow(T*& p, size_t want) {
-  if (p) cudaFree(p);
-  p = nullptr;
-  return cudaMalloc((void**)&p, want * sizeof(T));
-}
-
 }  // namespace
-
-void RtrbPngScratch::release() {
-  cudaFree(filtered); cudaFree(tokens); cudaFree(seg_out); cudaFree(seg_meta); cudaFree(seg_off); cudaFree(file);
-  cudaFree(total);
-  filtered = nullptr; tokens = nullptr; seg_out = nullptr; seg_meta = nullptr; seg_off = nullptr; file = nullptr;
-  total = nullptr;
-  cap_bytes = cap_segs = 0;
-}
 
 cudaError_t rtrb_png_encode(RtrbPngScratch& s, const uint8_t* src, int width, int height, int pixel_format,
                             cudaStream_t stream, uint8_t* host_mapped, unsigned long long* count_mapped,
                             unsigned long long* launches) {
   const size_t n = rtrb_png_filtered_bytes(width, height), nseg = rtrb_png_segments(width, height);
   cudaError_t e;
-  if (s.cap_bytes < n || s.cap_segs < nseg) {
-    const size_t cb = n > s.cap_bytes ? n : s.cap_bytes, cs = nseg > s.cap_segs ? nseg : s.cap_segs;
-    s.release();
-    if ((e = grow(s.filtered, cb)) != cudaSuccess || (e = grow(s.tokens, cs * SEG)) != cudaSuccess ||
-        (e = grow(s.seg_out, cs * RTRB_PNG_SEGMENT_WORST(SEG))) != cudaSuccess ||
-        (e = grow(s.seg_meta, cs * 3)) != cudaSuccess || (e = grow(s.seg_off, cs)) != cudaSuccess ||
-        (e = grow(s.file, RTRB_PNG_FIXED_BYTES + cs * (RTRB_PNG_CHUNK_BYTES + RTRB_PNG_SEGMENT_WORST(0)) + cb)) != cudaSuccess ||
-        (e = grow(s.total, 1)) != cudaSuccess) {
-      s.release();
-      return e;
-    }
-    s.cap_bytes = cb; s.cap_segs = cs;
-  }
+  if ((e = s.filtered.ensure(n)) != cudaSuccess || (e = s.tokens.ensure(nseg * SEG)) != cudaSuccess ||
+      (e = s.seg_out.ensure(nseg * RTRB_PNG_SEGMENT_WORST(SEG))) != cudaSuccess ||
+      (e = s.seg_meta.ensure(nseg * 3)) != cudaSuccess || (e = s.seg_off.ensure(nseg)) != cudaSuccess ||
+      (e = s.file.ensure(rtrb_png_bound(width, height))) != cudaSuccess || (e = s.total.ensure(1)) != cudaSuccess)
+    return e;
   if ((e = cudaFuncSetAttribute(png_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DEFLATE_SMEM)) != cudaSuccess)
     return e;
-  png_filter_kernel<<<height, 256, 0, stream>>>(src, width, pixel_format, s.filtered);
-  png_deflate_kernel<<<(unsigned)nseg, DT, DEFLATE_SMEM, stream>>>(s.filtered, n, 3 * width + 1, s.tokens, s.seg_out, s.seg_meta);
-  png_assemble_kernel<<<1, 1024, 0, stream>>>(s.seg_meta, (int)nseg, n, width, height, s.seg_off, s.file, s.total);
-  png_place_kernel<<<(unsigned)nseg, 256, 0, stream>>>(s.seg_out, s.seg_meta, s.seg_off, s.file);
+  png_filter_kernel<<<height, 256, 0, stream>>>(src, width, pixel_format, s.filtered.p);
+  png_deflate_kernel<<<(unsigned)nseg, DT, DEFLATE_SMEM, stream>>>(s.filtered.p, n, 3 * width + 1, s.tokens.p, s.seg_out.p,
+                                                                   s.seg_meta.p);
+  png_assemble_kernel<<<1, 1024, 0, stream>>>(s.seg_meta.p, (int)nseg, n, width, height, s.seg_off.p, s.file.p, s.total.p);
+  png_place_kernel<<<(unsigned)nseg, 256, 0, stream>>>(s.seg_out.p, s.seg_meta.p, s.seg_off.p, s.file.p);
   *launches += 4;
   if (host_mapped) {
-    png_publish_kernel<<<64, 256, 0, stream>>>(s.file, s.total, host_mapped, count_mapped);
+    png_publish_kernel<<<64, 256, 0, stream>>>(s.file.p, s.total.p, host_mapped, count_mapped);
     *launches += 1;
   }
   return cudaGetLastError();

@@ -15,6 +15,7 @@
 #include <stdint.h>
 
 #include "../../include/rtrb_b200.h"
+#include "rtrb_devbuf.h"
 
 // PNG framing around the segments: signature 8, IHDR chunk 25, IDAT with the 2-byte zlib header 14, IDAT with the
 // 4-byte Adler-32 trailer 16, IEND 12.  Each segment is one IDAT chunk (12 bytes of length, type and CRC).
@@ -36,19 +37,17 @@ inline size_t rtrb_png_bound(int width, int height) {
 
 // Device scratch of one renderer; grows with the largest frame encoded so far and is released with the renderer.
 struct RtrbPngScratch {
-  uint8_t* filtered = nullptr;       // the filtered stream
-  uint32_t* tokens = nullptr;        // LZ77 tokens, RTRB_PNG_SEGMENT_BYTES slots per segment
-  uint8_t* seg_out = nullptr;        // each segment's deflate bytes, RTRB_PNG_SEGMENT_WORST(segment) apart
-  uint32_t* seg_meta = nullptr;      // per segment: bytes, chunk CRC-32, Adler-32 of its input
-  unsigned long long* seg_off = nullptr;  // per segment: offset of its IDAT chunk in the file
-  uint8_t* file = nullptr;           // the finished PNG file
-  unsigned long long* total = nullptr;  // its byte count
-  size_t cap_bytes = 0, cap_segs = 0;
-  void release();
+  DevBuf<uint8_t> filtered;             // the filtered stream
+  DevBuf<uint32_t> tokens;              // LZ77 tokens, RTRB_PNG_SEGMENT_BYTES slots per segment
+  DevBuf<uint8_t> seg_out;              // each segment's deflate bytes, RTRB_PNG_SEGMENT_WORST(segment) apart
+  DevBuf<uint32_t> seg_meta;            // per segment: bytes, chunk CRC-32, Adler-32 of its input
+  DevBuf<unsigned long long> seg_off;   // per segment: offset of its IDAT chunk in the file
+  DevBuf<uint8_t> file;                 // the finished PNG file
+  DevBuf<unsigned long long> total;     // its byte count
 };
 
 // Queues the encoder for a width x height image at `src` (RTRB_FMT_RGB8 / RGBA8 / PNG_RGB8) on `stream`.  The file
-// lands in s.file and its size in *s.total; with host_mapped / count_mapped (device aliases of mapped host memory)
+// lands in s.file and its size in s.total; with host_mapped / count_mapped (device aliases of mapped host memory)
 // it is also stored there.  Adds the number of kernel launches to *launches.
 cudaError_t rtrb_png_encode(RtrbPngScratch& s, const uint8_t* src, int width, int height, int pixel_format,
                             cudaStream_t stream, uint8_t* host_mapped, unsigned long long* count_mapped,

@@ -302,6 +302,7 @@ def test_render_fork_json_files(tmp_path):
     (1, {}, None),                                   # default scene: adaptive 3..10 samples + Monte-Carlo rays
     (4, dict(width=96, height=54), None),            # 16 spp, MC rays in every shadow
     (3, dict(width=160, height=90), (40, 0, 80, 90)),  # a render_fork column strip: the stream restarts at its first pixel
+    (5, dict(width=64, height=36, spp=1, grid=4), None),  # 1 sample, threshold > 0: the counter-RNG frame fuses its resolve
 ])
 def test_mt19937_stream_mode_matches_oracle(oracle_mod, config_id, kw, window):
     """SURVEY 8f rank 4: RTRB_RNG_MT on the device - the reference's own random stream (Random.srand(1),
