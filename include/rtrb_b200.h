@@ -212,7 +212,10 @@ int rtrb_renderer_destroy(rtrb_renderer* r);
 
 /* -- the hot path ---------------------------------------------------------------------------- */
 /* Renders one frame into DEVICE buffers (async on opts->stream unless stats_out != NULL, which
- * synchronises).  Replaces the pixel loops camera.rb:59-63 and :102-106. */
+ * synchronises).  Replaces the pixel loops camera.rb:59-63 and :102-106.
+ * Consecutive depth-1, 1-spp FAST64 frames on one stream overlap on the device: a frame's kernel traces under the
+ * tail of the previous one and stores only after it has completed (results unchanged).  RTRB_FRAME_OVERLAP=0 in the
+ * environment when the renderer is created turns this off. */
 int rtrb_render_device(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts,
                        rtrb_stats* stats_out);
 

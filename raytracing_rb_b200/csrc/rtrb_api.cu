@@ -9,6 +9,7 @@
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include <atomic>
@@ -126,8 +127,10 @@ struct CtlMirror {
 };
 
 #define RTRB_PIPE_SLOTS 4  // frames that may be in flight between rtrb_submit and rtrb_wait
+#define RTRB_CTL_RING 4    // control blocks of the synchronous frame path (frame overlap, render_impl)
 struct FrameCtl {
-  DevBuf<CtlBlock> d;
+  DevBuf<CtlBlock> d;          // its control block, or the ring of them (main_ctl)
+  CtlBlock* blk = nullptr;     // the one the frame in this slot reports into
   CtlMirror* h = nullptr;      // pinned host mirror
   CtlMirror* h_dev = nullptr;  // ... and the address the device stores to (publish_ctl_kernel)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, evt0 = nullptr, evt1 = nullptr, copied = nullptr, ctl_copied = nullptr;
@@ -139,9 +142,10 @@ struct FrameCtl {
   unsigned ticket = 0;              // the rtrb_submit ticket occupying this slot while in_flight
   size_t px_count = 0;
   // Allocates on first use, so that slots a renderer never uses cost nothing.
-  cudaError_t init() {
+  cudaError_t init(size_t blocks = 1) {
     cudaError_t e;
-    if ((e = d.ensure(1)) != cudaSuccess) return e;
+    if ((e = d.ensure(blocks)) != cudaSuccess) return e;
+    blk = d.p;
     if ((e = cudaHostAlloc((void**)&h, sizeof(CtlMirror), cudaHostAllocMapped)) != cudaSuccess) return e;
     if ((e = cudaHostGetDevicePointer((void**)&h_dev, h, 0)) != cudaSuccess) return e;
     for (cudaEvent_t* ev : {&ev0, &ev1, &evt0, &evt1, &copied, &ctl_copied})
@@ -289,7 +293,7 @@ struct MtState {
       P.mt_stream = draws.p; P.mt_len = (uint32_t)std::min<size_t>(host.size(), 0xfffffff0u);
       P.mt_offset = offset.p; P.mt_count = count.p;
       CUDA_TRY(cudaMemcpyAsync(offset.p, off.data(), npx * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-      CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, sizeof(CtlBlock), s));
+      CUDA_TRY(cudaMemsetAsync(fc.blk, 0, sizeof(CtlBlock), s));
       if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
       CUDA_TRY(rtrb_launch_trace_mt_strict(P, stack_need, s));
       if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt1, s));
@@ -328,8 +332,13 @@ struct rtrb_renderer {
   cudaEvent_t push_ev = nullptr, push_done_ev = nullptr;  // rtrb_peer_push ordering (no timing)
   cudaEvent_t png_ev = nullptr;  // rtrb_encode_png waits for the pipelined encodes that share png
   RtrbPngScratch png;            // device PNG encoder scratch (rtrb_png.cu)
-  FrameCtl main_ctl;       // synchronous calls
+  FrameCtl main_ctl;       // synchronous calls: a ring of RTRB_CTL_RING control blocks
   FrameCtl pipe_ctl[RTRB_PIPE_SLOTS];  // rtrb_submit / rtrb_wait frame slots
+  // Frame overlap (render_impl): on unless RTRB_FRAME_OVERLAP=0 when the renderer is created.
+  bool frame_overlap = true;
+  unsigned ring_next = 0;              // the main_ctl ring slot the next synchronous frame takes
+  bool ring_zeroed = false;            // ... was zeroed by the last frame launched on ring_stream
+  cudaStream_t ring_stream = nullptr;
   bool pipe_ready = false;
   unsigned next_ticket = 0;
   // baked scene
@@ -859,7 +868,7 @@ void prefill_hits(int32_t* hit, int W, int H, cudaStream_t s) {
 
 // Where a launch reports into the control block.
 void bind_ctl(FrameParams& P, FrameCtl& fc) {
-  CtlBlock* b = fc.d.p;
+  CtlBlock* b = fc.blk;
   P.counters = b->counters; P.first_bad = &b->first_bad; P.work_counter = b->work;
   P.status = &b->status; P.extra_count = &b->extra_count; P.hot = b->hot;
 }
@@ -919,7 +928,7 @@ int finish_stats(FrameCtl& fc, rtrb_stats* stats_out) {
 
 // Copies the control block of the work queued on `s` back and finishes its stats.  Synchronises.
 int read_stats(FrameCtl& fc, cudaStream_t s, rtrb_stats* stats_out) {
-  CUDA_TRY(cudaMemcpyAsync(&fc.h->blk, fc.d.p, sizeof(CtlBlock), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaMemcpyAsync(&fc.h->blk, fc.blk, sizeof(CtlBlock), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   return finish_stats(fc, stats_out);
 }
@@ -992,6 +1001,21 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   if (E > 0) CUDA_TRY(r->extra_samples.ensure(n_slots * E * 3));
   if (E > 0 && fuse == 2) CUDA_TRY(r->pre_avg.ensure(n_slots * 3));
   FrameCtl& fc = ctl ? *ctl : r->main_ctl;
+  // Frame overlap: a frame that is one depth-1 FAST64 launch is launched with programmatic stream serialization, so its
+  // kernel traces under the tail of the kernel before it on the stream and waits for it only to write
+  // (trace_pre_body).  A synchronous frame takes the next control block of the main_ctl ring; an overlapping one also
+  // zeroes the block after it, and the next synchronous frame on the same stream then needs no memset between the
+  // two kernels.  Frames written into the same buffer stay ordered: every store waits for the previous grid.
+  const bool overlap = r->frame_overlap && !strict && !mt_mode && fuse == 1 && cam->trace_depth <= 1 && n_tiles > 0;
+  bool zeroed = false;
+  CtlBlock* next_blk = nullptr;
+  if (!ctl) {
+    fc.blk = fc.d.p + r->ring_next;
+    r->ring_next = (r->ring_next + 1) % RTRB_CTL_RING;
+    zeroed = r->ring_zeroed && r->ring_stream == stream;
+    r->ring_zeroed = false;
+    if (overlap) next_blk = fc.d.p + r->ring_next;
+  }
 
   FrameParams P;
   memset(&P, 0, sizeof(P));
@@ -1019,20 +1043,24 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   P.pixel_format = opts.pixel_format;
   // (1: a single sample with a positive threshold can never take the adaptive branch, variance == 0)
   P.fuse_resolve = fuse;
+  P.ctl_next = (unsigned long long*)next_blk;
+  P.ctl_next_words = next_blk ? (uint32_t)(sizeof(CtlBlock) / sizeof(unsigned long long)) : 0u;
 
-  // timing events only for the blocking calls that return stats: a timestamp between two kernels keeps
-  // frame i+1 from starting under frame i's tail, so pipelined frames (rtrb_submit) are not timed and
-  // report device_ms = trace_ms = 0
+  // timing events only for the blocking calls that return stats (the pipelined frames of rtrb_submit report
+  // device_ms = trace_ms = 0); the end-of-frame event only where something waits for it (timing, rtrb_submit's copy
+  // stream) or when frames do not overlap
   const bool timed = stats_out != nullptr;
   fc.timed = timed;
   if (timed) CUDA_TRY(cudaEventRecord(fc.ev0, stream));
-  CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, sizeof(CtlBlock), stream));
+  if (!zeroed) CUDA_TRY(cudaMemsetAsync(fc.blk, 0, sizeof(CtlBlock), stream));
   if (!win.whole && !tg.no_fill && tg.hit == r->hit.p && tg.hit) prefill_hits(tg.hit, W, H, stream);
   if (n_tiles > 0 && mt_mode) {
     if ((rc = r->mt.trace(P, fc, opts.seed, stack_need, stream))) return rc;
   } else if (n_tiles > 0) {
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt0, stream));
-    CUDA_TRY(strict ? rtrb_launch_trace_pre_strict(P, stack_need, stream) : rtrb_launch_trace_pre_fast(P, stack_need, stream));
+    CUDA_TRY(strict ? rtrb_launch_trace_pre_strict(P, stack_need, stream)
+                    : rtrb_launch_trace_pre_fast(P, stack_need, stream, overlap));
+    if (next_blk) { r->ring_zeroed = true; r->ring_stream = stream; }
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt1, stream));
     g_launches++;
     if (!P.fuse_resolve) {
@@ -1048,7 +1076,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
       g_launches++;
     }
   }
-  CUDA_TRY(cudaEventRecord(fc.ev1, stream));
+  if (timed || ctl || !r->frame_overlap) CUDA_TRY(cudaEventRecord(fc.ev1, stream));
   r->last_w = W; r->last_h = H;
   r->last_rgba_own = tg.rgba == r->rgba.p;
   r->last_has_rgb = tg.rgb == r->rgb.p && tg.rgb != nullptr;
@@ -1100,7 +1128,7 @@ int submit_finish(rtrb_renderer* r, FrameCtl& fc, int* ticket_out) {
   // stores it straight into the pinned (device-mapped) host mirror.  As a DMA of its own - even on its own stream - it
   // sat between the 6.2 MB frame copies of a PCIe-bound sequence and cost 6 % of the frame rate (8 057 -> 8 540 frames/s
   // on config 2); behind the frame on the copy stream it cost 14 % (round 1).
-  publish_ctl_kernel<<<1, 256, 0, r->stream>>>((unsigned long long*)&fc.h_dev->blk, (const unsigned long long*)fc.d.p,
+  publish_ctl_kernel<<<1, 256, 0, r->stream>>>((unsigned long long*)&fc.h_dev->blk, (const unsigned long long*)fc.blk,
                                                (int)(sizeof(CtlBlock) / sizeof(unsigned long long)));
   CUDA_TRY(cudaGetLastError());
   g_launches++;
@@ -1211,10 +1239,12 @@ int rtrb_renderer_create(const rtrb_scene_desc* scene, int device, rtrb_renderer
       (ce = cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking)) != cudaSuccess ||
       (ce = cudaEventCreateWithFlags(&r->push_ev, cudaEventDisableTiming)) != cudaSuccess ||
       (ce = cudaEventCreateWithFlags(&r->push_done_ev, cudaEventDisableTiming)) != cudaSuccess ||
-      (ce = r->main_ctl.init()) != cudaSuccess) {
+      (ce = r->main_ctl.init(RTRB_CTL_RING)) != cudaSuccess) {
     rtrb_renderer_destroy(r);
     return fail(RTRB_ERR_CUDA, "stream/event creation failed: %s", cudaGetErrorString(ce));
   }
+  const char* overlap = getenv("RTRB_FRAME_OVERLAP");
+  r->frame_overlap = !(overlap && strcmp(overlap, "0") == 0);
   rc = bake_scene(r, scene);
   if (rc) { rtrb_renderer_destroy(r); return rc; }
   *out = r;
@@ -1574,7 +1604,7 @@ int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rt
   fc.timed = stats_out != nullptr;
   fc.W = 1; fc.H = 1; fc.S = 1; fc.E = 0; fc.n_tiles = 1; fc.px_count = un; fc.detail = P.count_detail != 0;
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev0, s));
-  CUDA_TRY(cudaMemsetAsync(fc.d.p, 0, sizeof(CtlBlock), s));
+  CUDA_TRY(cudaMemsetAsync(fc.blk, 0, sizeof(CtlBlock), s));
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
   CUDA_TRY(rtrb_launch_trace_rays(P, B, opts->precision == RTRB_PREC_STRICT, (int)need, s));
   g_launches++;

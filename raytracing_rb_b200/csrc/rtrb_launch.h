@@ -40,6 +40,7 @@ using TraceKernel = void (*)(FrameParams);
 // stack_need = deepest work stack the frame can reach (trace_depth * (1 + mc) + 1).
 cudaError_t rtrb_launch_trace_pre_strict(const FrameParams& P, int stack_need, cudaStream_t s);
 cudaError_t rtrb_launch_trace_extra_strict(const FrameParams& P, int stack_need, cudaStream_t s);
-cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cudaStream_t s);
+// overlap: launch with programmatic stream serialization (depth-1 frames only; rtrb_api.cu, render_impl)
+cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cudaStream_t s, bool overlap = false);
 cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int stack_need, cudaStream_t s);
 cudaError_t rtrb_launch_trace_mt_strict(const FrameParams& P, int stack_need, cudaStream_t s);  // RTRB_RNG_MT

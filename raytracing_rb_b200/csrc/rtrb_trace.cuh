@@ -776,8 +776,15 @@ __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd,
 }
 
 // One thread per (pixel, sample j < pre_sample_times): the first loop of render_at (camera.rb:73-78).
+// The FAST64 depth-1 kernels may be launched with programmatic stream serialization (frame overlap, rtrb_api.cu): every
+// CTA lets the next frame's kernel launch as soon as it starts, and every thread traces before it waits for the
+// previous grid on the stream to complete, so the only things ordered behind that grid are this frame's global writes.
+// Everything before the wait reads only FrameParams, the scene tables and the lens tables.  Launched without the
+// attribute, the wait returns at once.
 template <class Pol, int MAXS, bool DETAIL, bool BVH = false>
 __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
+  constexpr bool kOverlap = Pol::fast && MAXS == 1;
+  if constexpr (kOverlap) cudaTriggerProgrammaticLaunchCompletion();
   const uint32_t S = (uint32_t)P.pre;
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   const unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * S;
@@ -803,6 +810,7 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
       int ph;
       d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
+      if constexpr (kOverlap) cudaGridDependencySynchronize();
       if (P.fuse_resolve) {
         // one sample, positive threshold: mean = s / 1.0 = s and variance = 0 < threshold (camera.rb:80-87)
         write_pixel(P, x, y, col.x, col.y, col.z);
@@ -813,7 +821,11 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
       if (j == 0 && P.hit) P.hit[(size_t)y * P.width + x] = ph;
     }
   }
+  if (kOverlap && !active) cudaGridDependencySynchronize();  // before flush_ctx's counters
   flush_ctx(P, ctx, x, y, active);
+  // the next frame's control block: that frame touches it only after its own wait, i.e. after this grid completed
+  if (kOverlap && blockIdx.x == 0u && P.ctl_next != nullptr)
+    for (uint32_t i = threadIdx.x; i < P.ctl_next_words; i += blockDim.x) P.ctl_next[i] = 0ull;
 }
 
 // Extra samples j in [pre, max) of the pixels that failed the variance test (camera.rb:88-93);

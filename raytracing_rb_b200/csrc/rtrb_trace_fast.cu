@@ -28,9 +28,10 @@ const FastKernels* build_for(const FrameParams& P, int stack_need) {
 
 }  // namespace
 
-cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cudaStream_t s) {
+cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cudaStream_t s, bool overlap) {
   const FastKernels* k = build_for(P, stack_need);
   if (!k) return cudaErrorInvalidValue;
+  if (overlap && k->capacity != 1) return cudaErrorInvalidValue;  // only the depth-1 kernels wait before their writes
   const TraceKernel kernel = k->pre[P.count_detail != 0][P.use_bvh != 0];
   // one thread per (pixel, sample); the ray-tree kernels run lockstep CTAs (rtrb_trace_fast.cuh, trace_pre_tree_body),
   // more and smaller ones on small frames
@@ -44,8 +45,22 @@ cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cud
   // both CTA sizes
   if (P.fuse_resolve == 2 && (block % P.pre) != 0) return cudaErrorInvalidConfiguration;
   const size_t smem = P.fuse_resolve == 2 ? (size_t)block * 3u * sizeof(double) : 0u;
-  kernel<<<(unsigned)blocks, block, smem, s>>>(P);
-  return cudaGetLastError();
+  if (!overlap) {
+    kernel<<<(unsigned)blocks, block, smem, s>>>(P);
+    return cudaGetLastError();
+  }
+  // programmatic dependent launch: may start under the tail of the previous kernel on the stream (trace_pre_body)
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)blocks);
+  cfg.blockDim = dim3((unsigned)block);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = s;
+  cfg.attrs = &attr;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, P);
 }
 
 cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int stack_need, cudaStream_t s) {

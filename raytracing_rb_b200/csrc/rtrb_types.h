@@ -152,6 +152,10 @@ struct FrameParams {
   // k / stx_count == __umulhi(k, tiles_magic), verified on the host for every k < n_tiles
   uint32_t tiles_magic;        // 0 = use tiles[]
   unsigned long long* hot;     // [RTRB_HOT_SLICES][2] sliced (rays, shadow queries) counters
+  // frame overlap (rtrb_api.cu, render_impl): the control block of the next frame on this stream, zeroed by CTA 0 of
+  // a depth-1 FAST64 kernel once the frame before it has completed, instead of a memset between the two launches
+  unsigned long long* ctl_next;  // [ctl_next_words] or nullptr
+  uint32_t ctl_next_words, pad_next;
   // RTRB_RNG_MT (stream-exact validation mode): the reference's MT19937 doubles, generated on the host, and
   // for every pixel of the window in the reference's order (x outer, y inner) where its draws start
   const double* mt_stream;     // [mt_len] genrand_res53 values after init_genrand(seed)
