@@ -63,8 +63,7 @@ RayKernel fast_trace(bool detail, bool bvh) {
   return bvh ? trace_rays_fast_kernel<MAXS, false, true> : trace_rays_fast_kernel<MAXS, false, false>;
 }
 
-// World#intersect for one ray into the ABI record.  delta as intersect_parameters forms it (sphere.rb:84, plane.rb:50;
-// a box delegates to the face that was hit, box.rb:102-107).
+// World#intersect for one ray into the ABI record, with intersect_parameters' delta.
 template <bool STRICT, bool BVH>
 __global__ void __launch_bounds__(kRayBlock) intersect_rays_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
   const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -87,19 +86,8 @@ __global__ void __launch_bounds__(kRayBlock) intersect_rays_kernel(const __grid_
   h.face = -1;
   if (best_i >= 0) {
     const DevGeom g = P.geom[best_i];
-    d3 delta;
-    if (g.type == RTRB_OBJ_SPHERE) {
-      delta = ((bh.p - mk(g.px, g.py, g.pz)) * RTRB_EPSILON) * (bh.dir_in ? 1.0 : -1.0);
-    } else {
-      d3 f = mk(g.nx, g.ny, g.nz);
-      if (g.type == RTRB_OBJ_BOX) {
-        const DevBoxFace& F = P.boxes[g.aux].f[bh.face];
-        f = mk(F.nx, F.ny, F.nz);
-        h.face = bh.face;
-      }
-      const double nfd = -dot(f, d);
-      delta = (f * RTRB_EPSILON) * (nfd > 0 ? 1.0 : (nfd < 0 ? -1.0 : 0.0));
-    }
+    const d3 delta = intersect_parameters<true>(P, g, P.mat[best_i], bh, d).delta;
+    if (g.type == RTRB_OBJ_BOX) h.face = bh.face;
     h.direction = bh.dir_in ? 1 : 0;
     h.distance = norm(o - bh.p);  // the expression World#intersect compared
     h.intersection[0] = bh.p.x; h.intersection[1] = bh.p.y; h.intersection[2] = bh.p.z;
@@ -108,7 +96,7 @@ __global__ void __launch_bounds__(kRayBlock) intersect_rays_kernel(const __grid_
   B.hits[i] = h;
 }
 
-// Camera#lens_func for (window pixel, sample j), with the aperture angle trace_pre_body draws for that sample.
+// Camera#lens_func for (window pixel, sample j): the frame kernels' camera_ray.
 __global__ void __launch_bounds__(kRayBlock) camera_rays_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (w >= (unsigned long long)B.n) return;
@@ -118,14 +106,8 @@ __global__ void __launch_bounds__(kRayBlock) camera_rays_kernel(const __grid_con
   const unsigned long long wx = (unsigned long long)(P.x1 - P.x0);
   const int y = P.y0 + (int)(px / wx), x = P.x0 + (int)(px % wx);
   const uint32_t pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
-  double theta = 0.0;
-  if (P.aperture_radius != 0.0) {
-    uint32_t c0 = pixel, c1 = j, c2 = 0u, c3 = 0u;
-    philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
-    theta = res53(c0, c1);  // Random.rand, camera.rb:135
-  }
   d3 ro, rd;
-  lens_ray<Generic>(P, x, y, theta, ro, rd);
+  camera_ray<Generic>(P, x, y, pixel, j, ro, rd);
   double* out = B.rays_out + w * 6ull;
   out[0] = ro.x; out[1] = ro.y; out[2] = ro.z;
   out[3] = rd.x; out[4] = rd.y; out[5] = rd.z;

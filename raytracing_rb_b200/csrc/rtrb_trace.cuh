@@ -270,13 +270,17 @@ struct CoverRay {
   d3 target, lp, lt, ltn, tl;
   double lt_r;
 };
+// lt_r = |lt| and ltn = lt / lt_r: Sphere#intersect's invariants of the probe ray
+__device__ __forceinline__ void cover_ray_unit(CoverRay& c) {
+  c.lt_r = norm(c.lt);
+  c.ltn = mk(c.lt.x / c.lt_r, c.lt.y / c.lt_r, c.lt.z / c.lt_r);
+}
 __device__ __forceinline__ CoverRay make_cover_ray(d3 target, const DevLight& L) {
   CoverRay c;
   c.target = target;
   c.lp = mk(L.px, L.py, L.pz);
   c.lt = c.lp - target;
-  c.lt_r = norm(c.lt);
-  c.ltn = mk(c.lt.x / c.lt_r, c.lt.y / c.lt_r, c.lt.z / c.lt_r);
+  cover_ray_unit(c);
   c.tl = target - c.lp;
   return c;
 }
@@ -411,6 +415,74 @@ struct StackItem {
   int32_t depth;
   uint32_t path;
 };
+// Fills a work item in place (a StackItem returned by value reorders the local-memory stores of the ray-tree kernels).
+__device__ __forceinline__ void set_item(StackItem& s, d3 o, d3 d, d3 att, int32_t depth, uint32_t path) {
+  s.ox = o.x; s.oy = o.y; s.oz = o.z;
+  s.dx = d.x; s.dy = d.y; s.dz = d.z;
+  s.ax = att.x; s.ay = att.y; s.az = att.z;
+  s.depth = depth; s.path = path;
+}
+
+// intersect_parameters (sphere.rb:88-101 / plane.rb:54-67) of the object g hit by direction d at bh: the normal n
+// (not normalised), the offset delta of the children's origins, the refractive rate and whether it may refract.
+// BOX = false compiles the box branch out.
+struct SurfaceParams {
+  d3 n, delta;
+  double rate;
+  bool can_refract;
+};
+template <bool BOX>
+__device__ __forceinline__ SurfaceParams intersect_parameters(const FrameParams& P, const DevGeom& g, const DevMat& M,
+                                                              const HitRec& bh, d3 d) {
+  d3 n, delta;
+  double rate;
+  bool can_refract;
+  if (g.type == RTRB_OBJ_SPHERE) {
+    d3 c = mk(g.px, g.py, g.pz);
+    delta = ((bh.p - c) * RTRB_EPSILON) * (bh.dir_in ? 1.0 : -1.0);  // sphere.rb:84
+    n = bh.dir_in ? (bh.p - c) : (c - bh.p);
+    rate = bh.dir_in ? M.refractive_rate : 1.0 / M.refractive_rate;
+    can_refract = true;
+  } else {
+    // a plane, or the face of a box that was hit (Box#intersect_parameters delegates, box.rb:102-107)
+    d3 f = mk(g.nx, g.ny, g.nz);
+    if constexpr (BOX) {
+      if (g.type == RTRB_OBJ_BOX) { const DevBoxFace& F = P.boxes[g.aux].f[bh.face]; f = mk(F.nx, F.ny, F.nz); }
+    }
+    double fd = dot(f, d);
+    double nfd = -fd;
+    double sgn = nfd > 0 ? 1.0 : (nfd < 0 ? -1.0 : 0.0);
+    delta = (f * RTRB_EPSILON) * sgn;  // plane.rb:50
+    n = fd > 0 ? -f : f;               // plane.rb:55
+    rate = M.refractive_rate;
+    can_refract = M.has_refraction != 0;
+  }
+  return {n, delta, rate, can_refract};
+}
+
+// Adds an emitted colour to the sample's sum in emission order (rt_reduce); a channel of the sum above 1 sets
+// RTRB_ST_COLOR_GT_1.
+__device__ __forceinline__ void emit(d3& sum, d3 c, ThreadCtx& ctx) {
+  sum = sum + c;
+  if (sum.x > 1 || sum.y > 1 || sum.z > 1) ctx.status |= RTRB_ST_COLOR_GT_1;
+}
+
+// Sphere#get_uv (sphere.rb:111-120) / Plane#get_uv (plane.rb:81-85) of the point p of the textured object g.
+__device__ __forceinline__ void object_uv(const DevGeom& g, const DevMat& M, d3 p, double& u, double& v, ThreadCtx& ctx) {
+  if (g.type == RTRB_OBJ_SPHERE) {
+    d3 vec = p - mk(g.px, g.py, g.pz);
+    double x = dot(vec, ld3(M.e0)) / g.radius;
+    double y = dot(vec, ld3(M.e1)) / g.radius;
+    double z = dot(vec, ld3(M.e2)) / g.radius;
+    double mm = rb_sqrt(x * x + y * y + z * z + 2 * x + 1, ctx);
+    u = (y / mm + 1) / 2;
+    v = (-z / mm + 1) / 2;
+  } else {
+    d3 rel = p - mk(g.px, g.py, g.pz);
+    u = dot(rel, ld3(M.e0)) / M.u_unit;
+    v = dot(rel, ld3(M.e1)) / M.v_unit;
+  }
+}
 
 // RayTracer#trace_sync for one sample.  Returns the summed colour; *primary_hit gets the root ray's
 // World#intersect winner (-1 miss, -2 highlight-terminated).
@@ -418,12 +490,8 @@ template <class Pol, int MAXS, bool MT = false>
 __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                            ThreadCtx& ctx, int* primary_hit, MtCursor* mt = nullptr) {
   StackItem stack[MAXS];
-  int sp = 0;
-  stack[0].ox = ro.x; stack[0].oy = ro.y; stack[0].oz = ro.z;
-  stack[0].dx = rd.x; stack[0].dy = rd.y; stack[0].dz = rd.z;
-  stack[0].ax = 1.0; stack[0].ay = 1.0; stack[0].az = 1.0;
-  stack[0].depth = P.trace_depth; stack[0].path = 1u;
-  sp = 1;
+  set_item(stack[0], ro, rd, mk(1.0, 1.0, 1.0), P.trace_depth, 1u);
+  int sp = 1;
   d3 sum = mk(0.0, 0.0, 0.0);
   bool first = true;
   const uint32_t K = (uint32_t)(P.mc + 2);
@@ -452,9 +520,7 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
     if (hl_n > 0) {
       for (int l = 0; l < P.n_lights; ++l) {
         if (!((hl_mask >> l) & 1ull)) continue;
-        d3 c = (att * ld3(P.lights[l].color_hl)) / (double)hl_n;  // ray_tracer.rb:65
-        sum = sum + c;
-        if (sum.x > 1 || sum.y > 1 || sum.z > 1) ctx.status |= RTRB_ST_COLOR_GT_1;
+        emit(sum, (att * ld3(P.lights[l].color_hl)) / (double)hl_n, ctx);  // ray_tracer.rb:65
       }
       RTRB_COUNT(ctx, RTRB_CNT_HIGHLIGHT);
       if (is_first) *primary_hit = -2;
@@ -496,28 +562,7 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
 
     const DevGeom g = P.geom[best_i];
     const DevMat& M = P.mat[best_i];
-    // ---- intersect_parameters (sphere.rb:88-101 / plane.rb:54-67) ----
-    d3 n, delta;
-    double rate;
-    bool can_refract;
-    if (g.type == RTRB_OBJ_SPHERE) {
-      d3 c = mk(g.px, g.py, g.pz);
-      delta = ((bh.p - c) * RTRB_EPSILON) * (bh.dir_in ? 1.0 : -1.0);  // sphere.rb:84
-      n = bh.dir_in ? (bh.p - c) : (c - bh.p);
-      rate = bh.dir_in ? M.refractive_rate : 1.0 / M.refractive_rate;
-      can_refract = true;
-    } else {
-      // a plane, or the face of a box that was hit (Box#intersect_parameters delegates, box.rb:102-107)
-      d3 f = mk(g.nx, g.ny, g.nz);
-      if (g.type == RTRB_OBJ_BOX) { const DevBoxFace& F = P.boxes[g.aux].f[bh.face]; f = mk(F.nx, F.ny, F.nz); }
-      double fd = dot(f, d);
-      double nfd = -fd;
-      double sgn = nfd > 0 ? 1.0 : (nfd < 0 ? -1.0 : 0.0);
-      delta = (f * RTRB_EPSILON) * sgn;  // plane.rb:50
-      n = fd > 0 ? -f : f;               // plane.rb:55
-      rate = M.refractive_rate;
-      can_refract = M.has_refraction != 0;
-    }
+    const auto [n, delta, rate, can_refract] = intersect_parameters<true>(P, g, M, bh, d);
     const d3 nn = normalize(n, ctx);
     // get_reflection_by_ray_and_n (world_object.rb:121-125)
     double cos_theta = vcos(d, -n, ctx);
@@ -540,22 +585,10 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
     }
     // push children: reflection first, refraction second (popped first)  ray_tracer.rb:87-121
     if (sp + 2 + P.mc > MAXS) { ctx.status |= RTRB_ST_STACK_OVERFLOW; continue; }
-    {
-      StackItem& s = stack[sp++];
-      d3 a2 = att * ld3(M.refl);
-      s.ox = refl_org.x; s.oy = refl_org.y; s.oz = refl_org.z;
-      s.dx = refl_dir.x; s.dy = refl_dir.y; s.dz = refl_dir.z;
-      s.ax = a2.x; s.ay = a2.y; s.az = a2.z;
-      s.depth = it.depth - 1; s.path = it.path * K + 0u;
-    }
+    set_item(stack[sp++], refl_org, refl_dir, att * ld3(M.refl), it.depth - 1, it.path * K + 0u);
     if (has_refr) {
       RTRB_COUNT(ctx, RTRB_CNT_REFR);
-      StackItem& s = stack[sp++];
-      d3 a2 = att * ld3(M.refr);
-      s.ox = refr_org.x; s.oy = refr_org.y; s.oz = refr_org.z;
-      s.dx = refr_dir.x; s.dy = refr_dir.y; s.dz = refr_dir.z;
-      s.ax = a2.x; s.ay = a2.y; s.az = a2.z;
-      s.depth = it.depth - 1; s.path = it.path * K + 1u;
+      set_item(stack[sp++], refr_org, refr_dir, att * ld3(M.refr), it.depth - 1, it.path * K + 1u);
     }
 
     // ---- World#local_lights (world.rb:72-80) fused with WorldObject#local_lighting (:51-74) ----
@@ -609,26 +642,12 @@ __device__ __forceinline__ d3 trace_sample(const FrameParams& P, d3 ro, d3 rd, u
       d3 filter = mk(1.0, 1.0, 1.0);
       if (M.tex != nullptr) {
         double u, v;
-        if (g.type == RTRB_OBJ_SPHERE) {  // Sphere#get_uv (sphere.rb:111-120)
-          d3 vec = bh.p - mk(g.px, g.py, g.pz);
-          double x = dot(vec, ld3(M.e0)) / g.radius;
-          double y = dot(vec, ld3(M.e1)) / g.radius;
-          double z = dot(vec, ld3(M.e2)) / g.radius;
-          double mm = rb_sqrt(x * x + y * y + z * z + 2 * x + 1, ctx);
-          u = (y / mm + 1) / 2;
-          v = (-z / mm + 1) / 2;
-        } else {  // Plane#get_uv (plane.rb:81-85)
-          d3 rel = bh.p - mk(g.px, g.py, g.pz);
-          u = dot(rel, ld3(M.e0)) / M.u_unit;
-          v = dot(rel, ld3(M.e1)) / M.v_unit;
-        }
+        object_uv(g, M, bh.p, u, v, ctx);
         RTRB_COUNT(ctx, RTRB_CNT_TEXEL);
         filter = texture_color<Pol>(M, u, v, ctx) * filter;
       }
       d3 local = ((contrib * ld3(M.diffuse)) * filter) + ld3(M.ambient);
-      d3 c = att * local;  // ray_tracer.rb:152
-      sum = sum + c;
-      if (sum.x > 1 || sum.y > 1 || sum.z > 1) ctx.status |= RTRB_ST_COLOR_GT_1;
+      emit(sum, att * local, ctx);  // ray_tracer.rb:152
     }
   }
   return sum;
@@ -653,6 +672,18 @@ __device__ __forceinline__ void lens_ray(const FrameParams& P, int x, int y, dou
   d3 target = retina_position + rf * t;
   ro = aperture;
   rd = target - aperture;
+}
+// The primary ray of sample j of a frame's pixel (x, y): lens_ray with the aperture angle drawn from Philox
+// (Random.rand, camera.rb:135).  The frame kernels and camera_rays share it, so traced camera rays reproduce frames.
+template <class Pol>
+__device__ __forceinline__ void camera_ray(const FrameParams& P, int x, int y, uint32_t pixel, uint32_t j, d3& ro, d3& rd) {
+  double theta = 0.0;
+  if (P.aperture_radius != 0.0) {
+    uint32_t c0 = pixel, c1 = j, c2 = 0u, c3 = 0u;
+    philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
+    theta = res53(c0, c1);
+  }
+  lens_ray<Pol>(P, x, y, theta, ro, rd);
 }
 
 // array_to_color (camera.rb:153-156) + the byte truncation of PNG::Color.new
@@ -684,6 +715,12 @@ __device__ __forceinline__ void write_pixel(const FrameParams& P, int x, int y, 
   }
   uchar4 q = make_uchar4(quantise_u8(r), quantise_u8(g), quantise_u8(b), 255);
   reinterpret_cast<uchar4*>(P.rgba)[px] = q;
+}
+
+// Work item w of a frame with S samples per pixel -> (tile slot, sample j); the samples of a slot are consecutive.
+__device__ __forceinline__ void decode_work(unsigned long long w, uint32_t S, uint32_t& slot, uint32_t& j) {
+  if (S == 1u) { slot = (uint32_t)w; j = 0u; }
+  else { slot = (uint32_t)(w / S); j = (uint32_t)(w - (unsigned long long)slot * S); }
 }
 
 // Decodes work item -> (tile slot k, in-tile q, x, y); returns false when the pixel is outside the window.
@@ -794,19 +831,12 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
   bool active = false;
   if (w < total) {
     uint32_t slot, j;
-    if (S == 1u) { slot = (uint32_t)w; j = 0u; }
-    else { slot = (uint32_t)(w / S); j = (uint32_t)(w - (unsigned long long)slot * S); }
+    decode_work(w, S, slot, j);
     active = decode_pixel(P, slot, x, y);
     if (active) {
       const uint32_t pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
-      double theta = 0.0;
-      if (P.aperture_radius != 0.0) {
-        uint32_t c0 = pixel, c1 = j, c2 = 0u, c3 = 0u;
-        philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
-        theta = res53(c0, c1);  // Random.rand, camera.rb:135
-      }
       d3 ro, rd;
-      lens_ray<Pol>(P, x, y, theta, ro, rd);
+      camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
       int ph;
       d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
@@ -845,14 +875,8 @@ __device__ __forceinline__ void trace_extra_body(const FrameParams& P) {
     if (!decode_pixel(P, slot, x, y)) continue;
     any = true;
     const uint32_t pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
-    double theta = 0.0;
-    if (P.aperture_radius != 0.0) {
-      uint32_t c0 = pixel, c1 = j, c2 = 0u, c3 = 0u;
-      philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
-      theta = res53(c0, c1);
-    }
     d3 ro, rd;
-    lens_ray<Pol>(P, x, y, theta, ro, rd);
+    camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
     int ph;
     d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
     RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);

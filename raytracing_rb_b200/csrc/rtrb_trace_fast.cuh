@@ -275,6 +275,23 @@ __device__ __forceinline__ bool bvh_traverse(const FrameParams& P, const BvhRay&
   return true;
 }
 
+// The probe ray of the filtered lit_area: the CoverRay without lt_r / ltn (cover_ray_unit forms them when an exact sphere
+// test first needs them), its CullRay, and `far`: hits farther than the light cannot cover, factor needs
+// dot(hit - L, T - L) > 0.
+__device__ __forceinline__ CoverRay make_cover_probe(const FrameParams& P, d3 target, const DevLight& L, CullRay& r,
+                                                     float& far) {
+  CoverRay c;
+  c.target = target;
+  c.lp = mk(L.px, L.py, L.pz);
+  c.lt = c.lp - target;
+  c.tl = target - c.lp;
+  c.lt_r = 0; c.ltn = mk(0, 0, 0);
+  r = make_cull_ray(P, target, c.lt);
+  const float lx = (float)c.lt.x, ly = (float)c.lt.y, lz = (float)c.lt.z;
+  far = sqrt_approx(fmaf(lz, lz, fmaf(ly, ly, lx * lx))) * 1.00001f + 2.0f * r.E;
+  return c;
+}
+
 // World#intersect (world.rb:37-59) = FP32 filter (planes + sphere BVH) + exact test of the survivors.
 template <class Pol, bool BOX>
 __device__ __forceinline__ int closest_hit_bvh(const FrameParams& P, d3 o, d3 d, const CullRay& r, HitRec& bh,
@@ -350,18 +367,9 @@ __device__ __forceinline__ int closest_hit_bvh(const FrameParams& P, d3 o, d3 d,
 // total - 0 == total, so skipping it leaves the running difference bit-identical.
 template <class Pol, bool BOX>
 __device__ __forceinline__ double lit_area_bvh(const FrameParams& P, d3 target, const DevLight& L, ThreadCtx& ctx) {
-  CoverRay c;
-  c.target = target;
-  c.lp = mk(L.px, L.py, L.pz);
-  c.lt = c.lp - target;
-  c.tl = target - c.lp;
-  c.lt_r = 0; c.ltn = mk(0, 0, 0);
-  const CullRay r = make_cull_ray(P, target, c.lt);
-  float far;  // hits farther than the light cannot cover: factor needs dot(hit - L, T - L) > 0
-  {
-    const float lx = (float)c.lt.x, ly = (float)c.lt.y, lz = (float)c.lt.z;
-    far = sqrt_approx(fmaf(lz, lz, fmaf(ly, ly, lx * lx))) * 1.00001f + 2.0f * r.E;
-  }
+  CullRay r;
+  float far;
+  CoverRay c = make_cover_probe(P, target, L, r, far);
   if (P.n_sph > 0x10000 || P.n_pl > 0xFFFF) return lit_area_call<Pol, BOX>(P, target, L, ctx);
   Pack8 S, Q;
   S.clear();
@@ -403,11 +411,7 @@ __device__ __forceinline__ double lit_area_bvh(const FrameParams& P, d3 target, 
       float lo, hi;
       const int kind = classify_sphere<BOX>(__ldg(&P.cull_sph[best_k]), r, lo, hi);
       if (kind == 0 || lo > far) continue;
-      if (!have_n) {
-        c.lt_r = norm(c.lt);
-        c.ltn = mk(c.lt.x / c.lt_r, c.lt.y / c.lt_r, c.lt.z / c.lt_r);
-        have_n = true;
-      }
+      if (!have_n) { cover_ray_unit(c); have_n = true; }
     }
     RTRB_COUNT(ctx, RTRB_CNT_EXACT);
     if (best_k >= 0) total -= cover_object_exact<Pol, BOX, 1>(P, P.geom[best_idx], c, L.radius, ctx);
@@ -554,18 +558,9 @@ __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3
 template <class Pol, bool BOX, bool KT>
 __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 target, const DevLight& L, const int light_index,
                                                   ThreadCtx& ctx) {
-  CoverRay c;
-  c.target = target;
-  c.lp = mk(L.px, L.py, L.pz);
-  c.lt = c.lp - target;
-  c.tl = target - c.lp;
-  c.lt_r = 0; c.ltn = mk(0, 0, 0);
-  const CullRay r = make_cull_ray(P, target, c.lt);
-  float far;  // hits farther than the light cannot cover: factor needs dot(hit - L, T - L) > 0
-  {
-    const float lx = (float)c.lt.x, ly = (float)c.lt.y, lz = (float)c.lt.z;
-    far = sqrt_approx(fmaf(lz, lz, fmaf(ly, ly, lx * lx))) * 1.00001f + 2.0f * r.E;
-  }
+  CullRay r;
+  float far;
+  CoverRay c = make_cover_probe(P, target, L, r, far);
   if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return lit_area_call<Pol, BOX>(P, target, L, ctx);
   // the probe ray's line passes through the light: apex table of this light when there is one
   uint32_t sm = (P.k_has_light_tab != 0) ? line_survivors_light<KT>(P, light_index, r) : line_survivors_generic<KT>(P, r);
@@ -587,11 +582,7 @@ __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 targe
       float lo, hi;
       const int kind = classify_sphere<BOX>(__ldg(&P.cull_sph[ks]), r, lo, hi);
       if (kind == 0 || lo > far) continue;
-      if (!have_n) {
-        c.lt_r = norm(c.lt);
-        c.ltn = mk(c.lt.x / c.lt_r, c.lt.y / c.lt_r, c.lt.z / c.lt_r);
-        have_n = true;
-      }
+      if (!have_n) { cover_ray_unit(c); have_n = true; }
       RTRB_COUNT(ctx, RTRB_CNT_EXACT);
       total -= cover_object_exact<Pol, BOX, 1>(P, P.geom[is], c, L.radius, ctx);
     } else {
@@ -712,8 +703,7 @@ __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackIte
         if (!((hl_mask >> l) & 1ull)) continue;
         d3 c = att * ld3(light_at<KT>(P, l).color_hl);
         if (hl_n != 1) c = c / (double)hl_n;  // x / 1.0 == x
-        sum = sum + c;
-        if (sum.x > 1 || sum.y > 1 || sum.z > 1) ctx.status |= RTRB_ST_COLOR_GT_1;
+        emit(sum, c, ctx);
       }
       RTRB_COUNT(ctx, RTRB_CNT_HIGHLIGHT);
       if (is_first) *primary_hit = -2;
@@ -763,29 +753,7 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
     (void)o;
     const DevGeom g = P.geom[best_i];
     const DevMat& M = P.mat[best_i];
-    d3 n, delta;
-    double rate;
-    bool can_refract;
-    if (g.type == RTRB_OBJ_SPHERE) {
-      d3 c = mk(g.px, g.py, g.pz);
-      delta = ((bh.p - c) * RTRB_EPSILON) * (bh.dir_in ? 1.0 : -1.0);
-      n = bh.dir_in ? (bh.p - c) : (c - bh.p);
-      rate = bh.dir_in ? M.refractive_rate : 1.0 / M.refractive_rate;
-      can_refract = true;
-    } else {
-      // a plane, or the face of a box that was hit (Box#intersect_parameters delegates, box.rb:102-107)
-      d3 f = mk(g.nx, g.ny, g.nz);
-      if constexpr (BOX) {
-        if (g.type == RTRB_OBJ_BOX) { const DevBoxFace& F = P.boxes[g.aux].f[bh.face]; f = mk(F.nx, F.ny, F.nz); }
-      }
-      double fd = dot(f, d);
-      double nfd = -fd;
-      double sgn = nfd > 0 ? 1.0 : (nfd < 0 ? -1.0 : 0.0);
-      delta = (f * RTRB_EPSILON) * sgn;
-      n = fd > 0 ? -f : f;
-      rate = M.refractive_rate;
-      can_refract = M.has_refraction != 0;
-    }
+    const auto [n, delta, rate, can_refract] = intersect_parameters<BOX>(P, g, M, bh, d);
     d3 nn;
     if ((BOX ? g.type == RTRB_OBJ_PLANE : g.type != RTRB_OBJ_SPHERE) && M.plane_nn_valid) {
       // n is +-front: its normalisation is a per-plane constant baked on the host (-(x / r) == (-x) / r)
@@ -816,12 +784,7 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
       const double cos_theta = vcos(d, -n, ctx);  // == vcos(d, n): both square the dot product
       const d3 refl_dir = normalize(nn * (2 * cos_theta * d_r) + d, ctx);
       if (refl_alive || near_normal) {
-        const d3 refl_org = bh.p + delta;
-        StackItem& s = stack[sp++];
-        s.ox = refl_org.x; s.oy = refl_org.y; s.oz = refl_org.z;
-        s.dx = refl_dir.x; s.dy = refl_dir.y; s.dz = refl_dir.z;
-        s.ax = a_refl.x; s.ay = a_refl.y; s.az = a_refl.z;
-        s.depth = it.depth - 1; s.path = it.path * K + 0u;
+        set_item(stack[sp++], bh.p + delta, refl_dir, a_refl, it.depth - 1, it.path * K + 0u);
       }
       if (can_refract && (refr_alive || near_normal)) {
         const double sin_i = rb_sqrt(1 - cos_theta * cos_theta, ctx);
@@ -832,11 +795,7 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
           const d3 refr_dir = nn * (-m_cos<Pol>(rr)) + normalize(refl_dir + d, ctx) * sin_r;
           const d3 refr_org = bh.p - nn * RTRB_EPSILON;
           RTRB_COUNT(ctx, RTRB_CNT_REFR);
-          StackItem& s = stack[sp++];
-          s.ox = refr_org.x; s.oy = refr_org.y; s.oz = refr_org.z;
-          s.dx = refr_dir.x; s.dy = refr_dir.y; s.dz = refr_dir.z;
-          s.ax = a_refr.x; s.ay = a_refr.y; s.az = a_refr.z;
-          s.depth = it.depth - 1; s.path = it.path * K + 1u;
+          set_item(stack[sp++], refr_org, refr_dir, a_refr, it.depth - 1, it.path * K + 1u);
         }
       }
     }
@@ -877,11 +836,7 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
             philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
             double theta = res53(c0, c1) * RTRB_PI / 2, phi = res53(c2, c3) * RTRB_PI * 2;
             d3 dir = nn * m_sin<Pol>(theta) + (leftv * m_cos<Pol>(phi) + upv * m_sin<Pol>(phi)) * m_cos<Pol>(theta);
-            StackItem& s = stack[sp++];
-            s.ox = shade_from.x; s.oy = shade_from.y; s.oz = shade_from.z;
-            s.dx = dir.x; s.dy = dir.y; s.dz = dir.z;
-            s.ax = a2.x; s.ay = a2.y; s.az = a2.z;
-            s.depth = it.depth - 1; s.path = child;
+            set_item(stack[sp++], shade_from, dir, a2, it.depth - 1, child);
           }
         }
         if (ctx.detail) ctx.c[RTRB_CNT_MC] += Pol::mc(P);
@@ -893,26 +848,12 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
       d3 filter = mk(1.0, 1.0, 1.0);
       if (Pol::textured(M)) {
         double u, v;
-        if (g.type == RTRB_OBJ_SPHERE) {
-          d3 vec = bh.p - mk(g.px, g.py, g.pz);
-          double x = dot(vec, ld3(M.e0)) / g.radius;
-          double y = dot(vec, ld3(M.e1)) / g.radius;
-          double z = dot(vec, ld3(M.e2)) / g.radius;
-          double mm = rb_sqrt(x * x + y * y + z * z + 2 * x + 1, ctx);
-          u = (y / mm + 1) / 2;
-          v = (-z / mm + 1) / 2;
-        } else {
-          d3 rel = bh.p - mk(g.px, g.py, g.pz);
-          u = dot(rel, ld3(M.e0)) / M.u_unit;
-          v = dot(rel, ld3(M.e1)) / M.v_unit;
-        }
+        object_uv(g, M, bh.p, u, v, ctx);
         RTRB_COUNT(ctx, RTRB_CNT_TEXEL);
         filter = texture_color<Pol>(M, u, v, ctx) * filter;
       }
       d3 local = ((contrib * ld3(M.diffuse)) * filter) + ld3(M.ambient);
-      d3 c = att * local;
-      sum = sum + c;
-      if (sum.x > 1 || sum.y > 1 || sum.z > 1) ctx.status |= RTRB_ST_COLOR_GT_1;
+      emit(sum, att * local, ctx);
     }
   }
 }
@@ -926,17 +867,15 @@ __device__ __forceinline__ void process_item_fast(const FrameParams& P, const St
   if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
 }
 
-// RayTracer#trace_sync for one sample (non-persistent form; used by tools and kept for reference).
+// RayTracer#trace_sync for one sample, free-running: the item loop of the depth-1, extra-sample and ray-query kernels
+// (the ray-tree frame kernels run trace_sample_fast_lockstep).
 template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                                 ThreadCtx& ctx, int* primary_hit) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
   // the root item starts in registers (no round trip through the local-memory stack)
   StackItem it;
-  it.ox = ro.x; it.oy = ro.y; it.oz = ro.z;
-  it.dx = rd.x; it.dy = rd.y; it.dz = rd.z;
-  it.ax = 1.0; it.ay = 1.0; it.az = 1.0;
-  it.depth = P.trace_depth; it.path = 1u;
+  set_item(it, ro, rd, mk(1.0, 1.0, 1.0), P.trace_depth, 1u);
   int sp = 0;
   d3 sum = mk(0.0, 0.0, 0.0);
   bool first = true;
@@ -971,10 +910,7 @@ __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d
                                                          ThreadCtx& ctx, int* primary_hit, bool active) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
   StackItem it;
-  it.ox = ro.x; it.oy = ro.y; it.oz = ro.z;
-  it.dx = rd.x; it.dy = rd.y; it.dz = rd.z;
-  it.ax = 1.0; it.ay = 1.0; it.az = 1.0;
-  it.depth = P.trace_depth; it.path = 1u;
+  set_item(it, ro, rd, mk(1.0, 1.0, 1.0), P.trace_depth, 1u);
   int sp = 0;
   d3 sum = mk(0.0, 0.0, 0.0);
   bool first = true, have = active;
@@ -1018,18 +954,11 @@ __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
   uint32_t slot = 0, j = 0, pixel = 0;
   d3 ro = mk(0, 0, 0), rd = mk(1, 0, 0);
   if (w < total) {
-    if (S == 1u) { slot = (uint32_t)w; j = 0u; }
-    else { slot = (uint32_t)(w / S); j = (uint32_t)(w - (unsigned long long)slot * S); }
+    decode_work(w, S, slot, j);
     active = decode_pixel(P, slot, x, y);
     if (active) {
       pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
-      double theta = 0.0;
-      if (P.aperture_radius != 0.0) {
-        uint32_t c0 = pixel, c1 = j, c2 = 0u, c3 = 0u;
-        philox4x32_10(P.key0, P.key1, c0, c1, c2, c3);
-        theta = res53(c0, c1);  // Random.rand, camera.rb:135
-      }
-      lens_ray<Pol>(P, x, y, theta, ro, rd);
+      camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
     }
   }
   int ph = -1;
