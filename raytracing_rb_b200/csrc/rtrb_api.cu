@@ -403,41 +403,20 @@ namespace {
 
 // ---- resolve kernels ---------------------------------------------------------------------------
 using rtrb::decode_pixel;
+using rtrb::final_average;
 using rtrb::pre_mean;
+using rtrb::queue_adaptive;
 using rtrb::write_pixel;
 
+// 256-thread blocks over n_tiles * 1024 slots: every warp is whole, as queue_adaptive requires
 __global__ void __launch_bounds__(256) resolve_kernel(const __grid_constant__ FrameParams P) {
   const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
   int x = 0, y = 0;
   const bool valid = slot < (uint32_t)P.n_tiles * RTRB_SUPER_PIXELS && decode_pixel(P, slot, x, y);
   double ax = 0, ay = 0, az = 0, variance = 0;
   if (valid) pre_mean(P, slot, ax, ay, az, variance);
-  const bool adaptive = valid && variance >= P.variant_threshold;
-  // warp-level compaction of the pixels that take the extra-sample branch (camera.rb:87-93): one ballot over
-  // the whole warp, one atomic per warp for the counter and one for the list, each lane's list position from a
-  // prefix popcount of the ballot
-  const unsigned amask = __ballot_sync(0xffffffffu, adaptive);
-  uint32_t base = 0;
-  if (amask != 0u) {
-    const int lane = threadIdx.x & 31;
-    const int leader = __ffs(amask) - 1;
-    if (lane == leader) {
-      const uint32_t n = __popc(amask);
-      atomicAdd(&P.counters[RTRB_CNT_ADAPTIVE], (unsigned long long)n);
-      if (P.max_samples > P.pre) base = atomicAdd(P.extra_count, n);
-    }
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (adaptive) {
-      if (P.max_samples > P.pre) {
-        P.extra_list[base + __popc(amask & ((1u << lane) - 1u))] = slot;
-        return;  // finished by resolve_extra_kernel
-      }
-      // empty extra loop: (average * pre + 0) / max  (camera.rb:93)
-      const double fp = (double)P.pre, fm = (double)P.max_samples;
-      ax = (ax * fp + 0.0) / fm; ay = (ay * fp + 0.0) / fm; az = (az * fp + 0.0) / fm;
-    }
-  }
-  if (valid) write_pixel(P, x, y, ax, ay, az);
+  const bool queued = queue_adaptive(P, valid && variance >= P.variant_threshold, slot, ax, ay, az);
+  if (valid && !queued) write_pixel(P, x, y, ax, ay, az);
 }
 
 __global__ void __launch_bounds__(256) resolve_extra_kernel(const __grid_constant__ FrameParams P) {
@@ -447,14 +426,12 @@ __global__ void __launch_bounds__(256) resolve_extra_kernel(const __grid_constan
     const uint32_t slot = P.extra_list[e];
     int x, y;
     if (!decode_pixel(P, slot, x, y)) continue;
-    double ax, ay, az, variance;
-    if (P.fuse_resolve == 2) { ax = P.pre_avg[(size_t)e * 3]; ay = P.pre_avg[(size_t)e * 3 + 1]; az = P.pre_avg[(size_t)e * 3 + 2]; }
-    else pre_mean(P, slot, ax, ay, az, variance);
+    const double* m = P.pre_avg + (size_t)e * 3;
+    double ax = m[0], ay = m[1], az = m[2];
     const double* s = P.extra_samples + (size_t)e * E * 3;
     double cx = 0.0, cy = 0.0, cz = 0.0;
     for (int j = 0; j < E; ++j) { cx += s[j * 3 + 0]; cy += s[j * 3 + 1]; cz += s[j * 3 + 2]; }
-    const double fp = (double)P.pre, fm = (double)P.max_samples;
-    ax = (ax * fp + cx) / fm; ay = (ay * fp + cy) / fm; az = (az * fp + cz) / fm;
+    final_average(ax, ay, az, P.pre, cx, cy, cz, P.max_samples);
     write_pixel(P, x, y, ax, ay, az);
   }
 }
@@ -991,22 +968,26 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   // 12.7 GB for one 4K / 64 spp frame) and no resolve launch.  RTRB_RNG_MT frames always go through the sample
   // buffer: trace_mt_body finishes render_at from it.
   const bool strict = opts.precision == RTRB_PREC_STRICT;
-  int fuse = (!mt_mode && S == 1 && cam->variant_threshold > 0) ? 1 : 0;
-  if (!strict && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0) fuse = 2;
-  const bool need_samples = fuse == 0;
+  int fuse = (!mt_mode && S == 1 && cam->variant_threshold > 0) ? RTRB_RESOLVE_IN_THREAD : RTRB_RESOLVE_SAMPLE_BUFFER;
+  if (!strict && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0)
+    fuse = RTRB_RESOLVE_IN_CTA;
+  const bool need_samples = fuse == RTRB_RESOLVE_SAMPLE_BUFFER;
   if ((need_samples && n_slots * (size_t)S * 3 * sizeof(double) > ((size_t)96 << 30)) || n_slots * (size_t)E * 3 * sizeof(double) > ((size_t)64 << 30))
     return fail(RTRB_ERR_UNSUPPORTED, "sample buffer would exceed the per-frame memory budget");
   if (need_samples) CUDA_TRY(r->samples.ensure(std::max<size_t>(1, n_slots * S * 3)));
   CUDA_TRY(r->extra_list.ensure(std::max<size_t>(1, n_slots)));
-  if (E > 0) CUDA_TRY(r->extra_samples.ensure(n_slots * E * 3));
-  if (E > 0 && fuse == 2) CUDA_TRY(r->pre_avg.ensure(n_slots * 3));
+  if (E > 0) {
+    CUDA_TRY(r->extra_samples.ensure(n_slots * E * 3));
+    CUDA_TRY(r->pre_avg.ensure(n_slots * 3));
+  }
   FrameCtl& fc = ctl ? *ctl : r->main_ctl;
   // Frame overlap: a frame that is one depth-1 FAST64 launch is launched with programmatic stream serialization, so its
   // kernel traces under the tail of the kernel before it on the stream and waits for it only to write
   // (trace_pre_body).  A synchronous frame takes the next control block of the main_ctl ring; an overlapping one also
   // zeroes the block after it, and the next synchronous frame on the same stream then needs no memset between the
   // two kernels.  Frames written into the same buffer stay ordered: every store waits for the previous grid.
-  const bool overlap = r->frame_overlap && !strict && !mt_mode && fuse == 1 && cam->trace_depth <= 1 && n_tiles > 0;
+  const bool overlap =
+      r->frame_overlap && !strict && !mt_mode && fuse == RTRB_RESOLVE_IN_THREAD && cam->trace_depth <= 1 && n_tiles > 0;
   bool zeroed = false;
   CtlBlock* next_blk = nullptr;
   if (!ctl) {
@@ -1041,7 +1022,6 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   // the Box code lives only in the full-counter kernel variants (rtrb_trace.cuh, trace_dispatch)
   P.count_detail = (opts.count_detail || r->n_boxes > 0) ? 1 : 0;
   P.pixel_format = opts.pixel_format;
-  // (1: a single sample with a positive threshold can never take the adaptive branch, variance == 0)
   P.fuse_resolve = fuse;
   P.ctl_next = (unsigned long long*)next_blk;
   P.ctl_next_words = next_blk ? (uint32_t)(sizeof(CtlBlock) / sizeof(unsigned long long)) : 0u;
@@ -1063,12 +1043,12 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
     if (next_blk) { r->ring_zeroed = true; r->ring_stream = stream; }
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt1, stream));
     g_launches++;
-    if (!P.fuse_resolve) {
+    if (fuse == RTRB_RESOLVE_SAMPLE_BUFFER) {
       resolve_kernel<<<(unsigned)((n_slots + 255) / 256), 256, 0, stream>>>(P);
       CUDA_TRY(cudaGetLastError());
       g_launches++;
     }
-    if (E > 0 && P.fuse_resolve != 1) {
+    if (E > 0 && fuse != RTRB_RESOLVE_IN_THREAD) {
       CUDA_TRY(strict ? rtrb_launch_trace_extra_strict(P, stack_need, stream) : rtrb_launch_trace_extra_fast(P, stack_need, stream));
       g_launches++;
       resolve_extra_kernel<<<296, 256, 0, stream>>>(P);

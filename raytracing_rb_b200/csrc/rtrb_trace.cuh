@@ -841,7 +841,7 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
       d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
       if constexpr (kOverlap) cudaGridDependencySynchronize();
-      if (P.fuse_resolve) {
+      if (P.fuse_resolve != RTRB_RESOLVE_SAMPLE_BUFFER) {  // RTRB_RESOLVE_IN_THREAD (IN_CTA is ray-tree only)
         // one sample, positive threshold: mean = s / 1.0 = s and variance = 0 < threshold (camera.rb:80-87)
         write_pixel(P, x, y, col.x, col.y, col.z);
       } else {
@@ -906,6 +906,47 @@ __device__ __forceinline__ void pre_mean(const FrameParams& P, uint32_t slot, do
   pre_mean_of(P.samples + (size_t)slot * P.pre * 3, P.pre, ax, ay, az, variance);
 }
 
+// (average * pre + extra) / max  (camera.rb:93), in place.  The empty extra loop passes an extra sum of literal 0.0:
+// the addition turns a -0.0 product into +0.0, and the FP RGB output keeps that sign.
+__device__ __forceinline__ void final_average(double& ax, double& ay, double& az, int pre, double cx, double cy,
+                                              double cz, int max_samples) {
+  const double fp = (double)pre, fm = (double)max_samples;
+  ax = (ax * fp + cx) / fm; ay = (ay * fp + cy) / fm; az = (az * fp + cz) / fm;
+}
+
+// The extra-sample branch of render_at (camera.rb:87-93) for the pixels whose variance test failed (`adaptive`):
+// counts them, and when max > pre queues each one for the extra-sample pass (slot in extra_list[], its mean (ax, ay,
+// az) in pre_avg[]) and returns true; when max <= pre the extra loop is empty and the mean is rescaled in place.
+// One ballot over the warp, one atomic per warp for the counter and one for the list, each lane's list position from
+// a prefix popcount of the ballot.  ALL 32 LANES OF THE WARP MUST CALL IT (full-mask ballot and shuffle).
+__device__ __forceinline__ bool queue_adaptive(const FrameParams& P, bool adaptive, uint32_t slot, double& ax, double& ay,
+                                               double& az) {
+  const unsigned amask = __ballot_sync(0xffffffffu, adaptive);
+  bool queued = false;
+  if (amask != 0u) {
+    const int lane = threadIdx.x & 31, leader = __ffs(amask) - 1;
+    uint32_t base = 0;
+    if (lane == leader) {
+      const uint32_t n = __popc(amask);
+      atomicAdd(&P.counters[RTRB_CNT_ADAPTIVE], (unsigned long long)n);
+      if (P.max_samples > P.pre) base = atomicAdd(P.extra_count, n);
+    }
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (adaptive) {
+      if (P.max_samples > P.pre) {
+        const uint32_t e = base + __popc(amask & ((1u << lane) - 1u));
+        P.extra_list[e] = slot;
+        double* m = P.pre_avg + (size_t)e * 3u;
+        m[0] = ax; m[1] = ay; m[2] = az;
+        queued = true;
+      } else {
+        final_average(ax, ay, az, P.pre, 0.0, 0.0, 0.0, P.max_samples);
+      }
+    }
+  }
+  return queued;
+}
+
 // RTRB_RNG_MT: Camera#render_at (camera.rb:70-99) for ONE pixel in ONE thread, because the reference's
 // MT19937 draws are consumed in program order: every sample's lens draw (camera.rb:135, drawn even when the
 // aperture is 0), its Monte-Carlo draws in LIFO ray order, then the next sample, then the adaptive samples.
@@ -951,8 +992,7 @@ __device__ __forceinline__ void trace_mt_body(const FrameParams& P) {
         RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
         cx += col.x; cy += col.y; cz += col.z;
       }
-      const double fp = (double)S, fm = (double)P.max_samples;
-      ax = (ax * fp + cx) / fm; ay = (ay * fp + cy) / fm; az = (az * fp + cz) / fm;  // camera.rb:93
+      final_average(ax, ay, az, S, cx, cy, cz, P.max_samples);
     }
     write_pixel(P, x, y, ax, ay, az);
     P.mt_count[order] = cur.overflow ? 0xFFFFFFFFu : cur.pos - start;

@@ -41,10 +41,10 @@ cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cud
   if (k->capacity > 1) block = threads < 4ull * (unsigned long long)sm_count() * kTreeBlock ? RTRB_TREE_MIN_BLOCK : kTreeBlock;
   const long long blocks = grid_size(threads, block);
   if (blocks < 0) return cudaErrorInvalidConfiguration;
-  // in-CTA resolve (fuse_resolve == 2, ray-tree frames only): the host only selects it for sample counts that divide
-  // both CTA sizes
-  if (P.fuse_resolve == 2 && (block % P.pre) != 0) return cudaErrorInvalidConfiguration;
-  const size_t smem = P.fuse_resolve == 2 ? (size_t)block * 3u * sizeof(double) : 0u;
+  // in-CTA resolve (ray-tree frames only): the host only selects it for sample counts that divide both CTA sizes
+  const bool in_cta = P.fuse_resolve == RTRB_RESOLVE_IN_CTA;
+  if (in_cta && (block % P.pre) != 0) return cudaErrorInvalidConfiguration;
+  const size_t smem = in_cta ? (size_t)block * 3u * sizeof(double) : 0u;
   if (!overlap) {
     kernel<<<(unsigned)blocks, block, smem, s>>>(P);
     return cudaGetLastError();

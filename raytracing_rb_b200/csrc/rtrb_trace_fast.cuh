@@ -903,8 +903,8 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
 // IN-CTA RESOLVE: when the CTA holds every sample of its pixels (pre_sample_times divides the CTA size), the sample
 // colours go to shared memory after the loop and one thread per pixel finishes render_at (camera.rb:79-98): ordered
 // mean, variance of the signed maximum, adaptive decision, quantisation.  No per-sample FP64 buffer crosses HBM
-// (24 B per sample: 12.7 GB for one 4K / 64 spp frame) and no resolve kernel runs.  FrameParams::fuse_resolve == 2
-// selects it; other sample counts (3, 10, ...) write the sample buffer for resolve_kernel as before.
+// (24 B per sample: 12.7 GB for one 4K / 64 spp frame) and no resolve kernel runs.  RTRB_RESOLVE_IN_CTA selects it;
+// other sample counts (3, 10, ...) write the sample buffer for resolve_kernel.
 template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                                          ThreadCtx& ctx, int* primary_hit, bool active) {
@@ -939,10 +939,10 @@ __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d
   return sum;
 }
 
-// Kernel body: the first loop of render_at (camera.rb:73-78) for the CTA's samples, then (fuse_resolve == 2) its tail.
+// Kernel body: the first loop of render_at (camera.rb:73-78) for the CTA's samples, then (RTRB_RESOLVE_IN_CTA) its tail.
 template <class Pol, int MAXS, bool BVH, bool DETAIL>
 __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
-  extern __shared__ double rtrb_cta_samples[];  // [blockDim.x][3] when fuse_resolve == 2
+  extern __shared__ double rtrb_cta_samples[];  // [blockDim.x][3] when RTRB_RESOLVE_IN_CTA
   const uint32_t S = (uint32_t)P.pre;
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   const unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * S;
@@ -967,7 +967,7 @@ __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
     RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
     if (j == 0 && P.hit) P.hit[(size_t)y * P.width + x] = ph;
   }
-  if (P.fuse_resolve == 2) {
+  if (P.fuse_resolve == RTRB_RESOLVE_IN_CTA) {
     // S divides blockDim.x, so the S samples of a pixel are S consecutive threads of this CTA
     double* mine = rtrb_cta_samples + (size_t)threadIdx.x * 3u;
     mine[0] = col.x; mine[1] = col.y; mine[2] = col.z;
@@ -1002,33 +1002,8 @@ __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
         variance /= (double)S;
       }
     }
-    const bool adaptive = resolver && variance >= P.variant_threshold;
-    // pixels that take the extra-sample branch (camera.rb:87-93): one ballot per warp, list positions by prefix
-    // popcount, one atomic per warp and counter
-    const unsigned amask = __ballot_sync(0xffffffffu, adaptive);
-    bool queued = false;
-    if (amask != 0u) {
-      const int lane = threadIdx.x & 31, leader = __ffs(amask) - 1;
-      uint32_t base = 0;
-      if (lane == leader) {
-        const uint32_t n = __popc(amask);
-        atomicAdd(&P.counters[RTRB_CNT_ADAPTIVE], (unsigned long long)n);
-        if (P.max_samples > P.pre) base = atomicAdd(P.extra_count, n);
-      }
-      base = __shfl_sync(0xffffffffu, base, leader);
-      if (adaptive) {
-        if (P.max_samples > P.pre) {
-          const uint32_t e = base + __popc(amask & ((1u << lane) - 1u));
-          P.extra_list[e] = slot;
-          double* m = P.pre_avg + (size_t)e * 3u;
-          m[0] = ax; m[1] = ay; m[2] = az;
-          queued = true;  // finished by resolve_extra_kernel
-        } else {  // empty extra loop: (average * pre + 0) / max  (camera.rb:93)
-          const double fp = (double)P.pre, fm = (double)P.max_samples;
-          ax = (ax * fp + 0.0) / fm; ay = (ay * fp + 0.0) / fm; az = (az * fp + 0.0) / fm;
-        }
-      }
-    }
+    // every thread of the CTA gets here (the barriers above), so every warp is whole
+    const bool queued = queue_adaptive(P, resolver && variance >= P.variant_threshold, slot, ax, ay, az);
     if (resolver && !queued) write_pixel(P, x, y, ax, ay, az);
   } else if (active) {
     double* out = P.samples + w * 3ull;

@@ -140,13 +140,11 @@ struct FrameParams {
   uint32_t* extra_count;       // number of pixels taking the extra-sample branch
   uint32_t* extra_list;        // [n_tiles*1024] pixel slots (tile k * 1024 + q)
   double* extra_samples;       // [extra][max-pre][3]
-  double* pre_avg;             // [extra][3] mean of the pre samples of the queued pixels (fuse_resolve == 2 only)
+  double* pre_avg;             // [extra][3] mean of the pre samples of the queued pixels, stored by the kernel that
+                               // queued them (rtrb_trace.cuh, queue_adaptive)
   unsigned long long* work_counter;  // [2] spare work-claim counters (zeroed with the control block)
   int32_t count_detail;
-  int32_t fuse_resolve;        // who finishes render_at: 0 = resolve_kernel from the sample buffer; 1 = the trace
-                               // kernel, one sample per pixel (mean = the sample, variance 0); 2 = the ray-tree
-                               // kernels, in the CTA that traced the pixel's samples (ordered mean + variance test
-                               // from shared memory)
+  int32_t fuse_resolve;        // RTRB_RESOLVE_*: who finishes render_at
   int32_t pixel_format;        // RTRB_FMT_*: 4 (RGBA8) or 3 (RGB8) bytes per pixel in `rgba`
   // whole frame on one renderer: tile k is (k % stx_count, k / stx_count), no table load at kernel start;
   // k / stx_count == __umulhi(k, tiles_magic), verified on the host for every k < n_tiles
@@ -176,6 +174,15 @@ struct FrameParams {
 };
 
 static_assert(sizeof(FrameParams) <= 4096, "FrameParams must fit the 4 KB kernel-parameter space");
+
+// FrameParams::fuse_resolve: who finishes render_at (camera.rb:79-98) after the first sample loop
+enum {
+  RTRB_RESOLVE_SAMPLE_BUFFER = 0,  // resolve_kernel, from the per-sample buffer
+  RTRB_RESOLVE_IN_THREAD = 1,      // the trace kernel: one sample per pixel and a positive threshold, so the mean is
+                                   // the sample and the variance 0 can never take the extra-sample branch
+  RTRB_RESOLVE_IN_CTA = 2,         // the ray-tree kernels, in the CTA that traced the pixel's samples (ordered mean
+                                   // and variance test from shared memory)
+};
 
 #define RTRB_HOT_SLICES 64     // one atomic per warp lands on one of 64 address pairs (no L2 atomic hot spot)
 

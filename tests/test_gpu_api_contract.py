@@ -118,7 +118,7 @@ def test_first_bad_pixel_in_the_adaptive_pass(oracle_mod, precision):
 @pytest.mark.parametrize("pre,mx,thr", [(4, 10, 0.001), (2, 8, 0.0), (8, 4, 0.0), (16, 16, 0.001), (3, 10, 0.001)])
 def test_in_cta_resolve_equals_the_sample_buffer_path(oracle_mod, pre, mx, thr):
     """The FAST64 ray-tree kernels finish render_at inside the CTA when pre_sample_times divides the CTA size
-    (fuse_resolve == 2; pre = 3 exercises the sample-buffer fallback); STRICT always goes through the sample buffer
+    (RTRB_RESOLVE_IN_CTA; pre = 3 exercises the sample-buffer fallback); STRICT always goes through the sample buffer
     and resolve_kernel.  Both must give the oracle's frame: same adaptive pixels, same extra samples, same bytes."""
     from raytracing_rb_b200 import Camera, World, scenes
     wdoc, cdoc = scenes.build(1)
