@@ -265,7 +265,7 @@ struct MtState {
   // Offsets = exclusive prefix sums of the per-pixel draw counts, iterated until stable.  The first pixel whose offset
   // is wrong is right after the next pass (its predecessors no longer move), so the loop ends after at most one pass
   // per pixel; in practice a handful of passes per data-dependent pixel.
-  int trace(FrameParams& P, FrameCtl& fc, uint64_t frame_seed, int stack_need, cudaStream_t s) {
+  int trace(FrameParams& P, FrameCtl& fc, uint64_t frame_seed, int capacity, cudaStream_t s) {
     const int S = P.pre;
     const size_t npx = (size_t)(P.x1 - P.x0) * (size_t)(P.y1 - P.y0);
     if (npx * (size_t)std::max(S, P.max_samples) > 0x3fffffffull) return fail(RTRB_ERR_UNSUPPORTED, "window too large for RTRB_RNG_MT");
@@ -295,7 +295,7 @@ struct MtState {
       CUDA_TRY(cudaMemcpyAsync(offset.p, off.data(), npx * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
       CUDA_TRY(cudaMemsetAsync(fc.blk, 0, sizeof(CtlBlock), s));
       if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
-      CUDA_TRY(rtrb_launch_trace_mt_strict(P, stack_need, s));
+      CUDA_TRY(rtrb_launch_trace_mt_strict(P, capacity, s));
       if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt1, s));
       g_launches++;
       CUDA_TRY(cudaMemcpyAsync(cnt.data(), count.p, npx * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
@@ -910,6 +910,20 @@ int read_stats(FrameCtl& fc, cudaStream_t s, rtrb_stats* stats_out) {
   return finish_stats(fc, stats_out);
 }
 
+// The trace kernels of a frame or ray batch: their work-stack capacity (rtrb_launch.h, trace_capacity) into *capacity,
+// or RTRB_ERR_UNSUPPORTED when none holds the stack; and their counter variant, P.count_detail.  The Box code lives
+// only in the full-counter variants (rtrb_trace.cuh, trace_dispatch), so scenes with a box always run those.  Called
+// with the other argument checks, before rtrb_trace_rays rejects a NULL renderer.
+int pick_trace_kernels(const rtrb_renderer* r, bool strict, int trace_depth, int mc, bool count_detail, FrameParams& P,
+                       int* capacity) {
+  *capacity = trace_capacity(strict, trace_depth, mc);
+  if (*capacity == 0)
+    return fail(RTRB_ERR_UNSUPPORTED, "trace_depth*(1+mc)+1 = %lld exceeds the device stack limit %d",
+                (long long)trace_depth * (1 + (long long)mc) + 1, kMaxStack);
+  P.count_detail = (count_detail || (r && r->n_boxes > 0)) ? 1 : 0;
+  return RTRB_OK;
+}
+
 int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts_in,
                 const FrameTargets* targets, rtrb_stats* stats_out, FrameCtl* ctl = nullptr) {
   if (!r || !cam) return fail(RTRB_ERR_INVALID, "renderer/camera is NULL");
@@ -936,10 +950,13 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   Window win;
   int rc = make_window(W, H, opts.x0, opts.y0, opts.x1, opts.y1, opts.tile_rank, opts.tile_world, win);
   if (rc) return rc;
-  const int stack_need = cam->trace_depth * (1 + cam->monte_carlo_diffusion_times) + 1;
-  if (stack_need > rtrb_max_stack_supported())
-    return fail(RTRB_ERR_UNSUPPORTED, "trace_depth*(1+mc)+1 = %d exceeds the device stack limit %d", stack_need,
-                rtrb_max_stack_supported());
+  const bool strict = opts.precision == RTRB_PREC_STRICT;
+  FrameParams P;
+  memset(&P, 0, sizeof(P));
+  int capacity;
+  if ((rc = pick_trace_kernels(r, strict, cam->trace_depth, cam->monte_carlo_diffusion_times, opts.count_detail != 0, P,
+                               &capacity)))
+    return rc;
 
   CUDA_TRY(cudaSetDevice(r->device));
   cudaStream_t stream = opts.stream ? (cudaStream_t)opts.stream : r->stream;
@@ -967,7 +984,6 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   // that traced its samples whenever the sample count divides the CTA size: no FP64 sample buffer (24 B per sample:
   // 12.7 GB for one 4K / 64 spp frame) and no resolve launch.  RTRB_RNG_MT frames always go through the sample
   // buffer: trace_mt_body finishes render_at from it.
-  const bool strict = opts.precision == RTRB_PREC_STRICT;
   int fuse = (!mt_mode && S == 1 && cam->variant_threshold > 0) ? RTRB_RESOLVE_IN_THREAD : RTRB_RESOLVE_SAMPLE_BUFFER;
   if (!strict && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0)
     fuse = RTRB_RESOLVE_IN_CTA;
@@ -998,8 +1014,6 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
     if (overlap) next_blk = fc.d.p + r->ring_next;
   }
 
-  FrameParams P;
-  memset(&P, 0, sizeof(P));
   bake_camera(P, cam);
   fill_scene_params(r, P);
   if (!P.use_bvh && r->n_sph > 0 && r->n_sph <= RTRB_APEX_MAX) {
@@ -1019,8 +1033,6 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   bind_ctl(P, fc);
   P.tiles_magic = win.whole ? r->tiles.magic : 0u;
   P.extra_list = r->extra_list.p; P.extra_samples = r->extra_samples.p;
-  // the Box code lives only in the full-counter kernel variants (rtrb_trace.cuh, trace_dispatch)
-  P.count_detail = (opts.count_detail || r->n_boxes > 0) ? 1 : 0;
   P.pixel_format = opts.pixel_format;
   P.fuse_resolve = fuse;
   P.ctl_next = (unsigned long long*)next_blk;
@@ -1035,11 +1047,11 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   if (!zeroed) CUDA_TRY(cudaMemsetAsync(fc.blk, 0, sizeof(CtlBlock), stream));
   if (!win.whole && !tg.no_fill && tg.hit == r->hit.p && tg.hit) prefill_hits(tg.hit, W, H, stream);
   if (n_tiles > 0 && mt_mode) {
-    if ((rc = r->mt.trace(P, fc, opts.seed, stack_need, stream))) return rc;
+    if ((rc = r->mt.trace(P, fc, opts.seed, capacity, stream))) return rc;
   } else if (n_tiles > 0) {
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt0, stream));
-    CUDA_TRY(strict ? rtrb_launch_trace_pre_strict(P, stack_need, stream)
-                    : rtrb_launch_trace_pre_fast(P, stack_need, stream, overlap));
+    CUDA_TRY(strict ? rtrb_launch_trace_pre_strict(P, capacity, stream)
+                    : rtrb_launch_trace_pre_fast(P, capacity, stream, overlap));
     if (next_blk) { r->ring_zeroed = true; r->ring_stream = stream; }
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt1, stream));
     g_launches++;
@@ -1049,7 +1061,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
       g_launches++;
     }
     if (E > 0 && fuse != RTRB_RESOLVE_IN_THREAD) {
-      CUDA_TRY(strict ? rtrb_launch_trace_extra_strict(P, stack_need, stream) : rtrb_launch_trace_extra_fast(P, stack_need, stream));
+      CUDA_TRY(strict ? rtrb_launch_trace_extra_strict(P, capacity, stream) : rtrb_launch_trace_extra_fast(P, capacity, stream));
       g_launches++;
       resolve_extra_kernel<<<296, 256, 0, stream>>>(P);
       CUDA_TRY(cudaGetLastError());
@@ -1546,9 +1558,13 @@ int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rt
   if (rc) return rc;
   if (n > 0 && (!rays || !rgb_out)) return fail(RTRB_ERR_INVALID, "rays / rgb_out is NULL");
   if (opts->trace_depth < 0 || opts->monte_carlo_diffusion_times < 0) return fail(RTRB_ERR_INVALID, "negative trace_depth / mc");
-  const long long need = (long long)opts->trace_depth * (1 + (long long)opts->monte_carlo_diffusion_times) + 1;
-  if (need > rtrb_max_stack_supported())
-    return fail(RTRB_ERR_UNSUPPORTED, "trace_depth*(1+mc)+1 = %lld exceeds the device stack limit %d", need, rtrb_max_stack_supported());
+  const bool strict = opts->precision == RTRB_PREC_STRICT;
+  FrameParams P;
+  memset(&P, 0, sizeof(P));
+  int capacity;
+  if ((rc = pick_trace_kernels(r, strict, opts->trace_depth, opts->monte_carlo_diffusion_times, opts->count_detail != 0,
+                               P, &capacity)))
+    return rc;
   if ((rc = ray_device(r))) return rc;
   const bool dev = opts->device_buffers == 1;
   if (dev && ((rc = check_device_ptr(r, rays, "rays")) || (rc = check_device_ptr(r, keys_or_null, "keys")) ||
@@ -1572,13 +1588,10 @@ int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rt
     if (keys_or_null) CUDA_TRY(cudaMemcpyAsync(p[1], keys_or_null, bytes[1], cudaMemcpyHostToDevice, s));
     B.rays = (const double*)p[0]; B.keys = (const uint32_t*)p[1]; B.rgb = (double*)p[2]; B.hit = (int32_t*)p[3];
   }
-  FrameParams P;
-  memset(&P, 0, sizeof(P));
   fill_scene_params(r, P);
   P.trace_depth = opts->trace_depth; P.mc = opts->monte_carlo_diffusion_times;
   P.width = 1; P.height = 1;  // status reports ray i as pixel (i, 0)
   P.key0 = (uint32_t)opts->seed; P.key1 = (uint32_t)(opts->seed >> 32);
-  P.count_detail = (opts->count_detail || r->n_boxes > 0) ? 1 : 0;  // the Box code lives in the detailed kernels
   FrameCtl& fc = r->ray_ctl;
   bind_ctl(P, fc);
   fc.timed = stats_out != nullptr;
@@ -1586,7 +1599,7 @@ int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rt
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev0, s));
   CUDA_TRY(cudaMemsetAsync(fc.blk, 0, sizeof(CtlBlock), s));
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
-  CUDA_TRY(rtrb_launch_trace_rays(P, B, opts->precision == RTRB_PREC_STRICT, (int)need, s));
+  CUDA_TRY(rtrb_launch_trace_rays(P, B, strict, capacity, s));
   g_launches++;
   if (fc.timed) { CUDA_TRY(cudaEventRecord(fc.evt1, s)); CUDA_TRY(cudaEventRecord(fc.ev1, s)); }
   if (!dev) {

@@ -15,8 +15,6 @@ namespace {
 
 using namespace rtrb;
 
-constexpr int kRayBlock = 128;
-
 // One thread per ray; the status of ray i is reported as pixel (i, 0) of a frame of height 1.
 template <class Pol, int MAXS, bool DETAIL, bool BVH>
 __device__ __forceinline__ void trace_rays_body(const FrameParams& P, const RayBatch& B) {
@@ -40,13 +38,13 @@ __device__ __forceinline__ void trace_rays_body(const FrameParams& P, const RayB
 }
 
 // Launch bounds as the frame kernels that run the same per-sample code free-running: the STRICT kernels, the generic
-// depth-1 kernel (Policy::d1_min_blocks) and the extra-sample ray-tree kernels (4 CTAs per SM).
+// depth-1 kernel (Policy::d1_min_blocks) and the extra-sample kernels (kExtraMinBlocks).
 template <int MAXS, bool DETAIL>
-__global__ void __launch_bounds__(kRayBlock) trace_rays_strict_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
+__global__ void __launch_bounds__(kBlock) trace_rays_strict_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
   trace_rays_body<Strict, MAXS, DETAIL, false>(P, B);
 }
 template <int MAXS, bool DETAIL, bool BVH>
-__global__ void __launch_bounds__(kRayBlock, MAXS == 1 ? Generic::d1_min_blocks : 4)
+__global__ void __launch_bounds__(kBlock, MAXS == 1 ? Generic::d1_min_blocks : kExtraMinBlocks)
     trace_rays_fast_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
   trace_rays_body<Generic::at<MAXS>, MAXS, DETAIL, BVH>(P, B);
 }
@@ -65,7 +63,7 @@ RayKernel fast_trace(bool detail, bool bvh) {
 
 // World#intersect for one ray into the ABI record, with intersect_parameters' delta.
 template <bool STRICT, bool BVH>
-__global__ void __launch_bounds__(kRayBlock) intersect_rays_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
+__global__ void __launch_bounds__(kBlock) intersect_rays_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
   const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (unsigned long long)B.n) return;
   const double* q = B.rays + i * 6ull;
@@ -97,7 +95,7 @@ __global__ void __launch_bounds__(kRayBlock) intersect_rays_kernel(const __grid_
 }
 
 // Camera#lens_func for (window pixel, sample j): the frame kernels' camera_ray.
-__global__ void __launch_bounds__(kRayBlock) camera_rays_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
+__global__ void __launch_bounds__(kBlock) camera_rays_kernel(const __grid_constant__ FrameParams P, const RayBatch B) {
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (w >= (unsigned long long)B.n) return;
   const unsigned long long S = (unsigned long long)(B.sample_end - B.sample_begin);
@@ -114,19 +112,10 @@ __global__ void __launch_bounds__(kRayBlock) camera_rays_kernel(const __grid_con
   if (B.keys_out) { B.keys_out[2ull * w] = pixel; B.keys_out[2ull * w + 1ull] = j; }
 }
 
-cudaError_t launch(RayKernel k, const FrameParams& P, const RayBatch& B, cudaStream_t s) {
-  const long long blocks = grid_size((unsigned long long)B.n, kRayBlock);
-  if (blocks <= 0) return blocks == 0 ? cudaSuccess : cudaErrorInvalidConfiguration;
-  k<<<(unsigned)blocks, kRayBlock, 0, s>>>(P, B);
-  return cudaGetLastError();
-}
-
 }  // namespace
 
-cudaError_t rtrb_launch_trace_rays(const FrameParams& P, const RayBatch& B, bool strict, int stack_need, cudaStream_t s) {
+cudaError_t rtrb_launch_trace_rays(const FrameParams& P, const RayBatch& B, bool strict, int capacity, cudaStream_t s) {
   const bool det = P.count_detail != 0, bvh = P.use_bvh != 0;
-  // the frames' capacities: STRICT always keeps a stack, FAST64 is stackless at depth <= 1
-  const int capacity = (!strict && P.trace_depth <= 1) ? 1 : stack_capacity(stack_need);
   RayKernel k = nullptr;
   switch (capacity) {
     case 1: k = fast_trace<1>(det, bvh); break;
@@ -135,15 +124,15 @@ cudaError_t rtrb_launch_trace_rays(const FrameParams& P, const RayBatch& B, bool
     case kMaxStack: k = strict ? strict_trace<kMaxStack>(det) : fast_trace<kMaxStack>(det, bvh); break;
     default: return cudaErrorInvalidValue;
   }
-  return launch(k, P, B, s);
+  return launch_cover(k, (unsigned long long)B.n, kBlock, 0, false, s, P, B);
 }
 
 cudaError_t rtrb_launch_intersect_rays(const FrameParams& P, const RayBatch& B, bool strict, cudaStream_t s) {
   RayKernel k = strict ? intersect_rays_kernel<true, false>
                        : (P.use_bvh ? intersect_rays_kernel<false, true> : intersect_rays_kernel<false, false>);
-  return launch(k, P, B, s);
+  return launch_cover(k, (unsigned long long)B.n, kBlock, 0, false, s, P, B);
 }
 
 cudaError_t rtrb_launch_camera_rays(const FrameParams& P, const RayBatch& B, cudaStream_t s) {
-  return launch(camera_rays_kernel, P, B, s);
+  return launch_cover(camera_rays_kernel, (unsigned long long)B.n, kBlock, 0, false, s, P, B);
 }

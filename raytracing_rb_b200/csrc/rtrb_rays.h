@@ -20,9 +20,9 @@ struct RayBatch {
   int32_t sample_begin, sample_end;  // camera_rays: samples j in [sample_begin, sample_end) of every window pixel
 };
 
-// stack_need = trace_depth * (1 + mc) + 1, as for frames.  P.count_detail selects the kernels with the full counters
-// (and the Box code); P.use_bvh the sphere filter.
-cudaError_t rtrb_launch_trace_rays(const FrameParams& P, const RayBatch& B, bool strict, int stack_need, cudaStream_t s);
+// capacity = trace_capacity() of the batch (rtrb_launch.h), as for frames.  P.count_detail selects the kernels with the
+// full counters (and the Box code); P.use_bvh the sphere filter.
+cudaError_t rtrb_launch_trace_rays(const FrameParams& P, const RayBatch& B, bool strict, int capacity, cudaStream_t s);
 cudaError_t rtrb_launch_intersect_rays(const FrameParams& P, const RayBatch& B, bool strict, cudaStream_t s);
 // one thread per (window pixel, sample); P holds the baked camera, the window and the lens tables
 cudaError_t rtrb_launch_camera_rays(const FrameParams& P, const RayBatch& B, cudaStream_t s);

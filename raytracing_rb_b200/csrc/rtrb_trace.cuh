@@ -804,7 +804,7 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
 
 // BVH: FAST64 with the sphere BVH instead of the linear filter.
 // BOX: the FAST64 kernels carry the Box code only in their full-counter (DETAIL) variants; scenes with a
-// box are always dispatched there (rtrb_api.cu), so the lean hot kernels stay sphere/plane-only.
+// box are always dispatched there (rtrb_api.cu, pick_trace_kernels), so the lean hot kernels stay sphere/plane-only.
 template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                              ThreadCtx& ctx, int* primary_hit) {

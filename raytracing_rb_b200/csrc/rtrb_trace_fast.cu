@@ -17,8 +17,7 @@ const FastKernels* const kBuilds[] = {
     &rtrb_fast::t128,
 };
 
-const FastKernels* build_for(const FrameParams& P, int stack_need) {
-  const int capacity = P.trace_depth <= 1 ? 1 : stack_capacity(stack_need);
+const FastKernels* build_for(const FrameParams& P, int capacity) {
   const bool one_light = (P.scene_class & RTRB_SCENE_CLASS_ONE_LIGHT) != 0;
   const bool lean = (P.scene_class & RTRB_SCENE_CLASS_LEAN) != 0;
   for (const FastKernels* k : kBuilds)
@@ -28,45 +27,26 @@ const FastKernels* build_for(const FrameParams& P, int stack_need) {
 
 }  // namespace
 
-cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int stack_need, cudaStream_t s, bool overlap) {
-  const FastKernels* k = build_for(P, stack_need);
+cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int capacity, cudaStream_t s, bool overlap) {
+  const FastKernels* k = build_for(P, capacity);
   if (!k) return cudaErrorInvalidValue;
   if (overlap && k->capacity != 1) return cudaErrorInvalidValue;  // only the depth-1 kernels wait before their writes
-  const TraceKernel kernel = k->pre[P.count_detail != 0][P.use_bvh != 0];
   // one thread per (pixel, sample); the ray-tree kernels run lockstep CTAs (rtrb_trace_fast.cuh, trace_pre_tree_body),
   // more and smaller ones on small frames
   const unsigned long long threads = pre_threads(P);
-  if (threads == 0) return cudaSuccess;
-  int block = kFastBlock;
+  int block = kBlock;
   if (k->capacity > 1) block = threads < 4ull * (unsigned long long)sm_count() * kTreeBlock ? RTRB_TREE_MIN_BLOCK : kTreeBlock;
-  const long long blocks = grid_size(threads, block);
-  if (blocks < 0) return cudaErrorInvalidConfiguration;
   // in-CTA resolve (ray-tree frames only): the host only selects it for sample counts that divide both CTA sizes
   const bool in_cta = P.fuse_resolve == RTRB_RESOLVE_IN_CTA;
   if (in_cta && (block % P.pre) != 0) return cudaErrorInvalidConfiguration;
   const size_t smem = in_cta ? (size_t)block * 3u * sizeof(double) : 0u;
-  if (!overlap) {
-    kernel<<<(unsigned)blocks, block, smem, s>>>(P);
-    return cudaGetLastError();
-  }
-  // programmatic dependent launch: may start under the tail of the previous kernel on the stream (trace_pre_body)
-  cudaLaunchAttribute attr;
-  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr.val.programmaticStreamSerializationAllowed = 1;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)blocks);
-  cfg.blockDim = dim3((unsigned)block);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cfg.attrs = &attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, P);
+  return launch_cover(k->pre[P.count_detail != 0][P.use_bvh != 0], threads, block, smem, overlap, s, P);
 }
 
-cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int stack_need, cudaStream_t s) {
-  const FastKernels* k = build_for(P, stack_need);
+cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int capacity, cudaStream_t s) {
+  const FastKernels* k = build_for(P, capacity);
   if (!k) return cudaErrorInvalidValue;
   const TraceKernel kernel = k->extra[P.count_detail != 0][P.use_bvh != 0];
-  kernel<<<extra_grid(), kFastBlock, 0, s>>>(P);
+  kernel<<<extra_grid(), kBlock, 0, s>>>(P);
   return cudaGetLastError();
 }

@@ -5,8 +5,6 @@
 
 namespace {
 
-constexpr int kBlock = 128;
-
 template <int MAXS, bool DETAIL>
 __global__ void __launch_bounds__(kBlock) trace_pre_strict_kernel(const __grid_constant__ FrameParams P) {
   rtrb::trace_pre_body<rtrb::Strict, MAXS, DETAIL>(P);
@@ -27,35 +25,27 @@ template <int MAXS, bool DETAIL>
 const StrictKernels kKernels = {trace_pre_strict_kernel<MAXS, DETAIL>, trace_extra_strict_kernel<MAXS, DETAIL>,
                                 trace_mt_strict_kernel<MAXS, DETAIL>};
 
-// the kernels of capacity stack_capacity(stack_need), with or without the detailed counters
-const StrictKernels& kernels(const FrameParams& P, int stack_need) {
+// the kernels of `capacity`, with or without the detailed counters
+const StrictKernels& kernels(const FrameParams& P, int capacity) {
   const bool det = P.count_detail != 0;
-  switch (stack_capacity(stack_need)) {
+  switch (capacity) {
     case 10: return det ? kKernels<10, true> : kKernels<10, false>;
     case 32: return det ? kKernels<32, true> : kKernels<32, false>;
     default: return det ? kKernels<128, true> : kKernels<128, false>;
   }
 }
 
-// `k` with one thread for each of `threads`
-cudaError_t launch_cover(TraceKernel k, unsigned long long threads, const FrameParams& P, cudaStream_t s) {
-  const long long blocks = grid_size(threads, kBlock);
-  if (blocks <= 0) return blocks == 0 ? cudaSuccess : cudaErrorInvalidConfiguration;
-  k<<<(unsigned)blocks, kBlock, 0, s>>>(P);
-  return cudaGetLastError();
-}
-
 }  // namespace
 
-cudaError_t rtrb_launch_trace_pre_strict(const FrameParams& P, int stack_need, cudaStream_t s) {
-  return launch_cover(kernels(P, stack_need).pre, pre_threads(P), P, s);
+cudaError_t rtrb_launch_trace_pre_strict(const FrameParams& P, int capacity, cudaStream_t s) {
+  return launch_cover(kernels(P, capacity).pre, pre_threads(P), kBlock, 0, false, s, P);
 }
-cudaError_t rtrb_launch_trace_extra_strict(const FrameParams& P, int stack_need, cudaStream_t s) {
-  const TraceKernel k = kernels(P, stack_need).extra;
+cudaError_t rtrb_launch_trace_extra_strict(const FrameParams& P, int capacity, cudaStream_t s) {
+  const TraceKernel k = kernels(P, capacity).extra;
   k<<<extra_grid(), kBlock, 0, s>>>(P);
   return cudaGetLastError();
 }
-cudaError_t rtrb_launch_trace_mt_strict(const FrameParams& P, int stack_need, cudaStream_t s) {
+cudaError_t rtrb_launch_trace_mt_strict(const FrameParams& P, int capacity, cudaStream_t s) {
   // one thread per PIXEL
-  return launch_cover(kernels(P, stack_need).mt, (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS, P, s);
+  return launch_cover(kernels(P, capacity).mt, (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS, kBlock, 0, false, s, P);
 }

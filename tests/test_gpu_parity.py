@@ -152,11 +152,14 @@ def test_device_rejects_what_it_cannot_do(oracle_mod):
         cam.renderer().render(cam.camera_desc(), make_opts(rng_mode=_abi.RNG_MT, tile_rank=0, tile_world=2))
     with pytest.raises(RtrbError):
         cam.renderer().render(cam.camera_desc(), make_opts(rng_mode=_abi.RNG_MT, seed=1 << 40))
-    c = cam.camera_desc()
-    c.trace_depth = 100
-    c.monte_carlo_diffusion_times = 4
-    with pytest.raises(RtrbError):
-        cam.renderer().render(c, make_opts())
+    # work stacks deeper than the largest kernel's: 100 * 5 + 1 = 501, and 2^30 * 2 + 1, which does not fit in 32 bits
+    for depth, mc in ((100, 4), (1 << 30, 1)):
+        c = cam.camera_desc()
+        c.trace_depth = depth
+        c.monte_carlo_diffusion_times = mc
+        with pytest.raises(RtrbError) as e:
+            cam.renderer().render(c, make_opts())
+        assert e.value.code == _abi.RTRB_ERR_UNSUPPORTED
 
 
 def test_multi_gpu_tiles_compose_in_process():

@@ -327,8 +327,9 @@ def test_ray_call_errors():
     bad = make_ray_opts(precision=7)
     assert L.rtrb_trace_rays(h, C.byref(bad), 4, rays.ctypes.data, None, rgb.ctypes.data, None, None) == inv
     assert L.rtrb_intersect_rays(h, C.byref(bad), 4, rays.ctypes.data, hits.ctypes.data) == inv
-    deep = make_ray_opts(trace_depth=43, mc=2)  # 43 * 3 + 1 = 130 > 128
-    assert L.rtrb_trace_rays(h, C.byref(deep), 4, rays.ctypes.data, None, rgb.ctypes.data, None, None) == uns
+    for depth, mc in ((43, 2), (1 << 30, 1)):  # 43 * 3 + 1 = 130 > 128; 2^30 * 2 + 1 does not fit in 32 bits
+        deep = make_ray_opts(trace_depth=depth, mc=mc)
+        assert L.rtrb_trace_rays(h, C.byref(deep), 4, rays.ctypes.data, None, rgb.ctypes.data, None, None) == uns
     assert L.rtrb_trace_rays(h, C.byref(make_ray_opts(trace_depth=-1)), 4, rays.ctypes.data, None, rgb.ctypes.data, None, None) == inv
     # device_buffers = 1 with host memory
     dv = make_ray_opts(device_buffers=True)
