@@ -11,6 +11,8 @@
  * ruby.h); INTEGRATION.md lists the build steps for a machine with Ruby.
  *
  *   Rtrb::Renderer.new(world)                      -> bakes the scene on GPU 0 (rtrb_renderer_create)
+ *   renderer.update(world)                         -> re-bakes the world's current objects and lights in place
+ *                                                     (rtrb_scene_update; nothing is queued when they did not change)
  *   renderer.render(camera, seed = 1, precision = 1) -> String of H*W*3 RGB8 bytes, row = y, col = x
  *                                                     (RTRB_FMT_RGB8: alpha is always 255, camera.rb:155)
  *   renderer.render_png(camera, seed = 1, precision = 1) -> binary String: the frame as an 8-bit RGB PNG file,
@@ -55,29 +57,36 @@ static double ivar_f(VALUE obj, const char* name, const char* what) {
 }
 static int is_a(VALUE obj, const char* klass_path) { return RTEST(rb_obj_is_kind_of(obj, rb_path2class(klass_path))); }
 
-/* Texture -> 8-bit RGB rows: Texture#to_a holds rows of Vec3(v8/256.0) (texture.rb:12-20,34-36).  The buffer is
- * entered into `td` BEFORE it is filled, so the rb_ensure cleanup frees it even when a texel conversion raises. */
-static void texture_bytes(VALUE tex, rtrb_texture_desc* td) {
+/* Texture -> 8-bit RGB rows: Texture#to_a holds rows of Vec3(v8/256.0) (texture.rb:12-20,34-36).  Converted once per
+ * Texture object: `cache` (an identity Hash held by the renderer) keeps the bytes as a String, so Renderer#update, which
+ * runs before every frame, does not walk the texels again.  A Texture is never edited after it was decoded
+ * (texture.rb:12-20). */
+static void texture_bytes(VALUE tex, VALUE cache, rtrb_texture_desc* td) {
   const int w = NUM2INT(rb_funcall(tex, rb_intern("width"), 0));
   const int h = NUM2INT(rb_funcall(tex, rb_intern("height"), 0));
-  VALUE rows = rb_funcall(tex, rb_intern("to_a"), 0);
-  uint8_t* px = (uint8_t*)malloc((size_t)w * h * 3);
-  if (!px) rb_raise(rb_eNoMemError, "rtrb_b200: texture buffer");
-  td->rgb8 = px; td->width = w; td->height = h;
-  for (int y = 0; y < h; ++y) {
-    VALUE row = rb_ary_entry(rows, y);
-    for (int x = 0; x < w; ++x) {
-      double c[3];
-      vec3_into(rb_ary_entry(row, x), c, "texel");
-      for (int k = 0; k < 3; ++k) px[((size_t)y * w + x) * 3 + k] = (uint8_t)(c[k] * 256.0 + 0.5);
+  VALUE bytes = rb_hash_aref(cache, tex);
+  if (NIL_P(bytes)) {
+    VALUE rows = rb_funcall(tex, rb_intern("to_a"), 0);
+    bytes = rb_str_new(NULL, (long)w * h * 3);
+    uint8_t* px = (uint8_t*)RSTRING_PTR(bytes);
+    for (int y = 0; y < h; ++y) {
+      VALUE row = rb_ary_entry(rows, y);
+      for (int x = 0; x < w; ++x) {
+        double c[3];
+        vec3_into(rb_ary_entry(row, x), c, "texel");
+        for (int k = 0; k < 3; ++k) px[((size_t)y * w + x) * 3 + k] = (uint8_t)(c[k] * 256.0 + 0.5);
+      }
     }
+    rb_hash_aset(cache, tex, bytes);  /* only once complete */
   }
+  td->rgb8 = (const uint8_t*)RSTRING_PTR(bytes); td->width = w; td->height = h;
 }
 
 /* Flattening World -> rtrb_scene_desc can raise half way (a nil ivar, a non-numeric value: vec3_into / ivar_f call
- * rb_raise).  The scratch arrays therefore live in a struct that rb_ensure frees whether the body returns or raises. */
+ * rb_raise).  The scratch arrays therefore live in a struct that rb_ensure frees whether the body returns or raises
+ * (texture bytes belong to the renderer's cache). */
 typedef struct {
-  VALUE self, world;
+  VALUE self, world, texture_cache;
   rtrb_object_desc* od;
   rtrb_light_desc* ld;
   rtrb_texture_desc* td;
@@ -86,13 +95,13 @@ typedef struct {
 
 static VALUE init_cleanup(VALUE p) {
   init_call* c = (init_call*)p;
-  for (int i = 0; i < c->n_tex; ++i) free((void*)c->td[i].rgb8);
   free(c->od); free(c->ld); free(c->td);
   return Qnil;
 }
 
-static VALUE init_body(VALUE p) {
-  init_call* c = (init_call*)p;
+/* World -> rtrb_scene_desc: what Renderer.new and Renderer#update hand to the library.  The scratch arrays stay in `c`
+ * until its rb_ensure cleanup runs. */
+static void flatten_world(init_call* c, rtrb_scene_desc* sd) {
   VALUE world = c->world;
   VALUE objs = ivar(world, "@world_objects"), lights = ivar(world, "@lights");
   long n_obj = RARRAY_LEN(objs), n_li = RARRAY_LEN(lights);
@@ -106,8 +115,8 @@ static VALUE init_body(VALUE p) {
     d->texture = -1;
     VALUE tex = ivar(o, "@texture");
     if (!NIL_P(tex)) {
-      d->texture = c->n_tex++;          /* counted first: init_cleanup then frees a half-filled buffer too */
-      texture_bytes(tex, &td[d->texture]);
+      d->texture = c->n_tex++;
+      texture_bytes(tex, c->texture_cache, &td[d->texture]);
       /* what Texture#color really uses (texture.rb:9-10,15-16,24-25): the Texture object's own scales and offsets.
        * Sphere passes its texture_u/v_offset on (sphere.rb:25); Plane and Box do not (plane.rb:35, box.rb:76), so
        * their textures keep 0.0 whatever the YAML says. */
@@ -166,13 +175,17 @@ static VALUE init_body(VALUE p) {
     ld[i].high_light_rate = ivar_f(l, "@high_light_rate", "high_light_rate");
     ld[i].high_light_angle = ivar_f(l, "@high_light_angle", "high_light_angle");
   }
-  rtrb_scene_desc sd;
-  memset(&sd, 0, sizeof(sd));
-  sd.max_distance = ivar_f(world, "@max_distance", "max_distance");
-  sd.soft_shadow_exponent = ivar_f(world, "@soft_shadow_exponent", "soft_shadow_exponent");
-  sd.n_objects = (int32_t)n_obj; sd.n_lights = (int32_t)n_li; sd.n_textures = c->n_tex;
-  sd.objects = od; sd.lights = ld; sd.textures = td;
+  memset(sd, 0, sizeof(*sd));
+  sd->max_distance = ivar_f(world, "@max_distance", "max_distance");
+  sd->soft_shadow_exponent = ivar_f(world, "@soft_shadow_exponent", "soft_shadow_exponent");
+  sd->n_objects = (int32_t)n_obj; sd->n_lights = (int32_t)n_li; sd->n_textures = c->n_tex;
+  sd->objects = od; sd->lights = ld; sd->textures = td;
+}
 
+static VALUE init_body(VALUE p) {
+  init_call* c = (init_call*)p;
+  rtrb_scene_desc sd;
+  flatten_world(c, &sd);
   shim_renderer* s;
   Data_Get_Struct(c->self, shim_renderer, s);
   int rc = rtrb_renderer_create(&sd, 0, &s->r);
@@ -180,11 +193,41 @@ static VALUE init_body(VALUE p) {
   return c->self;
 }
 
+/* The library compares the new bake with the current one: an unchanged world queues nothing. */
+static VALUE update_body(VALUE p) {
+  init_call* c = (init_call*)p;
+  rtrb_scene_desc sd;
+  flatten_world(c, &sd);
+  shim_renderer* s;
+  Data_Get_Struct(c->self, shim_renderer, s);
+  int rc = rtrb_scene_update(s->r, &sd, NULL);
+  if (rc != RTRB_OK) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());
+  return c->self;
+}
+
+/* The renderer's Texture -> bytes cache (texture_bytes), made on first use. */
+static VALUE texture_cache(VALUE self) {
+  VALUE cache = rb_iv_get(self, "@texture_bytes");
+  if (NIL_P(cache)) {
+    cache = rb_hash_new();
+    rb_funcall(cache, rb_intern("compare_by_identity"), 0);
+    rb_iv_set(self, "@texture_bytes", cache);
+  }
+  return cache;
+}
+
 static VALUE renderer_initialize(VALUE self, VALUE world) {
   init_call c;
   memset(&c, 0, sizeof(c));
-  c.self = self; c.world = world;
+  c.self = self; c.world = world; c.texture_cache = texture_cache(self);
   return rb_ensure(init_body, (VALUE)&c, init_cleanup, (VALUE)&c);
+}
+
+static VALUE renderer_update(VALUE self, VALUE world) {
+  init_call c;
+  memset(&c, 0, sizeof(c));
+  c.self = self; c.world = world; c.texture_cache = texture_cache(self);
+  return rb_ensure(update_body, (VALUE)&c, init_cleanup, (VALUE)&c);
 }
 
 static VALUE renderer_alloc(VALUE klass) {
@@ -349,6 +392,7 @@ void Init_rtrb_b200(void) {
   cRenderer = rb_define_class_under(mRtrb, "Renderer", rb_cObject);
   rb_define_alloc_func(cRenderer, renderer_alloc);
   rb_define_method(cRenderer, "initialize", renderer_initialize, 1);
+  rb_define_method(cRenderer, "update", renderer_update, 1);
   rb_define_method(cRenderer, "render", renderer_render, -1);
   rb_define_method(cRenderer, "render_png", renderer_render_png, -1);
   rb_define_method(cRenderer, "stats", renderer_stats, 0);

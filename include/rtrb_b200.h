@@ -210,6 +210,20 @@ int rtrb_device_count(int* count_out);
 int rtrb_renderer_create(const rtrb_scene_desc* scene, int device, rtrb_renderer** out);
 int rtrb_renderer_destroy(rtrb_renderer* r);
 
+/* Replaces the renderer's baked scene with `scene` (same description, rules and errors as rtrb_renderer_create), for
+ * scenes that change between frames (World edits, animation).  Ordered on `stream` (NULL = the renderer's own):
+ *   - every frame, rtrb_submit frame or ray call queued before the update, on any stream this renderer has launched
+ *     on, sees the old scene; everything issued after it sees the new one (the first such launch on each stream
+ *     waits for the update's copies, and a depth-1 frame does not overlap the kernel before it);
+ *   - a stream that such a call used should outlive the next update; if it was destroyed meanwhile, that update
+ *     waits for the whole device instead (the work the stream had queued still runs);
+ *   - a rejected scene (RTRB_ERR_INVALID / RTRB_ERR_UNSUPPORTED) leaves the old one fully in force;
+ *   - a scene whose bake equals the current one queues nothing;
+ *   - framebuffers (and exported device pointers / IPC handles), pipeline slots and tickets are not touched.
+ * The scene is copied from pinned staging memory: the call returns without waiting for the device, except for the
+ * previous update's copies, and for its device to go idle when that update had to grow a scene buffer. */
+int rtrb_scene_update(rtrb_renderer* r, const rtrb_scene_desc* scene, void* stream);
+
 /* -- the hot path ---------------------------------------------------------------------------- */
 /* Renders one frame into DEVICE buffers (async on opts->stream unless stats_out != NULL, which
  * synchronises).  Replaces the pixel loops camera.rb:59-63 and :102-106.

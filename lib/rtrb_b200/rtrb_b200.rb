@@ -4,6 +4,7 @@ module Rtrb
   class Renderer
     # method stubs
     def initialize(world); raise NotImplementedError; end
+    def update(world); raise NotImplementedError; end
     def render(camera, seed = 1, precision = 1); raise NotImplementedError; end
     def render_png(camera, seed = 1, precision = 1); raise NotImplementedError; end
     def stats; raise NotImplementedError; end
@@ -19,8 +20,9 @@ require_relative '../rtrb_b200'
 # returns the finished 8-bit rows, which go through the existing canvas + save_image (:36-39).
 module Alex
   class Camera
+    # Edits of @world's objects and lights since the last frame reach this one (Renderer#update re-bakes them in place).
     def render_cuda(file_path, seed = 1)
-      @rtrb ||= Rtrb::Renderer.new(@world)
+      rtrb_renderer
       rgb = @rtrb.render(self, seed)           # H*W*3 bytes (RGB8), row = y, column = x
       @height.times do |y|
         @width.times do |x|
@@ -34,8 +36,18 @@ module Alex
 
     # save_image's file without the canvas: the GPU renders and encodes the PNG (8-bit RGB), only the file crosses PCIe
     def render_cuda_png(file_path, seed = 1)
-      @rtrb ||= Rtrb::Renderer.new(@world)
+      rtrb_renderer
       File.binwrite(file_path, @rtrb.render_png(self, seed))
+    end
+
+    private
+
+    def rtrb_renderer
+      if @rtrb
+        @rtrb.update(@world)
+      else
+        @rtrb = Rtrb::Renderer.new(@world)
+      end
     end
   end
 end

@@ -11,7 +11,7 @@ LIB_PATH = os.environ.get("RTRB_B200_LIB") or os.path.join(_HERE, "csrc", "librt
 
 EXPORTS = (
     "rtrb_abi_version", "rtrb_last_error", "rtrb_device_count",
-    "rtrb_renderer_create", "rtrb_renderer_destroy",
+    "rtrb_renderer_create", "rtrb_renderer_destroy", "rtrb_scene_update",
     "rtrb_render_device", "rtrb_download", "rtrb_render", "rtrb_submit", "rtrb_wait",
     "rtrb_framebuffer_device_ptr", "rtrb_framebuffer_download", "rtrb_framebuffer_copy_async", "rtrb_framebuffer_ipc_export", "rtrb_ipc_open", "rtrb_ipc_close",
     "rtrb_peer_push", "rtrb_peer_push_join",
@@ -44,6 +44,7 @@ def lib():
     L.rtrb_device_count.argtypes = [P(C.c_int)]
     L.rtrb_renderer_create.argtypes = [P(_abi.SceneDesc), C.c_int, P(C.c_void_p)]
     L.rtrb_renderer_destroy.argtypes = [C.c_void_p]
+    L.rtrb_scene_update.argtypes = [C.c_void_p, P(_abi.SceneDesc), C.c_void_p]
     L.rtrb_render_device.argtypes = [C.c_void_p, P(_abi.CameraDesc), P(_abi.RenderOpts), P(_abi.Stats)]
     L.rtrb_download.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.rtrb_render.argtypes = [C.c_void_p, P(_abi.CameraDesc), P(_abi.RenderOpts), C.c_void_p, C.c_void_p,

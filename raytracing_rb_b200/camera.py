@@ -13,7 +13,8 @@ import numpy as np
 
 from . import _abi
 from .configurable_object import ConfigurableObject
-from .renderer import Renderer, make_opts, render_multi
+from .renderer import make_opts, render_multi
+from .world import synced_renderer
 
 
 def write_png(path, rgba):
@@ -84,10 +85,9 @@ class Camera(ConfigurableObject):
         return c
 
     def renderer(self, device=None):
-        device = self.device if device is None else device
-        if device not in self._renderers:
-            self._renderers[device] = Renderer(self.world.to_scene_desc(), device)
-        return self._renderers[device]
+        """This camera's renderer on `device` (one per device, made on first use), brought up to date with the world:
+        edits of its objects and lights since the last call reach the next frame."""
+        return synced_renderer(self._renderers, self.device if device is None else device, self.world)
 
     # -- the hot path -----------------------------------------------------------------------------
     def render_frame(self, gpus=1, seed=1, precision=_abi.PREC_DEFAULT, window=None, count_detail=False,

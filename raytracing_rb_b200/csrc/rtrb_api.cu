@@ -17,6 +17,8 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "../../include/rtrb_b200.h"
@@ -324,6 +326,57 @@ struct MtState {
   }
 };
 
+// The baked scene on the host: every fact the frames read from the renderer and the contents of every scene buffer.
+// build_scene_image makes it from a descriptor (pure host); apply_scene puts it on the device.  Two images of the same
+// description are equal byte for byte (same_image).
+struct SceneImage {
+  struct Facts {  // memset before use: compared as bytes
+    int n_objects, n_lights, n_boxes, n_sph, n_pl;
+    int scene_class;             // RTRB_SCENE_CLASS_* bits (FrameParams::scene_class)
+    int small_scene;             // <= 32 spheres/boxes, <= 8 planes, <= 2 lights: linear-filter kernels
+    double max_distance, soft_shadow_exponent;
+    float m_scene, max_distance_f;
+    // small scenes: the per-ray tables that travel in the kernel parameters (FrameParams::k_*)
+    struct SmallTables {
+      float4 light_tab[RTRB_K_LIGHTS][RTRB_APEX_MAX];
+      float4 cull_sph[RTRB_APEX_MAX];
+      float4 cull_pl[2 * RTRB_K_PLANES];
+      DevLight lights[RTRB_K_LIGHTS];
+      DevLightF lights_f[RTRB_K_LIGHTS];
+      int32_t pl_index[RTRB_K_PLANES];
+      int32_t has_light_tab;
+    } k;
+  } f;
+  std::vector<double> sph_world;       // (cx, cy, cz, R) in cull_sph[] order, FP64, for the per-frame camera table
+  std::vector<DevGeom> geom;
+  std::vector<DevMat> mat;             // DevMat::tex left NULL: the device copy points at textures[mat_tex[i]]
+  std::vector<int32_t> mat_tex;        // texture index of each object, -1 = none
+  std::vector<DevLight> lights;
+  std::vector<DevBox> boxes;
+  std::vector<float4> cull_sph, cull_pl;  // FP32 filter view (FAST64)
+  std::vector<int32_t> sph_index, pl_index;
+  std::vector<DevLightF> lights_f;
+  std::vector<BvhNode> bvh;
+  std::vector<float4> light_tab;       // apex tables of the lights (linear-filter scenes with spheres and lights)
+  std::vector<std::vector<uint8_t>> textures;
+};
+
+template <typename T>
+bool same_bytes(const std::vector<T>& a, const std::vector<T>& b) {
+  return a.size() == b.size() && (a.empty() || memcmp(a.data(), b.data(), a.size() * sizeof(T)) == 0);
+}
+
+bool same_image(const SceneImage& a, const SceneImage& b) {
+  if (memcmp(&a.f, &b.f, sizeof(a.f)) != 0 || a.textures.size() != b.textures.size()) return false;
+  for (size_t i = 0; i < a.textures.size(); ++i)
+    if (!same_bytes(a.textures[i], b.textures[i])) return false;
+  return same_bytes(a.sph_world, b.sph_world) && same_bytes(a.geom, b.geom) && same_bytes(a.mat, b.mat) &&
+         same_bytes(a.mat_tex, b.mat_tex) && same_bytes(a.lights, b.lights) && same_bytes(a.boxes, b.boxes) &&
+         same_bytes(a.cull_sph, b.cull_sph) && same_bytes(a.cull_pl, b.cull_pl) && same_bytes(a.sph_index, b.sph_index) &&
+         same_bytes(a.pl_index, b.pl_index) && same_bytes(a.lights_f, b.lights_f) && same_bytes(a.bvh, b.bvh) &&
+         same_bytes(a.light_tab, b.light_tab);
+}
+
 }  // namespace
 
 struct rtrb_renderer {
@@ -341,35 +394,26 @@ struct rtrb_renderer {
   cudaStream_t ring_stream = nullptr;
   bool pipe_ready = false;
   unsigned next_ticket = 0;
-  // baked scene
-  int n_objects = 0, n_lights = 0, n_boxes = 0;
-  double max_distance = 0, soft_shadow_exponent = 0;
+  // baked scene: its host image and the device buffers that hold it
+  SceneImage scene;
   DevBuf<DevGeom> geom;
   DevBuf<DevMat> mat;
   DevBuf<DevLight> lights;
   DevBuf<DevBox> boxes;
-  // FP32 filter view (FAST64)
   DevBuf<float4> cull_sph, cull_pl;
   DevBuf<BvhNode> bvh;
-  DevBuf<float4> light_tab;            // apex tables of the lights (linear-filter scenes)
-  // small scenes: host copy of the per-ray tables that travel in the kernel parameters (FrameParams::k_*)
-  struct SmallTables {
-    float4 light_tab[RTRB_K_LIGHTS][RTRB_APEX_MAX];
-    float4 cull_sph[RTRB_APEX_MAX];
-    float4 cull_pl[2 * RTRB_K_PLANES];
-    DevLight lights[RTRB_K_LIGHTS];
-    DevLightF lights_f[RTRB_K_LIGHTS];
-    int32_t pl_index[RTRB_K_PLANES];
-    int32_t has_light_tab;
-  } k;
-  int scene_class = 0;                 // RTRB_SCENE_CLASS_* bits (FrameParams::scene_class)
-  bool small_scene = false;            // <= 32 spheres/boxes, <= 8 planes, <= 2 lights: linear-filter kernels
-  std::vector<double> sph_world;       // (cx, cy, cz, R) in cull_sph[] order, FP64, for the per-frame camera table
+  DevBuf<float4> light_tab;
   DevBuf<int32_t> sph_index, pl_index;
   DevBuf<DevLightF> lights_f;
-  int n_sph = 0, n_pl = 0;
-  float m_scene = 0.0f, max_distance_f = 0.0f;
   std::vector<DevBuf<uint8_t>> textures;  // DevMat::tex holds their addresses
+  // rtrb_scene_update ordering (DESIGN.md §13)
+  unsigned scene_gen = 0;                 // updates so far
+  std::vector<cudaStream_t> scene_streams;  // streams that launched scene-reading work since the last bake
+  cudaEvent_t scene_prior_ev = nullptr;   // recorded on each of them by an update, waited for by its copies
+  cudaEvent_t scene_ready_ev = nullptr;   // the last update's copies are done
+  uint8_t* staging = nullptr;             // pinned: the host side of an update's copies
+  size_t staging_bytes = 0;
+  std::vector<void*> retired;             // scene buffers an update outgrew; freed once the work before it is done
   // per-frame caches and scratch
   TileList tiles;
   LensTable lens;
@@ -392,7 +436,9 @@ struct rtrb_renderer {
   LensTable ray_lens;                  // rtrb_camera_rays
   // The members free their own device memory; the renderer's device must be current (rtrb_renderer_destroy).
   ~rtrb_renderer() {
-    for (cudaEvent_t ev : {push_ev, push_done_ev, png_ev})
+    for (void* p : retired) cudaFree(p);
+    if (staging) cudaFreeHost(staging);
+    for (cudaEvent_t ev : {push_ev, push_done_ev, png_ev, scene_prior_ev, scene_ready_ev})
       if (ev) cudaEventDestroy(ev);
     for (cudaStream_t s : {stream, copy_stream})
       if (s) cudaStreamDestroy(s);
@@ -520,30 +566,33 @@ int validate_scene(const rtrb_scene_desc* s) {
   return RTRB_OK;
 }
 
-int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
-  r->n_objects = s->n_objects;
-  r->n_lights = s->n_lights;
-  r->max_distance = s->max_distance;
-  r->soft_shadow_exponent = s->soft_shadow_exponent;
+// Descriptor -> host image of the baked scene (validate_scene has accepted `s`).  Pure host: no device is needed.
+void build_scene_image(const rtrb_scene_desc* s, SceneImage& img) {
+  SceneImage::Facts& fa = img.f;
+  memset(&fa, 0, sizeof(fa));
+  fa.n_objects = s->n_objects;
+  fa.n_lights = s->n_lights;
+  fa.max_distance = s->max_distance;
+  fa.soft_shadow_exponent = s->soft_shadow_exponent;
   {
     bool textured = false;
     for (int i = 0; i < s->n_objects; ++i) textured = textured || (s->objects[i].texture >= 0 && s->objects[i].type != RTRB_OBJ_BOX);
-    r->scene_class = 0;
     if (s->n_lights == 1 && s->soft_shadow_exponent == 2.0) {
-      r->scene_class |= RTRB_SCENE_CLASS_ONE_LIGHT;
-      if (s->lights[0].radius == 0.0 && !textured) r->scene_class |= RTRB_SCENE_CLASS_LEAN;
+      fa.scene_class |= RTRB_SCENE_CLASS_ONE_LIGHT;
+      if (s->lights[0].radius == 0.0 && !textured) fa.scene_class |= RTRB_SCENE_CLASS_LEAN;
     }
   }
+  img.textures.resize(s->n_textures);
   for (int i = 0; i < s->n_textures; ++i) {
     const rtrb_texture_desc& t = s->textures[i];
-    size_t bytes = (size_t)t.width * t.height * 3;
-    r->textures.emplace_back();
-    CUDA_TRY(r->textures.back().ensure(bytes));
-    CUDA_TRY(cudaMemcpy(r->textures.back().p, t.rgb8, bytes, cudaMemcpyHostToDevice));
+    img.textures[i].assign(t.rgb8, t.rgb8 + (size_t)t.width * t.height * 3);
   }
-  std::vector<DevGeom> geom(s->n_objects);
-  std::vector<DevMat> mat(s->n_objects);
-  std::vector<DevBox> boxes;
+  std::vector<DevGeom>& geom = img.geom;
+  std::vector<DevMat>& mat = img.mat;
+  std::vector<DevBox>& boxes = img.boxes;
+  geom.resize(s->n_objects);
+  mat.resize(s->n_objects);
+  img.mat_tex.assign(s->n_objects, -1);
   std::vector<double> box_radius;  // filter bound per box (INFINITY = none)
   for (int i = 0; i < s->n_objects; ++i) {
     const rtrb_object_desc& o = s->objects[i];
@@ -607,7 +656,7 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
     m.hscale = o.texture_horizontal_scale; m.vscale = o.texture_vertical_scale;
     m.uoff = o.texture_u_offset; m.voff = o.texture_v_offset;
     if (o.texture >= 0 && o.type != RTRB_OBJ_BOX) {  // a box never samples its texture (box.rb has no local_lighting)
-      m.tex = r->textures[o.texture].p;
+      img.mat_tex[i] = o.texture;
       m.tex_w = s->textures[o.texture].width;
       m.tex_h = s->textures[o.texture].height;
       if (o.type == RTRB_OBJ_SPHERE) {
@@ -621,7 +670,8 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
       }
     }
   }
-  std::vector<DevLight> lights(s->n_lights);
+  std::vector<DevLight>& lights = img.lights;
+  lights.resize(s->n_lights);
   for (int i = 0; i < s->n_lights; ++i) {
     const rtrb_light_desc& l = s->lights[i];
     DevLight& d = lights[i];
@@ -634,8 +684,10 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
     d.hl_threshold = l.high_light_angle / 180.0 * 3.141592653589793;  // world.rb:92
   }
   // ---- FP32 filter view: conversions round to nearest; the filter's margins cover that error ----
-  std::vector<float4> csph, cpl;
-  std::vector<int32_t> isph, ipl;
+  std::vector<float4>& csph = img.cull_sph;
+  std::vector<float4>& cpl = img.cull_pl;
+  std::vector<int32_t>& isph = img.sph_index;
+  std::vector<int32_t>& ipl = img.pl_index;
   std::vector<BvhBuildSphere> bsph;
   float m_scene = 0.0f;
   for (int i = 0; i < s->n_objects; ++i) {
@@ -659,9 +711,8 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
     }
   }
   // the BVH build reorders the spheres so that every leaf is a contiguous run of cull_sph[]
-  std::vector<BvhNode> nodes;
-  r->small_scene = (int)bsph.size() <= RTRB_BVH_MIN_SPHERES && (int)ipl.size() <= RTRB_K_PLANES && s->n_lights <= RTRB_K_LIGHTS;
-  if (!r->small_scene) nodes = rtrb_bvh::build_tree(bsph);
+  fa.small_scene = (int)bsph.size() <= RTRB_BVH_MIN_SPHERES && (int)ipl.size() <= RTRB_K_PLANES && s->n_lights <= RTRB_K_LIGHTS;
+  if (!fa.small_scene) img.bvh = rtrb_bvh::build_tree(bsph);
   for (const BvhBuildSphere& bs : bsph) {
     float w = (float)bs.r;
     if (bs.bound_only) {  // rounded up, sign bit set
@@ -673,30 +724,26 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
     csph.push_back(make_float4((float)bs.c[0], (float)bs.c[1], (float)bs.c[2], w));
     isph.push_back(bs.world_index);
   }
-  CUDA_TRY(r->bvh.ensure(std::max<size_t>(1, nodes.size())));
-  if (!nodes.empty()) CUDA_TRY(cudaMemcpy(r->bvh.p, nodes.data(), nodes.size() * sizeof(BvhNode), cudaMemcpyHostToDevice));
-  r->n_sph = (int)isph.size(); r->n_pl = (int)ipl.size();
-  r->sph_world.clear();
-  for (const BvhBuildSphere& bs : bsph) { for (int k = 0; k < 3; ++k) r->sph_world.push_back(bs.c[k]); r->sph_world.push_back(bs.r); }
-  memset(&r->k, 0, sizeof(r->k));
-  if (r->small_scene && !bsph.empty() && s->n_lights > 0) {
-    std::vector<float4> lt((size_t)s->n_lights * bsph.size());
+  fa.n_sph = (int)isph.size(); fa.n_pl = (int)ipl.size();
+  for (const BvhBuildSphere& bs : bsph) { for (int k = 0; k < 3; ++k) img.sph_world.push_back(bs.c[k]); img.sph_world.push_back(bs.r); }
+  if (fa.small_scene && !bsph.empty() && s->n_lights > 0) {
+    std::vector<float4>& lt = img.light_tab;
+    lt.resize((size_t)s->n_lights * bsph.size());
     for (int l = 0; l < s->n_lights; ++l) {
       double lm = fmax(fabs(s->lights[l].position[0]), fmax(fabs(s->lights[l].position[1]), fabs(s->lights[l].position[2])));
       for (size_t k = 0; k < bsph.size(); ++k)
         lt[(size_t)l * bsph.size() + k] = apex_entry(s->lights[l].position, 0.0, bsph[k].c, bsph[k].r, (double)m_scene + lm);
     }
-    CUDA_TRY(r->light_tab.ensure(lt.size()));
-    CUDA_TRY(cudaMemcpy(r->light_tab.p, lt.data(), lt.size() * sizeof(float4), cudaMemcpyHostToDevice));
     for (int l = 0; l < RTRB_K_LIGHTS; ++l)
       for (int k = 0; k < RTRB_APEX_MAX; ++k)
-        r->k.light_tab[l][k] = (l < s->n_lights && k < (int)bsph.size()) ? lt[(size_t)l * bsph.size() + k]
+        fa.k.light_tab[l][k] = (l < s->n_lights && k < (int)bsph.size()) ? lt[(size_t)l * bsph.size() + k]
                                                                         : make_float4(0.0f, 0.0f, 0.0f, INFINITY);
-    r->k.has_light_tab = 1;
+    fa.k.has_light_tab = 1;
   }
-  r->m_scene = m_scene;
-  r->max_distance_f = nextafterf((float)s->max_distance, INFINITY);
-  std::vector<DevLightF> lf(s->n_lights);
+  fa.m_scene = m_scene;
+  fa.max_distance_f = nextafterf((float)s->max_distance, INFINITY);
+  std::vector<DevLightF>& lf = img.lights_f;
+  lf.resize(s->n_lights);
   for (int i = 0; i < s->n_lights; ++i) {
     const rtrb_light_desc& l = s->lights[i];
     double thr = l.high_light_angle / 180.0 * 3.141592653589793;
@@ -706,38 +753,110 @@ int bake_scene(rtrb_renderer* r, const rtrb_scene_desc* s) {
     double c = cos(thr);
     lf[i].cos2_thr = (float)(c * c);
   }
-  if (r->small_scene) {
-    for (size_t k = 0; k < csph.size(); ++k) r->k.cull_sph[k] = csph[k];
-    for (size_t k = 0; k < cpl.size(); ++k) r->k.cull_pl[k] = cpl[k];
-    for (size_t k = 0; k < ipl.size(); ++k) r->k.pl_index[k] = ipl[k];
-    for (int l = 0; l < s->n_lights; ++l) { r->k.lights[l] = lights[l]; r->k.lights_f[l] = lf[l]; }
+  if (fa.small_scene) {
+    for (size_t k = 0; k < csph.size(); ++k) fa.k.cull_sph[k] = csph[k];
+    for (size_t k = 0; k < cpl.size(); ++k) fa.k.cull_pl[k] = cpl[k];
+    for (size_t k = 0; k < ipl.size(); ++k) fa.k.pl_index[k] = ipl[k];
+    for (int l = 0; l < s->n_lights; ++l) { fa.k.lights[l] = lights[l]; fa.k.lights_f[l] = lf[l]; }
   }
-  CUDA_TRY(r->cull_sph.ensure(std::max<size_t>(1, csph.size())));
-  CUDA_TRY(r->sph_index.ensure(std::max<size_t>(1, isph.size())));
-  CUDA_TRY(r->cull_pl.ensure(std::max<size_t>(1, cpl.size())));
-  CUDA_TRY(r->pl_index.ensure(std::max<size_t>(1, ipl.size())));
-  CUDA_TRY(r->lights_f.ensure(std::max<size_t>(1, lf.size())));
-  if (!csph.empty()) {
-    CUDA_TRY(cudaMemcpy(r->cull_sph.p, csph.data(), csph.size() * sizeof(float4), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(r->sph_index.p, isph.data(), isph.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  fa.n_boxes = (int)boxes.size();
+}
+
+// Calls f(device buffer, host image of it, least element count) for every scene buffer; the textures come before `mat`,
+// whose device copy holds their addresses.
+template <class F>
+void for_each_scene_buffer(rtrb_renderer* r, const SceneImage& img, F&& f) {
+  for (size_t i = 0; i < img.textures.size(); ++i) f(r->textures[i], img.textures[i], 1);
+  f(r->mat, img.mat, 1);
+  f(r->geom, img.geom, 1);
+  f(r->lights, img.lights, 1);
+  f(r->boxes, img.boxes, 1);
+  f(r->cull_sph, img.cull_sph, 1);
+  f(r->sph_index, img.sph_index, 1);
+  f(r->cull_pl, img.cull_pl, 1);
+  f(r->pl_index, img.pl_index, 1);
+  f(r->lights_f, img.lights_f, 1);
+  f(r->bvh, img.bvh, 1);
+  f(r->light_tab, img.light_tab, 0);
+}
+
+// The allocations of one apply_scene that replace buffers too small for the new image, in for_each_scene_buffer order
+// (nullptr: the current buffer is kept).  What is not handed over is freed.
+struct FreshBuffers {
+  std::vector<std::pair<void*, size_t>> a;  // (allocation, elements)
+  ~FreshBuffers() {
+    for (const auto& x : a)
+      if (x.first) cudaFree(x.first);
   }
-  if (!ipl.empty()) {
-    CUDA_TRY(cudaMemcpy(r->cull_pl.p, cpl.data(), cpl.size() * sizeof(float4), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(r->pl_index.p, ipl.data(), ipl.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+};
+
+// Host image -> the renderer's device buffers, through the pinned staging buffer, asynchronously on `s` (the caller
+// orders `s` after every reader of the old contents and has made sure the staging buffer is free).  Then the image
+// becomes the renderer's scene.  Every allocation is made first: when one fails, the renderer is left as it was.  A
+// buffer that is outgrown is retired, not freed: work queued before the bake may still read it.
+int apply_scene(rtrb_renderer* r, SceneImage& img, cudaStream_t s) {
+  const size_t kAlign = 256;
+  auto padded = [&](size_t bytes) { return (bytes + kAlign - 1) & ~(kAlign - 1); };
+  if (r->textures.size() < img.textures.size()) r->textures.resize(img.textures.size());  // empty until committed
+  size_t total = 0;
+  FreshBuffers fresh;
+  cudaError_t e = cudaSuccess;
+  for_each_scene_buffer(r, img, [&](auto& buf, const auto& v, size_t min_n) {
+    total += padded(v.size() * sizeof(v[0]));
+    const size_t want = std::max(min_n, v.size());
+    void* q = nullptr;
+    if (e == cudaSuccess && want > 0 && (want > buf.n || !buf.p)) e = cudaMalloc(&q, want * sizeof(v[0]));
+    fresh.a.emplace_back(q, want);
+  });
+  if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "scene buffer allocation failed: %s", cudaGetErrorString(e));
+  if (total > r->staging_bytes) {
+    if (r->staging) CUDA_TRY(cudaFreeHost(r->staging));
+    r->staging = nullptr;
+    r->staging_bytes = 0;
+    CUDA_TRY(cudaHostAlloc((void**)&r->staging, total, cudaHostAllocDefault));
+    r->staging_bytes = total;
   }
-  if (!lf.empty()) CUDA_TRY(cudaMemcpy(r->lights_f.p, lf.data(), lf.size() * sizeof(DevLightF), cudaMemcpyHostToDevice));
-  CUDA_TRY(r->geom.ensure(std::max(1, s->n_objects)));
-  CUDA_TRY(r->mat.ensure(std::max(1, s->n_objects)));
-  CUDA_TRY(r->lights.ensure(std::max(1, s->n_lights)));
-  CUDA_TRY(r->boxes.ensure(std::max<size_t>(1, boxes.size())));
-  r->n_boxes = (int)boxes.size();
-  if (!boxes.empty()) CUDA_TRY(cudaMemcpy(r->boxes.p, boxes.data(), boxes.size() * sizeof(DevBox), cudaMemcpyHostToDevice));
-  if (s->n_objects) {
-    CUDA_TRY(cudaMemcpy(r->geom.p, geom.data(), geom.size() * sizeof(DevGeom), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(r->mat.p, mat.data(), mat.size() * sizeof(DevMat), cudaMemcpyHostToDevice));
+  // commit: nothing below allocates
+  while (r->textures.size() > img.textures.size()) {
+    r->retired.push_back(r->textures.back().detach());
+    r->textures.pop_back();
   }
-  if (s->n_lights)
-    CUDA_TRY(cudaMemcpy(r->lights.p, lights.data(), lights.size() * sizeof(DevLight), cudaMemcpyHostToDevice));
+  size_t k = 0;
+  for_each_scene_buffer(r, img, [&](auto& buf, const auto&, size_t) {
+    const std::pair<void*, size_t> x = fresh.a[k];
+    fresh.a[k++].first = nullptr;
+    if (!x.first) return;
+    if (buf.p) r->retired.push_back(buf.detach());
+    buf.adopt((std::remove_reference_t<decltype(*buf.p)>*)x.first, x.second);
+  });
+  uint8_t* at = r->staging;
+  for_each_scene_buffer(r, img, [&](auto& buf, const auto& v, size_t) {
+    const size_t bytes = v.size() * sizeof(v[0]);
+    if (e != cudaSuccess || bytes == 0) return;
+    uint8_t* staged = at;
+    at += padded(bytes);
+    memcpy(staged, v.data(), bytes);
+    if constexpr (std::is_same<std::decay_t<decltype(v)>, std::vector<DevMat>>::value)
+      for (size_t i = 0; i < v.size(); ++i)
+        if (img.mat_tex[i] >= 0) ((DevMat*)staged)[i].tex = r->textures[img.mat_tex[i]].p;
+    e = cudaMemcpyAsync(buf.p, staged, bytes, cudaMemcpyHostToDevice, s);
+  });
+  r->scene = std::move(img);
+  CUDA_TRY(e);
+  return RTRB_OK;
+}
+
+// Orders scene-reading work about to be queued on `s` after the last rtrb_scene_update: the first such launch on a
+// stream since that update waits for the update's copies.  *fresh: this is that first launch (it must not overlap the
+// work before it, render_impl).  The bake of rtrb_renderer_create completed before it returned.
+int enter_scene_stream(rtrb_renderer* r, cudaStream_t s, bool* fresh) {
+  *fresh = false;
+  for (cudaStream_t t : r->scene_streams)
+    if (t == s) return RTRB_OK;
+  r->scene_streams.push_back(s);
+  if (r->scene_gen == 0) return RTRB_OK;
+  *fresh = true;
+  CUDA_TRY(cudaStreamWaitEvent(s, r->scene_ready_ev, 0));
   return RTRB_OK;
 }
 
@@ -765,25 +884,26 @@ void bake_camera(FrameParams& P, const rtrb_camera_desc* c) {
 // The scene part of FrameParams: baked buffers, FP32 filter view, constant-bank tables of small scenes.  The camera
 // apex table is not part of it (it only holds for rays that start at the camera).
 void fill_scene_params(const rtrb_renderer* r, FrameParams& P) {
-  P.max_distance = r->max_distance; P.soft_shadow_exponent = r->soft_shadow_exponent;
-  P.n_objects = r->n_objects; P.n_lights = r->n_lights;
+  const SceneImage::Facts& f = r->scene.f;
+  P.max_distance = f.max_distance; P.soft_shadow_exponent = f.soft_shadow_exponent;
+  P.n_objects = f.n_objects; P.n_lights = f.n_lights;
   P.geom = r->geom.p; P.mat = r->mat.p; P.lights = r->lights.p; P.boxes = r->boxes.p;
   P.cull_sph = r->cull_sph.p; P.sph_index = r->sph_index.p; P.cull_pl = r->cull_pl.p; P.pl_index = r->pl_index.p;
-  P.lights_f = r->lights_f.p; P.n_sph = r->n_sph; P.n_pl = r->n_pl; P.bvh = r->bvh.p;
-  P.m_scene = r->m_scene; P.max_distance_f = r->max_distance_f;
-  P.use_bvh = r->small_scene ? 0 : 1;
-  P.scene_class = r->scene_class;
-  if (r->small_scene) {
-    static_assert(sizeof(r->k.light_tab) == sizeof(P.k_light_tab) && sizeof(r->k.lights) == sizeof(P.k_lights), "table layout");
-    memcpy(P.k_light_tab, r->k.light_tab, sizeof(P.k_light_tab));
-    memcpy(P.k_cull_sph, r->k.cull_sph, sizeof(P.k_cull_sph));
-    memcpy(P.k_cull_pl, r->k.cull_pl, sizeof(P.k_cull_pl));
-    memcpy(P.k_lights, r->k.lights, sizeof(P.k_lights));
-    memcpy(P.k_lights_f, r->k.lights_f, sizeof(P.k_lights_f));
-    memcpy(P.k_pl_index, r->k.pl_index, sizeof(P.k_pl_index));
-    P.k_has_light_tab = r->k.has_light_tab;
+  P.lights_f = r->lights_f.p; P.n_sph = f.n_sph; P.n_pl = f.n_pl; P.bvh = r->bvh.p;
+  P.m_scene = f.m_scene; P.max_distance_f = f.max_distance_f;
+  P.use_bvh = f.small_scene ? 0 : 1;
+  P.scene_class = f.scene_class;
+  if (f.small_scene) {
+    static_assert(sizeof(f.k.light_tab) == sizeof(P.k_light_tab) && sizeof(f.k.lights) == sizeof(P.k_lights), "table layout");
+    memcpy(P.k_light_tab, f.k.light_tab, sizeof(P.k_light_tab));
+    memcpy(P.k_cull_sph, f.k.cull_sph, sizeof(P.k_cull_sph));
+    memcpy(P.k_cull_pl, f.k.cull_pl, sizeof(P.k_cull_pl));
+    memcpy(P.k_lights, f.k.lights, sizeof(P.k_lights));
+    memcpy(P.k_lights_f, f.k.lights_f, sizeof(P.k_lights_f));
+    memcpy(P.k_pl_index, f.k.pl_index, sizeof(P.k_pl_index));
+    P.k_has_light_tab = f.k.has_light_tab;
   }
-  P.light_tab = r->light_tab.p;  // nullptr unless the scene uses the linear filter
+  P.light_tab = r->scene.light_tab.empty() ? nullptr : r->light_tab.p;  // only scenes that use the linear filter
   P.cam_tab_valid = 0;
 }
 
@@ -920,7 +1040,7 @@ int pick_trace_kernels(const rtrb_renderer* r, bool strict, int trace_depth, int
   if (*capacity == 0)
     return fail(RTRB_ERR_UNSUPPORTED, "trace_depth*(1+mc)+1 = %lld exceeds the device stack limit %d",
                 (long long)trace_depth * (1 + (long long)mc) + 1, kMaxStack);
-  P.count_detail = (count_detail || (r && r->n_boxes > 0)) ? 1 : 0;
+  P.count_detail = (count_detail || (r && r->scene.f.n_boxes > 0)) ? 1 : 0;
   return RTRB_OK;
 }
 
@@ -1014,14 +1134,20 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
     if (overlap) next_blk = fc.d.p + r->ring_next;
   }
 
+  // the first frame on a stream after rtrb_scene_update starts only after the update's copies: no overlap with the
+  // kernel before it, which would let it read the scene early
+  bool fresh_scene;
+  if ((rc = enter_scene_stream(r, stream, &fresh_scene))) return rc;
   bake_camera(P, cam);
   fill_scene_params(r, P);
-  if (!P.use_bvh && r->n_sph > 0 && r->n_sph <= RTRB_APEX_MAX) {
+  const int n_sph = r->scene.f.n_sph;
+  if (!P.use_bvh && n_sph > 0 && n_sph <= RTRB_APEX_MAX) {
     const double cm = fmax(fabs(cam->position[0]), fmax(fabs(cam->position[1]), fabs(cam->position[2])));
-    for (int k = 0; k < r->n_sph; ++k)
-      P.cam_tab[k] = apex_entry(cam->position, fabs(cam->aperture_radius), &r->sph_world[4 * (size_t)k],
-                                r->sph_world[4 * (size_t)k + 3], (double)r->m_scene + cm + fabs(cam->aperture_radius));
-    for (int k = r->n_sph; k < RTRB_APEX_MAX; ++k) P.cam_tab[k] = make_float4(0.0f, 0.0f, 0.0f, INFINITY);  // never survives
+    const std::vector<double>& sw = r->scene.sph_world;
+    for (int k = 0; k < n_sph; ++k)
+      P.cam_tab[k] = apex_entry(cam->position, fabs(cam->aperture_radius), &sw[4 * (size_t)k], sw[4 * (size_t)k + 3],
+                                (double)r->scene.f.m_scene + cm + fabs(cam->aperture_radius));
+    for (int k = n_sph; k < RTRB_APEX_MAX; ++k) P.cam_tab[k] = make_float4(0.0f, 0.0f, 0.0f, INFINITY);  // never survives
     P.cam_tab_valid = 1;
   }
   P.key0 = (uint32_t)opts.seed; P.key1 = (uint32_t)(opts.seed >> 32);
@@ -1051,7 +1177,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   } else if (n_tiles > 0) {
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt0, stream));
     CUDA_TRY(strict ? rtrb_launch_trace_pre_strict(P, capacity, stream)
-                    : rtrb_launch_trace_pre_fast(P, capacity, stream, overlap));
+                    : rtrb_launch_trace_pre_fast(P, capacity, stream, overlap && !fresh_scene));
     if (next_blk) { r->ring_zeroed = true; r->ring_stream = stream; }
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt1, stream));
     g_launches++;
@@ -1237,9 +1363,62 @@ int rtrb_renderer_create(const rtrb_scene_desc* scene, int device, rtrb_renderer
   }
   const char* overlap = getenv("RTRB_FRAME_OVERLAP");
   r->frame_overlap = !(overlap && strcmp(overlap, "0") == 0);
-  rc = bake_scene(r, scene);
+  SceneImage img;
+  build_scene_image(scene, img);
+  rc = apply_scene(r, img, r->stream);
+  if (!rc && cudaStreamSynchronize(r->stream) != cudaSuccess) rc = fail(RTRB_ERR_CUDA, "scene upload failed");
   if (rc) { rtrb_renderer_destroy(r); return rc; }
+  // a renderer that is never updated keeps no pinned staging memory
+  cudaFreeHost(r->staging);
+  r->staging = nullptr;
+  r->staging_bytes = 0;
   *out = r;
+  return RTRB_OK;
+}
+
+int rtrb_scene_update(rtrb_renderer* r, const rtrb_scene_desc* scene, void* stream) {
+  int rc = validate_scene(scene);
+  if (rc) return rc;
+  if (!r) return fail(RTRB_ERR_INVALID, "renderer is NULL");
+  SceneImage img;
+  build_scene_image(scene, img);
+  if (same_image(img, r->scene)) return RTRB_OK;  // nothing queued: frames keep overlapping
+  CUDA_TRY(cudaSetDevice(r->device));
+  const cudaStream_t s = stream ? (cudaStream_t)stream : r->stream;
+  if (!r->scene_ready_ev) {
+    CUDA_TRY(cudaEventCreateWithFlags(&r->scene_prior_ev, cudaEventDisableTiming));
+    CUDA_TRY(cudaEventCreateWithFlags(&r->scene_ready_ev, cudaEventDisableTiming));
+  }
+  // The last update's copies are done: its staging buffer is free, and so is every buffer it outgrew (the work that
+  // could read those was queued before it, and its copies waited for that work).
+  if (r->scene_gen > 0) CUDA_TRY(cudaEventSynchronize(r->scene_ready_ev));
+  cudaError_t freed = cudaSuccess;
+  for (void* p : r->retired) {
+    const cudaError_t e = cudaFree(p);
+    if (freed == cudaSuccess) freed = e;
+  }
+  r->retired.clear();
+  CUDA_TRY(freed);
+  // Work queued so far reads the old scene: the copies wait for it on every stream that has launched some.  A stream
+  // that can no longer be recorded on was destroyed by its owner; the work it had queued still runs, so then the copies
+  // wait for the whole device, and the stream is forgotten.
+  bool lost_stream = false;
+  for (size_t i = 0; i < r->scene_streams.size();) {
+    const cudaStream_t t = r->scene_streams[i];
+    if (t != s && cudaEventRecord(r->scene_prior_ev, t) != cudaSuccess) {
+      cudaGetLastError();  // not sticky: clear it so that later launch checks do not report it
+      lost_stream = true;
+      r->scene_streams.erase(r->scene_streams.begin() + i);
+      continue;
+    }
+    if (t != s) CUDA_TRY(cudaStreamWaitEvent(s, r->scene_prior_ev, 0));
+    ++i;
+  }
+  if (lost_stream) CUDA_TRY(cudaDeviceSynchronize());
+  if ((rc = apply_scene(r, img, s))) return rc;
+  CUDA_TRY(cudaEventRecord(r->scene_ready_ev, s));
+  r->scene_gen++;
+  r->scene_streams.clear();
   return RTRB_OK;
 }
 
@@ -1573,6 +1752,8 @@ int rtrb_trace_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, const rt
   if (stats_out) { memset(stats_out, 0, sizeof(*stats_out)); stats_out->first_bad_x = stats_out->first_bad_y = -1; }
   if (n == 0) return RTRB_OK;
   cudaStream_t s = opts->stream ? (cudaStream_t)opts->stream : r->stream;
+  bool fresh_scene;
+  if ((rc = enter_scene_stream(r, s, &fresh_scene))) return rc;
   const size_t un = (size_t)n;
   RayBatch B;
   memset(&B, 0, sizeof(B));
@@ -1620,6 +1801,8 @@ int rtrb_intersect_rays(rtrb_renderer* r, const rtrb_ray_opts* opts, int n, cons
   if (dev && ((rc = check_device_ptr(r, rays, "rays")) || (rc = check_device_ptr(r, hits_out, "hits_out")))) return rc;
   if (n == 0) return RTRB_OK;
   cudaStream_t s = opts->stream ? (cudaStream_t)opts->stream : r->stream;
+  bool fresh_scene;
+  if ((rc = enter_scene_stream(r, s, &fresh_scene))) return rc;
   const size_t un = (size_t)n;
   RayBatch B;
   memset(&B, 0, sizeof(B));

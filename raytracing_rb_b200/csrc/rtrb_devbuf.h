@@ -28,6 +28,21 @@ struct DevBuf {
     return e;
   }
 
+  // Takes over `q` (count elements, from cudaMalloc) in place of the current allocation, which is freed.
+  void adopt(T* q, size_t count) {
+    release();
+    p = q;
+    n = count;
+  }
+
+  // Hands the allocation over to the caller (who frees it with cudaFree) and leaves the array empty.
+  T* detach() {
+    T* q = p;
+    p = nullptr;
+    n = 0;
+    return q;
+  }
+
  private:
   void release() {
     if (p) cudaFree(p);

@@ -1,9 +1,10 @@
 """Mirror of Alex::Lights::Light / SpotLight (reference src/lights/light.rb:2-11,
 src/lights/spot_light.rb:4-5): plain property bags.  SpotLight#intersect? is dead code upstream
 (references an undefined `center`) and is not mirrored."""
+from ._edits import Tracked
 
 
-class Light:
+class Light(Tracked):
     position = name = color = high_light_rate = high_light_angle = None
 
     def __init__(self, properties):  # light.rb:6-10

@@ -3,6 +3,7 @@ sphere.rb:6-26, plane.rb:7-36, box.rb:9-74) as HOST-side property bags: same att
 vectors, same mandatory-in-practice keys.  Their per-ray methods (intersect, cover_area,
 local_lighting, ...) are the CUDA kernels' job; `to_desc` flattens one object for the C ABI."""
 from . import _abi
+from ._edits import Tracked
 from .texture import Texture
 from .vec3 import Vec3
 
@@ -19,7 +20,7 @@ def _v(x, what):
     return (_abi.D3)(*x.to_a())
 
 
-class WorldObject:
+class WorldObject(Tracked):
     # world_object.rb:9-13 accessors (nil when absent)
     name = None
     reflective_attenuation = refractive_attenuation = diffuse_rate = ambient = None

@@ -71,10 +71,11 @@ def _torch_stream(device):
 
 class Renderer:
     def __init__(self, scene, device=0):
-        self._scene = scene  # SceneDescHolder; only needed during create, kept for introspection
+        self._scene = scene  # SceneDescHolder of the last create / update; kept for introspection
         self._h = C.c_void_p()
         self.device = device
         self._png_pending = {}  # submit_png ticket -> (host buffer, byte count that rtrb_wait fills in)
+        self.synced_to = None   # (world, edit count) it was last brought up to date with (world.synced_renderer)
         check(lib().rtrb_renderer_create(C.byref(scene.desc), device, C.byref(self._h)))
 
     def close(self):
@@ -91,6 +92,15 @@ class Renderer:
     @property
     def handle(self):
         return self._h
+
+    def update(self, scene, stream=None):
+        """Replaces the baked scene with `scene` (a SceneDescHolder) in stream order (rtrb_scene_update): work queued
+        before the call sees the old scene, work issued after it the new one; an unchanged scene queues nothing.
+        stream: a cudaStream_t handle, a torch.cuda.Stream, or None for the renderer's own stream."""
+        if stream is not None and not isinstance(stream, int):
+            stream = stream.cuda_stream or 1  # torch's default stream reports 0: cudaStreamLegacy, as _torch_stream
+        check(lib().rtrb_scene_update(self._h, C.byref(scene.desc), C.c_void_p(stream) if stream else None))
+        self._scene = scene
 
     def render_device(self, cam, opts=None, want_stats=True):
         """Frame stays in device memory.  Returns (stats dict or None, status code)."""

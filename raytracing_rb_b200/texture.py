@@ -8,6 +8,8 @@ import os
 
 import numpy as np
 
+from ._edits import Tracked
+
 
 def resolve_texture_path(file_name, config_path=None):
     """The reference opens the path relative to the process CWD (texture.rb:12).  Fall back to the
@@ -23,7 +25,7 @@ def resolve_texture_path(file_name, config_path=None):
     raise FileNotFoundError("texture file not found: %s (tried %s)" % (file_name, cands))
 
 
-class Texture:
+class Texture(Tracked):
     def __init__(self, file_name, horizontal_scale, vertical_scale, u_off=None, v_off=None, config_path=None):
         from PIL import Image
         self.file_name = resolve_texture_path(file_name, config_path)

@@ -8,6 +8,8 @@ clamped to 1 and raises on a zero vector (c:109-129), `*`//`/` accept only Float
 (c:194,213), `to_s` prints 6 decimals (rb:7-13)."""
 import math
 
+from . import _edits
+
 
 class Vec3:
     __slots__ = ("values", "_r")
@@ -102,7 +104,8 @@ class Vec3:
         a = self.values
         return Vec3(-a[0], -a[1], -a[2])
 
-    def _recalc(self):
+    def _recalc(self):  # after an in-place operation: a Vec3 of a world object or light may have changed
+        _edits.touch()
         a = self.values
         self._r = math.sqrt(a[0] * a[0] + a[1] * a[1] + a[2] * a[2])
         return self
@@ -131,6 +134,7 @@ class Vec3:
 
     def normalize_bang(self):  # normalize!
         n = self.normalize()
+        _edits.touch()
         self.values = n.values
         self._r = 1.0
         return self

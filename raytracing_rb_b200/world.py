@@ -6,7 +6,7 @@ import ctypes as C
 
 from .vec3 import Vec3
 
-from . import _abi
+from . import _abi, _edits
 from .configurable_object import ConfigurableObject
 from .lights import LIGHT_CLASSES
 from .objects import OBJECT_CLASSES
@@ -20,6 +20,20 @@ class SceneDescHolder:
         self._keepalive = keepalive
 
 
+def synced_renderer(renderers, device, world):
+    """renderers[device]: made from `world` on first use, and brought up to date (rtrb_scene_update) when the world
+    is another one or the scene mirror was edited since (_edits).  An unchanged world costs an integer compare."""
+    stamp = _edits.count()  # before flattening: an edit made meanwhile is picked up by the next call
+    r = renderers.get(device)
+    if r is None:
+        from .renderer import Renderer
+        renderers[device] = r = Renderer(world.to_scene_desc(), device)
+    elif r.synced_to != (world, stamp):
+        r.update(world.to_scene_desc())
+    r.synced_to = (world, stamp)
+    return r
+
+
 class World(ConfigurableObject):
     max_distance = None
     trace_depth = None          # world.rb:12, unused upstream (depth comes from the camera)
@@ -30,13 +44,16 @@ class World(ConfigurableObject):
         self.world_objects = self.parse_objects(self.world_objects)  # world.rb:17
         self.lights = self.parse_lights(self.lights)                  # world.rb:18
 
+    def __setattr__(self, name, value):
+        if name in ("world_objects", "lights") and isinstance(value, list) and not isinstance(value, _edits.TrackedList):
+            value = _edits.TrackedList(value)
+        _edits.touch()
+        object.__setattr__(self, name, value)
+
     def renderer(self, device=0):
-        """The scene baked on `device` for ray-level queries (one per device, made on first use)."""
-        rs = self.__dict__.setdefault("_renderers", {})
-        if device not in rs:
-            from .renderer import Renderer
-            rs[device] = Renderer(self.to_scene_desc(), device)
-        return rs[device]
+        """The scene baked on `device` for ray-level queries (one per device, made on first use), brought up to date
+        with edits of the objects and lights since the last call."""
+        return synced_renderer(self.__dict__.setdefault("_renderers", {}), device, self)
 
     def intersect_batch(self, rays, precision=_abi.PREC_DEFAULT, device=0):
         """World#intersect on many rays (Ray objects or [n, 6] rows of position, front) -> RAY_HIT_DTYPE array."""
