@@ -17,6 +17,13 @@
  *                                                     (RTRB_FMT_RGB8: alpha is always 255, camera.rb:155)
  *   renderer.render_png(camera, seed = 1, precision = 1) -> binary String: the frame as an 8-bit RGB PNG file,
  *                                                     encoded on the GPU (only the file crosses PCIe)
+ *   renderer.render_progressive(camera, schedule, seed = 1) { |rgb8, samples_done| ... }
+ *                                                  -> the frame in passes (rtrb_progressive_*): after the pass to each
+ *                                                     entry of `schedule` (increasing sample counts, the last one
+ *                                                     pre_sample_times) yields the preview as render's RGB8 String;
+ *                                                     raises as render does when the final frame raised
+ *   renderer.render_progressive_png(camera, schedule, seed = 1) { |png, samples_done| ... }
+ *                                                  -> the same, each preview as render_png's PNG file
  *   renderer.stats                                 -> Hash of the last frame's (or ray batch's) counters
  *   renderer.trace_rays(packed_rays, trace_depth, mc, seed = 1) -> [rgb, hits]: RayTracer#trace_sync on n rays given as
  *                                                     n*6 doubles (position, front; Array#pack("d*")); rgb = n*3 doubles,
@@ -311,6 +318,82 @@ static VALUE renderer_render_png(int argc, VALUE* argv, VALUE self) {
   return out;
 }
 
+/* ---- progressive frames: one pass per schedule entry, the GVL released around each pass and its download / encode */
+typedef struct {
+  render_call* c;
+  rtrb_progressive* p;
+  VALUE schedule;
+  int png;
+} progressive_run;
+
+typedef struct {
+  render_call* c;
+  rtrb_progressive* p;
+  int sample_end, png;
+} pass_call;
+
+static void* pass_without_gvl(void* q) {
+  pass_call* pc = (pass_call*)q;
+  render_call* c = pc->c;
+  c->rc = rtrb_progressive_pass(pc->p, pc->sample_end, &c->s->last);
+  if (c->rc != RTRB_OK && c->rc != RTRB_ERR_RAISED) return NULL;
+  const int raised = c->rc == RTRB_ERR_RAISED;
+  if (pc->png) {
+    void* src = NULL;
+    c->rc = rtrb_progressive_frame_ptr(pc->p, &src);
+    if (c->rc == RTRB_OK)
+      c->rc = rtrb_encode_png(c->s->r, src, c->cam.width, c->cam.height, c->opts.pixel_format, NULL, c->rgba, c->capacity,
+                              &c->png_bytes);
+  } else {
+    c->rc = rtrb_progressive_download(pc->p, c->rgba, NULL, NULL);
+  }
+  if (c->rc == RTRB_OK && raised) c->rc = RTRB_ERR_RAISED;
+  return NULL;
+}
+
+static VALUE progressive_body(VALUE q) {
+  progressive_run* run = (progressive_run*)q;
+  render_call* c = run->c;
+  const long n = RARRAY_LEN(run->schedule);
+  for (long i = 0; i < n; ++i) {
+    pass_call pc = {c, run->p, NUM2INT(rb_ary_entry(run->schedule, i)), run->png};
+    const size_t bytes = run->png ? c->capacity : (size_t)c->cam.width * c->cam.height * 3;
+    VALUE out = rb_str_new(NULL, (long)bytes);
+    c->rgba = (uint8_t*)RSTRING_PTR(out);
+    rb_thread_call_without_gvl(pass_without_gvl, &pc, RUBY_UBF_IO, NULL);
+    const int final = pc.sample_end == c->cam.pre_sample_times;
+    if (c->rc != RTRB_OK && c->rc != RTRB_ERR_RAISED) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());
+    if (run->png) rb_str_set_len(out, (long)c->png_bytes);
+    rb_yield_values(2, out, INT2NUM(pc.sample_end));
+    if (final && c->rc == RTRB_ERR_RAISED) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());  /* as render */
+  }
+  return Qnil;
+}
+
+static VALUE progressive_cleanup(VALUE q) {
+  rtrb_progressive_destroy(((progressive_run*)q)->p);
+  return Qnil;
+}
+
+static VALUE renderer_progressive(int argc, VALUE* argv, VALUE self, int png) {
+  VALUE camera, schedule, seed;
+  rb_scan_args(argc, argv, "21", &camera, &schedule, &seed);
+  Check_Type(schedule, T_ARRAY);
+  rb_need_block();
+  VALUE args[2] = {camera, seed};
+  render_call c;
+  frame_call(2, args, self, &c);
+  c.opts.skip_outputs = RTRB_SKIP_RGB | RTRB_SKIP_HIT;           /* only the 8-bit frame is needed */
+  if (png && rtrb_png_max_bytes(c.cam.width, c.cam.height, &c.capacity) != RTRB_OK)
+    rb_raise(rb_eArgError, "%s", rtrb_last_error());
+  progressive_run run = {&c, NULL, schedule, png};
+  if (rtrb_progressive_create(c.s->r, &c.cam, &c.opts, &run.p) != RTRB_OK) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());
+  return rb_ensure(progressive_body, (VALUE)&run, progressive_cleanup, (VALUE)&run);
+}
+
+static VALUE renderer_render_progressive(int argc, VALUE* argv, VALUE self) { return renderer_progressive(argc, argv, self, 0); }
+static VALUE renderer_render_progressive_png(int argc, VALUE* argv, VALUE self) { return renderer_progressive(argc, argv, self, 1); }
+
 typedef struct {
   shim_renderer* s;
   rtrb_ray_opts opts;
@@ -395,6 +478,8 @@ void Init_rtrb_b200(void) {
   rb_define_method(cRenderer, "update", renderer_update, 1);
   rb_define_method(cRenderer, "render", renderer_render, -1);
   rb_define_method(cRenderer, "render_png", renderer_render_png, -1);
+  rb_define_method(cRenderer, "render_progressive", renderer_render_progressive, -1);
+  rb_define_method(cRenderer, "render_progressive_png", renderer_render_progressive_png, -1);
   rb_define_method(cRenderer, "stats", renderer_stats, 0);
   rb_define_method(cRenderer, "trace_rays", renderer_trace_rays, -1);
   rb_define_method(cRenderer, "intersect_rays", renderer_intersect_rays, 1);

@@ -279,6 +279,52 @@ int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int hei
 int rtrb_submit_png(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* png_host,
                     size_t capacity, size_t* png_bytes_out, int* ticket_out);
 
+/* -- progressive frames --------------------------------------------------------------------------- */
+/* One camera plus render options whose pre_sample_times samples are traced in passes the caller chooses, with a
+ * well-defined image after every pass (interactive previews, renders that stop when a time budget is spent):
+ *   - Preview: after a pass that brings the frame to e < pre_sample_times samples, its outputs (the 8-bit frame in
+ *     opts->pixel_format, the float RGB, the hit ids) and stats equal bit for bit those of rtrb_render_device for the
+ *     same camera with pre_sample_times = max_sample_times = e, including render_at's variance test and its rescale of
+ *     the adaptive pixels.
+ *   - Final: the pass that reaches pre_sample_times finishes render_at as the one-shot frame does (variance test and,
+ *     when max_sample_times > pre_sample_times, the extra samples of the adaptive pixels, traced whole in that pass);
+ *     outputs and stats then equal rtrb_render_device of the camera as given.
+ *   - Stats: a pass reports the stats of the frame its outputs equal.  Counters, status, first_bad_x/y and max_stack
+ *     accumulate over the passes so far; device_ms / trace_ms cover this pass only.
+ * Arguments and buffers:
+ *   - opts follow the rules of rtrb_render_device: window, tile_rank / tile_world, the three pixel formats,
+ *     skip_outputs, rgba_device_out and stream.  RTRB_RNG_MT returns RTRB_ERR_UNSUPPORTED.
+ *   - the handle owns its scratch (the per-sample buffer [slots][pre][3] FP64, the extra-sample buffers, a control
+ *     block, its tile list and lens table) and its outputs: the float RGB, the hit ids and, unless opts->rgba_device_out
+ *     is given, the 8-bit frame.  Pixels outside the window or the rank's tiles read 0 and hit id -3.
+ *   - frames, rtrb_submit frames, ray calls and other progressive frames on the same renderer may run between passes:
+ *     they do not disturb it, and it does not disturb them.
+ *   - rtrb_progressive_create fails with RTRB_ERR_UNSUPPORTED when the sample buffer exceeds the per-frame memory
+ *     budget of rtrb_render_device, and with RTRB_ERR_CUDA when no CUDA device is usable.
+ * Passes:
+ *   - rtrb_progressive_pass traces samples [done, sample_end) of every pixel, done being the samples of the passes
+ *     before it; sample_end must be in (done, pre_sample_times].  A pass after the final one returns RTRB_ERR_INVALID.
+ *   - passes are ordered on opts->stream (NULL = the renderer's own) and synchronise only when stats_out != NULL,
+ *     like rtrb_render_device.  They read the scene, so rtrb_scene_update orders them as it orders frames.
+ *   - when rtrb_scene_update has replaced the scene since create, the next pass returns RTRB_ERR_INVALID ("scene
+ *     changed"): one pixel mixing two scenes would be neither frame.  An update whose scene equals the current one
+ *     does not count.
+ *   - RTRB_ERR_RAISED when the frame the outputs equal would have raised (every output is written).
+ * A progressive frame must be destroyed before its renderer. */
+typedef struct rtrb_progressive rtrb_progressive;
+int rtrb_progressive_create(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts,
+                            rtrb_progressive** out);
+/* samples [done, sample_end) */
+int rtrb_progressive_pass(rtrb_progressive* p, int sample_end, rtrb_stats* stats_out);
+/* Copies the outputs of the passes so far to HOST buffers (layouts of rtrb_download; each pointer may be NULL).
+ * Blocking.  RTRB_ERR_INVALID before the first pass, for an 8-bit frame that went to rgba_device_out, and for an
+ * output that skip_outputs dropped. */
+int rtrb_progressive_download(rtrb_progressive* p, uint8_t* frame, double* rgb_or_null, int32_t* hit_or_null);
+/* Device pointer of the 8-bit frame (its own buffer, or rgba_device_out), e.g. for rtrb_encode_png. */
+int rtrb_progressive_frame_ptr(rtrb_progressive* p, void** ptr_out);
+/* Waits for the device and frees the frame's buffers.  NULL is a no-op. */
+int rtrb_progressive_destroy(rtrb_progressive* p);
+
 /* -- ray-level queries on caller-supplied rays ---------------------------------------------------- */
 /* The layers below the camera, for callers with their own rays (other projections, picking, probes of one ray):
  * RayTracer#trace_sync (ray_tracer.rb:16-46) and World#intersect (world.rb:37-59) on a batch of rays, one device

@@ -7,6 +7,8 @@ module Rtrb
     def update(world); raise NotImplementedError; end
     def render(camera, seed = 1, precision = 1); raise NotImplementedError; end
     def render_png(camera, seed = 1, precision = 1); raise NotImplementedError; end
+    def render_progressive(camera, schedule, seed = 1); raise NotImplementedError; end
+    def render_progressive_png(camera, schedule, seed = 1); raise NotImplementedError; end
     def stats; raise NotImplementedError; end
     def trace_rays(packed_rays, trace_depth, mc, seed = 1); raise NotImplementedError; end
     def intersect_rays(packed_rays); raise NotImplementedError; end
@@ -40,7 +42,25 @@ module Alex
       File.binwrite(file_path, @rtrb.render_png(self, seed))
     end
 
+    # render_cuda_png in passes: the file is rewritten after every pass of `schedule` (increasing sample counts ending
+    # at pre_sample_times; default 1, 2, 4, ... then pre_sample_times), each a preview of the samples traced so far
+    def render_cuda_progressive(file_path, schedule = nil)
+      rtrb_renderer
+      schedule ||= progressive_schedule(@pre_sample_times)
+      @rtrb.render_progressive_png(self, schedule) { |png, _samples_done| File.binwrite(file_path, png) }
+    end
+
     private
+
+    def progressive_schedule(pre)
+      out = []
+      e = 1
+      while e < pre
+        out << e
+        e *= 2
+      end
+      out << pre
+    end
 
     def rtrb_renderer
       if @rtrb

@@ -18,6 +18,8 @@ EXPORTS = (
     "rtrb_render_multi", "rtrb_tile_partition", "rtrb_measure_fma_peak", "rtrb_launch_count", "rtrb_last_mt_passes",
     "rtrb_png_max_bytes", "rtrb_encode_png", "rtrb_submit_png",
     "rtrb_trace_rays", "rtrb_intersect_rays", "rtrb_camera_rays",
+    "rtrb_progressive_create", "rtrb_progressive_pass", "rtrb_progressive_download", "rtrb_progressive_frame_ptr",
+    "rtrb_progressive_destroy",
 )
 
 _lib = None
@@ -75,6 +77,11 @@ def lib():
     L.rtrb_intersect_rays.argtypes = [C.c_void_p, P(_abi.RayOpts), C.c_int, C.c_void_p, C.c_void_p]
     L.rtrb_camera_rays.argtypes = [C.c_void_p, P(_abi.CameraDesc), P(_abi.RayOpts), C.c_int, C.c_int, C.c_void_p,
                                    C.c_void_p]
+    L.rtrb_progressive_create.argtypes = [C.c_void_p, P(_abi.CameraDesc), P(_abi.RenderOpts), P(C.c_void_p)]
+    L.rtrb_progressive_pass.argtypes = [C.c_void_p, C.c_int, P(_abi.Stats)]
+    L.rtrb_progressive_download.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.rtrb_progressive_frame_ptr.argtypes = [C.c_void_p, P(C.c_void_p)]
+    L.rtrb_progressive_destroy.argtypes = [C.c_void_p]
     for name in EXPORTS:
         getattr(L, name)
     if L.rtrb_abi_version() != _abi.ABI_VERSION:

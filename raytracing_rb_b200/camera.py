@@ -13,7 +13,7 @@ import numpy as np
 
 from . import _abi
 from .configurable_object import ConfigurableObject
-from .renderer import make_opts, render_multi
+from .renderer import make_opts, progressive_schedule, render_multi
 from .world import synced_renderer
 
 
@@ -140,6 +140,33 @@ class Camera(ConfigurableObject):
         if code == _abi.RTRB_ERR_RAISED:
             self._raise_for(stats)
         return stats
+
+    def render_progressive(self, file_path=None, schedule=None, seed=1, **kw):
+        """render_cuda in passes, for previews and time-budgeted renders: a generator that yields (samples_done, Frame)
+        after every pass of `schedule` (increasing sample counts, the last one pre_sample_times; default
+        progressive_schedule(pre_sample_times)).  A preview after e samples is the frame of pre = max = e samples; the
+        final pass gives render_frame's frame.  With file_path the PNG is rewritten after every pass by the GPU encoder,
+        as render_png writes it.  Raises RuntimeError as render_cuda does when the final frame raised.  kw: make_opts
+        options (precision, window, count_detail, pixel_format, ...)."""
+        cam = self.camera_desc()
+        r = self.renderer()
+        prog = r.progressive(cam, make_opts(seed=seed, **kw))
+        try:
+            frame = None
+            for e in schedule or progressive_schedule(cam.pre_sample_times):
+                prog.pass_to(e)
+                frame = prog.download()
+                if file_path:
+                    png = r.encode_png(self.width, self.height, prog.opts.pixel_format, src=prog.frame_ptr())
+                    os.makedirs(os.path.dirname(os.path.abspath(file_path)), exist_ok=True)
+                    with open(file_path, "wb") as f:
+                        f.write(png)
+                yield e, frame
+            self.last_frame = frame
+            if frame is not None and prog.done == cam.pre_sample_times and frame.raised:
+                self._raise_for(frame.stats)
+        finally:
+            prog.close()
 
     def render_fork(self, file_path, threads, out_dir="out", seed=1, **kw):
         """Drop-in for render_fork(file_path, threads) (camera.rb:41-68) for tooling that consumes its

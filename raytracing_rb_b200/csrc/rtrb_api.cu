@@ -445,12 +445,37 @@ struct rtrb_renderer {
   }
 };
 
+// A progressive frame (rtrb_progressive_*, DESIGN.md §14): one camera and its options, whose pre samples are traced in
+// passes.  It owns everything its passes write, so that other work on the renderer between two passes neither
+// disturbs it nor is disturbed by it.
+struct rtrb_progressive {
+  rtrb_renderer* r = nullptr;
+  cudaStream_t stream = nullptr;
+  FrameParams P;               // as baked at create; P.pre = S is the sample buffer's stride
+  int capacity = 0, S = 0, E = 0;
+  int done = 0;                // samples traced so far: every pass covers [done, sample_end)
+  unsigned scene_gen = 0;      // the renderer's scene_gen at create (an update that applied since invalidates the frame)
+  bool strict = false;
+  FrameCtl fc;                 // its control block: counters, status, first_bad and max_stack accumulate over the passes
+  TileList tiles;
+  LensTable lens;
+  DevBuf<double> samples, extra_samples, pre_avg, rgb;  // [slots][S][3], [slots][E][3], [slots][3], [H][W][3]
+  DevBuf<uint32_t> extra_list;
+  DevBuf<int32_t> hit;
+  DevBuf<uint8_t> frame;       // the 8-bit frame, unless it goes to opts.rgba_device_out
+  size_t frame_bytes = 0;
+  int W = 0, H = 0, format = RTRB_FMT_RGBA8;
+  bool own_frame = true;
+  // its buffers are freed with it; its device must be current (rtrb_progressive_destroy)
+};
+
 namespace {
 
 // ---- resolve kernels ---------------------------------------------------------------------------
 using rtrb::decode_pixel;
 using rtrb::final_average;
 using rtrb::pre_mean;
+using rtrb::pre_mean_of;
 using rtrb::queue_adaptive;
 using rtrb::write_pixel;
 
@@ -480,6 +505,19 @@ __global__ void __launch_bounds__(256) resolve_extra_kernel(const __grid_constan
     final_average(ax, ay, az, P.pre, cx, cy, cz, P.max_samples);
     write_pixel(P, x, y, ax, ay, az);
   }
+}
+
+// A progressive frame's preview: resolve_kernel over the first P.pre samples of each pixel of a sample buffer whose
+// pixels are `stride` samples apart.  The host sets P.max_samples = P.pre, so queue_adaptive counts the adaptive pixels
+// and rescales them in place, exactly as in a frame of pre = max = P.pre samples.
+__global__ void __launch_bounds__(256) resolve_prefix_kernel(const __grid_constant__ FrameParams P, int stride) {
+  const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
+  int x = 0, y = 0;
+  const bool valid = slot < (uint32_t)P.n_tiles * RTRB_SUPER_PIXELS && decode_pixel(P, slot, x, y);
+  double ax = 0, ay = 0, az = 0, variance = 0;
+  if (valid) pre_mean_of(P.samples + (size_t)slot * stride * 3, P.pre, ax, ay, az, variance);
+  const bool queued = queue_adaptive(P, valid && variance >= P.variant_threshold, slot, ax, ay, az);
+  if (valid && !queued) write_pixel(P, x, y, ax, ay, az);
 }
 
 // Frame control block -> its pinned host mirror by direct stores (zero-copy over PCIe): see rtrb_submit.
@@ -907,6 +945,22 @@ void fill_scene_params(const rtrb_renderer* r, FrameParams& P) {
   P.cam_tab_valid = 0;
 }
 
+// Camera and scene of a frame: bake_camera, fill_scene_params and the camera's apex table.
+void bake_frame(const rtrb_renderer* r, const rtrb_camera_desc* cam, FrameParams& P) {
+  bake_camera(P, cam);
+  fill_scene_params(r, P);
+  const int n_sph = r->scene.f.n_sph;
+  if (!P.use_bvh && n_sph > 0 && n_sph <= RTRB_APEX_MAX) {
+    const double cm = fmax(fabs(cam->position[0]), fmax(fabs(cam->position[1]), fabs(cam->position[2])));
+    const std::vector<double>& sw = r->scene.sph_world;
+    for (int k = 0; k < n_sph; ++k)
+      P.cam_tab[k] = apex_entry(cam->position, fabs(cam->aperture_radius), &sw[4 * (size_t)k], sw[4 * (size_t)k + 3],
+                                (double)r->scene.f.m_scene + cm + fabs(cam->aperture_radius));
+    for (int k = n_sph; k < RTRB_APEX_MAX; ++k) P.cam_tab[k] = make_float4(0.0f, 0.0f, 0.0f, INFINITY);  // never survives
+    P.cam_tab_valid = 1;
+  }
+}
+
 struct FrameTargets {  // where this renderer writes (own buffers, or rank 0's through a peer mapping)
   uint8_t* rgba = nullptr;
   double* rgb = nullptr;
@@ -1044,14 +1098,37 @@ int pick_trace_kernels(const rtrb_renderer* r, bool strict, int trace_depth, int
   return RTRB_OK;
 }
 
-int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts_in,
-                const FrameTargets* targets, rtrb_stats* stats_out, FrameCtl* ctl = nullptr) {
-  if (!r || !cam) return fail(RTRB_ERR_INVALID, "renderer/camera is NULL");
-  rtrb_render_opts opts = opts_or_default(opts_in);
+// The camera checks of a frame (rtrb_render_device and rtrb_progressive_create).
+int check_frame_camera(const rtrb_camera_desc* cam) {
   if (cam->width <= 0 || cam->height <= 0) return fail(RTRB_ERR_INVALID, "bad frame size %dx%d", cam->width, cam->height);
   if (cam->pre_sample_times < 1) return fail(RTRB_ERR_INVALID, "pre_sample_times must be >= 1");
   if (cam->max_sample_times < 0 || cam->monte_carlo_diffusion_times < 0 || cam->trace_depth < 0)
     return fail(RTRB_ERR_INVALID, "negative sampling parameter");
+  return RTRB_OK;
+}
+
+// The option checks of a frame after its RNG mode's: precision, pixel format, window and tile partition.
+int check_frame_opts(const rtrb_render_opts& opts, int W, int H, Window& win) {
+  if (opts.precision != RTRB_PREC_STRICT && opts.precision != RTRB_PREC_FAST64)
+    return fail(RTRB_ERR_INVALID, "unknown precision mode %d", opts.precision);
+  if (opts.pixel_format != RTRB_FMT_RGBA8 && opts.pixel_format != RTRB_FMT_RGB8 && opts.pixel_format != RTRB_FMT_PNG_RGB8)
+    return fail(RTRB_ERR_INVALID, "unknown pixel format %d", opts.pixel_format);
+  return make_window(W, H, opts.x0, opts.y0, opts.x1, opts.y1, opts.tile_rank, opts.tile_world, win);
+}
+
+// The per-frame memory budget of the sample buffers: S pre samples per slot (when the frame keeps them) and E extra.
+int check_sample_budget(size_t n_slots, int S, int E, bool need_samples) {
+  if ((need_samples && n_slots * (size_t)S * 3 * sizeof(double) > ((size_t)96 << 30)) || n_slots * (size_t)E * 3 * sizeof(double) > ((size_t)64 << 30))
+    return fail(RTRB_ERR_UNSUPPORTED, "sample buffer would exceed the per-frame memory budget");
+  return RTRB_OK;
+}
+
+int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts_in,
+                const FrameTargets* targets, rtrb_stats* stats_out, FrameCtl* ctl = nullptr) {
+  if (!r || !cam) return fail(RTRB_ERR_INVALID, "renderer/camera is NULL");
+  rtrb_render_opts opts = opts_or_default(opts_in);
+  int rc = check_frame_camera(cam);
+  if (rc) return rc;
   if (opts.rng_mode != RTRB_RNG_CTR && opts.rng_mode != RTRB_RNG_MT) return fail(RTRB_ERR_INVALID, "unknown rng_mode %d", opts.rng_mode);
   const bool mt_mode = opts.rng_mode == RTRB_RNG_MT;
   if (mt_mode) {
@@ -1062,14 +1139,9 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
     if ((opts.seed >> 32) != 0) return fail(RTRB_ERR_UNSUPPORTED, "RTRB_RNG_MT: seeds above 32 bits take Ruby's init_by_array path");
     opts.precision = RTRB_PREC_STRICT;
   }
-  if (opts.precision != RTRB_PREC_STRICT && opts.precision != RTRB_PREC_FAST64)
-    return fail(RTRB_ERR_INVALID, "unknown precision mode %d", opts.precision);
-  if (opts.pixel_format != RTRB_FMT_RGBA8 && opts.pixel_format != RTRB_FMT_RGB8 && opts.pixel_format != RTRB_FMT_PNG_RGB8)
-    return fail(RTRB_ERR_INVALID, "unknown pixel format %d", opts.pixel_format);
   const int W = cam->width, H = cam->height;
   Window win;
-  int rc = make_window(W, H, opts.x0, opts.y0, opts.x1, opts.y1, opts.tile_rank, opts.tile_world, win);
-  if (rc) return rc;
+  if ((rc = check_frame_opts(opts, W, H, win))) return rc;
   const bool strict = opts.precision == RTRB_PREC_STRICT;
   FrameParams P;
   memset(&P, 0, sizeof(P));
@@ -1108,8 +1180,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   if (!strict && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0)
     fuse = RTRB_RESOLVE_IN_CTA;
   const bool need_samples = fuse == RTRB_RESOLVE_SAMPLE_BUFFER;
-  if ((need_samples && n_slots * (size_t)S * 3 * sizeof(double) > ((size_t)96 << 30)) || n_slots * (size_t)E * 3 * sizeof(double) > ((size_t)64 << 30))
-    return fail(RTRB_ERR_UNSUPPORTED, "sample buffer would exceed the per-frame memory budget");
+  if ((rc = check_sample_budget(n_slots, S, E, need_samples))) return rc;
   if (need_samples) CUDA_TRY(r->samples.ensure(std::max<size_t>(1, n_slots * S * 3)));
   CUDA_TRY(r->extra_list.ensure(std::max<size_t>(1, n_slots)));
   if (E > 0) {
@@ -1138,18 +1209,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   // kernel before it, which would let it read the scene early
   bool fresh_scene;
   if ((rc = enter_scene_stream(r, stream, &fresh_scene))) return rc;
-  bake_camera(P, cam);
-  fill_scene_params(r, P);
-  const int n_sph = r->scene.f.n_sph;
-  if (!P.use_bvh && n_sph > 0 && n_sph <= RTRB_APEX_MAX) {
-    const double cm = fmax(fabs(cam->position[0]), fmax(fabs(cam->position[1]), fabs(cam->position[2])));
-    const std::vector<double>& sw = r->scene.sph_world;
-    for (int k = 0; k < n_sph; ++k)
-      P.cam_tab[k] = apex_entry(cam->position, fabs(cam->aperture_radius), &sw[4 * (size_t)k], sw[4 * (size_t)k + 3],
-                                (double)r->scene.f.m_scene + cm + fabs(cam->aperture_radius));
-    for (int k = n_sph; k < RTRB_APEX_MAX; ++k) P.cam_tab[k] = make_float4(0.0f, 0.0f, 0.0f, INFINITY);  // never survives
-    P.cam_tab_valid = 1;
-  }
+  bake_frame(r, cam, P);
   P.key0 = (uint32_t)opts.seed; P.key1 = (uint32_t)(opts.seed >> 32);
   P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
   P.n_tiles = n_tiles; P.stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER; P.tiles = r->tiles.dev.p;
@@ -1888,6 +1948,171 @@ int rtrb_tile_partition(int width, int height, const int32_t* window, int tile_r
   *count_out = (int)t.size();
   if (tiles_out)
     for (int i = 0; i < (int)t.size() && i < capacity; ++i) tiles_out[i] = t[i];
+  return RTRB_OK;
+}
+
+int rtrb_progressive_create(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts_in,
+                            rtrb_progressive** out) {
+  if (!out) return fail(RTRB_ERR_INVALID, "out is NULL");
+  *out = nullptr;
+  if (!r || !cam) return fail(RTRB_ERR_INVALID, "renderer/camera is NULL");
+  int rc = check_frame_camera(cam);
+  if (rc) return rc;
+  const rtrb_render_opts opts = opts_or_default(opts_in);
+  if (opts.rng_mode == RTRB_RNG_MT)
+    return fail(RTRB_ERR_UNSUPPORTED, "progressive frames draw from the counter RNG (RTRB_RNG_MT is a blocking validation mode)");
+  if (opts.rng_mode != RTRB_RNG_CTR) return fail(RTRB_ERR_INVALID, "unknown rng_mode %d", opts.rng_mode);
+  const int W = cam->width, H = cam->height;
+  Window win;
+  if ((rc = check_frame_opts(opts, W, H, win))) return rc;
+  if ((rc = require_device())) return rc;
+  CUDA_TRY(cudaSetDevice(r->device));
+  std::unique_ptr<rtrb_progressive> p(new rtrb_progressive());
+  FrameParams& P = p->P;
+  memset(&P, 0, sizeof(P));
+  const bool strict = opts.precision == RTRB_PREC_STRICT;
+  if ((rc = pick_trace_kernels(r, strict, cam->trace_depth, cam->monte_carlo_diffusion_times, opts.count_detail != 0, P,
+                               &p->capacity)))
+    return rc;
+  const cudaStream_t s = opts.stream ? (cudaStream_t)opts.stream : r->stream;
+  const int S = cam->pre_sample_times, E = cam->max_sample_times > S ? cam->max_sample_times - S : 0;
+  p->r = r; p->stream = s; p->strict = strict; p->S = S; p->E = E;
+  p->W = W; p->H = H; p->format = opts.pixel_format;
+  const cudaError_t ce = p->fc.init();
+  if (ce != cudaSuccess) return fail(RTRB_ERR_CUDA, "control block init failed: %s", cudaGetErrorString(ce));
+  if ((rc = p->tiles.ensure(W, H, win, s)) || (rc = p->lens.ensure(cam, s))) return rc;
+  const int n_tiles = (int)p->tiles.host.size();
+  const size_t n_slots = (size_t)n_tiles * RTRB_SUPER_PIXELS, px = (size_t)W * H;
+  if ((rc = check_sample_budget(n_slots, S, E, true))) return rc;
+  CUDA_TRY(p->samples.ensure(std::max<size_t>(1, n_slots * S * 3)));
+  CUDA_TRY(p->extra_list.ensure(std::max<size_t>(1, n_slots)));
+  if (E > 0) {
+    CUDA_TRY(p->extra_samples.ensure(n_slots * E * 3));
+    CUDA_TRY(p->pre_avg.ensure(n_slots * 3));
+  }
+  // its outputs: pixels outside the window or the rank's tiles read 0, hit id -3
+  p->frame_bytes = RTRB_FRAME_BYTES(W, H, opts.pixel_format);
+  p->own_frame = opts.rgba_device_out == nullptr;
+  if (p->own_frame) {
+    CUDA_TRY(p->frame.ensure(p->frame_bytes));
+    CUDA_TRY(cudaMemsetAsync(p->frame.p, 0, p->frame_bytes, s));
+  }
+  if (!(opts.skip_outputs & RTRB_SKIP_RGB)) {
+    CUDA_TRY(p->rgb.ensure(px * 3));
+    CUDA_TRY(cudaMemsetAsync(p->rgb.p, 0, px * 3 * sizeof(double), s));
+  }
+  if (!(opts.skip_outputs & RTRB_SKIP_HIT)) {
+    CUDA_TRY(p->hit.ensure(px));
+    if (!win.whole) prefill_hits(p->hit.p, W, H, s);
+  }
+  bake_frame(r, cam, P);
+  P.key0 = (uint32_t)opts.seed; P.key1 = (uint32_t)(opts.seed >> 32);
+  P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
+  P.n_tiles = n_tiles; P.stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER; P.tiles = p->tiles.dev.p;
+  P.tiles_magic = win.whole ? p->tiles.magic : 0u;
+  P.lens_sx = p->lens.tab.p; P.lens_sy = p->lens.tab.p + W;
+  P.samples = p->samples.p; P.rgb = p->rgb.p; P.hit = p->hit.p;
+  P.rgba = p->own_frame ? p->frame.p : (uint8_t*)opts.rgba_device_out;
+  P.pre_avg = p->pre_avg.p; P.extra_list = p->extra_list.p; P.extra_samples = p->extra_samples.p;
+  P.pixel_format = opts.pixel_format;
+  P.fuse_resolve = RTRB_RESOLVE_SAMPLE_BUFFER;
+  bind_ctl(P, p->fc);
+  CUDA_TRY(cudaMemsetAsync(p->fc.blk, 0, sizeof(CtlBlock), s));
+  FrameCtl& fc = p->fc;
+  fc.W = W; fc.H = H; fc.n_tiles = n_tiles; fc.detail = P.count_detail != 0; fc.px_count = p->tiles.px_count;
+  p->scene_gen = r->scene_gen;
+  *out = p.release();
+  return RTRB_OK;
+}
+
+int rtrb_progressive_pass(rtrb_progressive* p, int sample_end, rtrb_stats* stats_out) {
+  if (!p) return fail(RTRB_ERR_INVALID, "progressive frame is NULL");
+  if (p->done >= p->S) return fail(RTRB_ERR_INVALID, "the frame is final: its last pass has run");
+  if (sample_end <= p->done || sample_end > p->S)
+    return fail(RTRB_ERR_INVALID, "sample_end %d outside (%d, %d]", sample_end, p->done, p->S);
+  rtrb_renderer* r = p->r;
+  if (r->scene_gen != p->scene_gen)
+    return fail(RTRB_ERR_INVALID, "scene changed: rtrb_scene_update replaced the scene after the frame was created");
+  CUDA_TRY(cudaSetDevice(r->device));
+  const cudaStream_t s = p->stream;
+  bool fresh_scene;
+  int rc = enter_scene_stream(r, s, &fresh_scene);
+  if (rc) return rc;
+  FrameCtl& fc = p->fc;
+  FrameParams& P = p->P;
+  P.pass_begin = p->done; P.pass_end = sample_end;
+  const bool final = sample_end == p->S;
+  const size_t n_slots = (size_t)P.n_tiles * RTRB_SUPER_PIXELS;
+  const unsigned grid = (unsigned)((n_slots + 255) / 256);
+  fc.timed = stats_out != nullptr;
+  if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev0, s));
+  // the counters accumulate over the passes, except adaptive_pixels: each resolve counts the frame it resolves
+  CUDA_TRY(cudaMemsetAsync(&fc.blk->counters[RTRB_CNT_ADAPTIVE], 0, sizeof(unsigned long long), s));
+  if (P.n_tiles > 0) {
+    if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt0, s));
+    CUDA_TRY(p->strict ? rtrb_launch_trace_pass_strict(P, p->capacity, s) : rtrb_launch_trace_pass_fast(P, p->capacity, s));
+    g_launches++;
+    if (fc.timed) CUDA_TRY(cudaEventRecord(fc.evt1, s));
+    if (!final) {
+      // the preview is the frame of pre = max = sample_end samples
+      FrameParams Q = P;
+      Q.pre = sample_end; Q.max_samples = sample_end;
+      resolve_prefix_kernel<<<grid, 256, 0, s>>>(Q, p->S);
+      CUDA_TRY(cudaGetLastError());
+      g_launches++;
+    } else {
+      // render_at's tail as a one-shot sample-buffer frame runs it
+      resolve_kernel<<<grid, 256, 0, s>>>(P);
+      CUDA_TRY(cudaGetLastError());
+      g_launches++;
+      if (p->E > 0) {
+        CUDA_TRY(p->strict ? rtrb_launch_trace_extra_strict(P, p->capacity, s) : rtrb_launch_trace_extra_fast(P, p->capacity, s));
+        g_launches++;
+        resolve_extra_kernel<<<296, 256, 0, s>>>(P);
+        CUDA_TRY(cudaGetLastError());
+        g_launches++;
+      }
+    }
+  }
+  if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev1, s));
+  p->done = sample_end;
+  fc.S = sample_end; fc.E = final ? p->E : 0;
+  return stats_out ? read_stats(fc, s, stats_out) : RTRB_OK;
+}
+
+int rtrb_progressive_download(rtrb_progressive* p, uint8_t* frame, double* rgb_or_null, int32_t* hit_or_null) {
+  if (!p) return fail(RTRB_ERR_INVALID, "progressive frame is NULL");
+  if (p->done == 0) return fail(RTRB_ERR_INVALID, "no pass has run yet");
+  CUDA_TRY(cudaSetDevice(p->r->device));
+  const cudaStream_t s = p->stream;
+  const size_t px = (size_t)p->W * p->H;
+  if (frame) {
+    if (!p->own_frame) return fail(RTRB_ERR_INVALID, "the frame is written to rgba_device_out, not to its own buffer");
+    CUDA_TRY(cudaMemcpyAsync(frame, p->frame.p, p->frame_bytes, cudaMemcpyDeviceToHost, s));
+  }
+  if (rgb_or_null) {
+    if (!p->rgb.p) return fail(RTRB_ERR_INVALID, "the frame keeps no float RGB (RTRB_SKIP_RGB)");
+    CUDA_TRY(cudaMemcpyAsync(rgb_or_null, p->rgb.p, px * 3 * sizeof(double), cudaMemcpyDeviceToHost, s));
+  }
+  if (hit_or_null) {
+    if (!p->hit.p) return fail(RTRB_ERR_INVALID, "the frame keeps no hit ids (RTRB_SKIP_HIT)");
+    CUDA_TRY(cudaMemcpyAsync(hit_or_null, p->hit.p, px * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  }
+  CUDA_TRY(cudaStreamSynchronize(s));
+  return RTRB_OK;
+}
+
+int rtrb_progressive_frame_ptr(rtrb_progressive* p, void** ptr_out) {
+  if (!p || !ptr_out) return fail(RTRB_ERR_INVALID, "bad argument");
+  *ptr_out = p->P.rgba;
+  return RTRB_OK;
+}
+
+int rtrb_progressive_destroy(rtrb_progressive* p) {
+  if (!p) return RTRB_OK;
+  cudaSetDevice(p->r->device);
+  cudaDeviceSynchronize();  // its passes may still be writing its buffers
+  delete p;
   return RTRB_OK;
 }
 

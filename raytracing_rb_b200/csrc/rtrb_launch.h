@@ -44,6 +44,10 @@ inline int sm_count() {
 inline unsigned long long pre_threads(const FrameParams& P) {
   return (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * (unsigned long long)P.pre;
 }
+// Threads of a progressive frame's pass: one per (tile pixel, sample in [pass_begin, pass_end)).
+inline unsigned long long pass_threads(const FrameParams& P) {
+  return (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * (unsigned long long)(P.pass_end - P.pass_begin);
+}
 // Grid of the persistent grid-stride extra-sample kernels: 8 CTAs per SM.
 inline unsigned extra_grid() { return (unsigned)sm_count() * 8u; }
 
@@ -82,4 +86,7 @@ cudaError_t rtrb_launch_trace_extra_strict(const FrameParams& P, int capacity, c
 // overlap: launch with programmatic stream serialization (depth-1 frames only; rtrb_api.cu, render_impl)
 cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int capacity, cudaStream_t s, bool overlap = false);
 cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int capacity, cudaStream_t s);
+// progressive frames (rtrb_api.cu, rtrb_progressive_pass): samples [P.pass_begin, P.pass_end) into the sample buffer
+cudaError_t rtrb_launch_trace_pass_strict(const FrameParams& P, int capacity, cudaStream_t s);
+cudaError_t rtrb_launch_trace_pass_fast(const FrameParams& P, int capacity, cudaStream_t s);
 cudaError_t rtrb_launch_trace_mt_strict(const FrameParams& P, int capacity, cudaStream_t s);  // RTRB_RNG_MT

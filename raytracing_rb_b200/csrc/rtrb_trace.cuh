@@ -818,11 +818,13 @@ __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd,
 // previous grid on the stream to complete, so the only things ordered behind that grid are this frame's global writes.
 // Everything before the wait reads only FrameParams, the scene tables and the lens tables.  Launched without the
 // attribute, the wait returns at once.
-template <class Pol, int MAXS, bool DETAIL, bool BVH = false>
+// PASS: the pass kernels of a progressive frame.  One thread per (pixel, sample j in [pass_begin, pass_end)); the
+// colour goes to the sample buffer at (slot * pre + j), the stride of the whole frame.  No overlap, no in-thread resolve.
+template <class Pol, int MAXS, bool DETAIL, bool BVH = false, bool PASS = false>
 __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
-  constexpr bool kOverlap = Pol::fast && MAXS == 1;
+  constexpr bool kOverlap = Pol::fast && MAXS == 1 && !PASS;
   if constexpr (kOverlap) cudaTriggerProgrammaticLaunchCompletion();
-  const uint32_t S = (uint32_t)P.pre;
+  const uint32_t S = PASS ? (uint32_t)(P.pass_end - P.pass_begin) : (uint32_t)P.pre;
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   const unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * S;
   ThreadCtx ctx;
@@ -832,6 +834,7 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
   if (w < total) {
     uint32_t slot, j;
     decode_work(w, S, slot, j);
+    if constexpr (PASS) j += (uint32_t)P.pass_begin;
     active = decode_pixel(P, slot, x, y);
     if (active) {
       const uint32_t pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
@@ -841,7 +844,10 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
       d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
       if constexpr (kOverlap) cudaGridDependencySynchronize();
-      if (P.fuse_resolve != RTRB_RESOLVE_SAMPLE_BUFFER) {  // RTRB_RESOLVE_IN_THREAD (IN_CTA is ray-tree only)
+      if constexpr (PASS) {
+        double* out = P.samples + ((unsigned long long)slot * (uint32_t)P.pre + j) * 3ull;
+        out[0] = col.x; out[1] = col.y; out[2] = col.z;
+      } else if (P.fuse_resolve != RTRB_RESOLVE_SAMPLE_BUFFER) {  // RTRB_RESOLVE_IN_THREAD (IN_CTA is ray-tree only)
         // one sample, positive threshold: mean = s / 1.0 = s and variance = 0 < threshold (camera.rb:80-87)
         write_pixel(P, x, y, col.x, col.y, col.z);
       } else {

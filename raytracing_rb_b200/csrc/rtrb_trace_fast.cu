@@ -50,3 +50,15 @@ cudaError_t rtrb_launch_trace_extra_fast(const FrameParams& P, int capacity, cud
   kernel<<<extra_grid(), kBlock, 0, s>>>(P);
   return cudaGetLastError();
 }
+
+cudaError_t rtrb_launch_trace_pass_fast(const FrameParams& P, int capacity, cudaStream_t s) {
+  const FastKernels* k = nullptr;
+  for (const FastKernels* g : {&rtrb_fast::d1, &rtrb_fast::t10, &rtrb_fast::t32, &rtrb_fast::t128})
+    if (g->capacity == capacity) k = g;
+  if (!k) return cudaErrorInvalidValue;
+  // the pre kernels' launch shape for the pass's samples (the lockstep CTAs of the ray-tree kernels included)
+  const unsigned long long threads = pass_threads(P);
+  int block = kBlock;
+  if (k->capacity > 1) block = threads < 4ull * (unsigned long long)sm_count() * kTreeBlock ? RTRB_TREE_MIN_BLOCK : kTreeBlock;
+  return launch_cover(k->pass[P.count_detail != 0][P.use_bvh != 0], threads, block, 0, false, s, P);
+}

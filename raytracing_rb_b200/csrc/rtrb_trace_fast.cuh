@@ -905,7 +905,8 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
 // mean, variance of the signed maximum, adaptive decision, quantisation.  No per-sample FP64 buffer crosses HBM
 // (24 B per sample: 12.7 GB for one 4K / 64 spp frame) and no resolve kernel runs.  RTRB_RESOLVE_IN_CTA selects it;
 // other sample counts (3, 10, ...) write the sample buffer for resolve_kernel.
-template <class Pol, int MAXS, bool BVH, bool BOX>
+// PASS: a progressive frame's pass, whose launch holds pass_end - pass_begin samples of each pixel.
+template <class Pol, int MAXS, bool BVH, bool BOX, bool PASS = false>
 __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                                          ThreadCtx& ctx, int* primary_hit, bool active) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
@@ -916,7 +917,7 @@ __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d
   bool first = true, have = active;
   *primary_hit = -1;
   if (active) ctx.max_stack = max(ctx.max_stack, 1u);
-  const bool mid_barrier = BVH && P.pre < 32;
+  const bool mid_barrier = BVH && (PASS ? P.pass_end - P.pass_begin : P.pre) < 32;
   while (__syncthreads_or(have ? 1 : 0)) {
     HitRec bh;
     int best_i = -1;
@@ -940,10 +941,12 @@ __device__ __forceinline__ d3 trace_sample_fast_lockstep(const FrameParams& P, d
 }
 
 // Kernel body: the first loop of render_at (camera.rb:73-78) for the CTA's samples, then (RTRB_RESOLVE_IN_CTA) its tail.
-template <class Pol, int MAXS, bool BVH, bool DETAIL>
+// PASS: a progressive frame's pass, samples j in [pass_begin, pass_end) into the sample buffer at (slot * pre + j),
+// as trace_pre_body; never resolves in the CTA.
+template <class Pol, int MAXS, bool BVH, bool DETAIL, bool PASS = false>
 __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
   extern __shared__ double rtrb_cta_samples[];  // [blockDim.x][3] when RTRB_RESOLVE_IN_CTA
-  const uint32_t S = (uint32_t)P.pre;
+  const uint32_t S = PASS ? (uint32_t)(P.pass_end - P.pass_begin) : (uint32_t)P.pre;
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   const unsigned long long total = (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS * S;
   ThreadCtx ctx;
@@ -955,6 +958,7 @@ __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
   d3 ro = mk(0, 0, 0), rd = mk(1, 0, 0);
   if (w < total) {
     decode_work(w, S, slot, j);
+    if constexpr (PASS) j += (uint32_t)P.pass_begin;
     active = decode_pixel(P, slot, x, y);
     if (active) {
       pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
@@ -962,12 +966,17 @@ __device__ __forceinline__ void trace_pre_tree_body(const FrameParams& P) {
     }
   }
   int ph = -1;
-  const d3 col = trace_sample_fast_lockstep<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph, active);
+  const d3 col = trace_sample_fast_lockstep<Pol, MAXS, BVH, DETAIL, PASS>(P, ro, rd, pixel, j, ctx, &ph, active);
   if (active) {
     RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
     if (j == 0 && P.hit) P.hit[(size_t)y * P.width + x] = ph;
   }
-  if (P.fuse_resolve == RTRB_RESOLVE_IN_CTA) {
+  if constexpr (PASS) {
+    if (active) {
+      double* out = P.samples + ((unsigned long long)slot * (uint32_t)P.pre + j) * 3ull;
+      out[0] = col.x; out[1] = col.y; out[2] = col.z;
+    }
+  } else if (P.fuse_resolve == RTRB_RESOLVE_IN_CTA) {
     // S divides blockDim.x, so the S samples of a pixel are S consecutive threads of this CTA
     double* mine = rtrb_cta_samples + (size_t)threadIdx.x * 3u;
     mine[0] = col.x; mine[1] = col.y; mine[2] = col.z;

@@ -3,15 +3,18 @@
 // rtrb_fast_l1n (one light, no Monte-Carlo rays).  Each rtrb_trace_fast_*.cu translation unit instantiates one
 // (class, work-stack capacity) pair, so `make -j` compiles them in parallel; rtrb_trace_fast.cu launches them.
 #pragma once
+#include <type_traits>
+
 #include "rtrb_launch.h"
 #include "rtrb_trace_fast.cuh"
 
 // One class build's kernels for one work-stack capacity (1: the stackless depth-1 kernels), indexed
-// [count_detail][use_bvh], and the class they were compiled for.
+// [count_detail][use_bvh], and the class they were compiled for.  pass: progressive-frame passes (generic build only,
+// nullptr elsewhere).
 struct FastKernels {
   bool one_light, lean, no_mc;
   int capacity;
-  TraceKernel pre[2][2], extra[2][2];
+  TraceKernel pre[2][2], extra[2][2], pass[2][2];
 };
 
 namespace rtrb_fast { using Pol = rtrb::Generic;

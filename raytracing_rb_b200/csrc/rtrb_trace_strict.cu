@@ -14,16 +14,20 @@ __global__ void __launch_bounds__(kBlock) trace_extra_strict_kernel(const __grid
   rtrb::trace_extra_body<rtrb::Strict, MAXS, DETAIL>(P);
 }
 template <int MAXS, bool DETAIL>
+__global__ void __launch_bounds__(kBlock) trace_pass_strict_kernel(const __grid_constant__ FrameParams P) {
+  rtrb::trace_pre_body<rtrb::Strict, MAXS, DETAIL, false, true>(P);
+}
+template <int MAXS, bool DETAIL>
 __global__ void __launch_bounds__(kBlock) trace_mt_strict_kernel(const __grid_constant__ FrameParams P) {
   rtrb::trace_mt_body<rtrb::Strict, MAXS, DETAIL>(P);
 }
 
 struct StrictKernels {
-  TraceKernel pre, extra, mt;
+  TraceKernel pre, extra, mt, pass;
 };
 template <int MAXS, bool DETAIL>
 const StrictKernels kKernels = {trace_pre_strict_kernel<MAXS, DETAIL>, trace_extra_strict_kernel<MAXS, DETAIL>,
-                                trace_mt_strict_kernel<MAXS, DETAIL>};
+                                trace_mt_strict_kernel<MAXS, DETAIL>, trace_pass_strict_kernel<MAXS, DETAIL>};
 
 // the kernels of `capacity`, with or without the detailed counters
 const StrictKernels& kernels(const FrameParams& P, int capacity) {
@@ -48,4 +52,7 @@ cudaError_t rtrb_launch_trace_extra_strict(const FrameParams& P, int capacity, c
 cudaError_t rtrb_launch_trace_mt_strict(const FrameParams& P, int capacity, cudaStream_t s) {
   // one thread per PIXEL
   return launch_cover(kernels(P, capacity).mt, (unsigned long long)P.n_tiles * RTRB_SUPER_PIXELS, kBlock, 0, false, s, P);
+}
+cudaError_t rtrb_launch_trace_pass_strict(const FrameParams& P, int capacity, cudaStream_t s) {
+  return launch_cover(kernels(P, capacity).pass, pass_threads(P), kBlock, 0, false, s, P);
 }

@@ -171,6 +171,9 @@ struct FrameParams {
   DevLightF k_lights_f[RTRB_K_LIGHTS];               // = lights_f[]
   int32_t k_pl_index[RTRB_K_PLANES];                 // = pl_index[]
   int32_t k_has_light_tab, pad_k;
+  // progressive frames (rtrb_progressive_pass): the pass kernels trace samples j in [pass_begin, pass_end) of every
+  // slot into samples[slot * pre + j]; `pre` stays the frame's pre_sample_times (the buffer's stride)
+  int32_t pass_begin, pass_end;
 };
 
 static_assert(sizeof(FrameParams) <= 4096, "FrameParams must fit the 4 KB kernel-parameter space");

@@ -58,6 +58,26 @@ def make_ray_opts(precision=_abi.PREC_DEFAULT, seed=1, trace_depth=1, mc=0, coun
     return o
 
 
+def _frame_shape(width, height, pixel_format):
+    """numpy shape of an 8-bit frame in `pixel_format`."""
+    if pixel_format == _abi.FMT_PNG_RGB8:   # H scanlines of (filter byte 0, W x RGB8): IDAT's payload before deflate
+        return (height, width * 3 + 1)
+    return (height, width, 3 if pixel_format == _abi.FMT_RGB8 else 4)
+
+
+def progressive_schedule(pre, first=1):
+    """The doubling pass schedule of a progressive frame of `pre` samples per pixel: first, 2*first, 4*first, ... while
+    below pre, then pre itself (always the last entry).  Pure host logic."""
+    if pre < 1 or first < 1:
+        raise ValueError("pre and first must be >= 1")
+    out, e = [], first
+    while e < pre:
+        out.append(e)
+        e *= 2
+    out.append(pre)
+    return out
+
+
 def _is_tensor(x):
     return type(x).__module__.startswith("torch")
 
@@ -122,11 +142,7 @@ class Renderer:
         """The frame-level call the Ruby shim binds (host buffers in, host buffers out)."""
         opts = opts or make_opts()
         H, W = cam.height, cam.width
-        if opts.pixel_format == _abi.FMT_PNG_RGB8:   # H scanlines of (filter byte 0, W x RGB8): IDAT's payload before deflate
-            shape = (H, W * 3 + 1)
-        else:
-            shape = (H, W, 3 if opts.pixel_format == _abi.FMT_RGB8 else 4)
-        rgba = out_rgba if out_rgba is not None else np.empty(shape, np.uint8)
+        rgba = out_rgba if out_rgba is not None else np.empty(_frame_shape(W, H, opts.pixel_format), np.uint8)
         rgb = np.empty((H, W, 3), np.float64) if want_rgb else None
         hit = np.empty((H, W), np.int32) if want_hit else None
         st = _abi.Stats()
@@ -264,6 +280,10 @@ class Renderer:
         check(lib().rtrb_camera_rays(self._h, C.byref(cam), C.byref(opts), b, e, rays.ctypes.data, keys.ctypes.data))
         return rays, keys
 
+    def progressive(self, cam, opts=None):
+        """A progressive frame of `cam` on this renderer (rtrb_progressive_create) -> Progressive."""
+        return Progressive(self, cam, opts)
+
     def peer_push(self, src_ptr, dst_peer_ptr, nbytes, after_stream=None):
         """Copy-engine gather: queue a D2D copy to a peer mapping behind `after_stream` (see rtrb_peer_push)."""
         check(lib().rtrb_peer_push(self._h, C.c_void_p(src_ptr), C.c_void_p(dst_peer_ptr), nbytes,
@@ -293,6 +313,58 @@ class Renderer:
         buf = (C.c_uint8 * 64)()
         check(lib().rtrb_framebuffer_ipc_export(self._h, width, height, buf))
         return bytes(buf)
+
+
+class Progressive:
+    """A frame whose pre_sample_times samples are traced in passes (rtrb_progressive_*, include/rtrb_b200.h).  After a
+    pass to e < pre samples its outputs and stats are those of the frame with pre = max = e; the pass that reaches pre
+    gives the frame of the camera as given.  Holds a reference to its Renderer, which must outlive it."""
+
+    def __init__(self, renderer, cam, opts=None):
+        self.renderer = renderer
+        self.cam = cam
+        self.opts = opts or make_opts()
+        self.done = 0
+        self.stats, self.code = None, _abi.RTRB_OK
+        self._h = C.c_void_p()
+        check(lib().rtrb_progressive_create(renderer.handle, C.byref(cam), C.byref(self.opts), C.byref(self._h)))
+
+    def pass_to(self, sample_end, want_stats=True):
+        """Traces samples [done, sample_end) -> (stats dict or None, status code).  Synchronises only when want_stats."""
+        st = _abi.Stats()
+        code = lib().rtrb_progressive_pass(self._h, sample_end, C.byref(st) if want_stats else None)
+        check(code, allow_raised=True)
+        self.done = sample_end
+        self.stats, self.code = (st.as_dict() if want_stats else None), code
+        return self.stats, code
+
+    def download(self, want_rgb=True, want_hit=True):
+        """The outputs of the passes so far -> Frame (rgba is None when the 8-bit frame goes to rgba_device_out; stats
+        and code are those of the last pass)."""
+        H, W = self.cam.height, self.cam.width
+        rgba = None if self.opts.rgba_device_out else np.empty(_frame_shape(W, H, self.opts.pixel_format), np.uint8)
+        rgb = np.empty((H, W, 3), np.float64) if want_rgb else None
+        hit = np.empty((H, W), np.int32) if want_hit else None
+        check(lib().rtrb_progressive_download(self._h, rgba.ctypes.data if rgba is not None else None,
+                                              rgb.ctypes.data if want_rgb else None, hit.ctypes.data if want_hit else None))
+        return Frame(rgba, rgb, hit, self.stats, self.code)
+
+    def frame_ptr(self):
+        """Device pointer of the 8-bit frame (e.g. for Renderer.encode_png(src=...))."""
+        p = C.c_void_p()
+        check(lib().rtrb_progressive_frame_ptr(self._h, C.byref(p)))
+        return p.value
+
+    def close(self):
+        if self._h:
+            lib().rtrb_progressive_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def ipc_open(device, handle_bytes):
