@@ -358,6 +358,7 @@ struct SceneImage {
   std::vector<DevLightF> lights_f;
   std::vector<BvhNode> bvh;
   std::vector<float4> light_tab;       // apex tables of the lights (linear-filter scenes with spheres and lights)
+  std::vector<uint32_t> light_cand;    // their candidate masks (FrameParams::light_cand), with light_tab
   std::vector<std::vector<uint8_t>> textures;
 };
 
@@ -374,7 +375,7 @@ bool same_image(const SceneImage& a, const SceneImage& b) {
          same_bytes(a.mat_tex, b.mat_tex) && same_bytes(a.lights, b.lights) && same_bytes(a.boxes, b.boxes) &&
          same_bytes(a.cull_sph, b.cull_sph) && same_bytes(a.cull_pl, b.cull_pl) && same_bytes(a.sph_index, b.sph_index) &&
          same_bytes(a.pl_index, b.pl_index) && same_bytes(a.lights_f, b.lights_f) && same_bytes(a.bvh, b.bvh) &&
-         same_bytes(a.light_tab, b.light_tab);
+         same_bytes(a.light_tab, b.light_tab) && same_bytes(a.light_cand, b.light_cand);
 }
 
 }  // namespace
@@ -403,6 +404,7 @@ struct rtrb_renderer {
   DevBuf<float4> cull_sph, cull_pl;
   DevBuf<BvhNode> bvh;
   DevBuf<float4> light_tab;
+  DevBuf<uint32_t> light_cand;
   DevBuf<int32_t> sph_index, pl_index;
   DevBuf<DevLightF> lights_f;
   std::vector<DevBuf<uint8_t>> textures;  // DevMat::tex holds their addresses
@@ -777,6 +779,11 @@ void build_scene_image(const rtrb_scene_desc* s, SceneImage& img) {
         fa.k.light_tab[l][k] = (l < s->n_lights && k < (int)bsph.size()) ? lt[(size_t)l * bsph.size() + k]
                                                                         : make_float4(0.0f, 0.0f, 0.0f, INFINITY);
     fa.k.has_light_tab = 1;
+    const size_t per_light = 3 * 2 * RTRB_LIGHT_BINS;
+    img.light_cand.resize((size_t)s->n_lights * per_light);
+    for (int l = 0; l < s->n_lights; ++l)
+      rtrb_light_masks(&lt[(size_t)l * bsph.size()].x, (int)bsph.size(),
+                       (uint32_t(*)[2][RTRB_LIGHT_BINS])&img.light_cand[(size_t)l * per_light]);
   }
   fa.m_scene = m_scene;
   fa.max_distance_f = nextafterf((float)s->max_distance, INFINITY);
@@ -816,6 +823,7 @@ void for_each_scene_buffer(rtrb_renderer* r, const SceneImage& img, F&& f) {
   f(r->lights_f, img.lights_f, 1);
   f(r->bvh, img.bvh, 1);
   f(r->light_tab, img.light_tab, 0);
+  f(r->light_cand, img.light_cand, 0);
 }
 
 // The allocations of one apply_scene that replace buffers too small for the new image, in for_each_scene_buffer order
@@ -942,6 +950,7 @@ void fill_scene_params(const rtrb_renderer* r, FrameParams& P) {
     P.k_has_light_tab = f.k.has_light_tab;
   }
   P.light_tab = r->scene.light_tab.empty() ? nullptr : r->light_tab.p;  // only scenes that use the linear filter
+  P.light_cand = r->scene.light_cand.empty() ? nullptr : r->light_cand.p;
   P.cam_tab_valid = 0;
 }
 
@@ -958,6 +967,14 @@ void bake_frame(const rtrb_renderer* r, const rtrb_camera_desc* cam, FrameParams
                                 (double)r->scene.f.m_scene + cm + fabs(cam->aperture_radius));
     for (int k = n_sph; k < RTRB_APEX_MAX; ++k) P.cam_tab[k] = make_float4(0.0f, 0.0f, 0.0f, INFINITY);  // never survives
     P.cam_tab_valid = 1;
+    if (cam->aperture_radius == 0.0) {
+      rtrb_camera_masks(&P.cam_tab[0].x, n_sph, P.pos, P.focal_point, P.left, P.up_n, P.front, cam->image_distance,
+                        cam->retina_width, cam->retina_height, cam->width, cam->height, P.k_cam_tx, P.k_cam_ty);
+    } else {  // rays start anywhere on the lens: every sphere is a candidate
+      const uint32_t all = n_sph >= 32 ? 0xffffffffu : (1u << n_sph) - 1u;
+      for (uint32_t& m : P.k_cam_tx) m = all;
+      for (uint32_t& m : P.k_cam_ty) m = all;
+    }
   }
 }
 

@@ -797,18 +797,19 @@ __device__ __forceinline__ void merge_ctx(ThreadCtx& ctx, const ThreadCtx& t) {
   }
 }
 
-// FAST64 entry point, defined in rtrb_trace_fast.cuh (only instantiated by that translation unit).
-template <class Pol, int MAXS, bool BVH, bool BOX>
+// FAST64 entry point, defined in rtrb_trace_fast.cuh (only instantiated by that translation unit).  CULL: the depth-1
+// frame kernels' candidate masks (FrameParams::k_cam_tx, light_cand); cam_cand = those of the pixel's super-tile.
+template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
-                                                ThreadCtx& ctx, int* primary_hit);
+                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu);
 
 // BVH: FAST64 with the sphere BVH instead of the linear filter.
 // BOX: the FAST64 kernels carry the Box code only in their full-counter (DETAIL) variants; scenes with a
 // box are always dispatched there (rtrb_api.cu, pick_trace_kernels), so the lean hot kernels stay sphere/plane-only.
-template <class Pol, int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
-                                             ThreadCtx& ctx, int* primary_hit) {
-  if constexpr (Pol::fast) return trace_sample_fast<Pol, MAXS, BVH, BOX>(P, ro, rd, pixel, sample, ctx, primary_hit);
+                                             ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu) {
+  if constexpr (Pol::fast) return trace_sample_fast<Pol, MAXS, BVH, BOX, CULL>(P, ro, rd, pixel, sample, ctx, primary_hit, cam_cand);
   else return trace_sample<Pol, MAXS>(P, ro, rd, pixel, sample, ctx, primary_hit);
 }
 
@@ -820,9 +821,11 @@ __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd,
 // attribute, the wait returns at once.
 // PASS: the pass kernels of a progressive frame.  One thread per (pixel, sample j in [pass_begin, pass_end)); the
 // colour goes to the sample buffer at (slot * pre + j), the stride of the whole frame.  No overlap, no in-thread resolve.
+// The FAST64 depth-1 linear-filter kernels narrow the camera apex test to the candidate masks of the pixel's super-tile.
 template <class Pol, int MAXS, bool DETAIL, bool BVH = false, bool PASS = false>
 __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
   constexpr bool kOverlap = Pol::fast && MAXS == 1 && !PASS;
+  constexpr bool kCull = Pol::fast && MAXS == 1 && !BVH;
   if constexpr (kOverlap) cudaTriggerProgrammaticLaunchCompletion();
   const uint32_t S = PASS ? (uint32_t)(P.pass_end - P.pass_begin) : (uint32_t)P.pre;
   const unsigned long long w = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -841,7 +844,13 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
       d3 ro, rd;
       camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
       int ph;
-      d3 col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
+      d3 col;
+      if constexpr (kCull) {
+        const uint32_t cand = P.k_cam_tx[min(x >> 5, RTRB_CAM_TX - 1)] & P.k_cam_ty[min(y >> 5, RTRB_CAM_TY - 1)];
+        col = trace_dispatch<Pol, MAXS, BVH, DETAIL, true>(P, ro, rd, pixel, j, ctx, &ph, cand);
+      } else {
+        col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
+      }
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);
       if constexpr (kOverlap) cudaGridDependencySynchronize();
       if constexpr (PASS) {

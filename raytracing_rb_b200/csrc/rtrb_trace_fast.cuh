@@ -462,6 +462,45 @@ __device__ __forceinline__ uint32_t line_survivors_camera(const FrameParams& P, 
   }
   return m;
 }
+// The same tests over the candidate bits only (CULL kernels): the result is the full scan's, because a sphere outside
+// the candidate mask fails its apex test (rtrb_cull_tables.h).  Camera: the tile's mask is warp-uniform, so the
+// dynamically indexed constant-bank read does not serialise.
+__device__ __forceinline__ uint32_t camera_survivors_of(const FrameParams& P, const uint32_t cand, const CullRay& r) {
+  uint32_t m = 0u;
+  for (uint32_t c = cand; c != 0u; c &= c - 1u) {
+    const int k = __ffs(c) - 1;
+    m |= apex_test(P.cam_tab[k], r) << k;
+  }
+  return m;
+}
+// Shadow probes: the light's masks for the probe line's direction ratios (rtrb_light_masks: axis a of the largest
+// component, ratios w[(a+1)%3] / w[a] and w[(a+2)%3] / w[a], which the line's two directions share).  A direction
+// that is not finite (a probe from the light itself) keeps every sphere, as its apex tests do.  The candidates
+// differ between lanes, so the table entries come from global memory.
+__device__ __forceinline__ uint32_t light_survivors_of(const FrameParams& P, const int light_index, const CullRay& r) {
+  const float ax = fabsf(r.dx), ay = fabsf(r.dy), az = fabsf(r.dz);
+  int a;
+  float wa, wb, wc;
+  if (ax >= ay && ax >= az) { a = 0; wa = r.dx; wb = r.dy; wc = r.dz; }
+  else if (ay >= az) { a = 1; wa = r.dy; wb = r.dz; wc = r.dx; }
+  else { a = 2; wa = r.dz; wb = r.dx; wc = r.dy; }
+  const float inv = rcp_approx(wa);
+  const float s = wb * inv, t = wc * inv;
+  uint32_t cand = 0xffffffffu >> (32 - P.n_sph);
+  if (fabsf(s) <= 2.0f && fabsf(t) <= 2.0f) {
+    constexpr int N = RTRB_LIGHT_BINS;
+    const int i = min(max((int)((s + 1.0f) * (0.5f * N)), 0), N - 1), j = min(max((int)((t + 1.0f) * (0.5f * N)), 0), N - 1);
+    const uint32_t* cube = P.light_cand + (size_t)((light_index * 3 + a) * 2) * N;
+    cand = __ldg(&cube[i]) & __ldg(&cube[N + j]);
+  }
+  const float4* tab = P.light_tab + (size_t)light_index * P.n_sph;
+  uint32_t m = 0u;
+  for (uint32_t c = cand; c != 0u; c &= c - 1u) {
+    const int k = __ffs(c) - 1;
+    m |= apex_test(__ldg(&tab[k]), r) << k;
+  }
+  return m;
+}
 template <bool KT>
 __device__ __forceinline__ uint32_t line_survivors_light(const FrameParams& P, const int light_index, const CullRay& r) {
   uint32_t m = 0u;
@@ -483,11 +522,15 @@ __device__ __forceinline__ uint32_t line_survivors_light(const FrameParams& P, c
 }
 
 // World#intersect (world.rb:37-59) = FP32 filter over every object + exact test of the survivors.
-template <class Pol, bool BOX, bool KT>
+template <class Pol, bool BOX, bool KT, bool CULL = false>
 __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3 d, const CullRay& r, HitRec& bh,
-                                                ThreadCtx& ctx, const bool through_lens) {
+                                                ThreadCtx& ctx, const bool through_lens, const uint32_t cam_cand = 0xffffffffu) {
   if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return closest_hit_scan_call<Pol, BOX>(P, o, d, bh, ctx);
-  const uint32_t mask = (through_lens && P.cam_tab_valid) ? line_survivors_camera(P, r) : line_survivors_generic<KT>(P, r);
+  uint32_t mask;
+  if constexpr (CULL)
+    mask = (through_lens && P.cam_tab_valid) ? camera_survivors_of(P, cam_cand, r) : line_survivors_generic<KT>(P, r);
+  else
+    mask = (through_lens && P.cam_tab_valid) ? line_survivors_camera(P, r) : line_survivors_generic<KT>(P, r);
   // pass 1 (only when something can be pruned): the smallest certain upper bound; nothing at or beyond
   // max_distance can win (world.rb:39)
   float best_hi = P.max_distance_f;
@@ -555,7 +598,7 @@ __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3
 // An object the probe ray certainly misses (or certainly meets beyond the light) has factor 0, hence
 // cover exactly 0 (sphere.rb:29,45-53 multiply everything by factor; world_object.rb:43-47), and
 // total - 0 == total, so skipping it leaves the running difference bit-identical.
-template <class Pol, bool BOX, bool KT>
+template <class Pol, bool BOX, bool KT, bool CULL = false>
 __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 target, const DevLight& L, const int light_index,
                                                   ThreadCtx& ctx) {
   CullRay r;
@@ -563,7 +606,9 @@ __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 targe
   CoverRay c = make_cover_probe(P, target, L, r, far);
   if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return lit_area_call<Pol, BOX>(P, target, L, ctx);
   // the probe ray's line passes through the light: apex table of this light when there is one
-  uint32_t sm = (P.k_has_light_tab != 0) ? line_survivors_light<KT>(P, light_index, r) : line_survivors_generic<KT>(P, r);
+  uint32_t sm;
+  if constexpr (CULL) sm = (P.k_has_light_tab != 0) ? light_survivors_of(P, light_index, r) : line_survivors_generic<KT>(P, r);
+  else sm = (P.k_has_light_tab != 0) ? line_survivors_light<KT>(P, light_index, r) : line_survivors_generic<KT>(P, r);
   uint32_t qm = 0u;
   for (int k = 0; k < P.n_pl; ++k) {
     float lo, hi;
@@ -609,17 +654,17 @@ __device__ __forceinline__ const DevLightF& light_f_at(const FrameParams& P, int
 
 // Compile-time choice: kernels are instantiated once per filter so each stays compact (the linear
 // scan wins below ~32 spheres: measured 5.56 vs 6.05 ms on config 3; the BVH wins 5x on config 5).
-template <class Pol, bool BVH, bool BOX, bool KT>
+template <class Pol, bool BVH, bool BOX, bool KT, bool CULL = false>
 __device__ __forceinline__ int closest_hit_fast(const FrameParams& P, d3 o, d3 d, const CullRay& r, HitRec& bh,
-                                                ThreadCtx& ctx, const bool through_lens) {
+                                                ThreadCtx& ctx, const bool through_lens, const uint32_t cam_cand = 0xffffffffu) {
   if constexpr (BVH) return closest_hit_bvh<Pol, BOX>(P, o, d, r, bh, ctx);
-  else return closest_hit_linear<Pol, BOX, KT>(P, o, d, r, bh, ctx, through_lens);
+  else return closest_hit_linear<Pol, BOX, KT, CULL>(P, o, d, r, bh, ctx, through_lens, cam_cand);
 }
-template <class Pol, bool BVH, bool BOX, bool KT>
+template <class Pol, bool BVH, bool BOX, bool KT, bool CULL = false>
 __device__ __forceinline__ double lit_area_fast(const FrameParams& P, d3 target, const DevLight& L, const int light_index,
                                                 ThreadCtx& ctx) {
   if constexpr (BVH) return lit_area_bvh<Pol, BOX>(P, target, L, ctx);
-  else return lit_area_linear<Pol, BOX, KT>(P, target, L, light_index, ctx);
+  else return lit_area_linear<Pol, BOX, KT, CULL>(P, target, L, light_index, ctx);
 }
 
 // The reference's own expression of the highlight match (world.rb:86-93), register-only interface.  Only the depth-1
@@ -682,9 +727,9 @@ __device__ __forceinline__ bool attenuation_dead(d3 att) {
 //            here (dead, terminated by a highlight, or a miss);
 //   phase B  intersect_parameters, the children (pushed onto `stack`), World#local_lights and local_lighting.
 // Emitted colours are added to `sum` in emission order.
-template <class Pol, int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackItem& it, d3& sum, ThreadCtx& ctx, bool is_first,
-                                            int* primary_hit, HitRec& bh) {
+                                            int* primary_hit, HitRec& bh, const uint32_t cam_cand = 0xffffffffu) {
   constexpr bool KT = !BVH && MAXS == 1;  // constant-bank tables: depth-1 linear-filter kernels only (see pl_rec)
   const d3 o = mk(it.ox, it.oy, it.oz), d = mk(it.dx, it.dy, it.dz), att = mk(it.ax, it.ay, it.az);
   if (it.depth <= 0 || attenuation_dead(att)) return -1;  // rt_map :52
@@ -714,7 +759,7 @@ __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackIte
   // ---- World#intersect ----
   bh.p = mk(0, 0, 0); bh.dir_in = false;
   if constexpr (BOX) bh.face = 0;
-  const int best_i = closest_hit_fast<Pol, BVH, BOX, KT>(P, o, d, r, bh, ctx, is_first);
+  const int best_i = closest_hit_fast<Pol, BVH, BOX, KT, CULL>(P, o, d, r, bh, ctx, is_first, cam_cand);
   if (best_i < 0) return -1;
   if (is_first) *primary_hit = best_i;
   RTRB_COUNT(ctx, RTRB_CNT_HITS);
@@ -742,7 +787,7 @@ static __device__ __noinline__ uint32_t born_dead_children_status(double dx, dou
   return t.status;
 }
 
-template <class Pol, int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackItem& it, const int best_i, const HitRec& bh,
                                              StackItem* stack, int& sp, d3& sum, ThreadCtx& ctx, uint32_t pixel,
                                              uint32_t sample) {
@@ -807,7 +852,7 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
     for (int l = 0; l < Pol::n_lights(P); ++l) {
       const DevLight& L = light_at<KT>(P, l);
       ctx.shadow++;
-      const double area = lit_area_fast<Pol, BVH, BOX, KT>(P, shade_from, L, l, ctx);
+      const double area = lit_area_fast<Pol, BVH, BOX, KT, CULL>(P, shade_from, L, l, ctx);
       if (area > 0) {
         double w = rb_pow<Pol>(area, Pol::shadow_exponent(P));
         if (Pol::n_lights(P) != 1) w = w / (double)Pol::n_lights(P);  // x / 1.0 == x
@@ -858,20 +903,20 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
   }
 }
 
-template <class Pol, int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ void process_item_fast(const FrameParams& P, const StackItem& it, StackItem* stack, int& sp,
                                                   d3& sum, ThreadCtx& ctx, uint32_t pixel, uint32_t sample,
-                                                  bool is_first, int* primary_hit) {
+                                                  bool is_first, int* primary_hit, const uint32_t cam_cand = 0xffffffffu) {
   HitRec bh;
-  const int best_i = item_phase_a<Pol, MAXS, BVH, BOX>(P, it, sum, ctx, is_first, primary_hit, bh);
-  if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
+  const int best_i = item_phase_a<Pol, MAXS, BVH, BOX, CULL>(P, it, sum, ctx, is_first, primary_hit, bh, cam_cand);
+  if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX, CULL>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
 }
 
 // RayTracer#trace_sync for one sample, free-running: the item loop of the depth-1, extra-sample and ray-query kernels
 // (the ray-tree frame kernels run trace_sample_fast_lockstep).
-template <class Pol, int MAXS, bool BVH, bool BOX>
+template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
-                                                ThreadCtx& ctx, int* primary_hit) {
+                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
   // the root item starts in registers (no round trip through the local-memory stack)
   StackItem it;
@@ -882,7 +927,7 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
   *primary_hit = -1;
   ctx.max_stack = max(ctx.max_stack, 1u);
   while (true) {
-    process_item_fast<Pol, MAXS, BVH, BOX>(P, it, stack, sp, sum, ctx, pixel, sample, first, primary_hit);
+    process_item_fast<Pol, MAXS, BVH, BOX, CULL>(P, it, stack, sp, sum, ctx, pixel, sample, first, primary_hit, cam_cand);
     first = false;
     if (MAXS == 1 || sp == 0) break;
     if ((uint32_t)sp > ctx.max_stack) ctx.max_stack = (uint32_t)sp;

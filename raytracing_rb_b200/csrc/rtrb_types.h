@@ -11,6 +11,7 @@
 #include <stdint.h>
 
 #include "rtrb_bvh.h"
+#include "rtrb_cull_tables.h"
 
 #define RTRB_MAX_LIGHTS 64
 #define RTRB_SUPER 32                 // super-tile edge in pixels (tile partition unit across GPUs)
@@ -174,6 +175,11 @@ struct FrameParams {
   // progressive frames (rtrb_progressive_pass): the pass kernels trace samples j in [pass_begin, pass_end) of every
   // slot into samples[slot * pre + j]; `pre` stays the frame's pre_sample_times (the buffer's stride)
   int32_t pass_begin, pass_end;
+  // Candidate masks of the depth-1 linear-filter kernels (rtrb_cull_tables.h): camera rays of super-tile (tx, ty) need
+  // the apex test only for the spheres in k_cam_tx[tx] & k_cam_ty[ty] (tiles beyond the last entry share it), shadow
+  // probes of light l only for those in light_cand's bins of their direction.  Every set bit is a sphere < n_sph.
+  uint32_t k_cam_tx[RTRB_CAM_TX], k_cam_ty[RTRB_CAM_TY];  // valid with cam_tab_valid (all spheres: aperture frames)
+  const uint32_t* light_cand;  // [n_lights][3 axes][2 ratios][RTRB_LIGHT_BINS], valid with k_has_light_tab
 };
 
 static_assert(sizeof(FrameParams) <= 4096, "FrameParams must fit the 4 KB kernel-parameter space");
