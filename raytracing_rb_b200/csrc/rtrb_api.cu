@@ -338,7 +338,6 @@ struct SceneImage {
     float m_scene, max_distance_f;
     // small scenes: the per-ray tables that travel in the kernel parameters (FrameParams::k_*)
     struct SmallTables {
-      float4 light_tab[RTRB_K_LIGHTS][RTRB_APEX_MAX];
       float4 cull_sph[RTRB_APEX_MAX];
       float4 cull_pl[2 * RTRB_K_PLANES];
       DevLight lights[RTRB_K_LIGHTS];
@@ -774,10 +773,6 @@ void build_scene_image(const rtrb_scene_desc* s, SceneImage& img) {
       for (size_t k = 0; k < bsph.size(); ++k)
         lt[(size_t)l * bsph.size() + k] = apex_entry(s->lights[l].position, 0.0, bsph[k].c, bsph[k].r, (double)m_scene + lm);
     }
-    for (int l = 0; l < RTRB_K_LIGHTS; ++l)
-      for (int k = 0; k < RTRB_APEX_MAX; ++k)
-        fa.k.light_tab[l][k] = (l < s->n_lights && k < (int)bsph.size()) ? lt[(size_t)l * bsph.size() + k]
-                                                                        : make_float4(0.0f, 0.0f, 0.0f, INFINITY);
     fa.k.has_light_tab = 1;
     const size_t per_light = 3 * 2 * RTRB_LIGHT_BINS;
     img.light_cand.resize((size_t)s->n_lights * per_light);
@@ -940,8 +935,7 @@ void fill_scene_params(const rtrb_renderer* r, FrameParams& P) {
   P.use_bvh = f.small_scene ? 0 : 1;
   P.scene_class = f.scene_class;
   if (f.small_scene) {
-    static_assert(sizeof(f.k.light_tab) == sizeof(P.k_light_tab) && sizeof(f.k.lights) == sizeof(P.k_lights), "table layout");
-    memcpy(P.k_light_tab, f.k.light_tab, sizeof(P.k_light_tab));
+    static_assert(sizeof(f.k.lights) == sizeof(P.k_lights), "table layout");
     memcpy(P.k_cull_sph, f.k.cull_sph, sizeof(P.k_cull_sph));
     memcpy(P.k_cull_pl, f.k.cull_pl, sizeof(P.k_cull_pl));
     memcpy(P.k_lights, f.k.lights, sizeof(P.k_lights));
@@ -970,6 +964,13 @@ void bake_frame(const rtrb_renderer* r, const rtrb_camera_desc* cam, FrameParams
     if (cam->aperture_radius == 0.0) {
       rtrb_camera_masks(&P.cam_tab[0].x, n_sph, P.pos, P.focal_point, P.left, P.up_n, P.front, cam->image_distance,
                         cam->retina_width, cam->retina_height, cam->width, cam->height, P.k_cam_tx, P.k_cam_ty);
+      // only the depth-1 kernels read them; at trace_depth 0 a camera ray is not even counted, so the sky path's
+      // "one ray" would be wrong there
+      static_assert(sizeof(P.k_tile_rows) == RTRB_CAM_TX * 4, "tile rows layout");
+      if (cam->trace_depth == 1)
+        rtrb_tile_rows(&P.k_cull_pl[0].x, P.n_pl, P.k_lights_f, P.n_lights, P.pos, P.focal_point, P.left, P.up_n,
+                       P.front, cam->image_distance, cam->retina_width, cam->retina_height, cam->width, cam->height,
+                       (uint8_t(*)[4])P.k_tile_rows);
     } else {  // rays start anywhere on the lens: every sphere is a candidate
       const uint32_t all = n_sph >= 32 ? 0xffffffffu : (1u << n_sph) - 1u;
       for (uint32_t& m : P.k_cam_tx) m = all;

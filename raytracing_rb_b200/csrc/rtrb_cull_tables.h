@@ -59,11 +59,50 @@ inline bool rtrb_lens_pixels(double lo, double hi, double half, int W, int& i0, 
   return true;
 }
 
+// What the camera masks and the tile certificates know about the primary rays of a pinhole frame.  Pixel (x, y) looks
+// along rf = front^ * D - left * sx(x) - up^ * sy(y) from the camera (camera.rb:130-134; the ray's FP64 direction is a
+// positive or negative multiple of rf).  The FP32 u the kernel tests and the pixel's exact direction differ by the FP32
+// normalisation (< 2^-20 rad) and by the FP64 ray's own rounding: rd = target - pos = rf (t - 1) with |t - 1| = |od| /
+// |rf . front^| (od: distance of the focal plane), so |rd| >= |od| while the rounding of target is below 64 eps (|pos| +
+// |focal| + 2 rf_max (1 + |od| / c_min)).  `dir` bounds that angle; in retina units it moves (sx, sy) by at most
+// dir * rf_max^2 / c_min, which must stay under a quarter pixel for the one-pixel dilation.
+struct RtrbPinhole {
+  double f[3];    // front^
+  double c_min;   // |rf . front^| >= c_min over the frame
+  double rf_max;  // |rf| <= rf_max
+  double od;      // (focal_point - pos) . front^ (signed)
+  double dir;     // angle between the pixel's exact direction and the FP32 u of its ray
+  bool ok;        // the bounds hold and the direction error is under a quarter pixel
+};
+inline RtrbPinhole rtrb_pinhole(const double pos[3], const double focal_point[3], const double left[3], const double up_n[3],
+                                const double front[3], double D, double rw, double rh, int W, int H) {
+  RtrbPinhole c;
+  const double fl = sqrt(front[0] * front[0] + front[1] * front[1] + front[2] * front[2]);
+  for (int i = 0; i < 3; ++i) c.f[i] = front[i] / fl;
+  const double* f = c.f;
+  const double lf = fabs(left[0] * f[0] + left[1] * f[1] + left[2] * f[2]);
+  const double uf = fabs(up_n[0] * f[0] + up_n[1] * f[1] + up_n[2] * f[2]);
+  const double ln = sqrt(left[0] * left[0] + left[1] * left[1] + left[2] * left[2]);
+  const double un = sqrt(up_n[0] * up_n[0] + up_n[1] * up_n[1] + up_n[2] * up_n[2]);
+  c.c_min = fabs(D) - fabs(rw) * lf - fabs(rh) * uf;
+  c.rf_max = fabs(D) + fabs(rw) * ln + fabs(rh) * un;
+  const double dp[3] = {focal_point[0] - pos[0], focal_point[1] - pos[1], focal_point[2] - pos[2]};
+  c.od = dp[0] * f[0] + dp[1] * f[1] + dp[2] * f[2];
+  const double od = fabs(c.od);
+  const double pn = sqrt(pos[0] * pos[0] + pos[1] * pos[1] + pos[2] * pos[2]);
+  const double fn = sqrt(focal_point[0] * focal_point[0] + focal_point[1] * focal_point[1] + focal_point[2] * focal_point[2]);
+  c.dir = 9.5367431640625e-7 + 64.0 * 1.1102230246251565e-16 * (pn + fn + 2.0 * c.rf_max * (1.0 + od / c.c_min)) / od;
+  const double shift = c.dir * c.rf_max * c.rf_max / c.c_min;
+  const double pitch = fmin(2.0 * fabs(rw) / W, 2.0 * fabs(rh) / H);
+  c.ok = isfinite(fl) && fl > 0.0 && isfinite(D) && c.c_min > 1e-9 * c.rf_max && isfinite(shift) && isfinite(pitch) &&
+         shift < 0.25 * pitch && W > 0 && H > 0;
+  return c;
+}
+
 // Camera masks of a pinhole frame: tx[c] / ty[r] = the spheres whose camera apex test can keep the primary ray of some
-// pixel in super-tile column c / row r.  Pixel (x, y) looks along rf = front^ * D - left * sx(x) - up^ * sy(y) from the
-// camera (camera.rb:130-134; the ray's FP64 direction is a positive or negative multiple of rf), so a point
-// p = a left + b up^ + c front^ (relative to the camera) is on the line of (sx, sy) = (-D a / c, -D b / c).
-// A ball of radius rho around V lies in the box of half-widths rho |row_i(B^-1)| in (a, b, c) (B = [left up^ front^]).
+// pixel in super-tile column c / row r.  A point p = a left + b up^ + c front^ (relative to the camera) is on the line
+// of (sx, sy) = (-D a / c, -D b / c) (rtrb_pinhole).  A ball of radius rho around V lies in the box of half-widths
+// rho |row_i(B^-1)| in (a, b, c) (B = [left up^ front^]).
 // Everything is set when the camera is degenerate or the FP64 ray direction cannot be bounded to well under a pixel.
 inline void rtrb_camera_masks(const float* tab, int n, const double pos[3], const double focal_point[3], const double left[3],
                               const double up_n[3], const double front[3], double D, double rw, double rh, int W, int H,
@@ -75,8 +114,8 @@ inline void rtrb_camera_masks(const float* tab, int n, const double pos[3], cons
     for (int i = 0; i < RTRB_CAM_TX; ++i) tx[i] |= m;
     for (int i = 0; i < RTRB_CAM_TY; ++i) ty[i] |= m;
   };
-  const double fl = sqrt(front[0] * front[0] + front[1] * front[1] + front[2] * front[2]);
-  const double f[3] = {front[0] / fl, front[1] / fl, front[2] / fl};
+  const RtrbPinhole cam = rtrb_pinhole(pos, focal_point, left, up_n, front, D, rw, rh, W, H);
+  const double* f = cam.f;
   // rows of B^-1: cross products of the other two columns over det
   double inv[3][3];
   const double c0[3] = {up_n[1] * f[2] - up_n[2] * f[1], up_n[2] * f[0] - up_n[0] * f[2], up_n[0] * f[1] - up_n[1] * f[0]};
@@ -87,27 +126,7 @@ inline void rtrb_camera_masks(const float* tab, int n, const double pos[3], cons
   for (int k = 0; k < 3; ++k) { inv[0][k] = c0[k] / det; inv[1][k] = c1[k] / det; inv[2][k] = c2[k] / det; }
   double rown[3];
   for (int i = 0; i < 3; ++i) rown[i] = sqrt(inv[i][0] * inv[i][0] + inv[i][1] * inv[i][1] + inv[i][2] * inv[i][2]);
-  // |rf| <= rf_max, |rf . front^| >= c_min over the frame
-  const double lf = fabs(left[0] * f[0] + left[1] * f[1] + left[2] * f[2]);
-  const double uf = fabs(up_n[0] * f[0] + up_n[1] * f[1] + up_n[2] * f[2]);
-  const double ln = sqrt(left[0] * left[0] + left[1] * left[1] + left[2] * left[2]);
-  const double un = sqrt(up_n[0] * up_n[0] + up_n[1] * up_n[1] + up_n[2] * up_n[2]);
-  const double c_min = fabs(D) - fabs(rw) * lf - fabs(rh) * uf;
-  const double rf_max = fabs(D) + fabs(rw) * ln + fabs(rh) * un;
-  // The FP32 u the kernel tests and the pixel's exact direction differ by the FP32 normalisation (< 2^-20 rad) and by
-  // the FP64 ray's own rounding: rd = target - pos = rf (t - 1) with |t - 1| = |od| / |rf . front^| (od: distance of
-  // the focal plane), so |rd| >= |od| while the rounding of target is below 64 eps (|pos| + |focal| + 2 rf_max (1 +
-  // |od| / c_min)).  In retina units a direction error moves (sx, sy) by at most dir * rf_max^2 / c_min, which must
-  // stay under a quarter pixel for the one-pixel dilation.
-  const double dp[3] = {focal_point[0] - pos[0], focal_point[1] - pos[1], focal_point[2] - pos[2]};
-  const double od = fabs(dp[0] * f[0] + dp[1] * f[1] + dp[2] * f[2]);
-  const double pn = sqrt(pos[0] * pos[0] + pos[1] * pos[1] + pos[2] * pos[2]);
-  const double fn = sqrt(focal_point[0] * focal_point[0] + focal_point[1] * focal_point[1] + focal_point[2] * focal_point[2]);
-  const double dir = 9.5367431640625e-7 + 64.0 * 1.1102230246251565e-16 * (pn + fn + 2.0 * rf_max * (1.0 + od / c_min)) / od;
-  const double shift = dir * rf_max * rf_max / c_min;
-  const double pitch = fmin(2.0 * fabs(rw) / W, 2.0 * fabs(rh) / H);
-  bool ok = isfinite(det) && fabs(det) > 1e-6 && isfinite(D) && c_min > 1e-9 * rf_max && isfinite(shift) && isfinite(pitch) &&
-            shift < 0.25 * pitch && W > 0 && H > 0 && isfinite(rown[0] + rown[1] + rown[2]);
+  const bool ok = cam.ok && isfinite(det) && fabs(det) > 1e-6 && isfinite(rown[0] + rown[1] + rown[2]);
   if (!ok) { fill(all); return; }
   for (int k = 0; k < n; ++k) {
     const float* t = tab + 4 * (size_t)k;
@@ -158,5 +177,142 @@ inline void rtrb_light_masks(const float* tab, int n, uint32_t m[3][2][RTRB_LIGH
         for (int i = i0; i <= i1; ++i) m[a][j][i] |= 1u << k;
       }
     }
+  }
+}
+
+// FP32 view of a light for the highlight filter (DevLightF, rtrb_types.h).
+struct RtrbLightF {
+  float px, py, pz;
+  float pmax;       // |position|_inf
+  float cos2_thr;   // cos^2(high_light_angle), valid when mode == 1
+  int32_t mode;     // 1: threshold in (0, 90 deg) -> FP32 filter usable; 0: always take the exact path
+};
+
+// Tile certificates of a pinhole frame: rows[c] = {s0, s1, h0, h1} for super-tile column c < RTRB_CAM_TX.  Every primary
+// ray of the super-tiles (c, r), r in [s0, s1), is rejected by classify_plane for every plane as certainly behind its
+// origin (kind 0), and every primary ray of the rows [s0, s1) and [h0, h1) fails highlight_match_fast for every light
+// at its FP32 test (c2 + tol < cos2_thr): the kernels reach neither the exact plane test nor the exact highlight
+// expression there, so skipping those filters cannot change a frame, a hit id or a counter.  A column's certified rows
+// need not be contiguous (the light's image splits them); each interval is its longest run.  All zero = nothing.
+//
+// Bounds, per tile dilated by one pixel: the device's FP32 u is within dir + 2^-17 of the pixel's exact unit direction
+// (rtrb_pinhole; the 2^-17 covers |u| = 1 +- 2^-18).  With rf = D f - sx left - sy up (f = front^), any n . rf is linear
+// and separable in (sx, sy), so its range over a tile is the sum of a column term and a row term; |rf| <= rf_max and
+// |rf|^2 >= lam (D^2 + sx^2 + sy^2), lam a Gershgorin bound on the Gram matrix of (f, left, up).  The FP32 evaluations
+// of den, num, t, e_t (classify_plane) and of ret, a2, c2, rho, tol (highlight_match_fast) are bounded with margins
+// well above their documented error: a few ulp per fmaf chain, rcp.approx / rsqrt.approx within 2^-21 relative.
+// `o` is the FP32 ray origin (the camera position rounded to float); pl = k_cull_pl (8 floats per plane).
+inline void rtrb_tile_rows(const float* pl, int n_pl, const RtrbLightF* lf, int n_lights, const double pos[3],
+                           const double focal_point[3], const double left[3], const double up_n[3], const double front[3],
+                           double D, double rw, double rh, int W, int H, uint8_t rows[RTRB_CAM_TX][4]) {
+  for (int c = 0; c < RTRB_CAM_TX; ++c) rows[c][0] = rows[c][1] = rows[c][2] = rows[c][3] = 0;
+  const RtrbPinhole cam = rtrb_pinhole(pos, focal_point, left, up_n, front, D, rw, rh, W, H);
+  const double eps = 5.9604644775390625e-8;  // 2^-24
+  // the ray runs along +rf when D > 0 and the focal plane is in front (rd = rf (t - 1), t - 1 = od / (rf . f))
+  if (!cam.ok || !(D > 0.0) || !(cam.od > 0.0) || n_pl > 8 || n_lights > 2) return;
+  const double* f = cam.f;
+  const double dl = cam.dir + 7.62939453125e-6;  // |u - u_exact|
+  const float o32[3] = {(float)pos[0], (float)pos[1], (float)pos[2]};
+  const double o[3] = {o32[0], o32[1], o32[2]};
+  const double mo = fmax(fabs(o[0]), fmax(fabs(o[1]), fabs(o[2])));
+  auto dot = [](const double* a, const double* b) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; };
+  // a . rf over the tile = a.f D + X(sx) + Y(sy): range of the column / row terms
+  const int nc = (W + 31) / 32 < RTRB_CAM_TX ? (W + 31) / 32 : RTRB_CAM_TX;
+  const int nr = (H + 31) / 32 < 255 ? (H + 31) / 32 : 255;
+  auto sx = [&](int x) { return 2.0 * ((double)x / W - 0.5) * rw; };
+  auto sy = [&](int y) { return 2.0 * ((double)y / H - 0.5) * rh; };
+  auto range = [](double k, double s0, double s1, double& lo, double& hi) {  // of -k s over [s0, s1] (either order)
+    const double a = -k * s0, b = -k * s1;
+    lo = a < b ? a : b; hi = a < b ? b : a;
+  };
+  auto sq_min = [](double s0, double s1) { return (s0 <= 0.0) == (s1 <= 0.0) ? (s0 * s0 < s1 * s1 ? s0 * s0 : s1 * s1) : 0.0; };
+  // ---- planes: certainly behind the origin when s g >= g_th over the tile (s = -sign(num), g = n . rf) ----
+  double p_sgn[8], p_c[8], p_th[8], p_kl[8], p_ku[8];
+  bool planes_ok = true;
+  for (int k = 0; k < n_pl && planes_ok; ++k) {
+    const float* a = pl + 8 * k;
+    const double n[3] = {a[0], a[1], a[2]}, aw = a[3], pw = a[7];
+    const double num = ((double)a[4] - o[0]) * n[0] + ((double)a[5] - o[1]) * n[1] + ((double)a[6] - o[2]) * n[2];
+    const double e_num = 16.0 * eps * aw * (pw + mo) * 1.0001, e_den = 16.0 * eps * aw;
+    const double n_lo = fabs(num) - 0.5 * e_num;  // |num| on the device (its error is below 5/16 e_num)
+    const double q = 0.999 / 1.1002 - e_num / n_lo;
+    // |den| > 16 e_den (else kind 1), and t + e_t < 0 once 1.1002 (e_num / |num| + e_den / |den|) < 0.999
+    const double den_req = fmax(256.0 * eps * aw * 1.0001, e_den / q);
+    const double nn = sqrt(dot(n, n));
+    const double m_n = nn * dl + 8.0 * eps * aw * (1.0 + dl);  // |den - n . u_exact|
+    p_sgn[k] = num > 0.0 ? -1.0 : 1.0;
+    p_c[k] = p_sgn[k] * dot(n, f) * D;
+    p_th[k] = (den_req + m_n) * cam.rf_max * (1.0 + 1e-9) + 1e-300;
+    p_kl[k] = p_sgn[k] * dot(n, left);
+    p_ku[k] = p_sgn[k] * dot(n, up_n);
+    planes_ok = aw > 0.0 && n_lo > 0.0 && q > 0.0 && isfinite(num) && isfinite(p_th[k]) && isfinite(p_c[k]) &&
+                isfinite(p_kl[k]) && isfinite(p_ku[k]);
+  }
+  // ---- lights: |a . u| < cthr |a| with margin, i.e. h^2 < K (D^2 + sx^2 + sy^2), h = a . rf ----
+  double g[3][3];
+  const double* B[3] = {f, left, up_n};
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j) g[i][j] = dot(B[i], B[j]);
+  double lam = 1e300;
+  for (int i = 0; i < 3; ++i) lam = fmin(lam, g[i][i] - fabs(g[i][(i + 1) % 3]) - fabs(g[i][(i + 2) % 3]));
+  lam *= 1.0 - 1e-9;
+  double l_c[2], l_kl[2], l_ku[2], l_K[2];
+  bool lights_ok = lam > 0.0;
+  for (int l = 0; l < n_lights && lights_ok; ++l) {
+    const RtrbLightF& F = lf[l];
+    const double a[3] = {(double)F.px - o[0], (double)F.py - o[1], (double)F.pz - o[2]};
+    const double an = sqrt(dot(a, a)), a1 = fabs(a[0]) + fabs(a[1]) + fabs(a[2]);
+    const double ea = 8.0 * eps * ((double)F.pmax + mo) * 1.0001;
+    const double rho = 8.0 * (ea / (an * (1.0 - 1e-5)) + 8.0 * eps) * 1.0001;
+    const double tol = (rho * rho + 2.0 * rho) * 1.0001;
+    // c2 <= (ret / |a|)^2 (1 + 2^-18); the FP32 sum c2 + tol must not round up to cos2_thr
+    const double c2_room = ((double)F.cos2_thr * (1.0 - 1e-6) - tol) / (1.0 + 3.814697265625e-6);
+    const double m_a = an * (dl + 2.0 * eps) + 8.0 * eps * a1 * (1.0 + dl);           // |ret - a . u_exact|
+    const double room = c2_room > 0.0 ? sqrt(c2_room) * an - m_a : -1.0;
+    l_c[l] = dot(a, f) * D;
+    l_kl[l] = dot(a, left);
+    l_ku[l] = dot(a, up_n);
+    l_K[l] = room * room * lam * (1.0 - 1e-9);
+    lights_ok = F.mode == 1 && rho < 0.25 && room > 0.0 && isfinite(l_K[l]) && isfinite(l_c[l]) && isfinite(l_kl[l]) &&
+                isfinite(l_ku[l]) && an > 0.0;
+  }
+  if (!lights_ok) return;  // every certificate needs the highlight one
+  // per row: the row terms (tile rows r, dilated by one pixel)
+  double ry_lo[8][255], ry_hi[2][255], ry_hl[2][255], ry_s2[255];
+  for (int r = 0; r < nr; ++r) {
+    const double s0 = sy(32 * r - 1), s1 = sy(32 * r + 32);
+    ry_s2[r] = sq_min(s0, s1);
+    double lo, hi;
+    for (int k = 0; k < n_pl; ++k) { range(p_ku[k], s0, s1, lo, hi); ry_lo[k][r] = lo; }
+    for (int l = 0; l < n_lights; ++l) { range(l_ku[l], s0, s1, lo, hi); ry_hl[l][r] = lo; ry_hi[l][r] = hi; }
+  }
+  for (int c = 0; c < nc; ++c) {
+    const double s0 = sx(32 * c - 1), s1 = sx(32 * c + 32);
+    const double D2 = D * D + sq_min(s0, s1);
+    double cx_lo[8], hx_lo[2], hx_hi[2], lo, hi;
+    for (int k = 0; k < n_pl; ++k) { range(p_kl[k], s0, s1, lo, hi); cx_lo[k] = p_c[k] + lo; }
+    for (int l = 0; l < n_lights; ++l) { range(l_kl[l], s0, s1, lo, hi); hx_lo[l] = l_c[l] + lo; hx_hi[l] = l_c[l] + hi; }
+    // branch-free passes over the column's rows (they vectorise), then the longest run of each kind
+    uint8_t hl[256], sky[256];
+    for (int r = 0; r < nr; ++r) hl[r] = 1;
+    for (int l = 0; l < n_lights; ++l)
+      for (int r = 0; r < nr; ++r) {
+        const double h0 = -(hx_lo[l] + ry_hl[l][r]), h1 = hx_hi[l] + ry_hi[l][r], h = h0 > h1 ? h0 : h1;
+        hl[r] &= (uint8_t)(h * h < l_K[l] * (D2 + ry_s2[r]));
+      }
+    for (int r = 0; r < nr; ++r) sky[r] = hl[r] & (uint8_t)planes_ok;
+    for (int k = 0; k < n_pl; ++k)
+      for (int r = 0; r < nr; ++r) sky[r] &= (uint8_t)(cx_lo[k] + ry_lo[k][r] >= p_th[k]);
+    hl[nr] = sky[nr] = 0;
+    int run[2] = {0, 0}, best0[2] = {0, 0}, best1[2] = {0, 0};
+    for (int r = 0; r <= nr; ++r) {
+      const uint8_t in[2] = {sky[r], hl[r]};
+      for (int i = 0; i < 2; ++i) {
+        if (in[i]) { run[i]++; continue; }
+        if (run[i] > best1[i] - best0[i]) { best0[i] = r - run[i]; best1[i] = r; }
+        run[i] = 0;
+      }
+    }
+    for (int i = 0; i < 2; ++i) { rows[c][2 * i] = (uint8_t)best0[i]; rows[c][2 * i + 1] = (uint8_t)best1[i]; }
   }
 }

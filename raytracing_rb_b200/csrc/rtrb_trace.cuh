@@ -798,18 +798,22 @@ __device__ __forceinline__ void merge_ctx(ThreadCtx& ctx, const ThreadCtx& t) {
 }
 
 // FAST64 entry point, defined in rtrb_trace_fast.cuh (only instantiated by that translation unit).  CULL: the depth-1
-// frame kernels' candidate masks (FrameParams::k_cam_tx, light_cand); cam_cand = those of the pixel's super-tile.
+// frame kernels' candidate masks (FrameParams::k_cam_tx, light_cand); cam_cand = those of the pixel's super-tile, and
+// no_highlight = its tile certificate rules out every highlight (FrameParams::k_tile_rows).
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
-                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu);
+                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu,
+                                                bool no_highlight = false);
 
 // BVH: FAST64 with the sphere BVH instead of the linear filter.
 // BOX: the FAST64 kernels carry the Box code only in their full-counter (DETAIL) variants; scenes with a
 // box are always dispatched there (rtrb_api.cu, pick_trace_kernels), so the lean hot kernels stay sphere/plane-only.
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
-                                             ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu) {
-  if constexpr (Pol::fast) return trace_sample_fast<Pol, MAXS, BVH, BOX, CULL>(P, ro, rd, pixel, sample, ctx, primary_hit, cam_cand);
+                                             ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu,
+                                             bool no_highlight = false) {
+  if constexpr (Pol::fast)
+    return trace_sample_fast<Pol, MAXS, BVH, BOX, CULL>(P, ro, rd, pixel, sample, ctx, primary_hit, cam_cand, no_highlight);
   else return trace_sample<Pol, MAXS>(P, ro, rd, pixel, sample, ctx, primary_hit);
 }
 
@@ -821,7 +825,9 @@ __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd,
 // attribute, the wait returns at once.
 // PASS: the pass kernels of a progressive frame.  One thread per (pixel, sample j in [pass_begin, pass_end)); the
 // colour goes to the sample buffer at (slot * pre + j), the stride of the whole frame.  No overlap, no in-thread resolve.
-// The FAST64 depth-1 linear-filter kernels narrow the camera apex test to the candidate masks of the pixel's super-tile.
+// The FAST64 depth-1 linear-filter kernels (the pass kernels included) narrow the camera apex test to the candidate masks
+// of the pixel's super-tile, store sky tiles without tracing and skip the highlight test where the tile certificates
+// (FrameParams::k_tile_rows) allow.
 template <class Pol, int MAXS, bool DETAIL, bool BVH = false, bool PASS = false>
 __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
   constexpr bool kOverlap = Pol::fast && MAXS == 1 && !PASS;
@@ -842,13 +848,24 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
     if (active) {
       const uint32_t pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
       d3 ro, rd;
-      camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
       int ph;
       d3 col;
       if constexpr (kCull) {
-        const uint32_t cand = P.k_cam_tx[min(x >> 5, RTRB_CAM_TX - 1)] & P.k_cam_ty[min(y >> 5, RTRB_CAM_TY - 1)];
-        col = trace_dispatch<Pol, MAXS, BVH, DETAIL, true>(P, ro, rd, pixel, j, ctx, &ph, cand);
+        const int tx = x >> 5, ty = y >> 5;
+        const uint32_t cand = P.k_cam_tx[min(tx, RTRB_CAM_TX - 1)] & P.k_cam_ty[min(ty, RTRB_CAM_TY - 1)];
+        const uchar4 rows = tx < RTRB_CAM_TX ? P.k_tile_rows[tx] : make_uchar4(0, 0, 0, 0);
+        if (cand == 0u && ty >= rows.x && ty < rows.y) {
+          // sky tile: the ray meets no sphere (empty mask), no plane and no highlight cone, and no exact test runs, so
+          // rt_map's result is known: one ray, nothing emitted (sum stays +0.0), hit id -1
+          col = mk(0.0, 0.0, 0.0);
+          ph = -1;
+          ctx.rays = 1;
+        } else {
+          camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
+          col = trace_dispatch<Pol, MAXS, BVH, DETAIL, true>(P, ro, rd, pixel, j, ctx, &ph, cand, ty >= rows.z && ty < rows.w);
+        }
       } else {
+        camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
         col = trace_dispatch<Pol, MAXS, BVH, DETAIL>(P, ro, rd, pixel, j, ctx, &ph);
       }
       RTRB_COUNT(ctx, RTRB_CNT_SAMPLES);

@@ -501,23 +501,11 @@ __device__ __forceinline__ uint32_t light_survivors_of(const FrameParams& P, con
   }
   return m;
 }
-template <bool KT>
 __device__ __forceinline__ uint32_t line_survivors_light(const FrameParams& P, const int light_index, const CullRay& r) {
   uint32_t m = 0u;
-  if constexpr (!KT) {
-    const float4* tab = P.light_tab + (size_t)light_index * P.n_sph;
+  const float4* tab = P.light_tab + (size_t)light_index * P.n_sph;
 #pragma unroll 4
-    for (int k = 0; k < P.n_sph; ++k) m |= apex_test(__ldg(&tab[k]), r) << k;
-  } else {
-    // constant-bank table, eight spheres per uniform branch like the camera table
-#pragma unroll
-    for (int blk = 0; blk < RTRB_APEX_MAX / 8; ++blk) {
-      if (blk * 8 < P.n_sph) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) m |= apex_test(P.k_light_tab[light_index][blk * 8 + j], r) << (blk * 8 + j);
-      }
-    }
-  }
+  for (int k = 0; k < P.n_sph; ++k) m |= apex_test(__ldg(&tab[k]), r) << k;
   return m;
 }
 
@@ -598,17 +586,18 @@ __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3
 // An object the probe ray certainly misses (or certainly meets beyond the light) has factor 0, hence
 // cover exactly 0 (sphere.rb:29,45-53 multiply everything by factor; world_object.rb:43-47), and
 // total - 0 == total, so skipping it leaves the running difference bit-identical.
-template <class Pol, bool BOX, bool KT, bool CULL = false>
+template <class Pol, bool BOX, bool KT>
 __device__ __forceinline__ double lit_area_linear(const FrameParams& P, d3 target, const DevLight& L, const int light_index,
                                                   ThreadCtx& ctx) {
   CullRay r;
   float far;
   CoverRay c = make_cover_probe(P, target, L, r, far);
   if (P.n_sph > RTRB_APEX_MAX || P.n_pl > RTRB_K_PLANES) return lit_area_call<Pol, BOX>(P, target, L, ctx);
-  // the probe ray's line passes through the light: apex table of this light when there is one
+  // the probe ray's line passes through the light: apex table of this light when there is one (the depth-1 kernels test
+  // the candidates of the light's masks only)
   uint32_t sm;
-  if constexpr (CULL) sm = (P.k_has_light_tab != 0) ? light_survivors_of(P, light_index, r) : line_survivors_generic<KT>(P, r);
-  else sm = (P.k_has_light_tab != 0) ? line_survivors_light<KT>(P, light_index, r) : line_survivors_generic<KT>(P, r);
+  if constexpr (KT) sm = (P.k_has_light_tab != 0) ? light_survivors_of(P, light_index, r) : line_survivors_generic<KT>(P, r);
+  else sm = (P.k_has_light_tab != 0) ? line_survivors_light(P, light_index, r) : line_survivors_generic<KT>(P, r);
   uint32_t qm = 0u;
   for (int k = 0; k < P.n_pl; ++k) {
     float lo, hi;
@@ -660,11 +649,11 @@ __device__ __forceinline__ int closest_hit_fast(const FrameParams& P, d3 o, d3 d
   if constexpr (BVH) return closest_hit_bvh<Pol, BOX>(P, o, d, r, bh, ctx);
   else return closest_hit_linear<Pol, BOX, KT, CULL>(P, o, d, r, bh, ctx, through_lens, cam_cand);
 }
-template <class Pol, bool BVH, bool BOX, bool KT, bool CULL = false>
+template <class Pol, bool BVH, bool BOX, bool KT>
 __device__ __forceinline__ double lit_area_fast(const FrameParams& P, d3 target, const DevLight& L, const int light_index,
                                                 ThreadCtx& ctx) {
   if constexpr (BVH) return lit_area_bvh<Pol, BOX>(P, target, L, ctx);
-  else return lit_area_linear<Pol, BOX, KT, CULL>(P, target, L, light_index, ctx);
+  else return lit_area_linear<Pol, BOX, KT>(P, target, L, light_index, ctx);
 }
 
 // The reference's own expression of the highlight match (world.rb:86-93), register-only interface.  Only the depth-1
@@ -729,7 +718,8 @@ __device__ __forceinline__ bool attenuation_dead(d3 att) {
 // Emitted colours are added to `sum` in emission order.
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackItem& it, d3& sum, ThreadCtx& ctx, bool is_first,
-                                            int* primary_hit, HitRec& bh, const uint32_t cam_cand = 0xffffffffu) {
+                                            int* primary_hit, HitRec& bh, const uint32_t cam_cand = 0xffffffffu,
+                                            const bool no_highlight = false) {
   constexpr bool KT = !BVH && MAXS == 1;  // constant-bank tables: depth-1 linear-filter kernels only (see pl_rec)
   const d3 o = mk(it.ox, it.oy, it.oz), d = mk(it.dx, it.dy, it.dz), att = mk(it.ax, it.ay, it.az);
   if (it.depth <= 0 || attenuation_dead(att)) return -1;  // rt_map :52
@@ -737,8 +727,8 @@ __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackIte
 
   const CullRay r = make_cull_ray(P, o, d);
 
-  // ---- World#high_lights ----
-  {
+  // ---- World#high_lights ---- (CULL: not on a camera ray whose tile certificate shows every light's FP32 test false)
+  if (!(CULL && is_first && no_highlight)) {
     unsigned long long hl_mask = 0ull;
     int hl_n = 0;
     for (int l = 0; l < Pol::n_lights(P); ++l)
@@ -787,7 +777,7 @@ static __device__ __noinline__ uint32_t born_dead_children_status(double dx, dou
   return t.status;
 }
 
-template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
+template <class Pol, int MAXS, bool BVH, bool BOX>
 __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackItem& it, const int best_i, const HitRec& bh,
                                              StackItem* stack, int& sp, d3& sum, ThreadCtx& ctx, uint32_t pixel,
                                              uint32_t sample) {
@@ -852,7 +842,7 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
     for (int l = 0; l < Pol::n_lights(P); ++l) {
       const DevLight& L = light_at<KT>(P, l);
       ctx.shadow++;
-      const double area = lit_area_fast<Pol, BVH, BOX, KT, CULL>(P, shade_from, L, l, ctx);
+      const double area = lit_area_fast<Pol, BVH, BOX, KT>(P, shade_from, L, l, ctx);
       if (area > 0) {
         double w = rb_pow<Pol>(area, Pol::shadow_exponent(P));
         if (Pol::n_lights(P) != 1) w = w / (double)Pol::n_lights(P);  // x / 1.0 == x
@@ -906,17 +896,18 @@ __device__ __forceinline__ void item_phase_b(const FrameParams& P, const StackIt
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ void process_item_fast(const FrameParams& P, const StackItem& it, StackItem* stack, int& sp,
                                                   d3& sum, ThreadCtx& ctx, uint32_t pixel, uint32_t sample,
-                                                  bool is_first, int* primary_hit, const uint32_t cam_cand = 0xffffffffu) {
+                                                  bool is_first, int* primary_hit, const uint32_t cam_cand = 0xffffffffu,
+                                                  const bool no_highlight = false) {
   HitRec bh;
-  const int best_i = item_phase_a<Pol, MAXS, BVH, BOX, CULL>(P, it, sum, ctx, is_first, primary_hit, bh, cam_cand);
-  if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX, CULL>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
+  const int best_i = item_phase_a<Pol, MAXS, BVH, BOX, CULL>(P, it, sum, ctx, is_first, primary_hit, bh, cam_cand, no_highlight);
+  if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
 }
 
 // RayTracer#trace_sync for one sample, free-running: the item loop of the depth-1, extra-sample and ray-query kernels
 // (the ray-tree frame kernels run trace_sample_fast_lockstep).
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
-                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand) {
+                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand, bool no_highlight) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
   // the root item starts in registers (no round trip through the local-memory stack)
   StackItem it;
@@ -927,7 +918,8 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
   *primary_hit = -1;
   ctx.max_stack = max(ctx.max_stack, 1u);
   while (true) {
-    process_item_fast<Pol, MAXS, BVH, BOX, CULL>(P, it, stack, sp, sum, ctx, pixel, sample, first, primary_hit, cam_cand);
+    process_item_fast<Pol, MAXS, BVH, BOX, CULL>(P, it, stack, sp, sum, ctx, pixel, sample, first, primary_hit, cam_cand,
+                                                 no_highlight);
     first = false;
     if (MAXS == 1 || sp == 0) break;
     if ((uint32_t)sp > ctx.max_stack) ctx.max_stack = (uint32_t)sp;

@@ -66,13 +66,7 @@ struct DevLight {
   double hl_threshold;  // high_light_angle / 180.0 * PI (world.rb:92)
 };
 
-// FP32 view of a light for the highlight filter (rtrb_trace_fast.cuh).
-struct DevLightF {
-  float px, py, pz;
-  float pmax;       // |position|_inf
-  float cos2_thr;   // cos^2(high_light_angle), valid when mode == 1
-  int32_t mode;     // 1: threshold in (0, 90 deg) -> FP32 filter usable; 0: always take the exact path
-};
+typedef RtrbLightF DevLightF;  // FP32 view of a light for the highlight filter (rtrb_trace_fast.cuh)
 
 // Per-frame constants: thin-lens camera baked on the host in the reference's evaluation order
 // (camera.rb:129-151) + sampling + tiling.  Passed by value as a __grid_constant__ kernel parameter.
@@ -165,7 +159,6 @@ struct FrameParams {
   // spheres (+ boxes), <= RTRB_K_PLANES planes and <= RTRB_K_LIGHTS lights, and read every per-ray table from
   // here instead of global memory: uniform LDC/LDCU instead of LDG (L1 is cold at every launch boundary, and a
   // frame is one ~0.1 ms launch).  The BVH kernels ignore these fields.
-  float4 k_light_tab[RTRB_K_LIGHTS][RTRB_APEX_MAX];  // apex tables of the lights (padding: Kq = +inf)
   float4 k_cull_sph[RTRB_APEX_MAX];                  // = cull_sph[]
   float4 k_cull_pl[2 * RTRB_K_PLANES];               // = cull_pl[]
   DevLight k_lights[RTRB_K_LIGHTS];                  // = lights[]
@@ -180,6 +173,11 @@ struct FrameParams {
   // probes of light l only for those in light_cand's bins of their direction.  Every set bit is a sphere < n_sph.
   uint32_t k_cam_tx[RTRB_CAM_TX], k_cam_ty[RTRB_CAM_TY];  // valid with cam_tab_valid (all spheres: aperture frames)
   const uint32_t* light_cand;  // [n_lights][3 axes][2 ratios][RTRB_LIGHT_BINS], valid with k_has_light_tab
+  // Tile certificates of the same kernels (rtrb_tile_rows): for super-tile column tx < RTRB_CAM_TX, the camera rays of
+  // every super-tile row ty in [x, y) certainly meet no plane and no highlight cone, and those of rows [z, w) no
+  // highlight cone.  A tile of the first kind whose candidate mask is empty is sky: its pixels are black, hit id -1.
+  // All zero (no rows) for aperture frames and where the bounds do not hold; columns past the table share nothing.
+  uchar4 k_tile_rows[RTRB_CAM_TX];
 };
 
 static_assert(sizeof(FrameParams) <= 4096, "FrameParams must fit the 4 KB kernel-parameter space");
