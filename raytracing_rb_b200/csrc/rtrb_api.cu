@@ -253,6 +253,27 @@ struct TileList {
   }
 };
 
+// The per-frame buffers a frame's kernels read and write besides its 8-bit frame (setup_frame).  The renderer keeps one
+// set for its frames; a progressive frame owns its own.
+struct FrameBuffers {
+  TileList tiles;
+  LensTable lens;
+  DevBuf<double> samples, extra_samples, pre_avg, rgb;  // [slots][S][3], [slots][E][3], [slots][3], [H][W][3]
+  DevBuf<uint32_t> extra_list;
+  DevBuf<int32_t> hit;
+};
+
+// The outputs of a frame, as download_outputs copies them: the buffers that hold them (nullptr: the frame kept no such
+// output, or wrote its 8-bit frame elsewhere) and the stream its kernels ran on.  It points at the buffers, not at their
+// device memory, which moves when a buffer grows.
+struct FrameOutputs {
+  int W = 0, H = 0, format = RTRB_FMT_RGBA8;
+  const DevBuf<uint8_t>* frame = nullptr;
+  const DevBuf<double>* rgb = nullptr;
+  const DevBuf<int32_t>* hit = nullptr;
+  cudaStream_t stream = nullptr;
+};
+
 // RTRB_RNG_MT validation mode: serial by construction (every pixel's first draw depends on how many draws all earlier
 // pixels made), so the frame iterates to a fixed point of its per-pixel draw offsets.
 struct MtState {
@@ -416,20 +437,12 @@ struct rtrb_renderer {
   size_t staging_bytes = 0;
   std::vector<void*> retired;             // scene buffers an update outgrew; freed once the work before it is done
   // per-frame caches and scratch
-  TileList tiles;
-  LensTable lens;
-  DevBuf<double> samples, extra_samples, pre_avg, rgb;
-  DevBuf<uint32_t> extra_list;
+  FrameBuffers buf;
   MtState mt;
-  DevBuf<int32_t> hit;
   DevBuf<uint8_t> rgba;
   bool fb_exported = false;            // its address / IPC handle has been handed out: it may no longer move
   int fb_w = 0, fb_h = 0;
-  // last frame
-  int last_w = 0, last_h = 0;
-  bool last_has_rgb = false, last_has_hit = false, last_rgba_own = true;
-  int last_format = RTRB_FMT_RGBA8;
-  cudaStream_t last_stream = nullptr;
+  FrameOutputs last;                   // the last frame (rtrb_download); W = 0 until one has been rendered
   // ray-level calls (rtrb_trace_rays & co.): their own control block, scratch and lens tables, never the frames'
   FrameCtl ray_ctl;
   bool ray_ready = false;
@@ -451,22 +464,15 @@ struct rtrb_renderer {
 // disturbs it nor is disturbed by it.
 struct rtrb_progressive {
   rtrb_renderer* r = nullptr;
-  cudaStream_t stream = nullptr;
   FrameParams P;               // as baked at create; P.pre = S is the sample buffer's stride
   int capacity = 0, S = 0, E = 0;
   int done = 0;                // samples traced so far: every pass covers [done, sample_end)
   unsigned scene_gen = 0;      // the renderer's scene_gen at create (an update that applied since invalidates the frame)
   bool strict = false;
   FrameCtl fc;                 // its control block: counters, status, first_bad and max_stack accumulate over the passes
-  TileList tiles;
-  LensTable lens;
-  DevBuf<double> samples, extra_samples, pre_avg, rgb;  // [slots][S][3], [slots][E][3], [slots][3], [H][W][3]
-  DevBuf<uint32_t> extra_list;
-  DevBuf<int32_t> hit;
+  FrameBuffers buf;
   DevBuf<uint8_t> frame;       // the 8-bit frame, unless it goes to opts.rgba_device_out
-  size_t frame_bytes = 0;
-  int W = 0, H = 0, format = RTRB_FMT_RGBA8;
-  bool own_frame = true;
+  FrameOutputs out;            // out.stream is the stream its passes run on
   // its buffers are freed with it; its device must be current (rtrb_progressive_destroy)
 };
 
@@ -491,6 +497,8 @@ __global__ void __launch_bounds__(256) resolve_kernel(const __grid_constant__ Fr
   if (valid && !queued) write_pixel(P, x, y, ax, ay, az);
 }
 
+// A grid-stride loop over the adaptive pixels: launched as kResolveExtraBlocks blocks of 256 threads.
+constexpr unsigned kResolveExtraBlocks = 296;
 __global__ void __launch_bounds__(256) resolve_extra_kernel(const __grid_constant__ FrameParams P) {
   const uint32_t n = *P.extra_count;
   const int E = P.max_samples - P.pre;
@@ -1001,8 +1009,8 @@ int ensure_framebuffers(rtrb_renderer* r, int w, int h, bool rgba, bool rgb, boo
     CUDA_TRY(r->rgba.ensure(px * 4));
     CUDA_TRY(cudaMemset(r->rgba.p, 0, px * 4));
   }
-  if (rgb) CUDA_TRY(r->rgb.ensure(px * 3));
-  if (hit) CUDA_TRY(r->hit.ensure(px));
+  if (rgb) CUDA_TRY(r->buf.rgb.ensure(px * 3));
+  if (hit) CUDA_TRY(r->buf.hit.ensure(px));
   r->fb_w = w; r->fb_h = h;
   return RTRB_OK;
 }
@@ -1134,10 +1142,81 @@ int check_frame_opts(const rtrb_render_opts& opts, int W, int H, Window& win) {
   return make_window(W, H, opts.x0, opts.y0, opts.x1, opts.y1, opts.tile_rank, opts.tile_world, win);
 }
 
-// The per-frame memory budget of the sample buffers: S pre samples per slot (when the frame keeps them) and E extra.
-int check_sample_budget(size_t n_slots, int S, int E, bool need_samples) {
+// The setup every frame shares (render_impl, rtrb_progressive_create), after its checks: the tile list and lens table
+// in `buf`, the sample buffers the resolve mode (RTRB_RESOLVE_*) needs, P's camera, scene, window, buffers, outputs and
+// control block (P already holds pick_trace_kernels' choice), and the facts finish_stats needs in `fc`.  Queues nothing
+// on `s` but the uploads of the tile list and lens table.
+int setup_frame(const rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts& opts, const Window& win,
+                cudaStream_t s, FrameBuffers& buf, int resolve, uint8_t* rgba, double* rgb, int32_t* hit, FrameCtl& fc,
+                FrameParams& P) {
+  const int W = cam->width, H = cam->height;
+  int rc;
+  if ((rc = buf.tiles.ensure(W, H, win, s)) || (rc = buf.lens.ensure(cam, s))) return rc;
+  const int n_tiles = (int)buf.tiles.host.size();
+  const size_t n_slots = (size_t)n_tiles * RTRB_SUPER_PIXELS;
+  const int S = cam->pre_sample_times;
+  const int E = cam->max_sample_times > S ? cam->max_sample_times - S : 0;
+  // the per-frame memory budget: S pre samples per slot (when the frame keeps them) and E extra
+  const bool need_samples = resolve == RTRB_RESOLVE_SAMPLE_BUFFER;
   if ((need_samples && n_slots * (size_t)S * 3 * sizeof(double) > ((size_t)96 << 30)) || n_slots * (size_t)E * 3 * sizeof(double) > ((size_t)64 << 30))
     return fail(RTRB_ERR_UNSUPPORTED, "sample buffer would exceed the per-frame memory budget");
+  if (need_samples) CUDA_TRY(buf.samples.ensure(std::max<size_t>(1, n_slots * S * 3)));
+  CUDA_TRY(buf.extra_list.ensure(std::max<size_t>(1, n_slots)));
+  if (E > 0) {
+    CUDA_TRY(buf.extra_samples.ensure(n_slots * E * 3));
+    CUDA_TRY(buf.pre_avg.ensure(n_slots * 3));
+  }
+  bake_frame(r, cam, P);
+  P.key0 = (uint32_t)opts.seed; P.key1 = (uint32_t)(opts.seed >> 32);
+  P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
+  P.n_tiles = n_tiles; P.stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER; P.tiles = buf.tiles.dev.p;
+  P.tiles_magic = win.whole ? buf.tiles.magic : 0u;
+  P.lens_sx = buf.lens.tab.p; P.lens_sy = buf.lens.tab.p + W;
+  P.samples = need_samples ? buf.samples.p : nullptr; P.pre_avg = buf.pre_avg.p;
+  P.extra_list = buf.extra_list.p; P.extra_samples = buf.extra_samples.p;
+  P.rgba = rgba; P.rgb = rgb; P.hit = hit;
+  P.pixel_format = opts.pixel_format;
+  P.fuse_resolve = resolve;
+  bind_ctl(P, fc);
+  fc.W = W; fc.H = H; fc.S = S; fc.E = E; fc.n_tiles = n_tiles; fc.detail = P.count_detail != 0;
+  fc.px_count = buf.tiles.px_count;
+  return RTRB_OK;
+}
+
+// render_at's tail once the pre samples of a frame are traced: resolve_kernel when they are in the sample buffer, then,
+// unless the trace kernel finished the pixels itself, the extra samples of the adaptive pixels and their final average.
+int launch_render_at_tail(const FrameParams& P, bool strict, int capacity, cudaStream_t s) {
+  if (P.fuse_resolve == RTRB_RESOLVE_SAMPLE_BUFFER) {
+    resolve_kernel<<<(unsigned)(((size_t)P.n_tiles * RTRB_SUPER_PIXELS + 255) / 256), 256, 0, s>>>(P);
+    CUDA_TRY(cudaGetLastError());
+    g_launches++;
+  }
+  if (P.max_samples > P.pre && P.fuse_resolve != RTRB_RESOLVE_IN_THREAD) {
+    CUDA_TRY(strict ? rtrb_launch_trace_extra_strict(P, capacity, s) : rtrb_launch_trace_extra_fast(P, capacity, s));
+    g_launches++;
+    resolve_extra_kernel<<<kResolveExtraBlocks, 256, 0, s>>>(P);
+    CUDA_TRY(cudaGetLastError());
+    g_launches++;
+  }
+  return RTRB_OK;
+}
+
+// Copies the outputs of a frame into host buffers (NULL: not wanted) and waits for the copies.
+int download_outputs(const FrameOutputs& o, uint8_t* frame, double* rgb_or_null, int32_t* hit_or_null) {
+  const size_t px = (size_t)o.W * o.H;
+  if (frame) {
+    if (!o.frame) return fail(RTRB_ERR_INVALID, "the frame was written to rgba_device_out, not to a framebuffer of its own");
+    CUDA_TRY(cudaMemcpyAsync(frame, o.frame->p, RTRB_FRAME_BYTES(o.W, o.H, o.format), cudaMemcpyDeviceToHost, o.stream));
+  }
+  if (rgb_or_null) {
+    if (!o.rgb) return fail(RTRB_ERR_INVALID, "the frame kept no float RGB");
+    CUDA_TRY(cudaMemcpyAsync(rgb_or_null, o.rgb->p, px * 3 * sizeof(double), cudaMemcpyDeviceToHost, o.stream));
+  }
+  if (hit_or_null) {
+    if (!o.hit) return fail(RTRB_ERR_INVALID, "the frame kept no hit ids");
+    CUDA_TRY(cudaMemcpyAsync(hit_or_null, o.hit->p, px * sizeof(int32_t), cudaMemcpyDeviceToHost, o.stream));
+  }
+  CUDA_TRY(cudaStreamSynchronize(o.stream));
   return RTRB_OK;
 }
 
@@ -1180,16 +1259,12 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   if (!tg.rgba && opts.rgba_device_out) tg.rgba = (uint8_t*)opts.rgba_device_out;
   if ((rc = ensure_framebuffers(r, W, H, tg.rgba == nullptr, tg.want_rgb && !tg.rgb, tg.want_hit && !tg.hit))) return rc;
   if (!tg.rgba) tg.rgba = r->rgba.p;
-  if (tg.want_rgb && !tg.rgb) tg.rgb = r->rgb.p;
-  if (tg.want_hit && !tg.hit) tg.hit = r->hit.p;
+  if (tg.want_rgb && !tg.rgb) tg.rgb = r->buf.rgb.p;
+  if (tg.want_hit && !tg.hit) tg.hit = r->buf.hit.p;
   if (!tg.want_rgb) tg.rgb = nullptr;
   if (!tg.want_hit) tg.hit = nullptr;
 
-  if ((rc = r->tiles.ensure(W, H, win, stream)) || (rc = r->lens.ensure(cam, stream))) return rc;
-  const int n_tiles = (int)r->tiles.host.size();
-  const size_t n_slots = (size_t)n_tiles * RTRB_SUPER_PIXELS;
   const int S = cam->pre_sample_times;
-  const int E = cam->max_sample_times > S ? cam->max_sample_times - S : 0;
   // Who finishes render_at (FrameParams::fuse_resolve).  The FAST64 ray-tree kernels resolve a pixel inside the CTA
   // that traced its samples whenever the sample count divides the CTA size: no FP64 sample buffer (24 B per sample:
   // 12.7 GB for one 4K / 64 spp frame) and no resolve launch.  RTRB_RNG_MT frames always go through the sample
@@ -1197,50 +1272,33 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   int fuse = (!mt_mode && S == 1 && cam->variant_threshold > 0) ? RTRB_RESOLVE_IN_THREAD : RTRB_RESOLVE_SAMPLE_BUFFER;
   if (!strict && !mt_mode && cam->trace_depth > 1 && S <= RTRB_TREE_MIN_BLOCK && RTRB_TREE_MIN_BLOCK % S == 0)
     fuse = RTRB_RESOLVE_IN_CTA;
-  const bool need_samples = fuse == RTRB_RESOLVE_SAMPLE_BUFFER;
-  if ((rc = check_sample_budget(n_slots, S, E, need_samples))) return rc;
-  if (need_samples) CUDA_TRY(r->samples.ensure(std::max<size_t>(1, n_slots * S * 3)));
-  CUDA_TRY(r->extra_list.ensure(std::max<size_t>(1, n_slots)));
-  if (E > 0) {
-    CUDA_TRY(r->extra_samples.ensure(n_slots * E * 3));
-    CUDA_TRY(r->pre_avg.ensure(n_slots * 3));
-  }
+  // a synchronous frame takes the next control block of the main_ctl ring (the ring moves on below, once set up)
   FrameCtl& fc = ctl ? *ctl : r->main_ctl;
+  if (!ctl) fc.blk = fc.d.p + r->ring_next;
+  if ((rc = setup_frame(r, cam, opts, win, stream, r->buf, fuse, tg.rgba, tg.rgb, tg.hit, fc, P))) return rc;
+  const int n_tiles = P.n_tiles;
   // Frame overlap: a frame that is one depth-1 FAST64 launch is launched with programmatic stream serialization, so its
   // kernel traces under the tail of the kernel before it on the stream and waits for it only to write
-  // (trace_pre_body).  A synchronous frame takes the next control block of the main_ctl ring; an overlapping one also
-  // zeroes the block after it, and the next synchronous frame on the same stream then needs no memset between the
-  // two kernels.  Frames written into the same buffer stay ordered: every store waits for the previous grid.
+  // (trace_pre_body).  An overlapping synchronous frame also zeroes the ring's block after its own, and the next
+  // synchronous frame on the same stream then needs no memset between the two kernels.  Frames written into the same
+  // buffer stay ordered: every store waits for the previous grid.
   const bool overlap =
       r->frame_overlap && !strict && !mt_mode && fuse == RTRB_RESOLVE_IN_THREAD && cam->trace_depth <= 1 && n_tiles > 0;
   bool zeroed = false;
   CtlBlock* next_blk = nullptr;
   if (!ctl) {
-    fc.blk = fc.d.p + r->ring_next;
     r->ring_next = (r->ring_next + 1) % RTRB_CTL_RING;
     zeroed = r->ring_zeroed && r->ring_stream == stream;
     r->ring_zeroed = false;
     if (overlap) next_blk = fc.d.p + r->ring_next;
   }
+  P.ctl_next = (unsigned long long*)next_blk;
+  P.ctl_next_words = next_blk ? (uint32_t)(sizeof(CtlBlock) / sizeof(unsigned long long)) : 0u;
 
   // the first frame on a stream after rtrb_scene_update starts only after the update's copies: no overlap with the
   // kernel before it, which would let it read the scene early
   bool fresh_scene;
   if ((rc = enter_scene_stream(r, stream, &fresh_scene))) return rc;
-  bake_frame(r, cam, P);
-  P.key0 = (uint32_t)opts.seed; P.key1 = (uint32_t)(opts.seed >> 32);
-  P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
-  P.n_tiles = n_tiles; P.stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER; P.tiles = r->tiles.dev.p;
-  P.lens_sx = r->lens.tab.p; P.lens_sy = r->lens.tab.p + W;
-  P.samples = need_samples ? r->samples.p : nullptr; P.rgb = tg.rgb; P.hit = tg.hit; P.rgba = tg.rgba;
-  P.pre_avg = r->pre_avg.p;
-  bind_ctl(P, fc);
-  P.tiles_magic = win.whole ? r->tiles.magic : 0u;
-  P.extra_list = r->extra_list.p; P.extra_samples = r->extra_samples.p;
-  P.pixel_format = opts.pixel_format;
-  P.fuse_resolve = fuse;
-  P.ctl_next = (unsigned long long*)next_blk;
-  P.ctl_next_words = next_blk ? (uint32_t)(sizeof(CtlBlock) / sizeof(unsigned long long)) : 0u;
 
   // timing events only for the blocking calls that return stats (the pipelined frames of rtrb_submit report
   // device_ms = trace_ms = 0); the end-of-frame event only where something waits for it (timing, rtrb_submit's copy
@@ -1249,7 +1307,7 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
   fc.timed = timed;
   if (timed) CUDA_TRY(cudaEventRecord(fc.ev0, stream));
   if (!zeroed) CUDA_TRY(cudaMemsetAsync(fc.blk, 0, sizeof(CtlBlock), stream));
-  if (!win.whole && !tg.no_fill && tg.hit == r->hit.p && tg.hit) prefill_hits(tg.hit, W, H, stream);
+  if (!win.whole && !tg.no_fill && tg.hit == r->buf.hit.p && tg.hit) prefill_hits(tg.hit, W, H, stream);
   if (n_tiles > 0 && mt_mode) {
     if ((rc = r->mt.trace(P, fc, opts.seed, capacity, stream))) return rc;
   } else if (n_tiles > 0) {
@@ -1259,30 +1317,12 @@ int render_impl(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render
     if (next_blk) { r->ring_zeroed = true; r->ring_stream = stream; }
     if (timed) CUDA_TRY(cudaEventRecord(fc.evt1, stream));
     g_launches++;
-    if (fuse == RTRB_RESOLVE_SAMPLE_BUFFER) {
-      resolve_kernel<<<(unsigned)((n_slots + 255) / 256), 256, 0, stream>>>(P);
-      CUDA_TRY(cudaGetLastError());
-      g_launches++;
-    }
-    if (E > 0 && fuse != RTRB_RESOLVE_IN_THREAD) {
-      CUDA_TRY(strict ? rtrb_launch_trace_extra_strict(P, capacity, stream) : rtrb_launch_trace_extra_fast(P, capacity, stream));
-      g_launches++;
-      resolve_extra_kernel<<<296, 256, 0, stream>>>(P);
-      CUDA_TRY(cudaGetLastError());
-      g_launches++;
-    }
+    if ((rc = launch_render_at_tail(P, strict, capacity, stream))) return rc;
   }
   if (timed || ctl || !r->frame_overlap) CUDA_TRY(cudaEventRecord(fc.ev1, stream));
-  r->last_w = W; r->last_h = H;
-  r->last_rgba_own = tg.rgba == r->rgba.p;
-  r->last_has_rgb = tg.rgb == r->rgb.p && tg.rgb != nullptr;
-  r->last_has_hit = tg.hit == r->hit.p && tg.hit != nullptr;
-  r->last_stream = stream;
-  r->last_format = opts.pixel_format;
-
-  // facts needed to finish the stats once the control block has been copied back
-  fc.W = W; fc.H = H; fc.S = S; fc.E = E; fc.n_tiles = n_tiles; fc.detail = P.count_detail != 0;
-  fc.px_count = r->tiles.px_count;
+  r->last = FrameOutputs{W, H, opts.pixel_format, tg.rgba == r->rgba.p ? &r->rgba : nullptr,
+                         tg.rgb && tg.rgb == r->buf.rgb.p ? &r->buf.rgb : nullptr,
+                         tg.hit && tg.hit == r->buf.hit.p ? &r->buf.hit : nullptr, stream};
   return stats_out ? read_stats(fc, stream, stats_out) : RTRB_OK;
 }
 
@@ -1515,24 +1555,9 @@ int rtrb_render_device(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb
 
 int rtrb_download(rtrb_renderer* r, uint8_t* rgba, double* rgb_or_null, int32_t* hit_or_null) {
   if (!r) return fail(RTRB_ERR_INVALID, "renderer is NULL");
-  if (r->last_w == 0) return fail(RTRB_ERR_INVALID, "nothing rendered yet");
+  if (r->last.W == 0) return fail(RTRB_ERR_INVALID, "nothing rendered yet");
   CUDA_TRY(cudaSetDevice(r->device));
-  cudaStream_t s = r->last_stream ? r->last_stream : r->stream;
-  size_t px = (size_t)r->last_w * r->last_h;
-  if (rgba) {
-    if (!r->last_rgba_own) return fail(RTRB_ERR_INVALID, "the last frame was written to rgba_device_out, not to the renderer's framebuffer");
-    CUDA_TRY(cudaMemcpyAsync(rgba, r->rgba.p, RTRB_FRAME_BYTES(r->last_w, r->last_h, r->last_format), cudaMemcpyDeviceToHost, s));
-  }
-  if (rgb_or_null) {
-    if (!r->last_has_rgb) return fail(RTRB_ERR_INVALID, "the last frame kept no float RGB");
-    CUDA_TRY(cudaMemcpyAsync(rgb_or_null, r->rgb.p, px * 3 * sizeof(double), cudaMemcpyDeviceToHost, s));
-  }
-  if (hit_or_null) {
-    if (!r->last_has_hit) return fail(RTRB_ERR_INVALID, "the last frame kept no hit ids");
-    CUDA_TRY(cudaMemcpyAsync(hit_or_null, r->hit.p, px * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  }
-  CUDA_TRY(cudaStreamSynchronize(s));
-  return RTRB_OK;
+  return download_outputs(r->last, rgba, rgb_or_null, hit_or_null);
 }
 
 int rtrb_render(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* rgba,
@@ -1716,7 +1741,7 @@ int rtrb_render_multi(rtrb_renderer* const* renderers, int n, const rtrb_camera_
   if (want_hit && make_window(cam->width, cam->height, base.x0, base.y0, base.x1, base.y1, 0, 1, win) == RTRB_OK &&
       !win.whole) {
     CUDA_TRY(cudaSetDevice(root->device));
-    prefill_hits(root->hit.p, cam->width, cam->height, root->stream);
+    prefill_hits(root->buf.hit.p, cam->width, cam->height, root->stream);
     CUDA_TRY(cudaStreamSynchronize(root->stream));
   }
   std::vector<rtrb_stats> st(n);
@@ -1729,8 +1754,8 @@ int rtrb_render_multi(rtrb_renderer* const* renderers, int n, const rtrb_camera_
       o.tile_rank = i; o.tile_world = n; o.stream = nullptr; o.rgba_device_out = nullptr;
       FrameTargets tg;
       tg.rgba = root->rgba.p;
-      tg.rgb = want_rgb ? root->rgb.p : nullptr;
-      tg.hit = want_hit ? root->hit.p : nullptr;
+      tg.rgb = want_rgb ? root->buf.rgb.p : nullptr;
+      tg.hit = want_hit ? root->buf.hit.p : nullptr;
       tg.want_rgb = want_rgb; tg.want_hit = want_hit; tg.no_fill = true;
       rcs[i] = render_impl(renderers[i], cam, &o, &tg, &st[i]);
       errs[i] = g_last_error;
@@ -1993,51 +2018,27 @@ int rtrb_progressive_create(rtrb_renderer* r, const rtrb_camera_desc* cam, const
                                &p->capacity)))
     return rc;
   const cudaStream_t s = opts.stream ? (cudaStream_t)opts.stream : r->stream;
-  const int S = cam->pre_sample_times, E = cam->max_sample_times > S ? cam->max_sample_times - S : 0;
-  p->r = r; p->stream = s; p->strict = strict; p->S = S; p->E = E;
-  p->W = W; p->H = H; p->format = opts.pixel_format;
+  const int S = cam->pre_sample_times;
+  p->r = r; p->strict = strict; p->S = S; p->E = cam->max_sample_times > S ? cam->max_sample_times - S : 0;
   const cudaError_t ce = p->fc.init();
   if (ce != cudaSuccess) return fail(RTRB_ERR_CUDA, "control block init failed: %s", cudaGetErrorString(ce));
-  if ((rc = p->tiles.ensure(W, H, win, s)) || (rc = p->lens.ensure(cam, s))) return rc;
-  const int n_tiles = (int)p->tiles.host.size();
-  const size_t n_slots = (size_t)n_tiles * RTRB_SUPER_PIXELS, px = (size_t)W * H;
-  if ((rc = check_sample_budget(n_slots, S, E, true))) return rc;
-  CUDA_TRY(p->samples.ensure(std::max<size_t>(1, n_slots * S * 3)));
-  CUDA_TRY(p->extra_list.ensure(std::max<size_t>(1, n_slots)));
-  if (E > 0) {
-    CUDA_TRY(p->extra_samples.ensure(n_slots * E * 3));
-    CUDA_TRY(p->pre_avg.ensure(n_slots * 3));
-  }
-  // its outputs: pixels outside the window or the rank's tiles read 0, hit id -3
-  p->frame_bytes = RTRB_FRAME_BYTES(W, H, opts.pixel_format);
-  p->own_frame = opts.rgba_device_out == nullptr;
-  if (p->own_frame) {
-    CUDA_TRY(p->frame.ensure(p->frame_bytes));
-    CUDA_TRY(cudaMemsetAsync(p->frame.p, 0, p->frame_bytes, s));
-  }
-  if (!(opts.skip_outputs & RTRB_SKIP_RGB)) {
-    CUDA_TRY(p->rgb.ensure(px * 3));
-    CUDA_TRY(cudaMemsetAsync(p->rgb.p, 0, px * 3 * sizeof(double), s));
-  }
-  if (!(opts.skip_outputs & RTRB_SKIP_HIT)) {
-    CUDA_TRY(p->hit.ensure(px));
-    if (!win.whole) prefill_hits(p->hit.p, W, H, s);
-  }
-  bake_frame(r, cam, P);
-  P.key0 = (uint32_t)opts.seed; P.key1 = (uint32_t)(opts.seed >> 32);
-  P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
-  P.n_tiles = n_tiles; P.stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER; P.tiles = p->tiles.dev.p;
-  P.tiles_magic = win.whole ? p->tiles.magic : 0u;
-  P.lens_sx = p->lens.tab.p; P.lens_sy = p->lens.tab.p + W;
-  P.samples = p->samples.p; P.rgb = p->rgb.p; P.hit = p->hit.p;
-  P.rgba = p->own_frame ? p->frame.p : (uint8_t*)opts.rgba_device_out;
-  P.pre_avg = p->pre_avg.p; P.extra_list = p->extra_list.p; P.extra_samples = p->extra_samples.p;
-  P.pixel_format = opts.pixel_format;
-  P.fuse_resolve = RTRB_RESOLVE_SAMPLE_BUFFER;
-  bind_ctl(P, p->fc);
+  // its outputs, which the frame's setup points the kernels at
+  FrameBuffers& b = p->buf;
+  const size_t px = (size_t)W * H, frame_bytes = RTRB_FRAME_BYTES(W, H, opts.pixel_format);
+  const bool own_frame = opts.rgba_device_out == nullptr;
+  if (own_frame) CUDA_TRY(p->frame.ensure(frame_bytes));
+  if (!(opts.skip_outputs & RTRB_SKIP_RGB)) CUDA_TRY(b.rgb.ensure(px * 3));
+  if (!(opts.skip_outputs & RTRB_SKIP_HIT)) CUDA_TRY(b.hit.ensure(px));
+  if ((rc = setup_frame(r, cam, opts, win, s, b, RTRB_RESOLVE_SAMPLE_BUFFER,
+                        own_frame ? p->frame.p : (uint8_t*)opts.rgba_device_out, b.rgb.p, b.hit.p, p->fc, P)))
+    return rc;
+  // pixels outside the window or the rank's tiles read 0, hit id -3
+  if (own_frame) CUDA_TRY(cudaMemsetAsync(p->frame.p, 0, frame_bytes, s));
+  if (b.rgb.p) CUDA_TRY(cudaMemsetAsync(b.rgb.p, 0, px * 3 * sizeof(double), s));
+  if (b.hit.p && !win.whole) prefill_hits(b.hit.p, W, H, s);
   CUDA_TRY(cudaMemsetAsync(p->fc.blk, 0, sizeof(CtlBlock), s));
-  FrameCtl& fc = p->fc;
-  fc.W = W; fc.H = H; fc.n_tiles = n_tiles; fc.detail = P.count_detail != 0; fc.px_count = p->tiles.px_count;
+  p->out = FrameOutputs{W, H, opts.pixel_format, own_frame ? &p->frame : nullptr, b.rgb.p ? &b.rgb : nullptr,
+                        b.hit.p ? &b.hit : nullptr, s};
   p->scene_gen = r->scene_gen;
   *out = p.release();
   return RTRB_OK;
@@ -2052,7 +2053,7 @@ int rtrb_progressive_pass(rtrb_progressive* p, int sample_end, rtrb_stats* stats
   if (r->scene_gen != p->scene_gen)
     return fail(RTRB_ERR_INVALID, "scene changed: rtrb_scene_update replaced the scene after the frame was created");
   CUDA_TRY(cudaSetDevice(r->device));
-  const cudaStream_t s = p->stream;
+  const cudaStream_t s = p->out.stream;
   bool fresh_scene;
   int rc = enter_scene_stream(r, s, &fresh_scene);
   if (rc) return rc;
@@ -2060,8 +2061,6 @@ int rtrb_progressive_pass(rtrb_progressive* p, int sample_end, rtrb_stats* stats
   FrameParams& P = p->P;
   P.pass_begin = p->done; P.pass_end = sample_end;
   const bool final = sample_end == p->S;
-  const size_t n_slots = (size_t)P.n_tiles * RTRB_SUPER_PIXELS;
-  const unsigned grid = (unsigned)((n_slots + 255) / 256);
   fc.timed = stats_out != nullptr;
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev0, s));
   // the counters accumulate over the passes, except adaptive_pixels: each resolve counts the frame it resolves
@@ -2075,21 +2074,11 @@ int rtrb_progressive_pass(rtrb_progressive* p, int sample_end, rtrb_stats* stats
       // the preview is the frame of pre = max = sample_end samples
       FrameParams Q = P;
       Q.pre = sample_end; Q.max_samples = sample_end;
-      resolve_prefix_kernel<<<grid, 256, 0, s>>>(Q, p->S);
+      resolve_prefix_kernel<<<(unsigned)(((size_t)P.n_tiles * RTRB_SUPER_PIXELS + 255) / 256), 256, 0, s>>>(Q, p->S);
       CUDA_TRY(cudaGetLastError());
       g_launches++;
-    } else {
-      // render_at's tail as a one-shot sample-buffer frame runs it
-      resolve_kernel<<<grid, 256, 0, s>>>(P);
-      CUDA_TRY(cudaGetLastError());
-      g_launches++;
-      if (p->E > 0) {
-        CUDA_TRY(p->strict ? rtrb_launch_trace_extra_strict(P, p->capacity, s) : rtrb_launch_trace_extra_fast(P, p->capacity, s));
-        g_launches++;
-        resolve_extra_kernel<<<296, 256, 0, s>>>(P);
-        CUDA_TRY(cudaGetLastError());
-        g_launches++;
-      }
+    } else if ((rc = launch_render_at_tail(P, p->strict, p->capacity, s))) {  // as a one-shot sample-buffer frame
+      return rc;
     }
   }
   if (fc.timed) CUDA_TRY(cudaEventRecord(fc.ev1, s));
@@ -2102,22 +2091,7 @@ int rtrb_progressive_download(rtrb_progressive* p, uint8_t* frame, double* rgb_o
   if (!p) return fail(RTRB_ERR_INVALID, "progressive frame is NULL");
   if (p->done == 0) return fail(RTRB_ERR_INVALID, "no pass has run yet");
   CUDA_TRY(cudaSetDevice(p->r->device));
-  const cudaStream_t s = p->stream;
-  const size_t px = (size_t)p->W * p->H;
-  if (frame) {
-    if (!p->own_frame) return fail(RTRB_ERR_INVALID, "the frame is written to rgba_device_out, not to its own buffer");
-    CUDA_TRY(cudaMemcpyAsync(frame, p->frame.p, p->frame_bytes, cudaMemcpyDeviceToHost, s));
-  }
-  if (rgb_or_null) {
-    if (!p->rgb.p) return fail(RTRB_ERR_INVALID, "the frame keeps no float RGB (RTRB_SKIP_RGB)");
-    CUDA_TRY(cudaMemcpyAsync(rgb_or_null, p->rgb.p, px * 3 * sizeof(double), cudaMemcpyDeviceToHost, s));
-  }
-  if (hit_or_null) {
-    if (!p->hit.p) return fail(RTRB_ERR_INVALID, "the frame keeps no hit ids (RTRB_SKIP_HIT)");
-    CUDA_TRY(cudaMemcpyAsync(hit_or_null, p->hit.p, px * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  }
-  CUDA_TRY(cudaStreamSynchronize(s));
-  return RTRB_OK;
+  return download_outputs(p->out, frame, rgb_or_null, hit_or_null);
 }
 
 int rtrb_progressive_frame_ptr(rtrb_progressive* p, void** ptr_out) {
