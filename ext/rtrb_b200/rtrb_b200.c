@@ -30,6 +30,14 @@
  *                                                     hits = n int32 root-ray winners (unpack("d*") / unpack("l*"))
  *   renderer.intersect_rays(packed_rays)           -> String of n rtrb_ray_hit records (unpack("l4d7") each):
  *                                                     World#intersect's object, :in?, box face, distance, point, delta
+ *   Rtrb::Animation.new(renderer, w, h, delay_num, delay_den) -> an animated PNG on the renderer (rtrb_apng_create);
+ *                                                     keeps the renderer alive
+ *   animation.add_frame(camera, seed = 1)          -> binary String: the frame rendered and appended on the GPU
+ *                                                     (rtrb_apng_add), its fcTL and data chunks; a frame that raised
+ *                                                     is appended too, and frame_error holds what render would raise
+ *   animation.frame_error                          -> nil, or the message of the last add_frame's raising frame
+ *   animation.header(num_plays = 0)                -> binary String: signature, IHDR and acTL for the frames added;
+ *                                                     the file is header + every add_frame String + Rtrb::APNG_IEND
  */
 #include <ruby.h>
 #include <ruby/thread.h>
@@ -38,7 +46,7 @@
 
 #include "rtrb_b200.h"
 
-static VALUE mRtrb, cRenderer;
+static VALUE mRtrb, cRenderer, cAnimation;
 
 typedef struct {
   rtrb_renderer* r;
@@ -470,6 +478,103 @@ static VALUE renderer_stats(VALUE self) {
   return h;
 }
 
+/* ---- animated PNG files ---------------------------------------------------------------------------------------- */
+typedef struct {
+  rtrb_apng* a;
+  VALUE renderer;  /* marked: the animation must be destroyed before its renderer */
+  VALUE frame_error;
+  int width, height, frames;
+} shim_apng;
+
+static void apng_mark(void* p) {
+  rb_gc_mark(((shim_apng*)p)->renderer);
+  rb_gc_mark(((shim_apng*)p)->frame_error);
+}
+static void apng_free(void* p) {
+  shim_apng* s = (shim_apng*)p;
+  if (s->a) rtrb_apng_destroy(s->a);  /* does not touch the renderer, which the same GC pass may have freed */
+  free(s);
+}
+static VALUE apng_alloc(VALUE klass) {
+  shim_apng* s = (shim_apng*)calloc(1, sizeof(*s));
+  s->renderer = Qnil;
+  s->frame_error = Qnil;
+  return Data_Wrap_Struct(klass, apng_mark, apng_free, s);
+}
+
+static VALUE apng_initialize(VALUE self, VALUE renderer, VALUE w, VALUE h, VALUE delay_num, VALUE delay_den) {
+  shim_apng* s;
+  shim_renderer* sr;
+  Data_Get_Struct(self, shim_apng, s);
+  Data_Get_Struct(renderer, shim_renderer, sr);
+  s->renderer = renderer;
+  s->width = NUM2INT(w);
+  s->height = NUM2INT(h);
+  if (rtrb_apng_create(sr->r, s->width, s->height, NUM2INT(delay_num), NUM2INT(delay_den), &s->a) != RTRB_OK)
+    rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());
+  return self;
+}
+
+typedef struct {
+  render_call c;
+  rtrb_apng* a;
+  size_t bytes;
+} add_call;
+
+static void* add_frame_without_gvl(void* p) {  /* render into device memory, append there, fetch the chunks */
+  add_call* ac = (add_call*)p;
+  render_call* c = &ac->c;
+  c->rc = rtrb_render_device(c->s->r, &c->cam, &c->opts, &c->s->last);
+  if (c->rc != RTRB_OK && c->rc != RTRB_ERR_RAISED) return NULL;
+  const int raised = c->rc == RTRB_ERR_RAISED;
+  c->rc = rtrb_apng_add(ac->a, NULL, c->opts.pixel_format, NULL, c->rgba, c->capacity, &ac->bytes);
+  if (c->rc == RTRB_OK && raised) c->rc = RTRB_ERR_RAISED;
+  return NULL;
+}
+
+static VALUE apng_add_frame(int argc, VALUE* argv, VALUE self) {
+  shim_apng* s;
+  Data_Get_Struct(self, shim_apng, s);
+  VALUE camera, seed;
+  rb_scan_args(argc, argv, "11", &camera, &seed);
+  VALUE args[2] = {camera, seed};
+  add_call ac;
+  memset(&ac, 0, sizeof(ac));
+  frame_call(2, args, s->renderer, &ac.c);
+  if (ac.c.cam.width != s->width || ac.c.cam.height != s->height)
+    rb_raise(rb_eArgError, "a %dx%d camera does not fit the %dx%d animation", ac.c.cam.width, ac.c.cam.height, s->width,
+             s->height);
+  ac.c.opts.skip_outputs = RTRB_SKIP_RGB | RTRB_SKIP_HIT;
+  ac.a = s->a;
+  if (rtrb_apng_frame_max_bytes(s->width, s->height, &ac.c.capacity) != RTRB_OK) rb_raise(rb_eArgError, "%s", rtrb_last_error());
+  VALUE out = rb_str_new(NULL, (long)ac.c.capacity);
+  ac.c.rgba = (uint8_t*)RSTRING_PTR(out);
+  rb_thread_call_without_gvl(add_frame_without_gvl, &ac, RUBY_UBF_IO, NULL);
+  if (ac.c.rc != RTRB_OK && ac.c.rc != RTRB_ERR_RAISED) rb_raise(rb_eRuntimeError, "%s", rtrb_last_error());
+  s->frames++;
+  s->frame_error = ac.c.rc == RTRB_ERR_RAISED ? rb_str_new_cstr(rtrb_last_error()) : Qnil;
+  /* an animation keeps every frame's String: shrink the worst-case buffer to the frame's bytes (rb_str_set_len would
+   * keep the whole capacity allocated) */
+  return rb_str_resize(out, (long)ac.bytes);
+}
+
+static VALUE apng_frame_error(VALUE self) {
+  shim_apng* s;
+  Data_Get_Struct(self, shim_apng, s);
+  return s->frame_error;
+}
+
+static VALUE apng_header(int argc, VALUE* argv, VALUE self) {
+  shim_apng* s;
+  Data_Get_Struct(self, shim_apng, s);
+  VALUE plays;
+  rb_scan_args(argc, argv, "01", &plays);
+  VALUE out = rb_str_new(NULL, RTRB_APNG_HEADER_BYTES);
+  if (rtrb_apng_header(s->width, s->height, s->frames, NIL_P(plays) ? 0 : NUM2INT(plays), (uint8_t*)RSTRING_PTR(out)) != RTRB_OK)
+    rb_raise(rb_eArgError, "%s", rtrb_last_error());
+  return out;
+}
+
 void Init_rtrb_b200(void) {
   mRtrb = rb_define_module("Rtrb");
   cRenderer = rb_define_class_under(mRtrb, "Renderer", rb_cObject);
@@ -483,5 +588,12 @@ void Init_rtrb_b200(void) {
   rb_define_method(cRenderer, "stats", renderer_stats, 0);
   rb_define_method(cRenderer, "trace_rays", renderer_trace_rays, -1);
   rb_define_method(cRenderer, "intersect_rays", renderer_intersect_rays, 1);
+  cAnimation = rb_define_class_under(mRtrb, "Animation", rb_cObject);
+  rb_define_alloc_func(cAnimation, apng_alloc);
+  rb_define_method(cAnimation, "initialize", apng_initialize, 5);
+  rb_define_method(cAnimation, "add_frame", apng_add_frame, -1);
+  rb_define_method(cAnimation, "header", apng_header, -1);
+  rb_define_method(cAnimation, "frame_error", apng_frame_error, 0);
+  rb_define_const(mRtrb, "APNG_IEND", rb_str_new("\0\0\0\0IEND\xae\x42\x60\x82", 12));
   rb_define_const(mRtrb, "ABI_VERSION", INT2NUM(rtrb_abi_version()));
 }

@@ -279,6 +279,39 @@ int rtrb_encode_png(rtrb_renderer* r, const void* src_device, int width, int hei
 int rtrb_submit_png(rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_render_opts* opts, uint8_t* png_host,
                     size_t capacity, size_t* png_bytes_out, int* ticket_out);
 
+/* -- animated PNG files (ABI 4) ------------------------------------------------------------------- */
+/* An animation writes APNG frames (DESIGN.md 15) with the device PNG encoder.  Frame 0 is the whole canvas in IDAT
+ * chunks laid out as rtrb_encode_png lays them out.  Frame k >= 1 stores only the smallest rectangle holding every
+ * pixel whose RGB differs from frame k - 1 (1 x 1 at (0, 0) when none does), in fdAT chunks; its zlib stream is the
+ * one rtrb_encode_png gives for that rectangle as a standalone image.  Every fcTL has dispose NONE, blend SOURCE and
+ * the animation's delay.  A file is rtrb_apng_header, the frames' chunk bytes in the order they were added, then the
+ * 12-byte IEND chunk (00 00 00 00 'IEND' ae 42 60 82).
+ * Frames of one animation are appended in call order, whatever stream they run on; each animation has its own
+ * encoder scratch, so it neither waits for nor disturbs other encodes on the renderer.  A rejected call does not
+ * advance the animation. */
+typedef struct rtrb_apng rtrb_apng;
+#define RTRB_APNG_HEADER_BYTES 53 /* signature + IHDR + acTL */
+/* pure host: signature, IHDR and acTL of a width x height animation; num_frames >= 1, num_plays 0 = forever */
+int rtrb_apng_header(int width, int height, int num_frames, int num_plays, uint8_t out[RTRB_APNG_HEADER_BYTES]);
+/* pure host: bytes that always suffice for one frame's fcTL + data chunks (every segment stored) */
+int rtrb_apng_frame_max_bytes(int width, int height, size_t* bytes_out);
+/* An animation of width x height frames shown delay_num / delay_den seconds each (both < 65536; a denominator of 0
+ * means 100).  RTRB_ERR_CUDA when no CUDA device is usable. */
+int rtrb_apng_create(rtrb_renderer* r, int width, int height, int delay_num, int delay_den, rtrb_apng** out);
+/* Appends the frame at src_device (NULL = start of the renderer's framebuffer, as rtrb_encode_png) in pixel_format;
+ * ordered after the work on `stream` (NULL = the renderer's own); blocks until this frame's chunk bytes are in host
+ * (capacity >= rtrb_apng_frame_max_bytes).  With src_device NULL, RTRB_ERR_INVALID when the last frame rendered into
+ * the framebuffer has another size or pixel format than the animation's frame. */
+int rtrb_apng_add(rtrb_apng* a, const void* src_device, int pixel_format, void* stream,
+                  uint8_t* host, size_t capacity, size_t* bytes_out);
+/* Pipelined: renders the frame (rtrb_submit slots and tickets) and appends it on the copy stream; host_mapped must be
+ * page-locked and device-mapped; completed by the unchanged rtrb_wait, which stores the byte count into *bytes_out.
+ * opts->pixel_format is RTRB_FMT_RGBA8 or RTRB_FMT_RGB8; opts->rgba_device_out is rejected.  A frame that raises is
+ * still appended, and rtrb_wait returns RTRB_ERR_RAISED. */
+int rtrb_submit_apng(rtrb_renderer* r, rtrb_apng* a, const rtrb_camera_desc* cam, const rtrb_render_opts* opts,
+                     uint8_t* host_mapped, size_t capacity, size_t* bytes_out, int* ticket_out);
+int rtrb_apng_destroy(rtrb_apng* a); /* before its renderer; NULL is a no-op */
+
 /* -- progressive frames --------------------------------------------------------------------------- */
 /* One camera plus render options whose pre_sample_times samples are traced in passes the caller chooses, with a
  * well-defined image after every pass (interactive previews, renders that stop when a time budget is spent):

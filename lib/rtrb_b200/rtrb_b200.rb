@@ -13,6 +13,14 @@ module Rtrb
     def trace_rays(packed_rays, trace_depth, mc, seed = 1); raise NotImplementedError; end
     def intersect_rays(packed_rays); raise NotImplementedError; end
   end
+
+  class Animation
+    # method stubs
+    def initialize(renderer, width, height, delay_num, delay_den); raise NotImplementedError; end
+    def add_frame(camera, seed = 1); raise NotImplementedError; end
+    def header(num_plays = 0); raise NotImplementedError; end
+    def frame_error; raise NotImplementedError; end
+  end
 end
 
 require_relative '../rtrb_b200'
@@ -48,6 +56,25 @@ module Alex
       rtrb_renderer
       schedule ||= progressive_schedule(@pre_sample_times)
       @rtrb.render_progressive_png(self, schedule) { |png, _samples_done| File.binwrite(file_path, png) }
+    end
+
+    # n_frames frames as one animated PNG file, each shown 1 / fps seconds: the block, if given, runs before frame i and
+    # may edit @world and this camera; frame 0 is stored whole, every later frame only the rectangle of pixels that
+    # changed.  Each frame is rendered and appended on the GPU; only its chunks cross PCIe.  The file is written before a
+    # frame that raised is reported.
+    def render_cuda_animation(file_path, n_frames, fps = 25)
+      rtrb_renderer
+      anim = Rtrb::Animation.new(@rtrb, @width, @height, 1, fps)
+      chunks = []
+      error = nil
+      n_frames.times do |i|
+        yield i if block_given?
+        rtrb_renderer
+        chunks << anim.add_frame(self)
+        error ||= anim.frame_error
+      end
+      File.binwrite(file_path, anim.header + chunks.join + Rtrb::APNG_IEND)
+      raise RuntimeError, error if error
     end
 
     private

@@ -11,8 +11,9 @@ from .configurable_object import ConfigurableObject
 from .lights import Light, SpotLight
 from .objects import Box, Plane, Sphere, WorldObject
 from .ray_tracer import Ray, RayTracer
-from .renderer import (RAY_HIT_DTYPE, Frame, Progressive, Renderer, deal_frames, device_count, ipc_close, ipc_open,
-                       make_opts, make_ray_opts, measure_fma_peak, png_max_bytes, progressive_schedule, render_multi,
+from .renderer import (RAY_HIT_DTYPE, Apng, Frame, Progressive, Renderer, deal_frames, device_count, ipc_close, ipc_open,
+                       apng_frame_max_bytes, apng_header, make_opts, make_ray_opts,
+                       measure_fma_peak, png_max_bytes, progressive_schedule, render_multi,
                        tile_partition)
 from .texture import Texture
 from .vec3 import Vec3
@@ -22,6 +23,6 @@ __all__ = [
     "Camera", "World", "Sphere", "Plane", "Box", "WorldObject", "Light", "SpotLight", "Texture", "Vec3",
     "ConfigurableObject", "Renderer", "Frame", "make_opts", "render_multi", "measure_fma_peak",
     "device_count", "deal_frames", "ipc_open", "ipc_close", "write_png", "write_png_scanlines", "tile_partition",
-    "png_max_bytes", "Progressive", "progressive_schedule", "Ray", "RayTracer", "RAY_HIT_DTYPE", "make_ray_opts",
+    "png_max_bytes", "Apng", "apng_frame_max_bytes", "apng_header", "Progressive", "progressive_schedule", "Ray", "RayTracer", "RAY_HIT_DTYPE", "make_ray_opts",
     "PREC_STRICT", "PREC_FAST64", "PREC_DEFAULT", "RNG_CTR", "RNG_MT",
 ]

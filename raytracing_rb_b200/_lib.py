@@ -20,6 +20,8 @@ EXPORTS = (
     "rtrb_trace_rays", "rtrb_intersect_rays", "rtrb_camera_rays",
     "rtrb_progressive_create", "rtrb_progressive_pass", "rtrb_progressive_download", "rtrb_progressive_frame_ptr",
     "rtrb_progressive_destroy",
+    "rtrb_apng_header", "rtrb_apng_frame_max_bytes", "rtrb_apng_create", "rtrb_apng_add", "rtrb_submit_apng",
+    "rtrb_apng_destroy",
 )
 
 _lib = None
@@ -82,6 +84,13 @@ def lib():
     L.rtrb_progressive_download.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.rtrb_progressive_frame_ptr.argtypes = [C.c_void_p, P(C.c_void_p)]
     L.rtrb_progressive_destroy.argtypes = [C.c_void_p]
+    L.rtrb_apng_header.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
+    L.rtrb_apng_frame_max_bytes.argtypes = [C.c_int, C.c_int, P(C.c_size_t)]
+    L.rtrb_apng_create.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, P(C.c_void_p)]
+    L.rtrb_apng_add.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, P(C.c_size_t)]
+    L.rtrb_submit_apng.argtypes = [C.c_void_p, C.c_void_p, P(_abi.CameraDesc), P(_abi.RenderOpts), C.c_void_p,
+                                   C.c_size_t, P(C.c_size_t), P(C.c_int)]
+    L.rtrb_apng_destroy.argtypes = [C.c_void_p]
     for name in EXPORTS:
         getattr(L, name)
     if L.rtrb_abi_version() != _abi.ABI_VERSION:

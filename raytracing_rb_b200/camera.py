@@ -13,7 +13,7 @@ import numpy as np
 
 from . import _abi
 from .configurable_object import ConfigurableObject
-from .renderer import make_opts, progressive_schedule, render_multi
+from .renderer import Apng, apng_frame_max_bytes, make_opts, progressive_schedule, render_multi
 from .world import synced_renderer
 
 
@@ -140,6 +140,52 @@ class Camera(ConfigurableObject):
         if code == _abi.RTRB_ERR_RAISED:
             self._raise_for(stats)
         return stats
+
+    def render_animation(self, file_path, n_frames, step=None, fps=25, plays=0, seed=1, in_flight=3, **kw):
+        """n_frames frames written as one animated PNG file, encoded on the GPU: frame 0 whole, every later frame only the
+        rectangle of pixels that changed (DESIGN.md 15).  step(i), if given, runs before frame i and may edit the world
+        and this camera; world edits reach the GPU through renderer(), and the camera is re-read for every frame.
+        Frames are rendered and appended with up to in_flight (1..4) frames outstanding, and only the encoded chunks
+        cross PCIe.  Each frame is shown 1 / fps seconds; plays 0 loops forever.  Raises RuntimeError as render_cuda
+        does for the first frame that raised, after the file has been written.  kw: make_opts options.  Returns the
+        frames' stats dicts."""
+        import torch
+        if n_frames < 1 or not 1 <= in_flight <= 4:
+            raise ValueError("n_frames must be >= 1 and in_flight in 1..4")
+        opts = make_opts(seed=seed, pixel_format=_abi.FMT_RGB8, **kw)
+        r = self.renderer()
+        anim = r.apng(self.width, self.height, delay=(1, int(fps)))
+        cap = apng_frame_max_bytes(self.width, self.height)
+        bufs = [torch.zeros(cap, dtype=torch.uint8).pin_memory().numpy() for _ in range(in_flight)]
+        chunks, stats, pending = [], [], []
+
+        def retire():
+            data, st, code = anim.wait(pending.pop(0))
+            chunks.append(data)
+            stats.append((st, code))
+
+        try:
+            for i in range(n_frames):
+                if len(pending) == in_flight:
+                    retire()
+                if step is not None:
+                    step(i)
+                self.renderer()  # brings the renderer up to date with the world's edits
+                pending.append(anim.submit(self.camera_desc(), bufs[i % in_flight], opts))
+            while pending:
+                retire()
+            d = os.path.dirname(os.path.abspath(file_path))
+            os.makedirs(d, exist_ok=True)
+            with open(file_path, "wb") as f:
+                f.write(anim.header(plays))
+                f.writelines(chunks)
+                f.write(Apng.TRAILER)
+        finally:
+            anim.close()
+        for st, code in stats:
+            if code == _abi.RTRB_ERR_RAISED:
+                self._raise_for(st)
+        return [st for st, _ in stats]
 
     def render_progressive(self, file_path=None, schedule=None, seed=1, **kw):
         """render_cuda in passes, for previews and time-budgeted renders: a generator that yields (samples_done, Frame)

@@ -6,6 +6,7 @@
 // Compiled with -fmad=false: the host-side baking and the resolve arithmetic must round exactly
 // like the reference's scalar FP64 code.
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -474,6 +475,21 @@ struct rtrb_progressive {
   DevBuf<uint8_t> frame;       // the 8-bit frame, unless it goes to opts.rgba_device_out
   FrameOutputs out;            // out.stream is the stream its passes run on
   // its buffers are freed with it; its device must be current (rtrb_progressive_destroy)
+};
+
+// An APNG animation (rtrb_apng_*, DESIGN.md §15): the previous frame and the encoder's own scratch, so that its frames
+// neither wait for nor disturb other encodes on the renderer.
+struct rtrb_apng {
+  rtrb_renderer* r = nullptr;
+  int device = 0;                // r's, kept for rtrb_apng_destroy
+  int W = 0, H = 0, delay_num = 0, delay_den = 0;
+  int frames = 0;                // frames appended so far
+  DevBuf<uint8_t> rgb[2];        // compact RGB8 frames: frame k is stored in rgb[k & 1] and compared with the other
+  DevBuf<RtrbApngState> state;   // the rectangle, sizes and sequence counter, written by the device only
+  RtrbPngScratch png;
+  cudaEvent_t appended = nullptr;  // recorded after each append; the next one waits for it
+  ~rtrb_apng() { if (appended) cudaEventDestroy(appended); }
+  // its buffers are freed with it; its device must be current (rtrb_apng_destroy)
 };
 
 namespace {
@@ -1440,6 +1456,31 @@ int download_frame(rtrb_renderer* r, int rc, uint8_t* rgba, double* rgb_or_null,
   return rc;
 }
 
+// Checks shared by rtrb_apng_add and rtrb_submit_apng, before anything is queued.
+int apng_args(const rtrb_apng* a, int width, int height, size_t capacity) {
+  if (width != a->W || height != a->H)
+    return fail(RTRB_ERR_INVALID, "a %dx%d frame does not fit the %dx%d animation", width, height, a->W, a->H);
+  const size_t need = rtrb_apng_frame_bound(a->W, a->H);
+  if (capacity < need)
+    return fail(RTRB_ERR_INVALID, "apng capacity %zu < %zu bytes (rtrb_apng_frame_max_bytes)", capacity, need);
+  return RTRB_OK;
+}
+
+// Queues the next frame of `a` on `s`, after the previous append, whatever stream that ran on.
+int apng_append(rtrb_apng* a, const uint8_t* src, int pixel_format, cudaStream_t s, uint8_t* host_mapped,
+                unsigned long long* count_mapped) {
+  CUDA_TRY(cudaStreamWaitEvent(s, a->appended, 0));
+  const int k = a->frames;
+  unsigned long long launches = 0;
+  cudaError_t e = rtrb_apng_encode(a->png, a->state.p, a->rgb[(k + 1) & 1].p, a->rgb[k & 1].p, src, a->W, a->H,
+                                   pixel_format, k == 0, a->delay_num, a->delay_den, s, host_mapped, count_mapped,
+                                   &launches);
+  g_launches += launches;
+  if (e != cudaSuccess) return fail(RTRB_ERR_CUDA, "APNG encoder: %s", cudaGetErrorString(e));
+  CUDA_TRY(cudaEventRecord(a->appended, s));
+  a->frames = k + 1;
+  return RTRB_OK;
+}
 }  // namespace
 
 // ================================================================================================
@@ -2105,6 +2146,138 @@ int rtrb_progressive_destroy(rtrb_progressive* p) {
   cudaSetDevice(p->r->device);
   cudaDeviceSynchronize();  // its passes may still be writing its buffers
   delete p;
+  return RTRB_OK;
+}
+
+int rtrb_apng_header(int width, int height, int num_frames, int num_plays, uint8_t out[RTRB_APNG_HEADER_BYTES]) {
+  if (!out || width <= 0 || height <= 0 || num_frames < 1 || num_plays < 0)
+    return fail(RTRB_ERR_INVALID, "bad argument");
+  static const uint8_t sig[8] = {0x89, 'P', 'N', 'G', '\r', '\n', 0x1a, '\n'};
+  memcpy(out, sig, 8);
+  auto be32 = [](uint8_t* p, uint32_t v) { p[0] = (uint8_t)(v >> 24); p[1] = (uint8_t)(v >> 16); p[2] = (uint8_t)(v >> 8); p[3] = (uint8_t)v; };
+  auto crc = [](const uint8_t* p, size_t n) {
+    uint32_t c = 0xffffffffu;
+    for (size_t i = 0; i < n; ++i) {
+      c ^= p[i];
+      for (int k = 0; k < 8; ++k) c = c & 1u ? (c >> 1) ^ 0xedb88320u : c >> 1;
+    }
+    return ~c;
+  };
+  uint8_t* p = out + 8;
+  be32(p, 13); memcpy(p + 4, "IHDR", 4);
+  be32(p + 8, (uint32_t)width); be32(p + 12, (uint32_t)height);
+  p[16] = 8; p[17] = 2; p[18] = 0; p[19] = 0; p[20] = 0;  // 8-bit RGB, deflate, adaptive filters, no interlace
+  be32(p + 21, crc(p + 4, 17));
+  p += 25;
+  be32(p, 8); memcpy(p + 4, "acTL", 4);
+  be32(p + 8, (uint32_t)num_frames); be32(p + 12, (uint32_t)num_plays);
+  be32(p + 16, crc(p + 4, 12));
+  return RTRB_OK;
+}
+
+int rtrb_apng_frame_max_bytes(int width, int height, size_t* bytes_out) {
+  if (!bytes_out || width <= 0 || height <= 0) return fail(RTRB_ERR_INVALID, "bad argument");
+  *bytes_out = rtrb_apng_frame_bound(width, height);
+  return RTRB_OK;
+}
+
+int rtrb_apng_create(rtrb_renderer* r, int width, int height, int delay_num, int delay_den, rtrb_apng** out) {
+  if (!out) return fail(RTRB_ERR_INVALID, "out is NULL");
+  *out = nullptr;
+  if (width <= 0 || height <= 0) return fail(RTRB_ERR_INVALID, "bad animation size %dx%d", width, height);
+  if (delay_num < 0 || delay_num > 65535 || delay_den < 0 || delay_den > 65535)
+    return fail(RTRB_ERR_INVALID, "delay %d/%d does not fit 16 bits", delay_num, delay_den);
+  int rc = require_device();
+  if (rc) return rc;
+  if (!r) return fail(RTRB_ERR_INVALID, "renderer is NULL");
+  CUDA_TRY(cudaSetDevice(r->device));
+  rtrb_apng* a = new rtrb_apng();
+  a->r = r; a->device = r->device; a->W = width; a->H = height; a->delay_num = delay_num; a->delay_den = delay_den;
+  const size_t rgb_bytes = (size_t)width * height * 3;
+  RtrbApngState init;
+  memset(&init, 0, sizeof(init));
+  init.box[0] = init.box[1] = INT_MAX;
+  init.box[2] = init.box[3] = -1;
+  cudaError_t e;
+  if ((e = a->rgb[0].ensure(rgb_bytes)) != cudaSuccess || (e = a->rgb[1].ensure(rgb_bytes)) != cudaSuccess ||
+      (e = a->state.ensure(1)) != cudaSuccess ||
+      (e = cudaMemcpy(a->state.p, &init, sizeof(init), cudaMemcpyHostToDevice)) != cudaSuccess ||
+      (e = cudaEventCreateWithFlags(&a->appended, cudaEventDisableTiming)) != cudaSuccess) {
+    delete a;
+    return fail(RTRB_ERR_CUDA, "animation setup failed: %s", cudaGetErrorString(e));
+  }
+  *out = a;
+  return RTRB_OK;
+}
+
+int rtrb_apng_add(rtrb_apng* a, const void* src_device, int pixel_format, void* stream, uint8_t* host, size_t capacity,
+                  size_t* bytes_out) {
+  if (!a || !host || !bytes_out) return fail(RTRB_ERR_INVALID, "bad argument");
+  if (pixel_format != RTRB_FMT_RGBA8 && pixel_format != RTRB_FMT_RGB8 && pixel_format != RTRB_FMT_PNG_RGB8)
+    return fail(RTRB_ERR_INVALID, "unknown pixel format %d", pixel_format);
+  int rc = apng_args(a, a->W, a->H, capacity);
+  if (rc) return rc;
+  rtrb_renderer* r = a->r;
+  CUDA_TRY(cudaSetDevice(r->device));
+  const uint8_t* src = (const uint8_t*)src_device;
+  if (!src) {
+    if (r->rgba.n < RTRB_FRAME_BYTES(a->W, a->H, pixel_format))
+      return fail(RTRB_ERR_INVALID, "the framebuffer (%zu bytes) is smaller than a %dx%d frame", r->rgba.n, a->W, a->H);
+    // the last frame rendered into the framebuffer fixes its size and layout; a frame gathered there by other means
+    // (peer pushes, IPC) is taken as the caller says
+    const FrameOutputs& last = r->last;
+    if (last.frame == &r->rgba && (last.W != a->W || last.H != a->H || last.format != pixel_format))
+      return fail(RTRB_ERR_INVALID, "the framebuffer holds a %dx%d frame in format %d, not a %dx%d frame in format %d",
+                  last.W, last.H, last.format, a->W, a->H, pixel_format);
+    src = r->rgba.p;
+  }
+  cudaStream_t s = stream ? (cudaStream_t)stream : r->stream;
+  if ((rc = apng_append(a, src, pixel_format, s, nullptr, nullptr))) return rc;
+  unsigned long long total = 0;
+  CUDA_TRY(cudaMemcpyAsync(&total, a->png.total.p, sizeof(total), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  if (total > capacity) return fail(RTRB_ERR_CUDA, "APNG encoder produced %llu bytes, more than its bound %zu", total, capacity);
+  CUDA_TRY(cudaMemcpyAsync(host, a->png.file.p, total, cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  *bytes_out = (size_t)total;
+  return RTRB_OK;
+}
+
+int rtrb_submit_apng(rtrb_renderer* r, rtrb_apng* a, const rtrb_camera_desc* cam, const rtrb_render_opts* opts,
+                     uint8_t* host_mapped, size_t capacity, size_t* bytes_out, int* ticket_out) {
+  if (!r || !a || !cam || !host_mapped || !bytes_out || !ticket_out) return fail(RTRB_ERR_INVALID, "bad argument");
+  if (a->r != r) return fail(RTRB_ERR_INVALID, "the animation belongs to another renderer");
+  const int fmt = opts ? opts->pixel_format : RTRB_FMT_RGBA8;
+  if (fmt != RTRB_FMT_RGBA8 && fmt != RTRB_FMT_RGB8)
+    return fail(RTRB_ERR_INVALID, "rtrb_submit_apng encodes RTRB_FMT_RGBA8 or RTRB_FMT_RGB8 frames, not format %d", fmt);
+  if (opts && opts->rgba_device_out)
+    return fail(RTRB_ERR_INVALID, "rgba_device_out does not combine with rtrb_submit_apng (the frame stays in its slot)");
+  int rc = apng_args(a, cam->width, cam->height, capacity);
+  if (rc) return rc;
+  CUDA_TRY(cudaSetDevice(r->device));
+  void* host_dev = nullptr;
+  if (cudaHostGetDevicePointer(&host_dev, host_mapped, 0) != cudaSuccess) {
+    cudaGetLastError();  // not sticky: clear it so that later launch checks do not report it
+    return fail(RTRB_ERR_INVALID, "host_mapped is not page-locked, device-mapped host memory");
+  }
+  FrameCtl* fcp = nullptr;
+  uint8_t* frame = nullptr;
+  rc = submit_render(r, cam, opts, &fcp, &frame);
+  if (rc) return rc;
+  FrameCtl& fc = *fcp;
+  // appended on the copy stream behind the frame's kernels, as rtrb_submit_png encodes
+  CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, fc.ev1, 0));
+  if ((rc = apng_append(a, frame, fmt, r->copy_stream, (uint8_t*)host_dev, &fc.h_dev->png_bytes))) return rc;
+  CUDA_TRY(cudaEventRecord(fc.copied, r->copy_stream));
+  fc.png_bytes_out = bytes_out;
+  return submit_finish(r, fc, ticket_out);
+}
+
+int rtrb_apng_destroy(rtrb_apng* a) {
+  if (!a) return RTRB_OK;
+  cudaSetDevice(a->device);
+  cudaEventSynchronize(a->appended);  // every append ends with this record: then nothing reads or writes its buffers
+  delete a;
   return RTRB_OK;
 }
 

@@ -13,7 +13,10 @@
 //   - a non-final segment ends with an empty stored block (sync flush) so the next one starts on a byte boundary.
 // Every step is deterministic: the same input gives the same file whatever the scheduling.
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <stdint.h>
+
+#include <algorithm>
 
 #include "rtrb_png.h"
 
@@ -86,9 +89,11 @@ __device__ uint32_t crc_bytes(const uint8_t* p, size_t n, uint32_t crc, const ui
   return ~crc;
 }
 
-// CRC-32 of "IDAT" || data[0, n), all threads of the block; red needs 2 * (blockDim.x / 32) words
+// CRC-32 of "IDAT" || data[0, n), or with FDAT of "fdAT" || seq (big-endian) || data[0, n): the chunk CRC; all threads
+// of the block; red needs 2 * (blockDim.x / 32) words
+template <bool FDAT = false>
 __device__ uint32_t block_chunk_crc(const uint8_t* data, uint32_t n, const uint32_t* table, const uint32_t* x2n,
-                                    uint32_t* red) {
+                                    uint32_t* red, uint32_t seq = 0) {
   const uint32_t per = (n + blockDim.x - 1) / blockDim.x;
   const uint32_t b = min(n, threadIdx.x * per), e = min(n, b + per);
   uint32_t crc = crc_bytes(data + b, e - b, 0, table), len = e - b;
@@ -101,8 +106,14 @@ __device__ uint32_t block_chunk_crc(const uint8_t* data, uint32_t n, const uint3
   __syncthreads();
   uint32_t out = 0;
   if (threadIdx.x == 0) {
-    const uint8_t idat[4] = {'I', 'D', 'A', 'T'};
-    out = crc_bytes(idat, 4, 0, table);
+    if (FDAT) {
+      const uint8_t head[8] = {'f', 'd', 'A', 'T', (uint8_t)(seq >> 24), (uint8_t)(seq >> 16), (uint8_t)(seq >> 8),
+                               (uint8_t)seq};
+      out = crc_bytes(head, 8, 0, table);
+    } else {
+      const uint8_t idat[4] = {'I', 'D', 'A', 'T'};
+      out = crc_bytes(idat, 4, 0, table);
+    }
     for (int w = 0; w < (int)(blockDim.x >> 5); ++w) out = crc_combine(out, red[2 * w], red[2 * w + 1], x2n);
   }
   return out;  // valid in thread 0
@@ -140,12 +151,19 @@ __device__ __forceinline__ uint32_t paeth(int a, int b, int c) {
   return (uint32_t)((pa <= pb && pa <= pc) ? a : (pb <= pc ? b : c));
 }
 
+// One CTA per row.  CROP: the rows [0, h) of the APNG frame's w x h rectangle at (x0, y0) in `crop` (the grid covers
+// the whole frame; rows >= h exit), filtered as a standalone w x h image, whose first row has no row above.
+template <bool CROP>
 __global__ void __launch_bounds__(256) png_filter_kernel(const uint8_t* __restrict__ src, int W, int fmt,
-                                                         uint8_t* __restrict__ out) {
-  const int y = blockIdx.x, n = 3 * W;
+                                                         uint8_t* __restrict__ out,
+                                                         const RtrbApngState* __restrict__ crop) {
+  const int y = blockIdx.x;
+  if (CROP && y >= crop->h) return;
+  const int nw = 3 * W, n = CROP ? 3 * crop->w : nw;
   const int bpp = fmt == RTRB_FMT_RGBA8 ? 4 : 3;
-  const size_t stride = fmt == RTRB_FMT_PNG_RGB8 ? (size_t)n + 1 : (size_t)W * bpp;
+  const size_t stride = fmt == RTRB_FMT_PNG_RGB8 ? (size_t)nw + 1 : (size_t)W * bpp;
   const uint8_t* row = src + y * stride + (fmt == RTRB_FMT_PNG_RGB8 ? 1 : 0);
+  if (CROP) row += crop->y0 * stride + (size_t)crop->x0 * bpp;
   const uint8_t* up = y > 0 ? row - stride : row;
   auto at = [&](const uint8_t* r, int i) -> int { return r[(i / 3) * bpp + i % 3]; };
   uint32_t s[5] = {0, 0, 0, 0, 0};
@@ -341,9 +359,18 @@ struct DeflateShared {
   uint32_t hdr_bits, out_bytes;
 };
 
+// One CTA per segment.  CROP: the APNG frame's filtered stream, its size and row length read from `crop`; the grid
+// covers the whole frame's segments and those past the crop's exit; the chunk CRC is that of the segment's fdAT chunk.
+template <bool CROP>
 __global__ void __launch_bounds__(DT, 1) png_deflate_kernel(const uint8_t* __restrict__ in, unsigned long long n_in, int row_bytes,
                                                             uint32_t* __restrict__ tokens, uint8_t* __restrict__ seg_out,
-                                                            uint32_t* __restrict__ seg_meta) {
+                                                            uint32_t* __restrict__ seg_meta,
+                                                            const RtrbApngState* __restrict__ crop) {
+  if (CROP) {
+    if (blockIdx.x >= crop->nseg) return;
+    n_in = crop->n_in;
+    row_bytes = 3 * crop->w + 1;
+  }
   extern __shared__ __align__(16) uint8_t smem[];
   uint8_t* data = smem;                                                   // [REGION + 16]
   uint16_t* prev = reinterpret_cast<uint16_t*>(smem + REGION + 16);      // [REGION] chain links (distance, 0 = end)
@@ -616,7 +643,9 @@ __global__ void __launch_bounds__(DT, 1) png_deflate_kernel(const uint8_t* __res
     for (int i = tid; i < (int)out_bytes; i += DT) out[i] = bytes[i];
   }
   __syncthreads();
-  const uint32_t crc = block_chunk_crc(out, out_bytes, sh.crc_table, sh.x2n, sh.red);
+  // a crop's segment s is the fdAT chunk with sequence number seq + 2 + s (after the fcTL and zlib-header chunks)
+  const uint32_t crc = CROP ? block_chunk_crc<true>(out, out_bytes, sh.crc_table, sh.x2n, sh.red, crop->seq + 2 + seg)
+                           : block_chunk_crc(out, out_bytes, sh.crc_table, sh.x2n, sh.red);
   if (tid == 0) {
     const uint32_t a = (uint32_t)((1ull + sh.adler_a) % 65521ull);
     const uint32_t b = (uint32_t)(((unsigned long long)seg_len + sh.adler_b) % 65521ull);
@@ -733,6 +762,134 @@ __global__ void __launch_bounds__(256) png_publish_kernel(const uint8_t* __restr
   if (tid == 0) *count = n;
 }
 
+// ---- APNG frames -------------------------------------------------------------------------------------------------
+// Stores the frame `src` (W x H in fmt) as compact RGB8 into `cur` and, unless it is the first frame, compares its RGB
+// with the previous frame `prev`.  Each CTA merges the bounding box of its changed pixels into st->box with one atomic
+// per side; the last CTA turns the box into the frame's rectangle (the whole canvas for the first frame, 1 x 1 at
+// (0, 0) when nothing changed), derives the crop's stream size and segment count, and resets the box for the next frame.
+__global__ void __launch_bounds__(256) apng_diff_kernel(const uint8_t* __restrict__ src, int W, int H, int fmt,
+                                                        const uint8_t* __restrict__ prev, uint8_t* __restrict__ cur,
+                                                        int first, RtrbApngState* st) {
+  const int bpp = fmt == RTRB_FMT_RGBA8 ? 4 : 3;
+  const size_t stride = fmt == RTRB_FMT_PNG_RGB8 ? (size_t)W * 3 + 1 : (size_t)W * bpp;
+  const int off = fmt == RTRB_FMT_PNG_RGB8 ? 1 : 0;
+  int x0 = INT_MAX, y0 = INT_MAX, x1 = -1, y1 = -1;
+  const size_t npix = (size_t)W * H;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += (size_t)gridDim.x * blockDim.x) {
+    const int y = (int)(i / W), x = (int)(i - (size_t)y * W);
+    const uint8_t* p = src + y * stride + off + (size_t)x * bpp;
+    const uint8_t r = p[0], g = p[1], b = p[2];
+    uint8_t* c = cur + 3 * i;
+    c[0] = r; c[1] = g; c[2] = b;
+    if (!first) {
+      const uint8_t* q = prev + 3 * i;
+      if (q[0] != r || q[1] != g || q[2] != b) { x0 = min(x0, x); y0 = min(y0, y); x1 = max(x1, x); y1 = max(y1, y); }
+    }
+  }
+  x0 = __reduce_min_sync(0xffffffffu, x0); y0 = __reduce_min_sync(0xffffffffu, y0);
+  x1 = __reduce_max_sync(0xffffffffu, x1); y1 = __reduce_max_sync(0xffffffffu, y1);
+  __shared__ int red[8][4];
+  const int warp = threadIdx.x >> 5;
+  if ((threadIdx.x & 31) == 0) { red[warp][0] = x0; red[warp][1] = y0; red[warp][2] = x1; red[warp][3] = y1; }
+  __syncthreads();
+  if (threadIdx.x != 0) return;
+  for (int w = 1; w < (int)(blockDim.x >> 5); ++w) {
+    x0 = min(x0, red[w][0]); y0 = min(y0, red[w][1]); x1 = max(x1, red[w][2]); y1 = max(y1, red[w][3]);
+  }
+  if (x1 >= 0) {
+    atomicMin(&st->box[0], x0); atomicMin(&st->box[1], y0); atomicMax(&st->box[2], x1); atomicMax(&st->box[3], y1);
+  }
+  __threadfence();
+  if (atomicAdd(&st->ctas_done, 1u) != gridDim.x - 1) return;
+  x0 = atomicExch(&st->box[0], INT_MAX); y0 = atomicExch(&st->box[1], INT_MAX);
+  x1 = atomicExch(&st->box[2], -1); y1 = atomicExch(&st->box[3], -1);
+  st->ctas_done = 0;
+  if (first) { x0 = 0; y0 = 0; x1 = W - 1; y1 = H - 1; }
+  else if (x1 < 0) { x0 = 0; y0 = 0; x1 = 0; y1 = 0; }
+  const int w = x1 - x0 + 1, h = y1 - y0 + 1;
+  st->x0 = x0; st->y0 = y0; st->w = w; st->h = h;
+  st->n_in = (unsigned long long)h * (3ull * w + 1);
+  st->nseg = (unsigned)((st->n_in + SEG - 1) / SEG);
+  st->seq = st->next_seq;
+}
+
+constexpr int APNG_FCTL_BYTES = 12 + 26;
+
+// one CTA: segment offsets, the fcTL chunk, the zlib-header and Adler-32 chunks (IDAT for the first frame, else fdAT
+// with sequence numbers), the frame's byte count; advances the sequence counter
+__global__ void __launch_bounds__(1024) apng_assemble_kernel(const uint32_t* __restrict__ seg_meta, RtrbApngState* st,
+                                                             int idat, int delay_num, int delay_den,
+                                                             unsigned long long* __restrict__ seg_off,
+                                                             uint8_t* __restrict__ file,
+                                                             unsigned long long* __restrict__ total) {
+  __shared__ uint32_t crc_table[256], x2n[32], scan[32];
+  __shared__ unsigned long long carry;
+  const int nseg = (int)st->nseg;
+  const uint32_t seq = st->seq, extra = idat ? 0 : 4;  // an fdAT chunk has a sequence number in front of its data
+  crc_table_init(crc_table, x2n);
+  if (threadIdx.x == 0) carry = APNG_FCTL_BYTES + 14 + extra;  // after the fcTL and zlib-header chunks
+  __syncthreads();
+  for (int base = 0; base < nseg; base += blockDim.x) {
+    const int s = base + threadIdx.x;
+    const uint32_t sz = s < nseg ? seg_meta[3 * s] + RTRB_PNG_CHUNK_BYTES + extra : 0;
+    uint32_t tot;
+    const uint32_t incl = block_scan<false>(sz, scan, tot);
+    if (s < nseg) seg_off[s] = carry + incl - sz;
+    __syncthreads();
+    if (threadIdx.x == 0) carry += tot;
+    __syncthreads();
+  }
+  if (threadIdx.x != 0) return;
+  auto tag = [&](uint8_t* q, uint32_t q_seq) {
+    q[4] = idat ? 'I' : 'f'; q[5] = idat ? 'D' : 'd'; q[6] = 'A'; q[7] = 'T';
+    if (!idat) put_be32(q + 8, q_seq);
+  };
+  uint8_t* p = file;
+  put_be32(p, 26); p[4] = 'f'; p[5] = 'c'; p[6] = 'T'; p[7] = 'L';
+  put_be32(p + 8, seq);
+  put_be32(p + 12, (uint32_t)st->w); put_be32(p + 16, (uint32_t)st->h);
+  put_be32(p + 20, (uint32_t)st->x0); put_be32(p + 24, (uint32_t)st->y0);
+  p[28] = (uint8_t)(delay_num >> 8); p[29] = (uint8_t)delay_num; p[30] = (uint8_t)(delay_den >> 8); p[31] = (uint8_t)delay_den;
+  p[32] = 0; p[33] = 0;  // dispose NONE, blend SOURCE
+  put_be32(p + 34, crc_bytes(p + 4, 30, 0, crc_table));
+  p += APNG_FCTL_BYTES;
+  put_be32(p, 2 + extra); tag(p, seq + 1);
+  p[8 + extra] = 0x78; p[9 + extra] = 0x01;  // zlib: deflate, 32 KiB window
+  put_be32(p + 10 + extra, crc_bytes(p + 4, 6 + extra, 0, crc_table));
+  const unsigned long long n_in = st->n_in;
+  uint32_t adler = 1;
+  for (int s = 0; s < nseg; ++s) {
+    const unsigned long long len = min((unsigned long long)SEG, n_in - (unsigned long long)s * SEG);
+    adler = adler_combine(adler, seg_meta[3 * s + 2], len);
+  }
+  p = file + carry;
+  put_be32(p, 4 + extra); tag(p, seq + 2 + (uint32_t)nseg);
+  put_be32(p + 8 + extra, adler);
+  put_be32(p + 12 + extra, crc_bytes(p + 4, 8 + extra, 0, crc_table));
+  *total = carry + 16 + extra;
+  st->next_seq = idat ? seq + 1 : seq + 3 + (uint32_t)nseg;
+}
+
+// one CTA per segment of the whole frame (those past the crop's exit): the segment's fdAT chunk at its offset, with
+// the chunk CRC png_deflate_kernel<true> left in seg_meta
+__global__ void __launch_bounds__(256) apng_place_kernel(const uint8_t* __restrict__ seg_out,
+                                                         const uint32_t* __restrict__ seg_meta,
+                                                         const unsigned long long* __restrict__ seg_off,
+                                                         const RtrbApngState* __restrict__ st,
+                                                         uint8_t* __restrict__ file) {
+  const int s = blockIdx.x;
+  if (s >= (int)st->nseg) return;
+  const uint32_t n = seg_meta[3 * s];
+  uint8_t* p = file + seg_off[s];
+  const uint8_t* q = seg_out + (size_t)s * RTRB_PNG_SEGMENT_WORST(SEG);
+  if (threadIdx.x == 0) {
+    put_be32(p, n + 4); p[4] = 'f'; p[5] = 'd'; p[6] = 'A'; p[7] = 'T';
+    put_be32(p + 8, st->seq + 2 + (uint32_t)s);
+    put_be32(p + 12 + n, seg_meta[3 * s + 1]);
+  }
+  for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) p[12 + i] = q[i];
+}
+
 }  // namespace
 
 cudaError_t rtrb_png_encode(RtrbPngScratch& s, const uint8_t* src, int width, int height, int pixel_format,
@@ -745,14 +902,53 @@ cudaError_t rtrb_png_encode(RtrbPngScratch& s, const uint8_t* src, int width, in
       (e = s.seg_meta.ensure(nseg * 3)) != cudaSuccess || (e = s.seg_off.ensure(nseg)) != cudaSuccess ||
       (e = s.file.ensure(rtrb_png_bound(width, height))) != cudaSuccess || (e = s.total.ensure(1)) != cudaSuccess)
     return e;
-  if ((e = cudaFuncSetAttribute(png_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DEFLATE_SMEM)) != cudaSuccess)
+  if ((e = cudaFuncSetAttribute(png_deflate_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DEFLATE_SMEM)) != cudaSuccess)
     return e;
-  png_filter_kernel<<<height, 256, 0, stream>>>(src, width, pixel_format, s.filtered.p);
-  png_deflate_kernel<<<(unsigned)nseg, DT, DEFLATE_SMEM, stream>>>(s.filtered.p, n, 3 * width + 1, s.tokens.p, s.seg_out.p,
-                                                                   s.seg_meta.p);
+  png_filter_kernel<false><<<height, 256, 0, stream>>>(src, width, pixel_format, s.filtered.p, nullptr);
+  png_deflate_kernel<false><<<(unsigned)nseg, DT, DEFLATE_SMEM, stream>>>(s.filtered.p, n, 3 * width + 1, s.tokens.p,
+                                                                          s.seg_out.p, s.seg_meta.p, nullptr);
   png_assemble_kernel<<<1, 1024, 0, stream>>>(s.seg_meta.p, (int)nseg, n, width, height, s.seg_off.p, s.file.p, s.total.p);
   png_place_kernel<<<(unsigned)nseg, 256, 0, stream>>>(s.seg_out.p, s.seg_meta.p, s.seg_off.p, s.file.p);
   *launches += 4;
+  if (host_mapped) {
+    png_publish_kernel<<<64, 256, 0, stream>>>(s.file.p, s.total.p, host_mapped, count_mapped);
+    *launches += 1;
+  }
+  return cudaGetLastError();
+}
+
+cudaError_t rtrb_apng_encode(RtrbPngScratch& s, RtrbApngState* st, const uint8_t* prev, uint8_t* cur, const uint8_t* src,
+                             int width, int height, int pixel_format, bool first, int delay_num, int delay_den,
+                             cudaStream_t stream, uint8_t* host_mapped, unsigned long long* count_mapped,
+                             unsigned long long* launches) {
+  const size_t n = rtrb_png_filtered_bytes(width, height), nseg = rtrb_png_segments(width, height);
+  cudaError_t e;
+  if ((e = s.filtered.ensure(n)) != cudaSuccess || (e = s.tokens.ensure(nseg * SEG)) != cudaSuccess ||
+      (e = s.seg_out.ensure(nseg * RTRB_PNG_SEGMENT_WORST(SEG))) != cudaSuccess ||
+      (e = s.seg_meta.ensure(nseg * 3)) != cudaSuccess || (e = s.seg_off.ensure(nseg)) != cudaSuccess ||
+      (e = s.file.ensure(rtrb_apng_frame_bound(width, height))) != cudaSuccess || (e = s.total.ensure(1)) != cudaSuccess)
+    return e;
+  if ((e = cudaFuncSetAttribute(png_deflate_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DEFLATE_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(png_deflate_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DEFLATE_SMEM)) != cudaSuccess)
+    return e;
+  const size_t npix = (size_t)width * height;
+  apng_diff_kernel<<<(unsigned)std::min<size_t>((npix + 255) / 256, 148 * 8), 256, 0, stream>>>(
+      src, width, height, pixel_format, prev, cur, first ? 1 : 0, st);
+  // the first frame is the whole canvas, with sizes the host knows: rtrb_encode_png's kernels give its IDAT chunks
+  if (first) {
+    png_filter_kernel<false><<<height, 256, 0, stream>>>(cur, width, RTRB_FMT_RGB8, s.filtered.p, nullptr);
+    png_deflate_kernel<false><<<(unsigned)nseg, DT, DEFLATE_SMEM, stream>>>(s.filtered.p, n, 3 * width + 1, s.tokens.p,
+                                                                            s.seg_out.p, s.seg_meta.p, nullptr);
+  } else {
+    png_filter_kernel<true><<<height, 256, 0, stream>>>(cur, width, RTRB_FMT_RGB8, s.filtered.p, st);
+    png_deflate_kernel<true><<<(unsigned)nseg, DT, DEFLATE_SMEM, stream>>>(s.filtered.p, 0, 0, s.tokens.p, s.seg_out.p,
+                                                                           s.seg_meta.p, st);
+  }
+  apng_assemble_kernel<<<1, 1024, 0, stream>>>(s.seg_meta.p, st, first ? 1 : 0, delay_num, delay_den, s.seg_off.p,
+                                               s.file.p, s.total.p);
+  if (first) png_place_kernel<<<(unsigned)nseg, 256, 0, stream>>>(s.seg_out.p, s.seg_meta.p, s.seg_off.p, s.file.p);
+  else apng_place_kernel<<<(unsigned)nseg, 256, 0, stream>>>(s.seg_out.p, s.seg_meta.p, s.seg_off.p, st, s.file.p);
+  *launches += 5;
   if (host_mapped) {
     png_publish_kernel<<<64, 256, 0, stream>>>(s.file.p, s.total.p, host_mapped, count_mapped);
     *launches += 1;

@@ -284,6 +284,11 @@ class Renderer:
         """A progressive frame of `cam` on this renderer (rtrb_progressive_create) -> Progressive."""
         return Progressive(self, cam, opts)
 
+    def apng(self, width, height, delay=(1, 25)):
+        """An animated PNG of width x height frames on this renderer, each shown delay[0] / delay[1] seconds
+        (rtrb_apng_create) -> Apng."""
+        return Apng(self, width, height, delay)
+
     def peer_push(self, src_ptr, dst_peer_ptr, nbytes, after_stream=None):
         """Copy-engine gather: queue a D2D copy to a peer mapping behind `after_stream` (see rtrb_peer_push)."""
         check(lib().rtrb_peer_push(self._h, C.c_void_p(src_ptr), C.c_void_p(dst_peer_ptr), nbytes,
@@ -367,6 +372,69 @@ class Progressive:
             pass
 
 
+class Apng:
+    """An animated PNG built frame by frame on the device (rtrb_apng_*, include/rtrb_b200.h): frame 0 is the whole
+    canvas, every later frame only the rectangle of pixels that changed since the frame before.  The file is
+    header(), then the chunk bytes of every frame in the order they were added, then TRAILER.  Holds a reference to its
+    Renderer, which must outlive it."""
+
+    TRAILER = b"\x00\x00\x00\x00IEND\xaeB`\x82"
+
+    def __init__(self, renderer, width, height, delay=(1, 25)):
+        self.renderer = renderer
+        self.width, self.height = width, height
+        self.delay = tuple(delay)
+        self.frames = 0
+        self._pending = {}  # submit ticket -> (host buffer, byte count that rtrb_wait fills in)
+        self._h = C.c_void_p()
+        check(lib().rtrb_apng_create(renderer.handle, width, height, self.delay[0], self.delay[1], C.byref(self._h)))
+
+    def add(self, src=None, pixel_format=_abi.FMT_RGB8, stream=None):
+        """Appends the frame at device pointer `src` (None = the renderer's framebuffer) in pixel_format, ordered after
+        the work on `stream` (None = the renderer's own) -> the frame's chunk bytes."""
+        cap = apng_frame_max_bytes(self.width, self.height)
+        out = np.empty(cap, np.uint8)
+        n = C.c_size_t()
+        check(lib().rtrb_apng_add(self._h, C.c_void_p(src) if src else None, pixel_format,
+                                  C.c_void_p(stream) if stream else None, out.ctypes.data, cap, C.byref(n)))
+        self.frames += 1
+        return out[:n.value].tobytes()
+
+    def submit(self, cam, out_pinned, opts=None):
+        """Pipelined frame rendered and appended on the device (rtrb_submit_apng): returns a ticket at once; the chunk
+        bytes land in `out_pinned` (a uint8 numpy view of page-locked, device-mapped host memory of at least
+        apng_frame_max_bytes(W, H) bytes) by the time `wait(ticket)` returns.  Shares the renderer's four slots."""
+        opts = opts or make_opts(pixel_format=_abi.FMT_RGB8)
+        t = C.c_int()
+        n = C.c_size_t()
+        check(lib().rtrb_submit_apng(self.renderer.handle, self._h, C.byref(cam), C.byref(opts),
+                                     out_pinned.ctypes.data, out_pinned.nbytes, C.byref(n), C.byref(t)))
+        self.frames += 1
+        self._pending[t.value] = (out_pinned, n)
+        return t.value
+
+    def wait(self, ticket):
+        """-> (chunk bytes, stats dict, status code) of a submitted frame."""
+        out, n = self._pending.pop(ticket)
+        stats, code = self.renderer.wait(ticket)
+        return out[:n.value].tobytes(), stats, code
+
+    def header(self, num_plays=0):
+        """Signature, IHDR and acTL for the frames added so far; num_plays 0 loops forever."""
+        return apng_header(self.width, self.height, self.frames, num_plays)
+
+    def close(self):
+        if self._h:
+            lib().rtrb_apng_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def ipc_open(device, handle_bytes):
     buf = (C.c_uint8 * 64).from_buffer_copy(handle_bytes)
     p = C.c_void_p()
@@ -421,6 +489,20 @@ def png_max_bytes(width, height):
     n = C.c_size_t()
     check(lib().rtrb_png_max_bytes(width, height, C.byref(n)))
     return n.value
+
+
+def apng_frame_max_bytes(width, height):
+    """Bytes that always suffice for one APNG frame's chunks of a width x height animation.  Pure host logic."""
+    n = C.c_size_t()
+    check(lib().rtrb_apng_frame_max_bytes(width, height, C.byref(n)))
+    return n.value
+
+
+def apng_header(width, height, num_frames, num_plays=0):
+    """Signature, IHDR and acTL chunks of a width x height animation of num_frames frames.  Pure host logic."""
+    out = (C.c_uint8 * 53)()
+    check(lib().rtrb_apng_header(width, height, num_frames, num_plays, out))
+    return bytes(out)
 
 
 def measure_fma_peak(device=0, fp64=True):
