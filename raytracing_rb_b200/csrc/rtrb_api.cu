@@ -991,10 +991,14 @@ void bake_frame(const rtrb_renderer* r, const rtrb_camera_desc* cam, FrameParams
       // only the depth-1 kernels read them; at trace_depth 0 a camera ray is not even counted, so the sky path's
       // "one ray" would be wrong there
       static_assert(sizeof(P.k_tile_rows) == RTRB_CAM_TX * 4, "tile rows layout");
-      if (cam->trace_depth == 1)
+      if (cam->trace_depth == 1) {
         rtrb_tile_rows(&P.k_cull_pl[0].x, P.n_pl, P.k_lights_f, P.n_lights, P.pos, P.focal_point, P.left, P.up_n,
                        P.front, cam->image_distance, cam->retina_width, cam->retina_height, cam->width, cam->height,
                        (uint8_t(*)[4])P.k_tile_rows);
+        rtrb_ground_rows(&P.k_cull_pl[0].x, P.n_pl, P.max_distance_f, P.pos, P.focal_point, P.left, P.up_n, P.front,
+                         cam->image_distance, cam->retina_width, cam->retina_height, cam->width, cam->height,
+                         (const uint8_t(*)[4])P.k_tile_rows, (uint8_t(*)[2])P.k_ground_rows);
+      }
     } else {  // rays start anywhere on the lens: every sphere is a candidate
       const uint32_t all = n_sph >= 32 ? 0xffffffffu : (1u << n_sph) - 1u;
       for (uint32_t& m : P.k_cam_tx) m = all;

@@ -316,3 +316,64 @@ inline void rtrb_tile_rows(const float* pl, int n_pl, const RtrbLightF* lf, int 
     for (int i = 0; i < 2; ++i) { rows[c][2 * i] = (uint8_t)best0[i]; rows[c][2 * i + 1] = (uint8_t)best1[i]; }
   }
 }
+
+// Longest run of set flags in f[0, n): [b0, b1), empty = [0, 0).
+inline void rtrb_longest_run(const uint8_t* f, int n, int& b0, int& b1) {
+  b0 = b1 = 0;
+  int run = 0;
+  for (int r = 0; r <= n; ++r) {
+    if (r < n && f[r]) { run++; continue; }
+    if (run > b1 - b0) { b0 = r - run; b1 = r; }
+    run = 0;
+  }
+}
+
+// Ground certificates of a pinhole frame whose scene has exactly one plane: rows[c] = {g0, g1} for super-tile column
+// c < RTRB_CAM_TX, the longest run of rows in which, for every primary ray of the tile (dilated by one pixel),
+// classify_plane does not return kind 0 for the plane and its lo <= max_distance_f, inside tile_rows' no-highlight rows.
+// A ground tile whose camera candidate mask is empty therefore sends exactly the plane to the exact test, and nothing
+// else.  All zero = nothing.
+// Bounds: den = n . u is within m_n of n . rf / |rf| (rtrb_tile_rows), so s (n . rf) >= m_n rf_max, s = sign(num), gives
+// den the sign of num (or |den| below the grazing cut, kind 1): t = num rcp(den) >= 0, never kind 0; and lo <= t <=
+// (|num| + e_num / 2) (1 + 1e-5) / (s g_min / rf_max - m_n).
+inline void rtrb_ground_rows(const float* pl, int n_pl, float max_distance_f, const double pos[3], const double focal_point[3],
+                             const double left[3], const double up_n[3], const double front[3], double D, double rw,
+                             double rh, int W, int H, const uint8_t tile_rows[RTRB_CAM_TX][4],
+                             uint8_t rows[RTRB_CAM_TX][2]) {
+  for (int c = 0; c < RTRB_CAM_TX; ++c) rows[c][0] = rows[c][1] = 0;
+  const RtrbPinhole cam = rtrb_pinhole(pos, focal_point, left, up_n, front, D, rw, rh, W, H);
+  const double eps = 5.9604644775390625e-8;  // 2^-24
+  if (!cam.ok || !(D > 0.0) || !(cam.od > 0.0) || n_pl != 1) return;
+  auto dot = [](const double* a, const double* b) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; };
+  const double* f = cam.f;
+  const double dl = cam.dir + 7.62939453125e-6;
+  const double o[3] = {(float)pos[0], (float)pos[1], (float)pos[2]};
+  const double mo = fmax(fabs(o[0]), fmax(fabs(o[1]), fabs(o[2])));
+  const double n[3] = {pl[0], pl[1], pl[2]}, aw = pl[3], pw = pl[7];
+  const double num = ((double)pl[4] - o[0]) * n[0] + ((double)pl[5] - o[1]) * n[1] + ((double)pl[6] - o[2]) * n[2];
+  const double e_num = 16.0 * eps * aw * (pw + mo) * 1.0001;
+  const double s = num > 0.0 ? 1.0 : -1.0;
+  const double m_n = sqrt(dot(n, n)) * dl + 8.0 * eps * aw * (1.0 + dl);
+  const double g_th = m_n * cam.rf_max * (1.0 + 1e-9) + 1e-300;
+  if (!(aw > 0.0 && fabs(num) - 0.5 * e_num > 0.0 && isfinite(num) && isfinite(g_th))) return;
+  const double kc = s * dot(n, f) * D, kl = s * dot(n, left), ku = s * dot(n, up_n);
+  const int nc = (W + 31) / 32 < RTRB_CAM_TX ? (W + 31) / 32 : RTRB_CAM_TX;
+  const int nr = (H + 31) / 32 < 255 ? (H + 31) / 32 : 255;
+  auto sx = [&](int x) { return 2.0 * ((double)x / W - 0.5) * rw; };
+  auto sy = [&](int y) { return 2.0 * ((double)y / H - 0.5) * rh; };
+  double ry_lo[255];
+  for (int r = 0; r < nr; ++r) ry_lo[r] = fmin(-ku * sy(32 * r - 1), -ku * sy(32 * r + 32));
+  for (int c = 0; c < nc; ++c) {
+    const double cx_lo = kc + fmin(-kl * sx(32 * c - 1), -kl * sx(32 * c + 32));
+    uint8_t g[256];
+    for (int r = 0; r < nr; ++r) {
+      const double sg = cx_lo + ry_lo[r];  // min of s (n . rf) over the tile
+      const double t_max = (fabs(num) + 0.5 * e_num) * (1.0 + 1e-5) / (sg / cam.rf_max - m_n);
+      g[r] = (uint8_t)(sg >= g_th && r >= tile_rows[c][2] && r < tile_rows[c][3] &&
+                       (max_distance_f == INFINITY || t_max <= (double)max_distance_f));
+    }
+    int g0, g1;
+    rtrb_longest_run(g, nr, g0, g1);
+    rows[c][0] = (uint8_t)g0; rows[c][1] = (uint8_t)g1;
+  }
+}

@@ -799,11 +799,12 @@ __device__ __forceinline__ void merge_ctx(ThreadCtx& ctx, const ThreadCtx& t) {
 
 // FAST64 entry point, defined in rtrb_trace_fast.cuh (only instantiated by that translation unit).  CULL: the depth-1
 // frame kernels' candidate masks (FrameParams::k_cam_tx, light_cand); cam_cand = those of the pixel's super-tile, and
-// no_highlight = its tile certificate rules out every highlight (FrameParams::k_tile_rows).
+// no_highlight = its tile certificate rules out every highlight (FrameParams::k_tile_rows), and ground = its ground
+// certificate holds and its mask is empty (FrameParams::k_ground_rows).
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                                 ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu,
-                                                bool no_highlight = false);
+                                                bool no_highlight = false, bool ground = false);
 
 // BVH: FAST64 with the sphere BVH instead of the linear filter.
 // BOX: the FAST64 kernels carry the Box code only in their full-counter (DETAIL) variants; scenes with a
@@ -811,9 +812,10 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
                                              ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand = 0xffffffffu,
-                                             bool no_highlight = false) {
+                                             bool no_highlight = false, bool ground = false) {
   if constexpr (Pol::fast)
-    return trace_sample_fast<Pol, MAXS, BVH, BOX, CULL>(P, ro, rd, pixel, sample, ctx, primary_hit, cam_cand, no_highlight);
+    return trace_sample_fast<Pol, MAXS, BVH, BOX, CULL>(P, ro, rd, pixel, sample, ctx, primary_hit, cam_cand, no_highlight,
+                                                        ground);
   else return trace_sample<Pol, MAXS>(P, ro, rd, pixel, sample, ctx, primary_hit);
 }
 
@@ -827,7 +829,7 @@ __device__ __forceinline__ d3 trace_dispatch(const FrameParams& P, d3 ro, d3 rd,
 // colour goes to the sample buffer at (slot * pre + j), the stride of the whole frame.  No overlap, no in-thread resolve.
 // The FAST64 depth-1 linear-filter kernels (the pass kernels included) narrow the camera apex test to the candidate masks
 // of the pixel's super-tile, store sky tiles without tracing and skip the highlight test where the tile certificates
-// (FrameParams::k_tile_rows) allow.
+// (FrameParams::k_tile_rows) allow, and skip the camera filter on ground tiles (FrameParams::k_ground_rows).
 template <class Pol, int MAXS, bool DETAIL, bool BVH = false, bool PASS = false>
 __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
   constexpr bool kOverlap = Pol::fast && MAXS == 1 && !PASS;
@@ -861,8 +863,11 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
           ph = -1;
           ctx.rays = 1;
         } else {
+          const uchar2 gr = tx < RTRB_CAM_TX ? P.k_ground_rows[tx] : make_uchar2(0, 0);
+          const bool ground = cand == 0u && ty >= gr.x && ty < gr.y;
           camera_ray<Pol>(P, x, y, pixel, j, ro, rd);
-          col = trace_dispatch<Pol, MAXS, BVH, DETAIL, true>(P, ro, rd, pixel, j, ctx, &ph, cand, ty >= rows.z && ty < rows.w);
+          col = trace_dispatch<Pol, MAXS, BVH, DETAIL, true>(P, ro, rd, pixel, j, ctx, &ph, cand, ty >= rows.z && ty < rows.w,
+                                                             ground);
         }
       } else {
         camera_ray<Pol>(P, x, y, pixel, j, ro, rd);

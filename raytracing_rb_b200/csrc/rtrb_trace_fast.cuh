@@ -509,6 +509,21 @@ __device__ __forceinline__ uint32_t line_survivors_light(const FrameParams& P, c
   return m;
 }
 
+// Pass 2 of closest_hit_linear for plane k: the exact Plane#intersect, kept when it wins in (distance, index) order.
+template <bool KT, bool BOX>
+__device__ __forceinline__ void exact_plane_candidate(const FrameParams& P, const int k, d3 o, d3 d, double& best,
+                                                      int& best_i, HitRec& bh, ThreadCtx& ctx) {
+  const int i = pl_world_index<KT>(P, k);
+  const DevGeom g = P.geom[i];
+  HitRec h;
+  double den;
+  RTRB_COUNT(ctx, RTRB_CNT_EXACT);
+  if (plane_intersect(g, o, d, h, den)) {
+    const double new_dis = norm(o - h.p);
+    if (new_dis < best || (new_dis == best && best_i >= 0 && i < best_i)) { best = new_dis; best_i = i; keep_hit<BOX>(bh, h); }
+  }
+}
+
 // World#intersect (world.rb:37-59) = FP32 filter over every object + exact test of the survivors.
 template <class Pol, bool BOX, bool KT, bool CULL = false>
 __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3 d, const CullRay& r, HitRec& bh,
@@ -569,15 +584,7 @@ __device__ __forceinline__ int closest_hit_linear(const FrameParams& P, d3 o, d3
     else if (planes_cached && k == 1) { lo = plo1; kind = pkind1; }
     else kind = classify_plane(pl_rec<KT>(P, 2 * k), pl_rec<KT>(P, 2 * k + 1), r, lo, hi);
     if (kind == 0 || !(lo <= best_hi)) continue;
-    const int i = pl_world_index<KT>(P, k);
-    const DevGeom g = P.geom[i];
-    HitRec h;
-    double den;
-    RTRB_COUNT(ctx, RTRB_CNT_EXACT);
-    if (plane_intersect(g, o, d, h, den)) {
-      const double new_dis = norm(o - h.p);
-      if (new_dis < best || (new_dis == best && best_i >= 0 && i < best_i)) { best = new_dis; best_i = i; keep_hit<BOX>(bh, h); }
-    }
+    exact_plane_candidate<KT, BOX>(P, k, o, d, best, best_i, bh, ctx);
   }
   return best_i;
 }
@@ -719,11 +726,26 @@ __device__ __forceinline__ bool attenuation_dead(d3 att) {
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ int item_phase_a(const FrameParams& P, const StackItem& it, d3& sum, ThreadCtx& ctx, bool is_first,
                                             int* primary_hit, HitRec& bh, const uint32_t cam_cand = 0xffffffffu,
-                                            const bool no_highlight = false) {
+                                            const bool no_highlight = false, const bool ground = false) {
   constexpr bool KT = !BVH && MAXS == 1;  // constant-bank tables: depth-1 linear-filter kernels only (see pl_rec)
   const d3 o = mk(it.ox, it.oy, it.oz), d = mk(it.dx, it.dy, it.dz), att = mk(it.ax, it.ay, it.az);
   if (it.depth <= 0 || attenuation_dead(att)) return -1;  // rt_map :52
   ctx.rays++;
+
+  if constexpr (CULL) {
+    if (is_first && ground) {
+      // ground tile: no highlight, and the filter would send plane 0 alone to the exact test (rtrb_ground_rows)
+      bh.p = mk(0, 0, 0); bh.dir_in = false;
+      if constexpr (BOX) bh.face = 0;
+      double best = P.max_distance;
+      int best_i = -1;
+      exact_plane_candidate<KT, BOX>(P, 0, o, d, best, best_i, bh, ctx);
+      if (best_i < 0) return -1;
+      *primary_hit = best_i;
+      RTRB_COUNT(ctx, RTRB_CNT_HITS);
+      return best_i;
+    }
+  }
 
   const CullRay r = make_cull_ray(P, o, d);
 
@@ -897,9 +919,10 @@ template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL = false>
 __device__ __forceinline__ void process_item_fast(const FrameParams& P, const StackItem& it, StackItem* stack, int& sp,
                                                   d3& sum, ThreadCtx& ctx, uint32_t pixel, uint32_t sample,
                                                   bool is_first, int* primary_hit, const uint32_t cam_cand = 0xffffffffu,
-                                                  const bool no_highlight = false) {
+                                                  const bool no_highlight = false, const bool ground = false) {
   HitRec bh;
-  const int best_i = item_phase_a<Pol, MAXS, BVH, BOX, CULL>(P, it, sum, ctx, is_first, primary_hit, bh, cam_cand, no_highlight);
+  const int best_i = item_phase_a<Pol, MAXS, BVH, BOX, CULL>(P, it, sum, ctx, is_first, primary_hit, bh, cam_cand, no_highlight,
+                                                             ground);
   if (best_i >= 0) item_phase_b<Pol, MAXS, BVH, BOX>(P, it, best_i, bh, stack, sp, sum, ctx, pixel, sample);
 }
 
@@ -907,7 +930,8 @@ __device__ __forceinline__ void process_item_fast(const FrameParams& P, const St
 // (the ray-tree frame kernels run trace_sample_fast_lockstep).
 template <class Pol, int MAXS, bool BVH, bool BOX, bool CULL>
 __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 rd, uint32_t pixel, uint32_t sample,
-                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand, bool no_highlight) {
+                                                ThreadCtx& ctx, int* primary_hit, uint32_t cam_cand, bool no_highlight,
+                                                bool ground) {
   StackItem stack[MAXS > 1 ? MAXS : 1];
   // the root item starts in registers (no round trip through the local-memory stack)
   StackItem it;
@@ -919,7 +943,7 @@ __device__ __forceinline__ d3 trace_sample_fast(const FrameParams& P, d3 ro, d3 
   ctx.max_stack = max(ctx.max_stack, 1u);
   while (true) {
     process_item_fast<Pol, MAXS, BVH, BOX, CULL>(P, it, stack, sp, sum, ctx, pixel, sample, first, primary_hit, cam_cand,
-                                                 no_highlight);
+                                                 no_highlight, ground);
     first = false;
     if (MAXS == 1 || sp == 0) break;
     if ((uint32_t)sp > ctx.max_stack) ctx.max_stack = (uint32_t)sp;

@@ -178,6 +178,10 @@ struct FrameParams {
   // highlight cone.  A tile of the first kind whose candidate mask is empty is sky: its pixels are black, hit id -1.
   // All zero (no rows) for aperture frames and where the bounds do not hold; columns past the table share nothing.
   uchar4 k_tile_rows[RTRB_CAM_TX];
+  // Ground certificates (rtrb_ground_rows; scenes with exactly one plane): in rows [x, y) of column tx, a tile whose
+  // candidate mask is empty sends its camera rays to the exact test of plane 0 alone, with no highlight.  All zero =
+  // nothing.
+  uchar2 k_ground_rows[RTRB_CAM_TX];
 };
 
 static_assert(sizeof(FrameParams) <= 4096, "FrameParams must fit the 4 KB kernel-parameter space");

@@ -41,6 +41,7 @@ for name, cd in cams.items():
     tr, dv = [], []
     for _ in range(%(frames)d):
         flush.zero_()
+        torch.cuda.synchronize()  # the flush runs on torch's stream, the frame on the renderer's non-blocking one
         st, _ = r.render_device(cam, o)
         tr.append(st["trace_ms"]); dv.append(st["device_ms"])
     st, _ = r.render_device(cam, make_opts(seed=1, precision=PREC_FAST64, count_detail=True))
