@@ -998,6 +998,10 @@ void bake_frame(const rtrb_renderer* r, const rtrb_camera_desc* cam, FrameParams
         rtrb_ground_rows(&P.k_cull_pl[0].x, P.n_pl, P.max_distance_f, P.pos, P.focal_point, P.left, P.up_n, P.front,
                          cam->image_distance, cam->retina_width, cam->retina_height, cam->width, cam->height,
                          (const uint8_t(*)[4])P.k_tile_rows, (uint8_t(*)[2])P.k_ground_rows);
+        const int stx = (cam->width + RTRB_SUPER - 1) / RTRB_SUPER, sty = (cam->height + RTRB_SUPER - 1) / RTRB_SUPER;
+        P.sky_fill_tiles = (uint32_t)rtrb_sky_fill(P.k_cam_tx, P.k_cam_ty, (const uint8_t(*)[4])P.k_tile_rows, stx, sty,
+                                                   (uint8_t(*)[2])P.k_sky_run, P.k_trace_before);
+        P.sky_fill_traced = P.sky_fill_tiles ? (uint32_t)(stx * sty) - P.sky_fill_tiles : 0u;
       }
     } else {  // rays start anywhere on the lens: every sphere is a candidate
       const uint32_t all = n_sph >= 32 ? 0xffffffffu : (1u << n_sph) - 1u;
@@ -1191,6 +1195,8 @@ int setup_frame(const rtrb_renderer* r, const rtrb_camera_desc* cam, const rtrb_
   P.x0 = win.x0; P.y0 = win.y0; P.x1 = win.x1; P.y1 = win.y1;
   P.n_tiles = n_tiles; P.stx_count = (W + RTRB_SUPER - 1) / RTRB_SUPER; P.tiles = buf.tiles.dev.p;
   P.tiles_magic = win.whole ? buf.tiles.magic : 0u;
+  // the sky-fill grid covers the whole frame, one pixel per thread of the traced tiles, each resolved in its thread
+  if (P.tiles_magic == 0u || resolve != RTRB_RESOLVE_IN_THREAD) P.sky_fill_tiles = P.sky_fill_traced = 0u;
   P.lens_sx = buf.lens.tab.p; P.lens_sy = buf.lens.tab.p + W;
   P.samples = need_samples ? buf.samples.p : nullptr; P.pre_avg = buf.pre_avg.p;
   P.extra_list = buf.extra_list.p; P.extra_samples = buf.extra_samples.p;

@@ -328,6 +328,40 @@ inline void rtrb_longest_run(const uint8_t* f, int n, int& b0, int& b1) {
   }
 }
 
+// Sky-fill layout of a whole frame of stx x sty super-tiles (sty <= RTRB_CAM_TY): run[r] = {a, b}, the longest run of
+// columns c < RTRB_CAM_TX of super-tile row r whose tiles lie in their column's sky rows [tile_rows[c][0],
+// tile_rows[c][1]) and have an empty candidate mask cam_tx[c] & cam_ty[r], so every tile of it is one the kernels store
+// through their sky branch; before[r] = the tiles outside the runs (the traced tiles) of the rows < r.  The kernels trace
+// those in row-major order, traced tile t of row r being column t - before[r] left of a and t - before[r] + b - a from a
+// on, and store the runs' tiles from separate CTAs (trace_pre_body).  Returns the number of tiles in the runs; 0 (and no
+// runs) when the frame does not fit the tables.
+inline int rtrb_sky_fill(const uint32_t cam_tx[RTRB_CAM_TX], const uint32_t cam_ty[RTRB_CAM_TY],
+                         const uint8_t tile_rows[RTRB_CAM_TX][4], int stx, int sty, uint8_t run[RTRB_CAM_TY][2],
+                         uint16_t before[RTRB_CAM_TY]) {
+  for (int r = 0; r < RTRB_CAM_TY; ++r) run[r][0] = run[r][1] = 0, before[r] = 0;
+  if (stx < 1 || sty < 1 || sty > RTRB_CAM_TY || stx * sty > 0xffff) return 0;
+  const int nc = stx < RTRB_CAM_TX ? stx : RTRB_CAM_TX;
+  int r0 = 255, r1 = 0;  // rows that hold sky tiles at all
+  for (int c = 0; c < nc; ++c) {
+    if (tile_rows[c][0] >= tile_rows[c][1]) continue;
+    r0 = tile_rows[c][0] < r0 ? tile_rows[c][0] : r0;
+    r1 = tile_rows[c][1] > r1 ? tile_rows[c][1] : r1;
+  }
+  int n_sky = 0;
+  for (int r = 0; r < sty; ++r) {
+    before[r] = (uint16_t)(r * stx - n_sky);
+    int a = 0, b = 0, len = 0;  // the first longest run
+    for (int c = 0; c < (r >= r0 && r < r1 ? nc : 0); ++c) {
+      len = r >= tile_rows[c][0] && r < tile_rows[c][1] && (cam_tx[c] & cam_ty[r]) == 0u ? len + 1 : 0;
+      if (len > b - a) { a = c + 1 - len; b = c + 1; }
+    }
+    run[r][0] = (uint8_t)a; run[r][1] = (uint8_t)b;
+    n_sky += b - a;
+  }
+  if (n_sky == 0) for (int r = 0; r < sty; ++r) run[r][0] = run[r][1] = 0;
+  return n_sky;
+}
+
 // Ground certificates of a pinhole frame whose scene has exactly one plane: rows[c] = {g0, g1} for super-tile column
 // c < RTRB_CAM_TX, the longest run of rows in which, for every primary ray of the tile (dilated by one pixel),
 // classify_plane does not return kind 0 for the plane and its lo <= max_distance_f, inside tile_rows' no-highlight rows.

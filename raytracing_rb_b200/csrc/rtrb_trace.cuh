@@ -741,6 +741,70 @@ __device__ __forceinline__ bool decode_pixel(const FrameParams& P, uint32_t slot
   return x >= P.x0 && x < P.x1 && y >= P.y0 && y < P.y1;
 }
 
+// Super-tile row of the sky-fill order (rtrb_sky_fill) that holds item i of one kind, traced tiles or sky-run tiles, given
+// `before(r)`, the items of the rows < r: the last row r with before(r) <= i.  i comes from blockIdx, so the search runs on
+// the uniform datapath, once per warp.
+template <class Before>
+__device__ __forceinline__ int sky_fill_row(const FrameParams& P, uint32_t i, Before before) {
+  const int sty = (P.height + RTRB_SUPER - 1) / RTRB_SUPER;
+  int r = 0;
+#pragma unroll
+  for (int s = 64; s > 0; s >>= 1)
+    if (r + s < sty && before(r + s) <= i) r += s;
+  return r;
+}
+
+// decode_pixel of a sky-fill frame: slot k * 1024 + q is pixel q of the k-th traced tile in row-major order.  One sample
+// per pixel, so k comes from blockIdx alone.
+__device__ __forceinline__ bool decode_traced_pixel(const FrameParams& P, uint32_t slot, int& x, int& y) {
+  const uint32_t k = blockIdx.x / (RTRB_SUPER_PIXELS / blockDim.x), q = slot % RTRB_SUPER_PIXELS;
+  const int ty = sky_fill_row(P, k, [&](int r) { return (uint32_t)P.k_trace_before[r]; });
+  const uint32_t c = k - P.k_trace_before[ty];
+  const uchar2 run = P.k_sky_run[ty];
+  const uint32_t tx = c < run.x ? c : c + (uint32_t)(run.y - run.x);
+  int qx, qy;
+  rtrb_morton_decode(q, &qx, &qy);
+  x = (int)tx * RTRB_SUPER + qx;
+  y = ty * RTRB_SUPER + qy;
+  return x >= P.x0 && x < P.x1 && y >= P.y0 && y < P.y1;
+}
+
+// A fill CTA of a sky-fill frame: sky tiles [f, f + RTRB_SKY_FILL_TILES) of the runs in row-major order, f = the CTA's index
+// past the trace CTAs times RTRB_SKY_FILL_TILES, clipped to the frame.  Each pixel gets what trace_pre_body's sky branch
+// gives it: black in the pixel format, +0.0 in rgb, hit id -1, one ray and one sample in ctx.  A warp stores a pixel row
+// at a time, lane = pixel, with short independent stores: a lone warp's latency, not bandwidth, bounds the CTA.
+__device__ __forceinline__ void store_sky_tiles(const FrameParams& P, ThreadCtx& ctx) {
+  const uint32_t f0 = (blockIdx.x - P.sky_fill_traced * (RTRB_SUPER_PIXELS / blockDim.x)) * RTRB_SKY_FILL_TILES;
+  const uint32_t f1 = min(f0 + RTRB_SKY_FILL_TILES, P.sky_fill_tiles);
+  const int lane = threadIdx.x & 31;
+  uint32_t px = 0;
+  for (uint32_t i = f0; i < f1; ++i) {
+    auto sky_before = [&](int r) { return (uint32_t)(r * P.stx_count - P.k_trace_before[r]); };
+    const int ty = sky_fill_row(P, i, sky_before);
+    const int x = (P.k_sky_run[ty].x + (int)(i - sky_before(ty))) * RTRB_SUPER + lane, y0 = ty * RTRB_SUPER;
+    if (x >= P.width) continue;
+    const int y1 = min(y0 + RTRB_SUPER, P.height);
+    for (int y = y0 + (int)(threadIdx.x >> 5); y < y1; y += (int)(blockDim.x >> 5)) {
+      const size_t px_i = (size_t)y * P.width + x;
+      if (P.pixel_format == RTRB_FMT_RGBA8) {
+        reinterpret_cast<uchar4*>(P.rgba)[px_i] = make_uchar4(0, 0, 0, 255);
+      } else {
+        uint8_t* o = P.rgba + px_i * 3;
+        if (P.pixel_format == RTRB_FMT_PNG_RGB8) {  // PNG scanline: the filter-type byte 0 ahead of pixel 0
+          o = P.rgba + (size_t)y * ((size_t)P.width * 3 + 1) + 1 + (size_t)x * 3;
+          if (x == 0) o[-1] = 0;
+        }
+        o[0] = 0; o[1] = 0; o[2] = 0;
+      }
+      if (P.rgb) { P.rgb[px_i * 3 + 0] = 0.0; P.rgb[px_i * 3 + 1] = 0.0; P.rgb[px_i * 3 + 2] = 0.0; }
+      if (P.hit) P.hit[px_i] = -1;
+      ++px;
+    }
+  }
+  ctx.rays = px;
+  if (ctx.detail) ctx.c[RTRB_CNT_SAMPLES] = px;
+}
+
 // Records a pixel whose sample set a status bit (the reference would have raised there): status word and the
 // first offending pixel in the reference's pixel order (x outer, y inner).  Clears ctx.status so that a thread
 // which goes on to other pixels (grid-stride / persistent loops) attributes later bits to the right pixel.
@@ -842,11 +906,17 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
   init_ctx(ctx, DETAIL);
   int x = 0, y = 0;
   bool active = false;
-  if (w < total) {
+  // sky-fill frames (FrameParams::sky_fill_tiles): the CTAs past those of the traced tiles store the sky runs
+  bool fill = false, fill_frame = false;
+  if constexpr (kOverlap && kCull) {
+    fill_frame = P.sky_fill_tiles != 0u;
+    fill = fill_frame && blockIdx.x >= P.sky_fill_traced * (RTRB_SUPER_PIXELS / blockDim.x);
+  }
+  if (!fill && w < total) {
     uint32_t slot, j;
     decode_work(w, S, slot, j);
     if constexpr (PASS) j += (uint32_t)P.pass_begin;
-    active = decode_pixel(P, slot, x, y);
+    active = fill_frame ? decode_traced_pixel(P, slot, x, y) : decode_pixel(P, slot, x, y);
     if (active) {
       const uint32_t pixel = (uint32_t)y * (uint32_t)P.width + (uint32_t)x;
       d3 ro, rd;
@@ -889,6 +959,7 @@ __device__ __forceinline__ void trace_pre_body(const FrameParams& P) {
     }
   }
   if (kOverlap && !active) cudaGridDependencySynchronize();  // before flush_ctx's counters
+  if (fill) store_sky_tiles(P, ctx);
   flush_ctx(P, ctx, x, y, active);
   // the next frame's control block: that frame touches it only after its own wait, i.e. after this grid completed
   if (kOverlap && blockIdx.x == 0u && P.ctl_next != nullptr)

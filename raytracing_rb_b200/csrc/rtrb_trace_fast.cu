@@ -33,7 +33,11 @@ cudaError_t rtrb_launch_trace_pre_fast(const FrameParams& P, int capacity, cudaS
   if (overlap && k->capacity != 1) return cudaErrorInvalidValue;  // only the depth-1 kernels wait before their writes
   // one thread per (pixel, sample); the ray-tree kernels run lockstep CTAs (rtrb_trace_fast.cuh, trace_pre_tree_body),
   // more and smaller ones on small frames
-  const unsigned long long threads = pre_threads(P);
+  unsigned long long threads = pre_threads(P);
+  // sky-fill frames (FrameParams::sky_fill_tiles): the traced tiles' pixels, then the CTAs that store the sky runs
+  if (P.sky_fill_tiles != 0u)
+    threads = ((unsigned long long)P.sky_fill_traced * (RTRB_SUPER_PIXELS / kBlock) +
+               (P.sky_fill_tiles + RTRB_SKY_FILL_TILES - 1) / RTRB_SKY_FILL_TILES) * kBlock;
   int block = kBlock;
   if (k->capacity > 1) block = threads < 4ull * (unsigned long long)sm_count() * kTreeBlock ? RTRB_TREE_MIN_BLOCK : kTreeBlock;
   // in-CTA resolve (ray-tree frames only): the host only selects it for sample counts that divide both CTA sizes

@@ -23,6 +23,7 @@
 #define RTRB_SCENE_CLASS_LEAN 2
 #define RTRB_TREE_MIN_BLOCK 128        // smallest CTA the ray-tree kernels are launched with (the largest is 512): a
                                       // pre_sample_times that divides it has every sample of a pixel in one CTA
+#define RTRB_SKY_FILL_TILES 4         // sky tiles one fill CTA of a sky-fill frame stores (FrameParams::sky_fill_tiles)
 
 struct DevGeom {      // 64 B
   double px, py, pz;  // sphere centre / plane point
@@ -182,6 +183,14 @@ struct FrameParams {
   // candidate mask is empty sends its camera rays to the exact test of plane 0 alone, with no highlight.  All zero =
   // nothing.
   uchar2 k_ground_rows[RTRB_CAM_TX];
+  // Sky fill (rtrb_sky_fill; depth-1 FAST64 linear-filter frames resolved in the thread, whole frame on one renderer,
+  // pinhole camera): the grid is 8 CTAs for each of the sky_fill_traced tiles outside the sky runs k_sky_run (one run of
+  // columns per super-tile row), in row-major order (k_trace_before[r]: those of the rows < r), then
+  // ceil(sky_fill_tiles / RTRB_SKY_FILL_TILES) CTAs that store the runs' tiles without tracing.  sky_fill_tiles == 0:
+  // the one-thread-per-pixel grid over every tile, as for every other frame.
+  uchar2 k_sky_run[RTRB_CAM_TY];
+  uint16_t k_trace_before[RTRB_CAM_TY];
+  uint32_t sky_fill_tiles, sky_fill_traced;
 };
 
 static_assert(sizeof(FrameParams) <= 4096, "FrameParams must fit the 4 KB kernel-parameter space");
